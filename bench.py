@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frame-pairs/sec of the tracking hot path (window match + PnP).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     (N > 1: launched by torch.distributed.run, one rank per GPU)
 
 Workload (BASELINE.json configs[3], named in config.workload): a KITTI-00-length synthetic
@@ -221,6 +221,17 @@ def parity_against_port(resn, out, n):
             "what": "num_matches, ransac_inliers, pnp_inliers, best hypothesis exact; pose within 1e-5 rad / 1e-5"}
 
 
+def dump_outputs(out_dir: str, recs) -> None:
+    """One .npy per field of the pair records a caller of mv_track_sequence receives (all pairs, 64 B each):
+    float fields as float32, integer fields as float64 (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in recs.dtype.names:
+        if name == "pad":
+            continue
+        a = recs[name]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def run_reference(args, rank: int):
     if rank != 0:
         return
@@ -265,7 +276,14 @@ def main():
     ap.add_argument("--tensor-cores", action="store_true", help="same as --matcher tcgen05")
     ap.add_argument("--lanes", type=int, default=1,
                     help="PnP summation lanes per hypothesis (1: one thread; 2: one thread, packed FFMA2; 4..32: threads)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-pair results of the last timed step as DIR/<field>.npy (float32 / float64), "
+                         "so that two builds can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     args.tensor_cores = args.tensor_cores or args.matcher == "tcgen05"
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -339,6 +357,9 @@ def main():
     ms_max = float(t.item())
     ms_per_step = ms_max / args.steps
     value = n_pairs / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # `res` is every pair's record as the last timed step gathered it; the passes below overwrite it
+        dump_outputs(args.dump_outputs, tracking.results_to_numpy(res))
 
     # ---- per-kernel device time (CUDA events on the launch stream, separate short pass)
     tr.ctx.profile(True)

@@ -40,18 +40,38 @@ def _cpu_model() -> str:
     return "%s | %08x" % (name, zlib.crc32(flags.encode()))
 
 
-def build_fast() -> None:
+def build_fast(out_dir: str | None = None) -> str:
     """libmv_oracle_fast.so is compiled -march=native, so it must be built on the CPU that runs it:
     a sidecar file records the build host's CPU model + flag set and the library is rebuilt when
-    they differ (the GPU box receives this container's build)."""
-    so = os.path.join(_HERE, "libmv_oracle_fast.so")
-    tag = os.path.join(_HERE, "libmv_oracle_fast.host")
+    they differ.  __graft_entry__.build() builds it in oracle/ (out_dir = oracle/); at run time the
+    tree's copy is used when it fits this CPU, else a copy under the temporary directory, so that a
+    read-only tree still runs.  Returns the path of the library to load."""
+    import atexit
+    import shutil
+    import tempfile
     here = _cpu_model()
-    built_for = open(tag).read().strip() if os.path.exists(tag) else None
-    stale = (not os.path.exists(so)) or os.path.getmtime(so) < os.path.getmtime(os.path.join(_HERE, "mv_oracle.c"))
-    if stale or built_for != here:
-        subprocess.run(["make", "-C", _HERE, "-B", "libmv_oracle_fast.so"], check=True, capture_output=True)
-        open(tag, "w").write(here)
+    src_mtime = max(os.path.getmtime(os.path.join(_HERE, f)) for f in ("mv_oracle.c", "mv_oracle.h"))
+
+    def state(d):
+        so, tag = os.path.join(d, "libmv_oracle_fast.so"), os.path.join(d, "libmv_oracle_fast.host")
+        fresh = os.path.exists(so) and os.path.getmtime(so) >= src_mtime
+        return so, tag, fresh, fresh and os.path.exists(tag) and open(tag).read().strip() == here
+
+    if out_dir is None:
+        so, _, _, ok = state(_HERE)
+        if ok:
+            return so
+        # a fresh private directory (mode 0700), removed at exit: nothing another user placed is loaded
+        out_dir = tempfile.mkdtemp(prefix="mv_oracle_fast-")
+        atexit.register(shutil.rmtree, out_dir, True)
+    so, tag, fresh, ok = state(out_dir)
+    if not ok:
+        # -B: an up-to-date file built for another CPU is rebuilt all the same
+        subprocess.run(["make", "-C", _HERE] + (["-B"] if fresh else []) + ["FAST_SO=" + so, so],
+                       check=True, capture_output=True)
+        with open(tag, "w") as f:
+            f.write(here)
+    return so
 
 
 class MatchCfg(C.Structure):
@@ -107,10 +127,8 @@ class Oracle:
     """T2: the parametrised restatement."""
 
     def __init__(self, fast: bool = False):
-        if fast:
-            build_fast()
         build()
-        self.lib = C.CDLL(os.path.join(_HERE, "libmv_oracle_fast.so" if fast else "libmv_oracle.so"))
+        self.lib = C.CDLL(build_fast() if fast else os.path.join(_HERE, "libmv_oracle.so"))
         L = self.lib
         L.orc_softmax.restype = C.c_int
         L.orc_softmax.argtypes = [C.c_float, _i8p, C.c_int, _i32p, _f32p]

@@ -130,10 +130,16 @@ def _drive_pool(L, frames=60, per_frame=200, seed=0):
     return trace
 
 
-def test_local_feature_pool_matches_reference(reference):
+def _trace_digest(trace):
+    import hashlib
+    return hashlib.sha256(repr(trace).encode()).hexdigest()
+
+
+def test_local_feature_pool_matches_reference(t1_lib, t1):
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import lib
     ours = _drive_pool(lib.load())
-    theirs = _drive_pool(reference.lib)
-    assert ours == theirs
+    # the stored answer is a digest of T1's trace (the trace itself is 0.4 MB)
+    theirs = t1.next("_drive_pool", (), t1_lib and (lambda: _trace_digest(_drive_pool(t1_lib))))
+    assert _trace_digest(ours) == theirs
     assert ours[-1][0] > 0

@@ -30,7 +30,7 @@ def _quat_to_R(q):
                      [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
 
 
-def test_residual_matches_reference_projection_factor(oracle, reference):
+def test_residual_matches_reference_projection_factor(oracle, t1_lib, t1):
     class V2(C.Structure):
         _fields_ = [("x", C.c_float), ("y", C.c_float)]
 
@@ -59,10 +59,14 @@ def test_residual_matches_reference_projection_factor(oracle, reference):
         z = rng.uniform(0, 600, 2).astype(np.float32)
         lm, se3 = V3(*X), SE3(Q(*pose[:4]), V3(*pose[4:]))
         f = Factor(C.pointer(lm), C.pointer(se3), V2(*z), V2(0, 0), Cam(*cam))
-        reference.lib.compute_error_ProjectionFactor(C.byref(f))
+
+        def t1_error():
+            t1_lib.compute_error_ProjectionFactor(C.byref(f))
+            return np.array([f.error.x, f.error.y], np.float32)
+        want = t1.next("compute_error_ProjectionFactor", (pose, X, z, cam), t1_lib and t1_error)
         err = np.zeros(2, np.float32)
         oracle.lib.orc_projection_error(pose, X, z, cam, err)
-        assert err[0] == f.error.x and err[1] == f.error.y
+        assert err[0] == want[0] and err[1] == want[1]
 
 
 @pytest.mark.parametrize("seed", range(4))
