@@ -269,6 +269,23 @@ mv_status mv_build_corr_landmarks_batch(mv_ctx* ctx, int n_pairs, int top_n, int
                                         const int32_t* d_match_count, const int32_t* d_match_cell0,
                                         float* d_corr, int32_t* d_n_with_landmark);
 
+/* The whole sequence's table update in one call: frames 0 .. n_steps-1 with global frame numbers
+ * first_frame + f.  Step f is exactly
+ *     mv_landmarks_observe(first_frame + f, d_word[f][0 .. q_count), d_coords_in[f])
+ *     mv_landmarks_remove_old(first_frame + f)
+ * with q_count = min(d_q_count[f], top_n).  d_table is read at entry as the initial state and left in its final
+ * state, byte for byte the table of that per-frame loop (stale frames[] / coords of deleted records included).
+ * d_coords_out[f][q] receives what mv_landmarks_lookup of d_word[f][q] returns right after step f (0,0,0 where
+ * the word is outside [0, n_words) or q >= q_count).  A record keeps the coordinates of the occurrence that
+ * inserted it: update_local_feature never touches coords_3D, so a landmark older than frame f is expressed in the
+ * camera frame of the frame that inserted it, not in frame f's.
+ * Calls chain: [0, k) then [k, n) (first_frame advanced by k) equals one call over [0, n).
+ *   d_word int32 [n_steps][top_n], d_q_count int32 [n_steps], d_coords_in / d_coords_out float [n_steps][top_n][3]
+ * n_steps <= 65535, n_steps * top_n < 2^31. */
+mv_status mv_landmarks_sequence(mv_ctx* ctx, int n_words, mv_landmark* d_table, int first_frame, int n_steps,
+                                int top_n, const int32_t* d_word, const int32_t* d_q_count,
+                                const float* d_coords_in, float* d_coords_out);
+
 /* ------------------------------------------------------------------------- */
 /* Whole path over a sequence of frames (pair p = frames p, p+1)              */
 /* ------------------------------------------------------------------------- */
@@ -312,6 +329,30 @@ mv_status mv_track_sequence_host(mv_ctx* ctx, const mv_track_params* p, int n_fr
                                  const int8_t* h_desc, const float* h_depth,
                                  mv_pair_result* h_results,
                                  unsigned long long* h2d_bytes, unsigned long long* d2h_bytes);
+
+/* mv_track_sequence with the 3-D side of pair p's correspondences from the landmark table instead of depth
+ * (the reference's data flow, local_feature_matching.c:153-163 and local_feature_pool.h:16-22):
+ *   - the words of frames 0 .. n_frames-2 are mv_bow_assign_batch's with d_desc_scale (vocabulary set first);
+ *   - a query keypoint of frame f, pixel x = (cell / rows) * 8 + idx % 8, y = (cell % rows) * 8 + idx / 8, is
+ *     back-projected with frame f's depth at its cell by the fp32 operations of mv_build_corr_batch; those are
+ *     the coordinates its occurrence hands to observe;
+ *   - the table steps over frames 0 .. n_frames-2 exactly as mv_landmarks_sequence(first_frame, n_frames - 1)
+ *     (frame n_frames-1 is only the query side of the last pair): d_table in/out;
+ *   - pair p uses the table right after step p: match j -> its frame-0 cell -> that cell's place in frame p's
+ *     query list -> the coordinates of that query's word, mv_build_corr_landmarks_batch against that snapshot
+ *     (NaN without a landmark, lists keep order and length); d_n_with_landmark int32 [n_frames-1] (nullable)
+ *     receives the count per pair;
+ *   - match, RANSAC-E, the Gauss-Newton PnP (sampler keyed on pnp.first_pair + p) and the records are those of
+ *     mv_track_sequence.
+ * Landmark coordinates are in the camera frame of the frame that inserted the record (see mv_landmarks_sequence);
+ * a world-frame map would need solved poses fed back, which serialises the pairs, and is not done here.
+ * Two calls over frames [0, k] and [k, n-1] (one halo frame; first_frame and pnp.first_pair advanced by k) equal
+ * one call over [0, n-1]. */
+mv_status mv_track_sequence_landmarks(mv_ctx* ctx, const mv_track_params* p, int n_frames, int first_frame,
+                                      const int8_t* d_semi, const float* d_semi_scale,
+                                      const int8_t* d_desc, const float* d_desc_scale, const float* d_depth,
+                                      int n_words, mv_landmark* d_table,
+                                      mv_pair_result* d_results, int32_t* d_n_with_landmark);
 
 /* ------------------------------------------------------------------------- */
 /* NMS between the detector and the matcher (src/run_nms.c)                     */

@@ -634,11 +634,19 @@ static thread_local std::function<void(const char*)> g_seq_mark;  // MV_HOST_TRA
 // kernels -- the point where the next chunk's row gather is released (see below).
 static thread_local std::function<mv_status()> g_after_match;
 
+// 3-D side of the correspondences from the landmark table (mv_track_sequence_landmarks) instead of depth
+struct SeqLandmarks {
+  int n_words;
+  const int32_t* word;       // [n_frames - 1][top_n]
+  const float* coords_out;   // [n_frames - 1][top_n][3], mv_landmarks_sequence
+  int32_t* n_with_landmark;  // nullable
+};
+
 // Match + pose half: needs descriptors (only rows of candidate / query cells are read) and
-// depth (only at matched frame-0 cells).
+// depth (only at matched frame-0 cells), or the landmarks of frame 0's queries.
 static mv_status seq_match_pose(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
                                 const float* d_depth, const SeqScratch& w, mv_pair_result* d_results,
-                                int pair_offset) {
+                                int pair_offset, const SeqLandmarks* lm = nullptr) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
@@ -652,9 +660,14 @@ static mv_status seq_match_pose(mv_ctx* c, const mv_track_params* p, int n_frame
                                        w.rin, nullptr, nullptr)))
       return st;
   }
-  if ((st = mv_build_corr_batch(c, n_pairs, cells, p->match.rows, M, nullptr, d_depth, p->pnp.fx, p->pnp.fy,
-                                p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr)))
+  if (lm) {
+    if ((st = mv_build_corr_landmarks_seq(c, n_pairs, N, M, lm->n_words, w.qp, w.qc, lm->word, lm->coords_out, w.mp,
+                                          w.mc, w.mcell, w.corr, lm->n_with_landmark)))
+      return st;
+  } else if ((st = mv_build_corr_batch(c, n_pairs, cells, p->match.rows, M, nullptr, d_depth, p->pnp.fx, p->pnp.fy,
+                                       p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr))) {
     return st;
+  }
   if (g_seq_mark) g_seq_mark("corr_end");
   mv_pnp_params pnp = p->pnp;
   pnp.first_pair += pair_offset;
@@ -679,6 +692,49 @@ extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int 
   if ((st = seq_scratch(c, p, n_frames, "seq", &w))) return st;
   if ((st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w))) return st;
   return seq_match_pose(c, p, n_frames, d_desc, d_depth, w, d_results, 0);
+}
+
+// Pair p = frames (p, p+1) with the 3-D side from the landmark table right after step p: detector, word
+// assignment of frames 0..n-2 with their query keypoints back-projected in the same launch, the table walked over
+// those frames in one batch (mv_landmarks_sequence), then match / RANSAC-E / correspondences / K3 / pack.
+extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_params* p, int n_frames, int first_frame,
+                                                 const int8_t* d_semi, const float* d_semi_scale, const int8_t* d_desc,
+                                                 const float* d_desc_scale, const float* d_depth, int n_words,
+                                                 mv_landmark* d_table, mv_pair_result* d_results,
+                                                 int32_t* d_n_with_landmark) {
+  MV_ENTER(c);
+  if (!p || n_frames < 2 || !d_semi || !d_semi_scale || !d_desc || !d_desc_scale || !d_depth || !d_results)
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks");
+  if (!seq_params_ok(p))
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks: rows, cols, top_n, max_valid and max_matches must be positive");
+  if (n_frames > 65535) MV_BAD_ARG(c, "mv_track_sequence_landmarks: at most 65535 frames per call");
+  if (c->bow_n_base <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks: no vocabulary (mv_bow_set_vocabulary first)");
+  if (n_words <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks: n_words must be positive");
+  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks: NULL landmark table");
+  if (reinterpret_cast<uintptr_t>(d_desc) & 15) MV_BAD_ARG(c, "mv_track_sequence_landmarks: d_desc must be 16-byte aligned");
+  if ((long long)(n_frames - 1) * p->top_n > 0x7fffffffLL)
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks: (n_frames - 1) * top_n must be below 2^31");
+  const int cells = p->match.rows * p->match.cols;
+  const int n_steps = n_frames - 1, N = p->top_n;
+  SeqScratch w;
+  void *word, *cin, *cout;
+  mv_status st;
+  if ((st = seq_scratch(c, p, n_frames, "lmseq", &w))) return st;
+  if ((st = mv_scratch(c, "lmseq.word", sizeof(int32_t) * (size_t)n_steps * N, &word))) return st;
+  if ((st = mv_scratch(c, "lmseq.coords_in", sizeof(float) * 3 * (size_t)n_steps * N, &cin))) return st;
+  if ((st = mv_scratch(c, "lmseq.coords_out", sizeof(float) * 3 * (size_t)n_steps * N, &cout))) return st;
+  if ((st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w))) return st;
+  MvBackProject bp;
+  bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
+  bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
+  bp.coords = (float*)cin;
+  if ((st = mv_bow_assign_impl(c, n_steps, cells, N, d_desc, d_desc_scale, w.qp, w.qc, (int32_t*)word, nullptr, bp)))
+    return st;
+  if ((st = mv_landmarks_sequence_impl(c, n_words, d_table, first_frame, n_steps, N, (const int32_t*)word, w.qc,
+                                       (const float*)cin, (float*)cout)))
+    return st;
+  const SeqLandmarks lm = {n_words, (const int32_t*)word, (const float*)cout, d_n_with_landmark};
+  return seq_match_pose(c, p, n_frames, d_desc, nullptr, w, d_results, 0, &lm);
 }
 
 // ---- selective staging of descriptors from pinned host memory ------------------------

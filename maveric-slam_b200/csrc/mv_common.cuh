@@ -37,6 +37,7 @@ struct mv_ctx {
   bool pnp_work_live = false;           // profile mode: the PnP work counter holds launches not yet read
   int match_items = 0;                  // tiles of the last tensor-core matcher launch (mv_ctx_match_work)
   int bow_n_base = 0, bow_wpb = 0;      // vocabulary on the device (mv_bow_set_vocabulary)
+  size_t bow_smem_attr = 0;             // dynamic shared memory the word-assignment kernel is allowed so far
   int lm_words = 0;                     // size the landmark scratch was initialised for
   std::map<std::string, mv_prof_slot> prof;
   std::vector<mv_pending_event> pending;
@@ -125,6 +126,28 @@ struct mv_device_guard {
 
 mv_status mv_scratch(mv_ctx* ctx, const char* name, size_t bytes, void** out);
 mv_status mv_pinned(mv_ctx* ctx, size_t bytes, void** out);
+
+// ---- landmark sequence path (bow.cu), called by mv_track_sequence_landmarks (api.cu)
+// Back-projection of every query keypoint with its frame's depth, fused into the word assignment launch:
+// coords [n_frames][top_n][3] (zeros beyond the query count); nothing is written when coords is NULL.
+struct MvBackProject {
+  const int32_t* q_idx = nullptr;
+  const float* depth = nullptr;
+  int rows = 0;
+  float fx = 0.0f, fy = 0.0f, cx = 0.0f, cy = 0.0f;
+  float* coords = nullptr;
+};
+mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, const int8_t* d_desc,
+                             const float* d_desc_scale, const int32_t* d_q_patch, const int32_t* d_q_count,
+                             int32_t* d_word, int32_t* d_base, const MvBackProject& bp);
+mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_table, int first_frame, int n_steps,
+                                     int top_n, const int32_t* d_word, const int32_t* d_q_count,
+                                     const float* d_coords_in, float* d_coords_out);
+// mv_build_corr_landmarks_batch for pairs (p, p+1) with the 3-D side from mv_landmarks_sequence's coords_out
+mv_status mv_build_corr_landmarks_seq(mv_ctx* ctx, int n_pairs, int top_n, int stride, int n_words,
+                                      const int32_t* d_q_patch, const int32_t* d_q_count, const int32_t* d_word,
+                                      const float* d_coords_out, const float* d_match_pts, const int32_t* d_match_count,
+                                      const int32_t* d_match_cell0, float* d_corr, int32_t* d_n_with_landmark);
 
 // float bounds that make a float-vs-double comparison exact in fp32:
 //   (double)s >  T  <=>  s >  mv_round_down(T)

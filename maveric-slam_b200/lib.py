@@ -27,7 +27,8 @@ NEW_SYMBOLS = [
     "mv_lba_schur_batch",
     "mv_lba_solve_batch",
     "mv_bow_set_vocabulary", "mv_bow_assign_batch", "mv_landmarks_init", "mv_landmarks_observe",
-    "mv_landmarks_remove_old", "mv_landmarks_lookup", "mv_build_corr_landmarks_batch",
+    "mv_landmarks_remove_old", "mv_landmarks_lookup", "mv_build_corr_landmarks_batch", "mv_landmarks_sequence",
+    "mv_track_sequence_landmarks",
 ]
 LEGACY_SYMBOLS = [
     "add_Vector2f", "add_Vector3f", "mult_Quaternionf", "create_Quaternionf", "Quaternionf_from_Vector3f",
@@ -137,6 +138,8 @@ def load() -> C.CDLL:
     L.mv_landmarks_remove_old.argtypes = [vp, i32, vp, i32]
     L.mv_landmarks_lookup.argtypes = [vp, i32, vp, i32, vp, vp, vp]
     L.mv_build_corr_landmarks_batch.argtypes = [vp, i32, i32, i32, i32] + [vp] * 10
+    L.mv_landmarks_sequence.argtypes = [vp, i32, vp, i32, i32, i32, vp, vp, vp, vp]
+    L.mv_track_sequence_landmarks.argtypes = [vp, C.POINTER(TrackParams), i32, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     L.mv_synth_frames.argtypes = [vp, C.POINTER(SynthParams), i32, i32, vp, vp, vp, vp]
     L.mv_nms_batch.argtypes = [vp, i32, i32, i32, vp, vp]
     L.run_nms_ex.argtypes = [vp, i32, i32, vp, vp]

@@ -449,6 +449,35 @@ class Tracker:
             self._d(q_count), self._d(word), self._d(pts), self._d(cnt), self._d(cell0), self._d(corr), self._d(nl)))
         return corr, nl
 
+    def landmarks_sequence(self, table, first_frame, word, q_count, coords_in, coords_out=None):
+        """The table update of a whole sequence in one call (mv_landmarks_sequence): step f observes frame
+        first_frame + f (word int32 [n_steps, top_n], the first q_count[f] of them, coordinates float32
+        [n_steps, top_n, 3]) and then removes old frames.  `table` is updated in place; returns coords_out float32
+        [n_steps, top_n, 3], each occurrence's landmark right after its frame's step (0 where there is none)."""
+        n_steps, top_n = word.shape
+        if coords_out is None:
+            coords_out = self.torch.empty((n_steps, top_n, 3), dtype=self.torch.float32, device=self.device)
+        self.ctx.check(self.lib.mv_landmarks_sequence(self.ctx.h, table.shape[0], self._d(table), int(first_frame), n_steps,
+                                                      top_n, self._d(word), self._d(q_count), self._d(coords_in),
+                                                      self._d(coords_out)))
+        return coords_out
+
+    def track_sequence_landmarks(self, params: _lib.TrackParams, semi, semi_scale, desc, desc_scale, depth, table,
+                                 first_frame=0, out=None, n_with_landmark=None):
+        """:meth:`track_sequence` with the 3-D side of each pair from the landmark table (vocabulary set first with
+        :meth:`bow_set_vocabulary`): the table steps over frames 0 .. n-2 (global numbers first_frame + f) and is
+        updated in place.  Returns (uint8 [n_pairs, 64] results, int32 [n_pairs] matches with a landmark)."""
+        torch = self.torch
+        n = semi.shape[0]
+        if out is None:
+            out = torch.empty((n - 1, 64), dtype=torch.uint8, device=self.device)
+        if n_with_landmark is None:
+            n_with_landmark = torch.empty((n - 1,), dtype=torch.int32, device=self.device)
+        self.ctx.check(self.lib.mv_track_sequence_landmarks(
+            self.ctx.h, C.byref(params), n, int(first_frame), self._d(semi), self._d(semi_scale), self._d(desc),
+            self._d(desc_scale), self._d(depth), table.shape[0], self._d(table), self._d(out), self._d(n_with_landmark)))
+        return out, n_with_landmark
+
     def chain_transforms(self, transforms):
         """python/compute_trajectory.py:49-51,76-77 as a parallel scan: float64 [n, 3, 4] relative
         transforms -> float64 [n+1, 3, 4] frame poses, pose 0 the identity."""
