@@ -24,9 +24,9 @@
  *     host thread or per GPU is the intended use); different contexts are independent.  The
  *     legacy void symbols share one process-global context on device 0 behind a mutex
  *   - batched calls take at most 65535 pairs / frames (MV_ERR_BAD_ARG beyond that; the
- *     host-buffer sequence call chunks internally and has no such limit)
- *   - on any error return of mv_track_sequence_host the library has drained its streams:
- *     the caller's host buffers are no longer read when the call returns
+ *     host-buffer sequence calls chunk internally and have no such limit)
+ *   - on any error return of mv_track_sequence_host or mv_track_sequence_landmarks_host the library has
+ *     drained its streams: the caller's host buffers are no longer read when the call returns
  */
 #ifndef MAVERIC_B200_H
 #define MAVERIC_B200_H
@@ -353,6 +353,30 @@ mv_status mv_track_sequence_landmarks(mv_ctx* ctx, const mv_track_params* p, int
                                       const int8_t* d_desc, const float* d_desc_scale, const float* d_depth,
                                       int n_words, mv_landmark* d_table,
                                       mv_pair_result* d_results, int32_t* d_n_with_landmark);
+
+/* mv_track_sequence_landmarks from host (ideally pinned) frames: the staging pipeline of mv_track_sequence_host
+ * (chunks of pairs sharing one halo frame, the pair index of the PnP sampler global) with the table carried
+ * from chunk to chunk on the device.  Returns when the results are in h_results.
+ *   - results, h_n_with_landmark (int32 [n_frames-1], nullable) and the final d_table are byte for byte those of
+ *     mv_track_sequence_landmarks on the same frames, whatever the chunk size, pinned or pageable buffers, and
+ *     selective staging on or off;
+ *   - d_table is caller-owned device memory of n_words records (it is the map, and small), read at entry and left
+ *     in its final state;
+ *   - two calls over frames [0, k] and [k, n-1] (first_frame and pnp.first_pair advanced by k) equal one call;
+ *     there is no limit on n_frames;
+ *   - h2d_bytes: those of mv_track_sequence_host (logits, semi scales, depth planes, the descriptor rows the
+ *     matcher reads -- the word assignment reads only query rows, which are among them) plus the desc scales;
+ *     d2h_bytes: the records, plus h_n_with_landmark when given;
+ *   - argument errors (no vocabulary, NULL table, n_words <= 0, non-positive sizes, n_frames < 2) are
+ *     MV_ERR_BAD_ARG before anything is enqueued: the table is untouched.  After a CUDA error the streams are
+ *     drained and the host buffers no longer read, but the table's state is unspecified.
+ * Not sharded over GPUs: a rank's initial table would depend on every earlier frame. */
+mv_status mv_track_sequence_landmarks_host(mv_ctx* ctx, const mv_track_params* p, int n_frames, int first_frame,
+                                           const int8_t* h_semi, const float* h_semi_scale,
+                                           const int8_t* h_desc, const float* h_desc_scale, const float* h_depth,
+                                           int n_words, mv_landmark* d_table,
+                                           mv_pair_result* h_results, int32_t* h_n_with_landmark /* nullable */,
+                                           unsigned long long* h2d_bytes, unsigned long long* d2h_bytes);
 
 /* ------------------------------------------------------------------------- */
 /* NMS between the detector and the matcher (src/run_nms.c)                     */

@@ -12,6 +12,7 @@
 #include <math.h>
 #include <stdlib.h>
 
+#include <algorithm>
 #include <mutex>
 
 #include "../../include/maveric_slam_compat.h"
@@ -861,20 +862,26 @@ struct StreamSwap {  // run the context's kernels on another stream for a scope
   ~StreamSwap() { c->stream = saved; }
 };
 
+// Landmark mode of the host pipeline (mv_track_sequence_landmarks_host): the caller's table and the inputs only
+// that path reads.
+struct HostLandmarks {
+  int first_frame, n_words;
+  mv_landmark* table;
+  const float* h_desc_scale;
+  int32_t* h_n_with_landmark;  // nullable
+};
+
 // Host inputs.  Chunks of frames are double-buffered: on the staging stream the logits are
 // copied and the detector runs, then descriptors arrive (selectively when the host buffers
 // are pinned, else as a plain copy); the compute stream matches and solves the previous chunk
-// meanwhile.  Consecutive chunks share one halo frame.
-extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p, int n_frames,
-                                            const int8_t* h_semi, const float* h_semi_scale,
-                                            const int8_t* h_desc, const float* h_depth,
-                                            mv_pair_result* h_results, unsigned long long* h2d_bytes,
-                                            unsigned long long* d2h_bytes) {
-  MV_ENTER(c);
-  if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_depth || !h_results)
-    MV_BAD_ARG(c, "mv_track_sequence_host");
-  if (!seq_params_ok(p))
-    MV_BAD_ARG(c, "mv_track_sequence_host: rows, cols, top_n, max_valid and max_matches must be positive");
+// meanwhile.  Consecutive chunks share one halo frame.  With `lm` the compute stream also assigns
+// the words of the chunk's frames but its halo and steps the caller's landmark table over them
+// before matching; chunks run in order on that stream, so the table chains from chunk to chunk.
+// Arguments are validated by the callers: nothing here returns MV_ERR_BAD_ARG before it enqueues.
+static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* h_semi,
+                                          const float* h_semi_scale, const int8_t* h_desc, const float* h_depth,
+                                          mv_pair_result* h_results, unsigned long long* h2d_bytes,
+                                          unsigned long long* d2h_bytes, const HostLandmarks* lm) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see below); the
@@ -891,7 +898,12 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
     if (v > 0) chunk_pairs = v;
   }
   if (chunk_pairs > n_pairs) chunk_pairs = n_pairs;
+  if (lm) {  // one table step per pair: mv_landmarks_sequence's limits on one call
+    const int most = (int)std::min<long long>(65535, 0x7fffffffLL / p->top_n);
+    if (chunk_pairs > most) chunk_pairs = most;
+  }
   const int cf = chunk_pairs + 1;
+  const int N = p->top_n;
 
   // zero-copy gather needs device-visible (pinned) descriptor and depth buffers
   bool gather = true;
@@ -914,6 +926,7 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
 
   constexpr int NB = 3;  // chunks in flight: staging DMA / row gather / compute
   void *bs[NB], *bd[NB], *bz[NB], *bsc[NB], *dres, *dmoved;
+  void *bdsc[NB], *bword[NB], *bcin[NB], *bcout[NB], *dnwl = nullptr;   // landmark mode
   SeqScratch w[NB];
   mv_status st;
   const size_t semi_pad = ((size_t)cf * cells * 65 + 255) & ~(size_t)255;
@@ -924,6 +937,23 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
     if ((st = mv_scratch(c, (n + ".depth").c_str(), sizeof(float) * (size_t)cf * cells, &bz[b]))) return st;
     if ((st = mv_scratch(c, (n + ".scale").c_str(), sizeof(float) * (size_t)cf, &bsc[b]))) return st;
     if ((st = seq_scratch(c, p, cf, n.c_str(), &w[b]))) return st;
+    if (lm) {
+      const size_t q = (size_t)chunk_pairs * N;
+      if ((st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
+      if ((st = mv_scratch(c, (n + ".word").c_str(), sizeof(int32_t) * q, &bword[b]))) return st;
+      if ((st = mv_scratch(c, (n + ".coords_in").c_str(), sizeof(float) * 3 * q, &bcin[b]))) return st;
+      if ((st = mv_scratch(c, (n + ".coords_out").c_str(), sizeof(float) * 3 * q, &bcout[b]))) return st;
+    }
+  }
+  if (lm) {
+    // the table update's shared sort scratch, for the full chunk and the last one: growing it between
+    // enqueues would free memory (cudaFree) while the three streams run
+    const int last_steps = n_pairs - (n_pairs - 1) / chunk_pairs * chunk_pairs;
+    if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, chunk_pairs, N))) return st;
+    if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, last_steps, N))) return st;
+    if (lm->h_n_with_landmark &&
+        (st = mv_scratch(c, "host.n_with_landmark", sizeof(int32_t) * (size_t)n_pairs, &dnwl)))
+      return st;
   }
   if ((st = mv_scratch(c, "host.results", sizeof(mv_pair_result) * (size_t)n_pairs, &dres))) return st;
   if ((st = mv_scratch(c, "host.moved", 16, &dmoved))) return st;
@@ -1003,6 +1033,11 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
     MV_CUDA(c, cudaMemcpyAsync(bz[b], h_depth + (size_t)p0 * cells, sizeof(float) * (size_t)nf * cells,
                                cudaMemcpyHostToDevice, cs));
     up += (unsigned long long)nf * ((size_t)cells * (65 + 4) + 4);
+    if (lm) {
+      MV_CUDA(c, cudaMemcpyAsync(bdsc[b], lm->h_desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice,
+                                 cs));
+      up += (unsigned long long)nf * 4;
+    }
     if (!gather) {
       MV_CUDA(c, cudaMemcpyAsync(bd[b], h_desc + (size_t)p0 * cells * 256, (size_t)nf * cells * 256,
                                  cudaMemcpyHostToDevice, cs));
@@ -1081,7 +1116,26 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
       MV_CUDA(c, cudaEventRecord(matched, c->stream));
       return launch_gather(k + 1, matched);
     };
-    s2 = seq_match_pose(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0);
+    if (lm) {
+      // after the chunk's `ready` and before its matcher: the word-assignment kernel (a persistent CTA per SM
+      // with the vocabulary in shared memory) never runs beside a row gather, which is released after the matcher
+      MvBackProject bp;
+      bp.q_idx = w[b].qi; bp.depth = (const float*)bz[b]; bp.rows = p->match.rows;
+      bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
+      bp.coords = (float*)bcin[b];
+      if ((s2 = mv_bow_assign_impl(c, nf - 1, cells, N, (const int8_t*)bd[b], (const float*)bdsc[b], w[b].qp,
+                                   w[b].qc, (int32_t*)bword[b], nullptr, bp)))
+        return s2;
+      if ((s2 = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame + p0, nf - 1, N,
+                                           (const int32_t*)bword[b], w[b].qc, (const float*)bcin[b],
+                                           (float*)bcout[b])))
+        return s2;
+      const SeqLandmarks sl = {lm->n_words, (const int32_t*)bword[b], (const float*)bcout[b],
+                               dnwl ? (int32_t*)dnwl + p0 : nullptr};
+      s2 = seq_match_pose(c, p, nf, (const int8_t*)bd[b], nullptr, w[b], (mv_pair_result*)dres + p0, p0, &sl);
+    } else {
+      s2 = seq_match_pose(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0);
+    }
     g_after_match = nullptr;
     g_seq_mark = nullptr;
     if (s2) return s2;
@@ -1099,8 +1153,14 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
     if ((st = stage_compute(k))) return st;
   }
   unsigned long long moved = 0;
+  unsigned long long down = sizeof(mv_pair_result) * (unsigned long long)n_pairs;
   MV_CUDA(c, cudaMemcpyAsync(h_results, dres, sizeof(mv_pair_result) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
                              c->stream));
+  if (dnwl) {
+    MV_CUDA(c, cudaMemcpyAsync(lm->h_n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
+                               c->stream));
+    down += sizeof(int32_t) * (unsigned long long)n_pairs;
+  }
   MV_CUDA(c, cudaStreamSynchronize(c->stream));
   MV_CUDA(c, cudaStreamSynchronize(c->copy_stream));
   MV_CUDA(c, cudaMemcpyAsync(&moved, dmoved, 8, cudaMemcpyDeviceToHost, c->gather_stream));
@@ -1115,8 +1175,42 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
   }
   if (gather) up += moved * 256ull;  // one 256 B descriptor row per staged cell
   if (h2d_bytes) *h2d_bytes = up;
-  if (d2h_bytes) *d2h_bytes = sizeof(mv_pair_result) * (unsigned long long)n_pairs;
+  if (d2h_bytes) *d2h_bytes = down;
   return MV_OK;
+}
+
+extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p, int n_frames,
+                                            const int8_t* h_semi, const float* h_semi_scale,
+                                            const int8_t* h_desc, const float* h_depth,
+                                            mv_pair_result* h_results, unsigned long long* h2d_bytes,
+                                            unsigned long long* d2h_bytes) {
+  MV_ENTER(c);
+  if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_depth || !h_results)
+    MV_BAD_ARG(c, "mv_track_sequence_host");
+  if (!seq_params_ok(p))
+    MV_BAD_ARG(c, "mv_track_sequence_host: rows, cols, top_n, max_valid and max_matches must be positive");
+  return track_sequence_host_impl(c, p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
+                                  d2h_bytes, nullptr);
+}
+
+extern "C" mv_status mv_track_sequence_landmarks_host(mv_ctx* c, const mv_track_params* p, int n_frames,
+                                                      int first_frame, const int8_t* h_semi, const float* h_semi_scale,
+                                                      const int8_t* h_desc, const float* h_desc_scale,
+                                                      const float* h_depth, int n_words, mv_landmark* d_table,
+                                                      mv_pair_result* h_results, int32_t* h_n_with_landmark,
+                                                      unsigned long long* h2d_bytes, unsigned long long* d2h_bytes) {
+  MV_ENTER(c);
+  if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_desc_scale || !h_depth || !h_results)
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks_host");
+  if (!seq_params_ok(p))
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: rows, cols, top_n, max_valid and max_matches must be positive");
+  if (c->bow_n_base <= 0)
+    MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: no vocabulary (mv_bow_set_vocabulary first)");
+  if (n_words <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: n_words must be positive");
+  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: NULL landmark table");
+  const HostLandmarks lm = {first_frame, n_words, d_table, h_desc_scale, h_n_with_landmark};
+  return track_sequence_host_impl(c, p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
+                                  d2h_bytes, &lm);
 }
 
 // ------------------------------------------------------------------------------------

@@ -617,6 +617,31 @@ extern "C" mv_status mv_landmarks_lookup(mv_ctx* ctx, int n_words, const mv_land
   return MV_OK;
 }
 
+// The counting sort's tiling (tiles of fb frames: at most 512 of them, the column scan's serial length, and 2^24
+// counters) and its scratch, shared by the call and by mv_landmarks_sequence_reserve.
+static void lmseq_tiles(int n_words, int n_steps, int* n_tiles, int* fb) {
+  int t = (int)std::min<long long>(std::min<long long>(512, (1LL << 24) / n_words), n_steps);
+  if (t < 1) t = 1;
+  *fb = (n_steps + t - 1) / t;
+  *n_tiles = (n_steps + *fb - 1) / *fb;
+}
+
+static mv_status lmseq_scratch(mv_ctx* ctx, int n_words, int n_steps, int top_n, void** cnt, void** tot, void** start,
+                               void** sorted) {
+  int n_tiles, fb;
+  lmseq_tiles(n_words, n_steps, &n_tiles, &fb);
+  mv_status st;
+  if ((st = mv_scratch(ctx, "lms.cnt", sizeof(int32_t) * (size_t)n_tiles * n_words, cnt))) return st;
+  if ((st = mv_scratch(ctx, "lms.total", sizeof(int32_t) * (size_t)n_words, tot))) return st;
+  if ((st = mv_scratch(ctx, "lms.start", sizeof(int32_t) * ((size_t)n_words + 1), start))) return st;
+  return mv_scratch(ctx, "lms.sorted", sizeof(int32_t) * (size_t)n_steps * top_n, sorted);
+}
+
+mv_status mv_landmarks_sequence_reserve(mv_ctx* ctx, int n_words, int n_steps, int top_n) {
+  void *cnt, *tot, *start, *sorted;
+  return lmseq_scratch(ctx, n_words, n_steps, top_n, &cnt, &tot, &start, &sorted);
+}
+
 mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_table, int first_frame, int n_steps,
                                      int top_n, const int32_t* d_word, const int32_t* d_q_count,
                                      const float* d_coords_in, float* d_coords_out) {
@@ -626,18 +651,12 @@ mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_ta
     MV_BAD_ARG(ctx, "mv_landmarks_sequence: 0..65535 steps of top_n > 0 queries, fewer than 2^31 in all");
   if (n_steps == 0) return MV_OK;
   if (!d_word || !d_q_count || !d_coords_in || !d_coords_out) MV_BAD_ARG(ctx, "mv_landmarks_sequence");
-  // tiles of fb frames: at most 512 of them (the column scan's serial length) and 2^24 counters
-  int n_tiles = (int)std::min<long long>(std::min<long long>(512, (1LL << 24) / n_words), n_steps);
-  if (n_tiles < 1) n_tiles = 1;
-  const int fb = (n_steps + n_tiles - 1) / n_tiles;
-  n_tiles = (n_steps + fb - 1) / fb;
+  int n_tiles, fb;
+  lmseq_tiles(n_words, n_steps, &n_tiles, &fb);
   const long long total = (long long)n_steps * top_n;
   void *cnt, *tot, *start, *sorted;
   mv_status st;
-  if ((st = mv_scratch(ctx, "lms.cnt", sizeof(int32_t) * (size_t)n_tiles * n_words, &cnt))) return st;
-  if ((st = mv_scratch(ctx, "lms.total", sizeof(int32_t) * (size_t)n_words, &tot))) return st;
-  if ((st = mv_scratch(ctx, "lms.start", sizeof(int32_t) * ((size_t)n_words + 1), &start))) return st;
-  if ((st = mv_scratch(ctx, "lms.sorted", sizeof(int32_t) * (size_t)total, &sorted))) return st;
+  if ((st = lmseq_scratch(ctx, n_words, n_steps, top_n, &cnt, &tot, &start, &sorted))) return st;
   {
     mv_prof_scope ps(ctx, "sort");
     MV_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)n_tiles * n_words, ctx->stream));

@@ -143,6 +143,9 @@ mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, co
 mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_table, int first_frame, int n_steps,
                                      int top_n, const int32_t* d_word, const int32_t* d_q_count,
                                      const float* d_coords_in, float* d_coords_out);
+// allocates the scratch mv_landmarks_sequence_impl needs for n_steps steps (callers that must not grow scratch
+// while other streams run, i.e. the host-buffer pipeline, reserve it for their largest call up front)
+mv_status mv_landmarks_sequence_reserve(mv_ctx* ctx, int n_words, int n_steps, int top_n);
 // mv_build_corr_landmarks_batch for pairs (p, p+1) with the 3-D side from mv_landmarks_sequence's coords_out
 mv_status mv_build_corr_landmarks_seq(mv_ctx* ctx, int n_pairs, int top_n, int stride, int n_words,
                                       const int32_t* d_q_patch, const int32_t* d_q_count, const int32_t* d_word,

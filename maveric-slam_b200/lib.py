@@ -28,7 +28,7 @@ NEW_SYMBOLS = [
     "mv_lba_solve_batch",
     "mv_bow_set_vocabulary", "mv_bow_assign_batch", "mv_landmarks_init", "mv_landmarks_observe",
     "mv_landmarks_remove_old", "mv_landmarks_lookup", "mv_build_corr_landmarks_batch", "mv_landmarks_sequence",
-    "mv_track_sequence_landmarks",
+    "mv_track_sequence_landmarks", "mv_track_sequence_landmarks_host",
 ]
 LEGACY_SYMBOLS = [
     "add_Vector2f", "add_Vector3f", "mult_Quaternionf", "create_Quaternionf", "Quaternionf_from_Vector3f",
@@ -140,6 +140,8 @@ def load() -> C.CDLL:
     L.mv_build_corr_landmarks_batch.argtypes = [vp, i32, i32, i32, i32] + [vp] * 10
     L.mv_landmarks_sequence.argtypes = [vp, i32, vp, i32, i32, i32, vp, vp, vp, vp]
     L.mv_track_sequence_landmarks.argtypes = [vp, C.POINTER(TrackParams), i32, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp]
+    L.mv_track_sequence_landmarks_host.argtypes = [vp, C.POINTER(TrackParams), i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
+                                                   vp, C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]
     L.mv_synth_frames.argtypes = [vp, C.POINTER(SynthParams), i32, i32, vp, vp, vp, vp]
     L.mv_nms_batch.argtypes = [vp, i32, i32, i32, vp, vp]
     L.run_nms_ex.argtypes = [vp, i32, i32, vp, vp]

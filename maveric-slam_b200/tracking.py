@@ -478,6 +478,26 @@ class Tracker:
             self._d(desc_scale), self._d(depth), table.shape[0], self._d(table), self._d(out), self._d(n_with_landmark)))
         return out, n_with_landmark
 
+    def track_sequence_landmarks_host(self, params: _lib.TrackParams, semi, semi_scale, desc, desc_scale, depth, table,
+                                      first_frame=0, out=None, n_with_landmark=None):
+        """:meth:`track_sequence_landmarks` from host tensors/arrays (pinned for full copy bandwidth, as
+        :meth:`track_sequence_host`); `table` stays on the device and is updated in place.  Blocks until the results
+        are on the host.  Returns (results structured array, int32 [n_pairs] matches with a landmark, h2d_bytes,
+        d2h_bytes)."""
+        n = semi.shape[0]
+        if out is None:
+            out = np.zeros(n - 1, PAIR_RESULT_DTYPE)
+        if n_with_landmark is None:
+            n_with_landmark = np.zeros(n - 1, np.int32)
+
+        def hp(a):
+            return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else _p(a)
+        up = C.c_ulonglong(0); down = C.c_ulonglong(0)
+        self.ctx.check(self.lib.mv_track_sequence_landmarks_host(
+            self.ctx.h, C.byref(params), n, int(first_frame), hp(semi), hp(semi_scale), hp(desc), hp(desc_scale),
+            hp(depth), table.shape[0], self._d(table), hp(out), hp(n_with_landmark), C.byref(up), C.byref(down)))
+        return out, n_with_landmark, up.value, down.value
+
     def chain_transforms(self, transforms):
         """python/compute_trajectory.py:49-51,76-77 as a parallel scan: float64 [n, 3, 4] relative
         transforms -> float64 [n+1, 3, 4] frame poses, pose 0 the identity."""

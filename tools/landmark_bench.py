@@ -6,7 +6,11 @@ tests/golden/ref_vocab.npz), against the depth path (mv_track_sequence) in the s
 Reports device-resident pairs/s of both paths (host clock around work ending in a device synchronise), the per-stage
 device times of the landmark path from the context's profile mode (bow, sort, walk, corr), the per-frame loop of
 mv_landmarks_observe / mv_landmarks_remove_old over the same words for contrast, the longest word list and the mean
-landmarks per pair.   python tools/landmark_bench.py [frames] [steps] > out.json"""
+landmarks per pair.
+
+End to end from pinned host buffers (the frames a caller gets off a camera or a file), alternated in one process:
+the depth path (mv_track_sequence_host) and the landmark path (mv_track_sequence_landmarks_host); median pairs/s,
+h2d bytes and the host-to-device rate they imply.   python tools/landmark_bench.py [frames] [steps] > out.json"""
 import json
 import os
 import subprocess
@@ -104,6 +108,44 @@ per_frame_loop(); batched()
 loop_s = min(timed(per_frame_loop) for _ in range(3))
 seq_s = min(timed(batched) for _ in range(3))
 
+# end to end from pinned host buffers
+def pinned(t):
+    return torch.empty(t.shape, dtype=t.dtype, pin_memory=True).copy_(t)
+
+
+hs, hsc, hd, hds, hz = (pinned(t) for t in (semi, sscale, desc, dscale, depth))
+host_nl = np.zeros(NF - 1, np.int32)
+e2e = {}
+
+
+def depth_host():
+    e2e["depth_host"] = tr.track_sequence_host(p, hs, hsc, hd, hz)
+
+
+def landmark_host():
+    tr.ctx.check(tr.lib.mv_landmarks_init(tr.ctx.h, tr.n_words, tr._d(table)))
+    e2e["landmark_host"] = tr.track_sequence_landmarks_host(p, hs, hsc, hd, hds, hz, table, n_with_landmark=host_nl)
+
+
+legs = {"depth_host": depth_host, "landmark_host": landmark_host}
+for fn in legs.values():   # warm-up: pinned pages, scratch of the host pipeline
+    fn()
+e2e_times = {k: [] for k in legs}
+for _ in range(STEPS):
+    for k, fn in legs.items():
+        e2e_times[k].append(timed(fn))
+host_table = table.clone()
+landmark_step()
+device_res, device_nl = out.cpu().numpy().tobytes(), nl.cpu().numpy()
+host_equals_device = (e2e["landmark_host"][0].tobytes() == device_res and (host_nl == device_nl).all()
+                      and bool(torch.equal(host_table, table)))
+e2e_out = {}
+for k in legs:
+    med = float(np.median(e2e_times[k]))
+    up = e2e[k][-2]
+    e2e_out[k] = {"median_s": med, "pairs_per_s": (NF - 1) / med, "h2d_bytes": up, "d2h_bytes": e2e[k][-1],
+                  "h2d_GB_per_s": up / med / 1e9, "h2d_bytes_per_frame": up / NF, "all_s": e2e_times[k]}
+
 w = word.cpu().numpy()
 valid = w[(w >= 0) & (w < tr.n_words)]
 hist = np.bincount(valid, minlength=tr.n_words)
@@ -123,4 +165,5 @@ print(json.dumps({
     "occurrences": int(valid.size), "distinct_words": int((hist > 0).sum()), "longest_word_list": int(hist.max()),
     "longest_word": int(hist.argmax()), "mean_landmarks_per_pair": float(nl.float().mean().item()),
     "mean_matches_per_pair": float(res["num_matches"].mean()),
+    "e2e_pinned": e2e_out, "e2e_landmark_host_equals_device": bool(host_equals_device),
 }, indent=1))
