@@ -290,6 +290,16 @@ mv_status mv_landmarks_sequence(mv_ctx* ctx, int n_words, mv_landmark* d_table, 
 /* Whole path over a sequence of frames (pair p = frames p, p+1)              */
 /* ------------------------------------------------------------------------- */
 
+/* Argument errors of the four sequence calls (mv_track_sequence, mv_track_sequence_host,
+ * mv_track_sequence_landmarks, mv_track_sequence_landmarks_host) are MV_ERR_BAD_ARG before anything is
+ * allocated or enqueued, so a landmark table is untouched.  They cover every refusal of the batched calls the
+ * path is made of: NULL inputs, n_frames < 2, non-positive rows / cols / top_n / max_valid / max_matches,
+ * match.radius < 0, max_matches > 65535, the PnP limits of mv_pnp_gn_batch (hypotheses, sample_size,
+ * lanes_per_hypothesis), use_tensor_cores = 1 on a shape the tensor-core matcher does not take (for the host
+ * calls: their largest chunk), more than 65535 frames in the device calls, a d_desc that is not 16-byte aligned
+ * in the device calls; in landmark mode also no vocabulary, a vocabulary larger than the word assignment's
+ * shared memory, n_words <= 0, a NULL table and (n_frames - 1) * top_n >= 2^31 in the device call. */
+
 typedef struct {
   mv_match_params match;
   mv_pnp_params   pnp;
@@ -367,9 +377,9 @@ mv_status mv_track_sequence_landmarks(mv_ctx* ctx, const mv_track_params* p, int
  *   - h2d_bytes: those of mv_track_sequence_host (logits, semi scales, depth planes, the descriptor rows the
  *     matcher reads -- the word assignment reads only query rows, which are among them) plus the desc scales;
  *     d2h_bytes: the records, plus h_n_with_landmark when given;
- *   - argument errors (no vocabulary, NULL table, n_words <= 0, non-positive sizes, n_frames < 2) are
- *     MV_ERR_BAD_ARG before anything is enqueued: the table is untouched.  After a CUDA error the streams are
- *     drained and the host buffers no longer read, but the table's state is unspecified.
+ *   - argument errors are MV_ERR_BAD_ARG before anything is enqueued (see above): the table is untouched.  After
+ *     a CUDA error the streams are drained and the host buffers no longer read, but the table's state is
+ *     unspecified.
  * Not sharded over GPUs: a rank's initial table would depend on every earlier frame. */
 mv_status mv_track_sequence_landmarks_host(mv_ctx* ctx, const mv_track_params* p, int n_frames, int first_frame,
                                            const int8_t* h_semi, const float* h_semi_scale,

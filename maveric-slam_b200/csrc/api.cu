@@ -13,6 +13,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <functional>
 #include <mutex>
 
 #include "../../include/maveric_slam_compat.h"
@@ -577,21 +578,60 @@ __global__ void pack_results_kernel(int n_pairs, const float* __restrict__ pose,
   out[p] = r;
 }
 
+// Landmark mode of the sequence calls: the 3-D side of pair p's correspondences comes from the caller's table right
+// after step p instead of depth.  seq_step reads the descriptor of its batch, with device pointers; the host pipeline
+// keeps one for the whole call, with the caller's host desc_scale / n_with_landmark, and derives each chunk's.
+struct SeqLandmarks {
+  int first_frame, n_words;
+  mv_landmark* table;
+  const float* desc_scale;    // one per frame
+  int32_t* n_with_landmark;   // one per pair, nullable
+};
+
 // Scratch of one in-flight batch of frames ("ns" = arena namespace, so two batches can be
 // in flight in the double-buffered host path).
 struct SeqScratch {
   int32_t *idx, *qp, *qi, *qc, *ov, *mc, *mcell, *rin;
   float *prob, *qpr, *mp, *corr, *pose, *stats;
   uint8_t* flags;
+  int32_t* word;              // landmark mode: [n_frames - 1][top_n]
+  float *coords_in, *coords_out;   // landmark mode: [n_frames - 1][top_n][3]
 };
 
-// sizes every scratch buffer of the sequence calls is computed from
-static bool seq_params_ok(const mv_track_params* p) {
-  return p->match.rows > 0 && p->match.cols > 0 && p->top_n > 0 && p->max_valid > 0 && p->match.max_matches > 0 &&
-         (long long)p->match.rows * p->match.cols <= 0x7fffffffLL;
+// Every refusal seq_detect and seq_step could make from the arguments, so that a sequence call refuses before it
+// allocates or enqueues anything.  n_frames: the largest batch the call runs (the whole sequence for the
+// device-resident calls, the largest chunk for the host ones); d_desc: the caller's descriptors, or NULL when they
+// are staged into scratch.
+static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+                           const SeqLandmarks* lm) {
+  auto refuse = [&](const char* why) {
+    snprintf(c->err, sizeof(c->err), "bad argument: %s: %s", fn, why);
+    return MV_ERR_BAD_ARG;
+  };
+  const mv_match_params& m = p->match;
+  if (m.rows <= 0 || m.cols <= 0 || p->top_n <= 0 || p->max_valid <= 0 || m.max_matches <= 0 ||
+      (long long)m.rows * m.cols > 0x7fffffffLL)
+    return refuse("rows, cols, top_n, max_valid and max_matches must be positive");
+  if (m.radius < 0) return refuse("match.radius must be >= 0");
+  if (!mv_pnp_params_ok(&p->pnp, m.max_matches))
+    return refuse("max_matches <= 65535, pnp.hypotheses in [1,65536], pnp.sample_size in [1,255], "
+                  "pnp.lanes_per_hypothesis 1 or 32");
+  if (n_frames > 65535)
+    return refuse("at most 65535 frames per call (grid y dimension); mv_track_sequence_host chunks longer sequences");
+  if (m.use_tensor_cores != 0 && m.use_tensor_cores != 2 && !mv_match_tc_feasible(&m, n_frames, n_frames - 1, p->top_n))
+    return refuse("use_tensor_cores = 1 on a shape the tensor-core matcher does not take (2 picks the matcher)");
+  if (d_desc && (reinterpret_cast<uintptr_t>(d_desc) & 15)) return refuse("d_desc must be 16-byte aligned");
+  if (!lm) return MV_OK;
+  if (c->bow_n_base <= 0) return refuse("no vocabulary (mv_bow_set_vocabulary first)");
+  if (!mv_bow_vocab_fits(c)) return refuse("vocabulary larger than an SM's shared memory");
+  if (lm->n_words <= 0) return refuse("n_words must be positive");
+  if (!lm->table) return refuse("NULL landmark table");
+  if ((long long)(n_frames - 1) * p->top_n > 0x7fffffffLL) return refuse("(n_frames - 1) * top_n must be below 2^31");
+  return MV_OK;
 }
 
-static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, const char* ns, SeqScratch* o) {
+static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, const char* ns, bool landmarks,
+                             SeqScratch* o) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
@@ -616,6 +656,11 @@ static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, 
   SCR(corr, float, ".corr", sizeof(float) * 5 * (size_t)n_pairs * M);
   SCR(pose, float, ".pose", sizeof(float) * 7 * (size_t)n_pairs);
   SCR(stats, float, ".stats", sizeof(float) * 4 * (size_t)n_pairs);
+  if (landmarks) {
+    SCR(word, int32_t, ".word", sizeof(int32_t) * (size_t)n_pairs * N);
+    SCR(coords_in, float, ".coords_in", sizeof(float) * 3 * (size_t)n_pairs * N);
+    SCR(coords_out, float, ".coords_out", sizeof(float) * 3 * (size_t)n_pairs * N);
+  }
 #undef SCR
   return MV_OK;
 }
@@ -629,49 +674,51 @@ static mv_status seq_detect(mv_ctx* c, const mv_track_params* p, int n_frames, c
   return mv_top_n_batch(c, n_frames, cells, p->top_n, p->max_valid, w.idx, w.prob, w.qp, w.qi, w.qpr, w.qc, w.ov);
 }
 
-#include <functional>
-static thread_local std::function<void(const char*)> g_seq_mark;  // MV_HOST_TRACE debug hook
-// Host-pipelined path: called right after the matcher has been enqueued, before the pose
-// kernels -- the point where the next chunk's row gather is released (see below).
-static thread_local std::function<mv_status()> g_after_match;
+// Called by seq_step once the matcher ("match_end") and the correspondences ("corr_end") are enqueued.
+using SeqStageFn = std::function<mv_status(const char* stage)>;
 
-// 3-D side of the correspondences from the landmark table (mv_track_sequence_landmarks) instead of depth
-struct SeqLandmarks {
-  int n_words;
-  const int32_t* word;       // [n_frames - 1][top_n]
-  const float* coords_out;   // [n_frames - 1][top_n][3], mv_landmarks_sequence
-  int32_t* n_with_landmark;  // nullable
-};
-
-// Match + pose half: needs descriptors (only rows of candidate / query cells are read) and
-// depth (only at matched frame-0 cells), or the landmarks of frame 0's queries.
-static mv_status seq_match_pose(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                                const float* d_depth, const SeqScratch& w, mv_pair_result* d_results,
-                                int pair_offset, const SeqLandmarks* lm = nullptr) {
+// The rest of a batch whose detector has run: with `lm`, the word assignment of frames 0..n-2 with their query
+// keypoints back-projected in the same launch and the table walked over those frames from lm->first_frame; then
+// match / RANSAC-E / correspondences / K3 / pack.  Only descriptor rows of candidate / query cells are read, and
+// depth only at matched frame-0 cells (or, with `lm`, at query cells).
+static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+                          const float* d_depth, const SeqScratch& w, mv_pair_result* d_results, int first_pair,
+                          const SeqLandmarks* lm, const SeqStageFn& on_stage = nullptr) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
   mv_status st;
+  if (lm) {
+    MvBackProject bp;
+    bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
+    bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
+    bp.coords = w.coords_in;
+    if ((st = mv_bow_assign_impl(c, n_pairs, cells, N, d_desc, lm->desc_scale, w.qp, w.qc, w.word, nullptr, bp)))
+      return st;
+    if ((st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_pairs, N, w.word, w.qc,
+                                         w.coords_in, w.coords_out)))
+      return st;
+  }
   if ((st = mv_match_batch(c, &p->match, n_frames, n_pairs, N, nullptr, nullptr, d_desc, w.idx, w.prob, w.qp, w.qi,
                            w.qc, w.mp, w.mc, w.mcell, nullptr, nullptr)))
     return st;
-  if (g_after_match && (st = g_after_match())) return st;
+  if (on_stage && (st = on_stage("match_end"))) return st;
   if (p->ransac_iterations > 0) {
     if ((st = mv_ransac_identity_batch(c, n_pairs, M, w.mp, w.mc, p->ransac_iterations, p->ransac_threshold,
                                        w.rin, nullptr, nullptr)))
       return st;
   }
   if (lm) {
-    if ((st = mv_build_corr_landmarks_seq(c, n_pairs, N, M, lm->n_words, w.qp, w.qc, lm->word, lm->coords_out, w.mp,
+    if ((st = mv_build_corr_landmarks_seq(c, n_pairs, N, M, lm->n_words, w.qp, w.qc, w.word, w.coords_out, w.mp,
                                           w.mc, w.mcell, w.corr, lm->n_with_landmark)))
       return st;
   } else if ((st = mv_build_corr_batch(c, n_pairs, cells, p->match.rows, M, nullptr, d_depth, p->pnp.fx, p->pnp.fy,
                                        p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr))) {
     return st;
   }
-  if (g_seq_mark) g_seq_mark("corr_end");
+  if (on_stage && (st = on_stage("corr_end"))) return st;
   mv_pnp_params pnp = p->pnp;
-  pnp.first_pair += pair_offset;
+  pnp.first_pair += first_pair;
   if ((st = mv_pnp_gn_batch(c, &pnp, n_pairs, M, w.corr, w.mc, nullptr, w.pose, w.stats, nullptr))) return st;
   pack_results_kernel<<<(n_pairs + 127) / 128, 128, 0, c->stream>>>(
       n_pairs, w.pose, w.stats, w.mc, p->ransac_iterations > 0 ? w.rin : nullptr, w.ov, d_results);
@@ -685,19 +732,16 @@ extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int 
   MV_ENTER(c);
   if (!p || n_frames < 2 || !d_semi || !d_semi_scale || !d_desc || !d_depth || !d_results)
     MV_BAD_ARG(c, "mv_track_sequence");
-  if (!seq_params_ok(p)) MV_BAD_ARG(c, "mv_track_sequence: rows, cols, top_n, max_valid and max_matches must be positive");
-  if (n_frames > 65535)
-    MV_BAD_ARG(c, "mv_track_sequence: at most 65535 frames per call (grid y dimension); mv_track_sequence_host chunks longer sequences");
   SeqScratch w;
   mv_status st;
-  if ((st = seq_scratch(c, p, n_frames, "seq", &w))) return st;
-  if ((st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w))) return st;
-  return seq_match_pose(c, p, n_frames, d_desc, d_depth, w, d_results, 0);
+  if ((st = seq_check(c, "mv_track_sequence", p, n_frames, d_desc, nullptr)) ||
+      (st = seq_scratch(c, p, n_frames, "seq", false, &w)) || (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
+    return st;
+  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, 0, nullptr);
 }
 
-// Pair p = frames (p, p+1) with the 3-D side from the landmark table right after step p: detector, word
-// assignment of frames 0..n-2 with their query keypoints back-projected in the same launch, the table walked over
-// those frames in one batch (mv_landmarks_sequence), then match / RANSAC-E / correspondences / K3 / pack.
+// Pair p = frames (p, p+1) with the 3-D side from the landmark table right after step p: detector, then seq_step in
+// landmark mode over the whole sequence.
 extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_params* p, int n_frames, int first_frame,
                                                  const int8_t* d_semi, const float* d_semi_scale, const int8_t* d_desc,
                                                  const float* d_desc_scale, const float* d_depth, int n_words,
@@ -706,36 +750,14 @@ extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_param
   MV_ENTER(c);
   if (!p || n_frames < 2 || !d_semi || !d_semi_scale || !d_desc || !d_desc_scale || !d_depth || !d_results)
     MV_BAD_ARG(c, "mv_track_sequence_landmarks");
-  if (!seq_params_ok(p))
-    MV_BAD_ARG(c, "mv_track_sequence_landmarks: rows, cols, top_n, max_valid and max_matches must be positive");
-  if (n_frames > 65535) MV_BAD_ARG(c, "mv_track_sequence_landmarks: at most 65535 frames per call");
-  if (c->bow_n_base <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks: no vocabulary (mv_bow_set_vocabulary first)");
-  if (n_words <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks: n_words must be positive");
-  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks: NULL landmark table");
-  if (reinterpret_cast<uintptr_t>(d_desc) & 15) MV_BAD_ARG(c, "mv_track_sequence_landmarks: d_desc must be 16-byte aligned");
-  if ((long long)(n_frames - 1) * p->top_n > 0x7fffffffLL)
-    MV_BAD_ARG(c, "mv_track_sequence_landmarks: (n_frames - 1) * top_n must be below 2^31");
-  const int cells = p->match.rows * p->match.cols;
-  const int n_steps = n_frames - 1, N = p->top_n;
+  const SeqLandmarks lm = {first_frame, n_words, d_table, d_desc_scale, d_n_with_landmark};
   SeqScratch w;
-  void *word, *cin, *cout;
   mv_status st;
-  if ((st = seq_scratch(c, p, n_frames, "lmseq", &w))) return st;
-  if ((st = mv_scratch(c, "lmseq.word", sizeof(int32_t) * (size_t)n_steps * N, &word))) return st;
-  if ((st = mv_scratch(c, "lmseq.coords_in", sizeof(float) * 3 * (size_t)n_steps * N, &cin))) return st;
-  if ((st = mv_scratch(c, "lmseq.coords_out", sizeof(float) * 3 * (size_t)n_steps * N, &cout))) return st;
-  if ((st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w))) return st;
-  MvBackProject bp;
-  bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
-  bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
-  bp.coords = (float*)cin;
-  if ((st = mv_bow_assign_impl(c, n_steps, cells, N, d_desc, d_desc_scale, w.qp, w.qc, (int32_t*)word, nullptr, bp)))
+  if ((st = seq_check(c, "mv_track_sequence_landmarks", p, n_frames, d_desc, &lm)) ||
+      (st = seq_scratch(c, p, n_frames, "lmseq", true, &w)) ||
+      (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
     return st;
-  if ((st = mv_landmarks_sequence_impl(c, n_words, d_table, first_frame, n_steps, N, (const int32_t*)word, w.qc,
-                                       (const float*)cin, (float*)cout)))
-    return st;
-  const SeqLandmarks lm = {n_words, (const int32_t*)word, (const float*)cout, d_n_with_landmark};
-  return seq_match_pose(c, p, n_frames, d_desc, nullptr, w, d_results, 0, &lm);
+  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, 0, &lm);
 }
 
 // ---- selective staging of descriptors from pinned host memory ------------------------
@@ -855,33 +877,17 @@ struct PnpResidencyCap {  // cap the PnP kernel's CTAs per SM for a scope
   ~PnpResidencyCap() { c->pnp_max_ctas_per_sm = saved; }
 };
 
-struct StreamSwap {  // run the context's kernels on another stream for a scope
-  mv_ctx* c;
-  cudaStream_t saved;
-  StreamSwap(mv_ctx* ctx, cudaStream_t s) : c(ctx), saved(ctx->stream) { ctx->stream = s; }
-  ~StreamSwap() { c->stream = saved; }
-};
-
-// Landmark mode of the host pipeline (mv_track_sequence_landmarks_host): the caller's table and the inputs only
-// that path reads.
-struct HostLandmarks {
-  int first_frame, n_words;
-  mv_landmark* table;
-  const float* h_desc_scale;
-  int32_t* h_n_with_landmark;  // nullable
-};
-
 // Host inputs.  Chunks of frames are double-buffered: on the staging stream the logits are
 // copied and the detector runs, then descriptors arrive (selectively when the host buffers
-// are pinned, else as a plain copy); the compute stream matches and solves the previous chunk
-// meanwhile.  Consecutive chunks share one halo frame.  With `lm` the compute stream also assigns
-// the words of the chunk's frames but its halo and steps the caller's landmark table over them
-// before matching; chunks run in order on that stream, so the table chains from chunk to chunk.
-// Arguments are validated by the callers: nothing here returns MV_ERR_BAD_ARG before it enqueues.
-static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* h_semi,
-                                          const float* h_semi_scale, const int8_t* h_desc, const float* h_depth,
-                                          mv_pair_result* h_results, unsigned long long* h2d_bytes,
-                                          unsigned long long* d2h_bytes, const HostLandmarks* lm) {
+// are pinned, else as a plain copy); the compute stream runs seq_step on the previous chunk
+// meanwhile.  Consecutive chunks share one halo frame.  With `lm` (host desc_scale and
+// n_with_landmark) seq_step also steps the caller's landmark table over the chunk's frames but its
+// halo before matching; chunks run in order on that stream, so the table chains from chunk to chunk.
+static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames,
+                                          const int8_t* h_semi, const float* h_semi_scale, const int8_t* h_desc,
+                                          const float* h_depth, mv_pair_result* h_results,
+                                          unsigned long long* h2d_bytes, unsigned long long* d2h_bytes,
+                                          const SeqLandmarks* lm) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see below); the
@@ -898,12 +904,14 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
     if (v > 0) chunk_pairs = v;
   }
   if (chunk_pairs > n_pairs) chunk_pairs = n_pairs;
-  if (lm) {  // one table step per pair: mv_landmarks_sequence's limits on one call
-    const int most = (int)std::min<long long>(65535, 0x7fffffffLL / p->top_n);
+  if (lm) {  // one table step per pair: mv_landmarks_sequence's limits on one call (top_n > 0 is checked below)
+    const int most = (int)std::min<long long>(65535, 0x7fffffffLL / std::max(p->top_n, 1));
     if (chunk_pairs > most) chunk_pairs = most;
   }
   const int cf = chunk_pairs + 1;
   const int N = p->top_n;
+  mv_status st;
+  if ((st = seq_check(c, fn, p, cf, nullptr, lm))) return st;
 
   // zero-copy gather needs device-visible (pinned) descriptor and depth buffers
   bool gather = true;
@@ -926,9 +934,8 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
 
   constexpr int NB = 3;  // chunks in flight: staging DMA / row gather / compute
   void *bs[NB], *bd[NB], *bz[NB], *bsc[NB], *dres, *dmoved;
-  void *bdsc[NB], *bword[NB], *bcin[NB], *bcout[NB], *dnwl = nullptr;   // landmark mode
+  void *bdsc[NB], *dnwl = nullptr;   // landmark mode
   SeqScratch w[NB];
-  mv_status st;
   const size_t semi_pad = ((size_t)cf * cells * 65 + 255) & ~(size_t)255;
   for (int b = 0; b < NB; b++) {
     const std::string n = "host.buf" + std::to_string(b);
@@ -936,14 +943,8 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
     if ((st = mv_scratch(c, (n + ".desc").c_str(), (size_t)cf * cells * 256, &bd[b]))) return st;
     if ((st = mv_scratch(c, (n + ".depth").c_str(), sizeof(float) * (size_t)cf * cells, &bz[b]))) return st;
     if ((st = mv_scratch(c, (n + ".scale").c_str(), sizeof(float) * (size_t)cf, &bsc[b]))) return st;
-    if ((st = seq_scratch(c, p, cf, n.c_str(), &w[b]))) return st;
-    if (lm) {
-      const size_t q = (size_t)chunk_pairs * N;
-      if ((st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
-      if ((st = mv_scratch(c, (n + ".word").c_str(), sizeof(int32_t) * q, &bword[b]))) return st;
-      if ((st = mv_scratch(c, (n + ".coords_in").c_str(), sizeof(float) * 3 * q, &bcin[b]))) return st;
-      if ((st = mv_scratch(c, (n + ".coords_out").c_str(), sizeof(float) * 3 * q, &bcout[b]))) return st;
-    }
+    if ((st = seq_scratch(c, p, cf, n.c_str(), lm != nullptr, &w[b]))) return st;
+    if (lm && (st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
   }
   if (lm) {
     // the table update's shared sort scratch, for the full chunk and the last one: growing it between
@@ -951,7 +952,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
     const int last_steps = n_pairs - (n_pairs - 1) / chunk_pairs * chunk_pairs;
     if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, chunk_pairs, N))) return st;
     if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, last_steps, N))) return st;
-    if (lm->h_n_with_landmark &&
+    if (lm->n_with_landmark &&
         (st = mv_scratch(c, "host.n_with_landmark", sizeof(int32_t) * (size_t)n_pairs, &dnwl)))
       return st;
   }
@@ -1034,7 +1035,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
                                cudaMemcpyHostToDevice, cs));
     up += (unsigned long long)nf * ((size_t)cells * (65 + 4) + 4);
     if (lm) {
-      MV_CUDA(c, cudaMemcpyAsync(bdsc[b], lm->h_desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice,
+      MV_CUDA(c, cudaMemcpyAsync(bdsc[b], lm->desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice,
                                  cs));
       up += (unsigned long long)nf * 4;
     }
@@ -1052,8 +1053,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
   // queued on the same SM stretch its global loads; the pose kernel (FP32-bound, its inputs in
   // shared memory) does not care.
   int pending_gather = -1;
-  // MV_HOST_EAGER_GATHER=1: start a chunk's row gather as soon as its detector is done (A/B knob)
-  const bool eager_gather = getenv("MV_HOST_EAGER_GATHER") && atoi(getenv("MV_HOST_EAGER_GATHER"));
   cudaEvent_t matched;
   if ((st = new_event(&matched))) return st;
   auto launch_gather = [&](int k, cudaEvent_t after) -> mv_status {
@@ -1096,48 +1095,32 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
     mark("det_end", k, c->stream);
     if (!gather) {
       MV_CUDA(c, cudaEventRecord(ready[b], c->stream));
-    } else if (k == 0 || eager_gather) {
+    } else if (k == 0) {
       return launch_gather(k, nullptr);
     } else {
       pending_gather = k;   // released by chunk k-1's matcher, see stage_compute
     }
     return MV_OK;
   };
+  // In landmark mode seq_step runs the word assignment (a persistent CTA per SM with the vocabulary in shared
+  // memory) after the chunk's `ready` and before its matcher, so it never runs beside a row gather.
   auto stage_compute = [&](int k) -> mv_status {
     const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
-    mv_status s2;
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, ready[b], 0));
     mark("cmp_beg", k, c->stream);
-    if (trace) g_seq_mark = [&, k](const char* what) { mark(what, k, c->stream); };
-    g_after_match = [&, k]() -> mv_status {
-      mark("match_end", k, c->stream);
-      if (pending_gather != k + 1) return MV_OK;
+    const SeqStageFn on_stage = [&](const char* stage) -> mv_status {
+      mark(stage, k, c->stream);
+      if (strcmp(stage, "match_end") || pending_gather != k + 1) return MV_OK;
       pending_gather = -1;
       MV_CUDA(c, cudaEventRecord(matched, c->stream));
       return launch_gather(k + 1, matched);
     };
-    if (lm) {
-      // after the chunk's `ready` and before its matcher: the word-assignment kernel (a persistent CTA per SM
-      // with the vocabulary in shared memory) never runs beside a row gather, which is released after the matcher
-      MvBackProject bp;
-      bp.q_idx = w[b].qi; bp.depth = (const float*)bz[b]; bp.rows = p->match.rows;
-      bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
-      bp.coords = (float*)bcin[b];
-      if ((s2 = mv_bow_assign_impl(c, nf - 1, cells, N, (const int8_t*)bd[b], (const float*)bdsc[b], w[b].qp,
-                                   w[b].qc, (int32_t*)bword[b], nullptr, bp)))
-        return s2;
-      if ((s2 = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame + p0, nf - 1, N,
-                                           (const int32_t*)bword[b], w[b].qc, (const float*)bcin[b],
-                                           (float*)bcout[b])))
-        return s2;
-      const SeqLandmarks sl = {lm->n_words, (const int32_t*)bword[b], (const float*)bcout[b],
-                               dnwl ? (int32_t*)dnwl + p0 : nullptr};
-      s2 = seq_match_pose(c, p, nf, (const int8_t*)bd[b], nullptr, w[b], (mv_pair_result*)dres + p0, p0, &sl);
-    } else {
-      s2 = seq_match_pose(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0);
-    }
-    g_after_match = nullptr;
-    g_seq_mark = nullptr;
+    SeqLandmarks chunk_lm{};
+    if (lm)
+      chunk_lm = {lm->first_frame + p0, lm->n_words, lm->table, (const float*)bdsc[b],
+                  dnwl ? (int32_t*)dnwl + p0 : nullptr};
+    mv_status s2 = seq_step(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0,
+                            lm ? &chunk_lm : nullptr, on_stage);
     if (s2) return s2;
     MV_CUDA(c, cudaEventRecord(consumed[b], c->stream));
     mark("cmp_end", k, c->stream);
@@ -1157,7 +1140,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const mv_track_params* p, i
   MV_CUDA(c, cudaMemcpyAsync(h_results, dres, sizeof(mv_pair_result) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
                              c->stream));
   if (dnwl) {
-    MV_CUDA(c, cudaMemcpyAsync(lm->h_n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
+    MV_CUDA(c, cudaMemcpyAsync(lm->n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
                                c->stream));
     down += sizeof(int32_t) * (unsigned long long)n_pairs;
   }
@@ -1187,9 +1170,7 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
   MV_ENTER(c);
   if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_depth || !h_results)
     MV_BAD_ARG(c, "mv_track_sequence_host");
-  if (!seq_params_ok(p))
-    MV_BAD_ARG(c, "mv_track_sequence_host: rows, cols, top_n, max_valid and max_matches must be positive");
-  return track_sequence_host_impl(c, p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
+  return track_sequence_host_impl(c, "mv_track_sequence_host", p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
                                   d2h_bytes, nullptr);
 }
 
@@ -1202,14 +1183,8 @@ extern "C" mv_status mv_track_sequence_landmarks_host(mv_ctx* c, const mv_track_
   MV_ENTER(c);
   if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_desc_scale || !h_depth || !h_results)
     MV_BAD_ARG(c, "mv_track_sequence_landmarks_host");
-  if (!seq_params_ok(p))
-    MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: rows, cols, top_n, max_valid and max_matches must be positive");
-  if (c->bow_n_base <= 0)
-    MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: no vocabulary (mv_bow_set_vocabulary first)");
-  if (n_words <= 0) MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: n_words must be positive");
-  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: NULL landmark table");
-  const HostLandmarks lm = {first_frame, n_words, d_table, h_desc_scale, h_n_with_landmark};
-  return track_sequence_host_impl(c, p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
+  const SeqLandmarks lm = {first_frame, n_words, d_table, h_desc_scale, h_n_with_landmark};
+  return track_sequence_host_impl(c, "mv_track_sequence_landmarks_host", p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
                                   d2h_bytes, &lm);
 }
 

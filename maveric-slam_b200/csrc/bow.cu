@@ -526,6 +526,14 @@ extern "C" mv_status mv_bow_assign_batch(mv_ctx* ctx, int n_frames, int cells, i
                             MvBackProject());
 }
 
+// dynamic shared memory of the word-assignment kernel: the whole vocabulary
+static size_t bow_smem(int n_base, int wpb) {
+  const size_t n_leaf = (size_t)n_base * wpb * 4 + 4;
+  return sizeof(int32_t) * ((n_leaf + 3) & ~(size_t)3) + (size_t)n_base * 256 + sizeof(float) * 2 * n_base;
+}
+
+bool mv_bow_vocab_fits(const mv_ctx* ctx) { return bow_smem(ctx->bow_n_base, ctx->bow_wpb) <= 227 * 1024; }
+
 mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, const int8_t* d_desc,
                              const float* d_desc_scale, const int32_t* d_q_patch, const int32_t* d_q_count,
                              int32_t* d_word, int32_t* d_base, const MvBackProject& bp) {
@@ -533,6 +541,7 @@ mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, co
     MV_BAD_ARG(ctx, "mv_bow_assign_batch");
   if (ctx->bow_n_base <= 0) MV_BAD_ARG(ctx, "mv_bow_assign_batch: no vocabulary (mv_bow_set_vocabulary first)");
   if (reinterpret_cast<uintptr_t>(d_desc) & 15) MV_BAD_ARG(ctx, "mv_bow_assign_batch: d_desc must be 16-byte aligned");
+  if (!mv_bow_vocab_fits(ctx)) MV_BAD_ARG(ctx, "mv_bow_assign_batch: vocabulary larger than an SM's shared memory");
   BowVocabDev v;
   v.n_base = ctx->bow_n_base; v.wpb = ctx->bow_wpb;
   void *dl, *db, *ds;
@@ -543,8 +552,7 @@ mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, co
   if ((st = mv_scratch(ctx, "bow.scale_bias", sizeof(float) * 2 * v.n_base, &ds))) return st;
   v.leaves = (const int32_t*)dl; v.base_t = (const int8_t*)db;
   v.scale = (const float*)ds; v.bias = (const float*)ds + v.n_base;
-  const size_t smem = sizeof(int32_t) * ((n_leaf + 3) & ~(size_t)3) + (size_t)v.n_base * 256 + sizeof(float) * 2 * v.n_base;
-  if (smem > 227 * 1024) MV_BAD_ARG(ctx, "mv_bow_assign_batch: vocabulary larger than an SM's shared memory");
+  const size_t smem = bow_smem(v.n_base, v.wpb);
   if (smem > ctx->bow_smem_attr) {   // a function attribute of the context's device: set once per size
     MV_CUDA(ctx, cudaFuncSetAttribute(bow_assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ctx->bow_smem_attr = smem;

@@ -246,7 +246,6 @@ extern "C" void mv_match_params_default(mv_match_params* p, int rows, int cols) 
 }
 
 int mv_match_tc_parts();
-bool mv_match_tc_feasible(const mv_match_params* p, int n_frames, int n_pairs, int top_n);
 mv_status mv_match_tc_launch(mv_ctx* ctx, const mv_match_params* p, int n_frames, int n_pairs, int top_n,
                              const int32_t* d_f0, const int32_t* d_f1, const int8_t* d_desc,
                              const int32_t* d_max_idx, const float* d_prob, const int32_t* d_q_patch,

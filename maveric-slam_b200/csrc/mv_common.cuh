@@ -127,6 +127,15 @@ struct mv_device_guard {
 mv_status mv_scratch(mv_ctx* ctx, const char* name, size_t bytes, void** out);
 mv_status mv_pinned(mv_ctx* ctx, size_t bytes, void** out);
 
+// Parameter rules of the batched calls, shared with the sequence calls (api.cu), which check them before they
+// enqueue anything.
+// mv_pnp_gn_batch's parameters for correspondence lists of `stride` entries (pnp_gn.cu)
+bool mv_pnp_params_ok(const mv_pnp_params* p, int stride);
+// the tensor-core matcher runs this shape; use_tensor_cores = 1 is MV_ERR_BAD_ARG where it does not (match_tc.cu)
+bool mv_match_tc_feasible(const mv_match_params* p, int n_frames, int n_pairs, int top_n);
+// the context's vocabulary fits the word-assignment kernel's shared memory (bow.cu)
+bool mv_bow_vocab_fits(const mv_ctx* ctx);
+
 // ---- landmark sequence path (bow.cu), called by mv_track_sequence_landmarks (api.cu)
 // Back-projection of every query keypoint with its frame's depth, fused into the word assignment launch:
 // coords [n_frames][top_n][3] (zeros beyond the query count); nothing is written when coords is NULL.

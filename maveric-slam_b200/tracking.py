@@ -61,6 +61,11 @@ def _p(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
 
 
+def _hp(a):
+    """Host buffer of a sequence call: a (pinned) CPU tensor or a numpy array."""
+    return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else _p(a)
+
+
 # --------------------------------------------------------------------------------------
 # single-pair, host arrays (reference names)
 # --------------------------------------------------------------------------------------
@@ -350,12 +355,9 @@ class Tracker:
         n = semi.shape[0]
         if out is None:
             out = np.zeros(n - 1, PAIR_RESULT_DTYPE)
-
-        def hp(a):
-            return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else _p(a)
         up = C.c_ulonglong(0); down = C.c_ulonglong(0)
-        self.ctx.check(self.lib.mv_track_sequence_host(self.ctx.h, C.byref(params), n, hp(semi), hp(semi_scale),
-                                                       hp(desc), hp(depth), hp(out), C.byref(up), C.byref(down)))
+        self.ctx.check(self.lib.mv_track_sequence_host(self.ctx.h, C.byref(params), n, _hp(semi), _hp(semi_scale),
+                                                       _hp(desc), _hp(depth), _hp(out), C.byref(up), C.byref(down)))
         return out, up.value, down.value
 
 
@@ -489,13 +491,10 @@ class Tracker:
             out = np.zeros(n - 1, PAIR_RESULT_DTYPE)
         if n_with_landmark is None:
             n_with_landmark = np.zeros(n - 1, np.int32)
-
-        def hp(a):
-            return C.c_void_p(a.data_ptr()) if hasattr(a, "data_ptr") else _p(a)
         up = C.c_ulonglong(0); down = C.c_ulonglong(0)
         self.ctx.check(self.lib.mv_track_sequence_landmarks_host(
-            self.ctx.h, C.byref(params), n, int(first_frame), hp(semi), hp(semi_scale), hp(desc), hp(desc_scale),
-            hp(depth), table.shape[0], self._d(table), hp(out), hp(n_with_landmark), C.byref(up), C.byref(down)))
+            self.ctx.h, C.byref(params), n, int(first_frame), _hp(semi), _hp(semi_scale), _hp(desc), _hp(desc_scale),
+            _hp(depth), table.shape[0], self._d(table), _hp(out), _hp(n_with_landmark), C.byref(up), C.byref(down)))
         return out, n_with_landmark, up.value, down.value
 
     def chain_transforms(self, transforms):

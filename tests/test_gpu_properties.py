@@ -324,7 +324,8 @@ def test_two_frame_sequence_and_single_pair_batches(tracker, tk, oracle, synth):
 
 def test_sequence_calls_reject_nonpositive_sizes(tracker, tk, synth):
     """Status codes instead of the reference's undefined behaviour: a non-positive grid, query count or
-    match capacity is MV_ERR_BAD_ARG from both sequence entry points, before anything is allocated."""
+    match capacity, a negative match radius and PnP parameters mv_pnp_gn_batch refuses are MV_ERR_BAD_ARG from
+    both sequence entry points, before anything is allocated or launched."""
     import torch
     from maveric_slam_b200 import lib
     rows, cols = 24, 80
@@ -337,20 +338,27 @@ def test_sequence_calls_reject_nonpositive_sizes(tracker, tk, synth):
     def broken(**kw):
         p = tk.track_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=32)
         for k, v in kw.items():
-            if k in ("rows", "cols", "max_matches"):
+            if k in ("rows", "cols", "max_matches", "radius"):
                 setattr(p.match, k, v)
+            elif k in ("lanes_per_hypothesis", "hypotheses", "sample_size"):
+                setattr(p.pnp, k, v)
             else:
                 setattr(p, k, v)
         return p
 
-    for kw in ({"rows": 0}, {"cols": -3}, {"top_n": 0}, {"max_valid": 0}, {"max_matches": 0}):
+    want = tracker.track_sequence(broken(), semi, scale, desc, depth).cpu().numpy().tobytes()
+    for kw in ({"rows": 0}, {"cols": -3}, {"top_n": 0}, {"max_valid": 0}, {"max_matches": 0},
+               {"lanes_per_hypothesis": 4}, {"hypotheses": 0}, {"sample_size": 0}, {"radius": -1}):
+        launches = tracker.ctx.launches
         with pytest.raises(lib.MvError, match="bad argument"):
             tracker.track_sequence(broken(**kw), semi, scale, desc, depth)
         with pytest.raises(lib.MvError, match="bad argument"):
             tracker.track_sequence_host(broken(**kw), hs, hsc, hd, hz)
-    # and the context is still usable afterwards
+        assert tracker.ctx.launches == launches, kw
+    # and the context is still usable afterwards, with the same answer
     res = tk.results_to_numpy(tracker.track_sequence(broken(), semi, scale, desc, depth))
-    assert res.shape == (1,)
+    assert res.shape == (1,) and res.tobytes() == want
+    assert tracker.track_sequence_host(broken(), hs, hsc, hd, hz)[0].tobytes() == want
 
 
 def test_contexts_of_two_gpus_from_one_thread(synth):

@@ -227,9 +227,42 @@ def test_argument_errors(tracker, lmseq):
         setattr(p.match if field in ("rows", "cols", "max_matches") else p, field, val)
         with pytest.raises(lib.MvError, match="bad argument"):
             call(p=p)
+    # refusals of the PnP and the matcher: checked before the table is stepped, nothing launched
+    for part, field, val in (("pnp", "lanes_per_hypothesis", 4), ("pnp", "hypotheses", 0), ("pnp", "sample_size", 0),
+                             ("match", "radius", -1)):
+        p = tracking.kitti_track_params(hypotheses=256)
+        setattr(getattr(p, part), field, val)
+        launches = tracker.ctx.launches
+        with pytest.raises(lib.MvError, match="bad argument"):
+            call(p=p)
+        assert tracker.ctx.launches == launches, field
+        assert _table_bytes(table) == before, field
     assert _table_bytes(table) == before
     # the context still works and continues the same table
     res, nl, table, _, _ = _host(tracker, s, first=FIRST + 3, lo=3, table=table,
                                  p=tracking.kitti_track_params(hypotheses=256, first_pair=3))
     assert res.tobytes() == s["res"][3 * 64:] and nl.tobytes() == s["nl"][3:].tobytes()
     assert _table_bytes(table) == s["table"]
+
+
+def test_oversize_vocabulary_refused_up_front(tracker, lmseq):
+    """A vocabulary mv_bow_set_vocabulary accepts but the word-assignment kernel's shared memory cannot hold (64 bases
+    of 211 words) is refused by both landmark calls before they launch anything; the depth paths on the same context
+    and thread then give their usual answer."""
+    from maveric_slam_b200 import lib, tracking
+    s, h, d = lmseq, lmseq["h"], lmseq["d"]
+    want = tracker.track_sequence(s["p"], d["semi"], d["sscale"], d["desc"], d["depth"]).cpu().numpy().tobytes()
+    fresh = tracking.Tracker(0)
+    fresh.bow_set_vocabulary(np.zeros((256, 64), np.int8), np.ones(64, np.float32), np.zeros(64, np.float32),
+                             np.zeros((64, 211, 4), np.int32))
+    table = fresh.landmarks_new(fresh.n_words)
+    before, launches = _table_bytes(table), fresh.ctx.launches
+    with pytest.raises(lib.MvError, match="shared memory"):
+        fresh.track_sequence_landmarks(s["p"], d["semi"], d["sscale"], d["desc"], d["dscale"], d["depth"], table)
+    with pytest.raises(lib.MvError, match="shared memory"):
+        fresh.track_sequence_landmarks_host(s["p"], h["semi"], h["sscale"], h["desc"], h["dscale"], h["depth"], table)
+    assert fresh.ctx.launches == launches
+    assert _table_bytes(table) == before
+    assert fresh.track_sequence(s["p"], d["semi"], d["sscale"], d["desc"], d["depth"]).cpu().numpy().tobytes() == want
+    res, _, _ = fresh.track_sequence_host(s["p"], h["semi"], h["sscale"], h["desc"], h["depth"])
+    assert res.tobytes() == want

@@ -294,3 +294,18 @@ def test_track_sequence_landmarks_argument_errors(tracker, seq):
     with pytest.raises(lib.MvError, match="n_words must be positive"):
         tracker.ctx.check(tracker.lib.mv_landmarks_sequence(tracker.ctx.h, 0, tracker._d(table), 0, 1, 1, None, None,
                                                             None, None))
+    # refusals of the PnP and the matcher: checked before the table is stepped, nothing launched
+    before = _table_bytes(table)
+    for part, field, val in (("pnp", "lanes_per_hypothesis", 4), ("pnp", "hypotheses", 0), ("pnp", "sample_size", 0),
+                             ("match", "radius", -1)):
+        bad = tracking.kitti_track_params(hypotheses=256)
+        setattr(getattr(bad, part), field, val)
+        launches = tracker.ctx.launches
+        with pytest.raises(lib.MvError, match="bad argument"):
+            tracker.track_sequence_landmarks(bad, semi, sscale, desc, dscale, depth, table, first_frame=seq["first"])
+        assert tracker.ctx.launches == launches, field
+        assert _table_bytes(table) == before, field
+    # the context still works and the table gives the stored answer
+    res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=seq["first"])
+    assert tracking.results_to_numpy(res).tobytes() == seq["res"].tobytes() and (nl.cpu().numpy() == seq["nl"]).all()
+    assert _table_bytes(table) == seq["table"]

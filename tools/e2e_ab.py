@@ -17,9 +17,8 @@ del semi, desc, depth
 torch.cuda.synchronize()
 out = np.zeros(NF - 1, tracking.PAIR_RESULT_DTYPE)
 ref = None
-for label, env in [("default", {}), ("eager", {"MV_HOST_EAGER_GATHER": "1"}), ("chunk185", {"MV_HOST_CHUNK_PAIRS": "185"}), ("chunk740", {"MV_HOST_CHUNK_PAIRS": "740"}), ("eager185", {"MV_HOST_EAGER_GATHER": "1", "MV_HOST_CHUNK_PAIRS": "185"})]:
-    for k in ("MV_HOST_EAGER_GATHER", "MV_HOST_CHUNK_PAIRS"):
-        os.environ.pop(k, None)
+for label, env in [("default", {}), ("chunk185", {"MV_HOST_CHUNK_PAIRS": "185"}), ("chunk740", {"MV_HOST_CHUNK_PAIRS": "740"})]:
+    os.environ.pop("MV_HOST_CHUNK_PAIRS", None)
     os.environ.update(env)
     for _ in range(2):
         tr.track_sequence_host(params, hs, hsc, hd, hz, out=out)
