@@ -179,8 +179,8 @@ typedef struct {
   float min_depth;          /* cheirality guard on the camera-frame z */
   float damping;            /* relative Levenberg damping added to diag(JtJ) */
   uint64_t seed;            /* counter-based sampling: splitmix64(seed, pair, h, i) */
-  int   lanes_per_hypothesis; /* threads cooperating on one hypothesis: 1 (one thread each) ..
-                               32 (one warp each), a power of two */
+  int   lanes_per_hypothesis; /* threads cooperating on one hypothesis: 1 (one thread each) or
+                               32 (one warp each) */
   int   first_pair;         /* global index of pair 0 of this call: the sampler is keyed on the
                                global pair index, so results do not depend on chunking/sharding */
 } mv_pnp_params;
@@ -197,8 +197,8 @@ void mv_pnp_params_default(mv_pnp_params* p);
  *   d_stats     float [n_pairs][4]  {inliers, cost, best_h, valid}
  *   d_hyp_pose  float [n_pairs][H][8] every hypothesis {q,t,inliers} (nullable) */
 /* lanes_per_hypothesis: 1 = one thread per hypothesis (throughput form), 32 = one warp per hypothesis
- * (latency form).  2, 4, 8, 16 are superseded A/B forms that exist only in a library built with
- * -DMV_PNP_AB (mv_pnp_has_ab_forms() == 1); the product library answers MV_ERR_BAD_ARG for them. */
+ * (latency form); any other value is MV_ERR_BAD_ARG.  mv_pnp_has_ab_forms() always returns 0: the
+ * library has no other kernel forms, and the symbol is kept so that existing callers still link. */
 int mv_pnp_has_ab_forms(void);
 mv_status mv_pnp_gn_batch(mv_ctx* ctx, const mv_pnp_params* p, int n_pairs, int stride,
                           const float* d_corr, const int32_t* d_count,

@@ -20,8 +20,6 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-fmad=false", "-Xcompiler", "-fPIC,-Wall,-Wno-unused-function",
           "-I", os.path.join(HERE, "..", "include")]
-if os.environ.get("MV_PNP_AB"):   # also compile the superseded K3 forms (A/B timing, tools/k3_ab.py)
-    COMMON.append("-DMV_PNP_AB")
 # A/B builds of a tuning constant: MV_EXTRA_NVCC="-DMV_LEAD_CTAS=2" MV_OUT=/path/variant.so python build.py
 # (objects go to a directory of their own; load the variant with MV_LIB_PATH=/path/variant.so)
 if os.environ.get("MV_EXTRA_NVCC"):

@@ -38,6 +38,13 @@ def test_library_exports_every_declared_symbol():
     assert set(lib.NEW_SYMBOLS) <= new and set(lib.LEGACY_SYMBOLS) <= legacy
 
 
+def test_pnp_has_ab_forms_is_zero():
+    # kept exported so that existing callers link; the library has no other PnP kernel forms
+    import maveric_slam_b200  # noqa: F401
+    from maveric_slam_b200 import lib
+    assert lib.load().mv_pnp_has_ab_forms() == 0
+
+
 def test_forwarding_headers_compile_as_c99(tmp_path):
     # a reference-style C caller: the reference's include names, C99, no C++
     src = tmp_path / "caller.c"

@@ -288,17 +288,9 @@ def _pnp_params(tk, H, lanes, seed=0, refine=10, sample_size=8):
 
 
 # lanes = 1: one thread per hypothesis (two-phase kernel for n <= 480, streaming kernel above); lanes = 32: one warp
-# per hypothesis.  lanes = 2 (packed-FP32 single thread), 4, 8 are A/B forms of a library built with -DMV_PNP_AB.
+# per hypothesis.
 def _pnp_lane_forms():
-    forms = [(1, 8), (1, 7), (32, 8)]
-    try:   # the superseded forms exist only in a library built with -DMV_PNP_AB
-        import maveric_slam_b200  # noqa: F401
-        from maveric_slam_b200 import lib
-        if lib.load().mv_pnp_has_ab_forms():
-            forms += [(2, 8), (2, 7), (4, 8), (8, 8)]
-    except Exception:
-        pass
-    return forms
+    return [(1, 8), (1, 7), (32, 8)]
 
 
 @pytest.mark.parametrize("lanes,sample_size", _pnp_lane_forms())

@@ -61,10 +61,8 @@ def test_pnp_forms_return_identical_bytes(tracker, synth, n, stride):
     """configs[2]: the product's two one-thread-per-hypothesis kernels -- the two-phase kernel (gate every
     slot, re-deal by exact count, packed-FFMA2 walk; pairs of up to 480 correspondences) and the streaming
     kernel (larger pairs; MV_PNP_STREAM=1 forces it for every pair) -- with 128 or 256 hypotheses per CTA:
-    same bytes for every one of 1024 hypotheses and for the selected pose.  A library built with
-    -DMV_PNP_AB adds the superseded forms (no re-deal, mask kernel, dense kernel) to the comparison."""
+    same bytes for every one of 1024 hypotheses and for the selected pose."""
     import torch
-    from maveric_slam_b200 import lib
     P, H = 3, 1024
     corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
     cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
@@ -79,14 +77,6 @@ def test_pnp_forms_return_identical_bytes(tracker, synth, n, stride):
             assert run() == want, ("two-phase", gpw)
             with _Env("MV_PNP_STREAM", "1"):
                 assert run() == want, ("streaming", gpw)
-    if lib.load().mv_pnp_has_ab_forms():
-        for form in ("nosort", "mask", "dense"):
-            with _Env("MV_PNP_FORM", form):
-                assert run() == want, form
-        # the fused kernel with the re-deal (and its barriers) left out after some or all passes
-        for mask in ("155", "00f", "000"):
-            with _Env("MV_PNP_FORM", "fused"), _Env("MV_PNP_SORTMASK", mask):
-                assert run() == want, mask
 
 
 def test_pnp_split_launch_returns_identical_bytes(tracker, synth):
@@ -112,6 +102,25 @@ def test_pnp_split_launch_returns_identical_bytes(tracker, synth):
                 assert run() == want, ("tail pairs", tail)
         with _Env("MV_PNP_ORDER", "0"):            # index order: no split
             assert run() == want, "index order"
+
+
+@pytest.mark.parametrize("lanes", [0, 2, 3, 4, 8, 16, 64])
+def test_pnp_refuses_lanes_without_a_kernel(tracker, synth, lanes):
+    """lanes_per_hypothesis is 1 (one thread per hypothesis) or 32 (one warp): any other value is
+    MV_ERR_BAD_ARG from mv_pnp_gn_batch before anything is launched."""
+    import torch
+    from maveric_slam_b200 import lib
+    P, n, stride = 2, 100, 128
+    corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
+    cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
+    pose = torch.zeros((P, 7), dtype=torch.float32, device=tracker.device)
+    stats = torch.zeros((P, 4), dtype=torch.float32, device=tracker.device)
+    launches = tracker.ctx.launches
+    st = tracker.lib.mv_pnp_gn_batch(tracker.ctx.h, C.byref(_pnp_params(64, lanes=lanes)), P, stride,
+                                     tracker._d(corr), tracker._d(cnt), None, tracker._d(pose), tracker._d(stats),
+                                     None)
+    assert st == lib.MV_ERR_BAD_ARG, (lanes, st)
+    assert tracker.ctx.launches == launches, lanes
 
 
 def test_pnp_hypothesis_does_not_depend_on_hypothesis_count(tracker, synth):

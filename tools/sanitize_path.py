@@ -27,7 +27,7 @@ scale = torch.full((nf,), float(synth.SEMI_SCALE), device=tr.device)
 if "seq" in stages:
     ref = None
     for tc in (True, False):
-        for lanes, hyp in ((1, 300), (32, 32)):     # the product's two K3 mappings (2..16 lanes: -DMV_PNP_AB builds)
+        for lanes, hyp in ((1, 300), (32, 32)):     # the two K3 mappings
             p = tracking.track_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=hyp,
                                       lanes=lanes, use_tensor_cores=tc)
             res = tr.track_sequence(p, semi, scale, desc, depth)
