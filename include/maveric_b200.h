@@ -286,6 +286,31 @@ mv_status mv_landmarks_sequence(mv_ctx* ctx, int n_words, mv_landmark* d_table, 
                                 int top_n, const int32_t* d_word, const int32_t* d_q_count,
                                 const float* d_coords_in, float* d_coords_out);
 
+/* mv_landmarks_sequence split at the point where the entry table is needed, so that a block of frames can be walked
+ * before the table it starts from exists (the table relay of tracking.track_sequence_landmarks_sharded).
+ *   speculate  walks the block's steps first_frame .. first_frame+n_steps-1 from a GUESSED entry table: the table
+ *              that the n_warm steps before it (global frames first_frame-n_warm ..) produce from an empty table.
+ *              Reads no caller table.  d_word int32 [n_warm + n_steps][top_n], d_q_count int32 [n_warm + n_steps],
+ *              d_coords_in float [n_steps][top_n][3] (warm-up frames need words only); d_coords_in must stay valid
+ *              until the resolve has run.  n_warm >= 0, n_steps >= 1, n_warm + n_steps <= 65535,
+ *              (n_warm + n_steps) * top_n < 2^31.  *out owns its device memory (stream-ordered on the context's
+ *              stream) until mv_lm_spec_release.
+ *   resolve    d_table in/out, d_coords_out float [n_steps][top_n][3]: byte for byte
+ *              mv_landmarks_sequence(first_frame, n_steps) on the same table, for every n_warm >= 0.  A word whose
+ *              true entry record has the guess's shape (word_id; if alive, num_frames and the live frames in ring
+ *              order) is patched, any other is walked again from the true record, so a wrong guess costs time and
+ *              never changes a byte.  d_n_rewalked int32 [1] (nullable): the number of words walked again.  Refused
+ *              (MV_ERR_BAD_ARG, nothing enqueued): a speculation of another context, a second resolve, a NULL table.
+ *   release    frees the speculation (after its context's stream work; resolved or not).  Call it before the context
+ *              is destroyed. */
+typedef struct mv_lm_spec mv_lm_spec;
+mv_status mv_landmarks_speculate(mv_ctx* ctx, int n_words, int first_frame, int n_warm, int n_steps, int top_n,
+                                 const int32_t* d_word, const int32_t* d_q_count, const float* d_coords_in,
+                                 mv_lm_spec** out);
+mv_status mv_landmarks_resolve(mv_ctx* ctx, mv_lm_spec* spec, mv_landmark* d_table, float* d_coords_out,
+                               int32_t* d_n_rewalked);
+void mv_lm_spec_release(mv_lm_spec* spec);
+
 /* ------------------------------------------------------------------------- */
 /* Whole path over a sequence of frames (pair p = frames p, p+1)              */
 /* ------------------------------------------------------------------------- */
@@ -380,13 +405,45 @@ mv_status mv_track_sequence_landmarks(mv_ctx* ctx, const mv_track_params* p, int
  *   - argument errors are MV_ERR_BAD_ARG before anything is enqueued (see above): the table is untouched.  After
  *     a CUDA error the streams are drained and the host buffers no longer read, but the table's state is
  *     unspecified.
- * Not sharded over GPUs: a rank's initial table would depend on every earlier frame. */
+ * Not sharded over GPUs: its pipeline steps the table chunk by chunk while it stages, so a rank could not run its
+ * table-free half before the previous rank's table arrives.  The device call shards (below). */
 mv_status mv_track_sequence_landmarks_host(mv_ctx* ctx, const mv_track_params* p, int n_frames, int first_frame,
                                            const int8_t* h_semi, const float* h_semi_scale,
                                            const int8_t* h_desc, const float* h_desc_scale, const float* h_depth,
                                            int n_words, mv_landmark* d_table,
                                            mv_pair_result* h_results, int32_t* h_n_with_landmark /* nullable */,
                                            unsigned long long* h2d_bytes, unsigned long long* d2h_bytes);
+
+/* mv_track_sequence_landmarks split at the table, so that blocks of a sequence can run on several GPUs with only
+ * the table passed from block to block (tracking.track_sequence_landmarks_sharded):
+ *   prepare     frames: n_warm warm-up frames (global first_frame-n_warm ..) then the block's n_frames frames
+ *               (pair p = block frames p, p+1; d_semi .. d_depth hold all n_warm + n_frames frames).  Enqueues the
+ *               detector, the word assignment (with the back-projection), mv_landmarks_speculate, the matcher and
+ *               RANSAC-E.  Reads no table.  Allocates everything the three calls need (stream-ordered, owned by *out).
+ *   step_table  resolves the speculation against d_table (in/out), which is stepped over the block's frames
+ *               0 .. n_frames-2 as mv_track_sequence_landmarks steps it; d_n_rewalked int32 [1] (nullable) as
+ *               mv_landmarks_resolve.  Its first launch is the first read of d_table.
+ *   solve       correspondences from the resolved coordinates, K3, records: d_results [n_frames-1],
+ *               d_n_with_landmark int32 [n_frames-1] (nullable).
+ *   release     frees the block (after its context's stream work), in any phase; before the context is destroyed.
+ * Equivalence: prepare, step_table, solve on frames [0, n) equal mv_track_sequence_landmarks on them byte for byte --
+ * records, counts and final table -- for every n_warm.  Chaining: blocks [0, k] and [k, n-1] (first_frame and
+ * pnp.first_pair advanced by k, n_warm frames before each) may be prepared in either order, on one context or on
+ * two; stepped in frame order they equal one call.  Other calls on the same context between prepare and solve do
+ * not disturb a block.
+ * Errors: prepare refuses what mv_track_sequence_landmarks refuses (bar the table, which it does not take) and
+ * n_warm < 0 or more than 65535 frames in all, before any allocation or enqueue.  step_table and solve allocate
+ * nothing and refuse, with nothing enqueued: a NULL block, a block of another context, a call out of phase (step
+ * once after prepare, solve once after step_table) and a NULL table. */
+typedef struct mv_lm_block mv_lm_block;
+mv_status mv_track_landmarks_prepare(mv_ctx* ctx, const mv_track_params* p, int n_warm, int n_frames, int first_frame,
+                                     const int8_t* d_semi, const float* d_semi_scale, const int8_t* d_desc,
+                                     const float* d_desc_scale, const float* d_depth, int n_words, mv_lm_block** out);
+mv_status mv_track_landmarks_step_table(mv_ctx* ctx, mv_lm_block* block, mv_landmark* d_table,
+                                        int32_t* d_n_rewalked);
+mv_status mv_track_landmarks_solve(mv_ctx* ctx, mv_lm_block* block, mv_pair_result* d_results,
+                                   int32_t* d_n_with_landmark);
+void mv_track_landmarks_release(mv_lm_block* block);
 
 /* ------------------------------------------------------------------------- */
 /* NMS between the detector and the matcher (src/run_nms.c)                     */

@@ -79,6 +79,7 @@ extern "C" void mv_ctx_destroy(mv_ctx* c) {
   cudaStreamSynchronize(c->gather_stream);
   for (auto& ev : c->pending) { cudaEventDestroy(ev.beg); cudaEventDestroy(ev.end); }
   for (auto& kv : c->scratch) cudaFree(kv.second.first);
+  if (c->block_pool) cudaMemPoolDestroy(c->block_pool);
   if (c->pinned) cudaFreeHost(c->pinned);
   if (c->abort_host) cudaFreeHost(c->abort_host);
   if (c->own_stream) cudaStreamDestroy(c->stream);
@@ -147,6 +148,20 @@ mv_status mv_scratch(mv_ctx* c, const char* name, size_t bytes, void** out) {
     slot.second = want;
   }
   *out = slot.first;
+  return MV_OK;
+}
+
+mv_status mv_block_alloc(mv_ctx* c, size_t bytes, void** out) {
+  if (!c->block_pool) {
+    cudaMemPoolProps props = {};
+    props.allocType = cudaMemAllocationTypePinned;
+    props.location.type = cudaMemLocationTypeDevice;
+    props.location.id = c->device;
+    MV_CUDA(c, cudaMemPoolCreate(&c->block_pool, &props));
+    uint64_t keep = ~0ull;
+    MV_CUDA(c, cudaMemPoolSetAttribute(c->block_pool, cudaMemPoolAttrReleaseThreshold, &keep));
+  }
+  MV_CUDA(c, cudaMallocFromPoolAsync(out, bytes, c->block_pool, c->stream));
   return MV_OK;
 }
 
@@ -603,7 +618,7 @@ struct SeqScratch {
 // device-resident calls, the largest chunk for the host ones); d_desc: the caller's descriptors, or NULL when they
 // are staged into scratch.
 static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                           const SeqLandmarks* lm) {
+                           const SeqLandmarks* lm, bool with_table = true) {
   auto refuse = [&](const char* why) {
     snprintf(c->err, sizeof(c->err), "bad argument: %s: %s", fn, why);
     return MV_ERR_BAD_ARG;
@@ -625,21 +640,27 @@ static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, 
   if (c->bow_n_base <= 0) return refuse("no vocabulary (mv_bow_set_vocabulary first)");
   if (!mv_bow_vocab_fits(c)) return refuse("vocabulary larger than an SM's shared memory");
   if (lm->n_words <= 0) return refuse("n_words must be positive");
-  if (!lm->table) return refuse("NULL landmark table");
+  if (with_table && !lm->table) return refuse("NULL landmark table");
   if ((long long)(n_frames - 1) * p->top_n > 0x7fffffffLL) return refuse("(n_frames - 1) * top_n must be below 2^31");
   return MV_OK;
 }
 
+// own: allocate on the compute stream into this list instead of the context's arena (a block's scratch)
 static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, const char* ns, bool landmarks,
-                             SeqScratch* o) {
+                             SeqScratch* o, std::vector<void*>* own = nullptr) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
   std::string s(ns);
   mv_status st;
   void* v;
-#define SCR(field, type, name, bytes) \
-  if ((st = mv_scratch(c, (s + name).c_str(), (bytes), &v))) return st; \
+#define SCR(field, type, name, bytes)                                        \
+  if (own) {                                                                 \
+    if ((st = mv_block_alloc(c, (bytes), &v))) return st;                   \
+    own->push_back(v);                                                       \
+  } else if ((st = mv_scratch(c, (s + name).c_str(), (bytes), &v))) {        \
+    return st;                                                               \
+  }                                                                          \
   o->field = (type*)v
   SCR(idx, int32_t, ".idx", sizeof(int32_t) * (size_t)n_frames * cells);
   SCR(prob, float, ".prob", sizeof(float) * (size_t)n_frames * cells);
@@ -677,37 +698,42 @@ static mv_status seq_detect(mv_ctx* c, const mv_track_params* p, int n_frames, c
 // Called by seq_step once the matcher ("match_end") and the correspondences ("corr_end") are enqueued.
 using SeqStageFn = std::function<mv_status(const char* stage)>;
 
-// The rest of a batch whose detector has run: with `lm`, the word assignment of frames 0..n-2 with their query
-// keypoints back-projected in the same launch and the table walked over those frames from lm->first_frame; then
-// match / RANSAC-E / correspondences / K3 / pack.  Only descriptor rows of candidate / query cells are read, and
-// depth only at matched frame-0 cells (or, with `lm`, at query cells).
-static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                          const float* d_depth, const SeqScratch& w, mv_pair_result* d_results, int first_pair,
-                          const SeqLandmarks* lm, const SeqStageFn& on_stage = nullptr) {
+// The rest of a batch whose detector has run, in three parts that the landmark block calls apart (prepare: words,
+// speculation, matcher; step_table: the table; solve).  With `lm`, the word assignment of frames 0..n-2 with their
+// query keypoints back-projected in the same launch.
+static mv_status seq_words(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+                           const float* d_depth, const SeqScratch& w, const SeqLandmarks* lm) {
+  MvBackProject bp;
+  bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
+  bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
+  bp.coords = w.coords_in;
+  return mv_bow_assign_impl(c, n_frames - 1, p->match.rows * p->match.cols, p->top_n, d_desc, lm->desc_scale, w.qp,
+                            w.qc, w.word, nullptr, bp);
+}
+
+// Match and RANSAC-E.
+static mv_status seq_match(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+                           const SeqScratch& w, const SeqStageFn& on_stage) {
+  const int n_pairs = n_frames - 1;
+  mv_status st;
+  if ((st = mv_match_batch(c, &p->match, n_frames, n_pairs, p->top_n, nullptr, nullptr, d_desc, w.idx, w.prob, w.qp,
+                           w.qi, w.qc, w.mp, w.mc, w.mcell, nullptr, nullptr)))
+    return st;
+  if (on_stage && (st = on_stage("match_end"))) return st;
+  if (p->ransac_iterations > 0)
+    return mv_ransac_identity_batch(c, n_pairs, p->match.max_matches, w.mp, w.mc, p->ransac_iterations,
+                                    p->ransac_threshold, w.rin, nullptr, nullptr);
+  return MV_OK;
+}
+
+// Correspondences (with `lm`: from w.coords_out, each query's record right after its frame's step), K3, records.
+static mv_status seq_solve(mv_ctx* c, const mv_track_params* p, int n_frames, const float* d_depth,
+                           const SeqScratch& w, mv_pair_result* d_results, int first_pair, const SeqLandmarks* lm,
+                           const SeqStageFn& on_stage) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
   mv_status st;
-  if (lm) {
-    MvBackProject bp;
-    bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
-    bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
-    bp.coords = w.coords_in;
-    if ((st = mv_bow_assign_impl(c, n_pairs, cells, N, d_desc, lm->desc_scale, w.qp, w.qc, w.word, nullptr, bp)))
-      return st;
-    if ((st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_pairs, N, w.word, w.qc,
-                                         w.coords_in, w.coords_out)))
-      return st;
-  }
-  if ((st = mv_match_batch(c, &p->match, n_frames, n_pairs, N, nullptr, nullptr, d_desc, w.idx, w.prob, w.qp, w.qi,
-                           w.qc, w.mp, w.mc, w.mcell, nullptr, nullptr)))
-    return st;
-  if (on_stage && (st = on_stage("match_end"))) return st;
-  if (p->ransac_iterations > 0) {
-    if ((st = mv_ransac_identity_batch(c, n_pairs, M, w.mp, w.mc, p->ransac_iterations, p->ransac_threshold,
-                                       w.rin, nullptr, nullptr)))
-      return st;
-  }
   if (lm) {
     if ((st = mv_build_corr_landmarks_seq(c, n_pairs, N, M, lm->n_words, w.qp, w.qc, w.word, w.coords_out, w.mp,
                                           w.mc, w.mcell, w.corr, lm->n_with_landmark)))
@@ -724,6 +750,23 @@ static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, con
       n_pairs, w.pose, w.stats, w.mc, p->ransac_iterations > 0 ? w.rin : nullptr, w.ov, d_results);
   MV_CHECK_LAUNCH(c);
   return MV_OK;
+}
+
+// The whole rest of a batch: with `lm` the words, then the table walked over frames 0..n-2 from lm->first_frame;
+// then match / RANSAC-E / correspondences / K3 / pack.  Only descriptor rows of candidate / query cells are read,
+// and depth only at matched frame-0 cells (or, with `lm`, at query cells).
+static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+                          const float* d_depth, const SeqScratch& w, mv_pair_result* d_results, int first_pair,
+                          const SeqLandmarks* lm, const SeqStageFn& on_stage = nullptr) {
+  mv_status st;
+  if (lm) {
+    if ((st = seq_words(c, p, n_frames, d_desc, d_depth, w, lm))) return st;
+    if ((st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_frames - 1, p->top_n, w.word,
+                                         w.qc, w.coords_in, w.coords_out)))
+      return st;
+  }
+  if ((st = seq_match(c, p, n_frames, d_desc, w, on_stage))) return st;
+  return seq_solve(c, p, n_frames, d_depth, w, d_results, first_pair, lm, on_stage);
 }
 
 extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_semi,
@@ -758,6 +801,100 @@ extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_param
       (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
     return st;
   return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, 0, &lm);
+}
+
+// ---- the landmark path split at the table (mv_track_landmarks_prepare / step_table / solve)
+// A block owns a SeqScratch over its n_warm + n_frames frames and a speculation; `b` is the view of the scratch
+// that starts at the block's first frame, the scratch seq_step would have had for the block alone.
+struct mv_lm_block {
+  mv_ctx* ctx;
+  mv_track_params p;
+  int n_warm, n_frames, n_words;
+  SeqScratch w, b;
+  std::vector<void*> mem;
+  mv_lm_spec* spec = nullptr;
+  int phase = 0;   // 1 prepared, 2 table stepped, 3 solved
+};
+
+static void lm_block_free(mv_lm_block* k) {
+  mv_device_guard guard(k->ctx->device);
+  mv_lm_spec_free(k->spec);
+  for (void* v : k->mem) cudaFreeAsync(v, k->ctx->stream);
+  delete k;
+}
+
+extern "C" mv_status mv_track_landmarks_prepare(mv_ctx* c, const mv_track_params* p, int n_warm, int n_frames,
+                                                int first_frame, const int8_t* d_semi, const float* d_semi_scale,
+                                                const int8_t* d_desc, const float* d_desc_scale, const float* d_depth,
+                                                int n_words, mv_lm_block** out) {
+  MV_ENTER(c);
+  if (!out) MV_BAD_ARG(c, "mv_track_landmarks_prepare: NULL out");
+  *out = nullptr;
+  if (!p || n_frames < 2 || n_warm < 0 || !d_semi || !d_semi_scale || !d_desc || !d_desc_scale || !d_depth)
+    MV_BAD_ARG(c, "mv_track_landmarks_prepare");
+  if ((long long)n_warm + n_frames > 65535) MV_BAD_ARG(c, "mv_track_landmarks_prepare: at most 65535 frames in all");
+  const int T = n_warm + n_frames;
+  const SeqLandmarks lm = {first_frame - n_warm, n_words, nullptr, d_desc_scale, nullptr};
+  mv_status st;
+  if ((st = seq_check(c, "mv_track_landmarks_prepare", p, T, d_desc, &lm, false))) return st;
+  if (p->match.use_tensor_cores == 1 && !mv_match_tc_feasible(&p->match, n_frames, n_frames - 1, p->top_n))
+    MV_BAD_ARG(c, "mv_track_landmarks_prepare: use_tensor_cores = 1 on a shape the tensor-core matcher does not take");
+  const int cells = p->match.rows * p->match.cols, N = p->top_n;
+  mv_lm_block* k = new mv_lm_block();
+  k->ctx = c; k->p = *p; k->n_warm = n_warm; k->n_frames = n_frames; k->n_words = n_words;
+  auto fail = [&](mv_status e) { lm_block_free(k); return e; };
+  if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem)) || (st = seq_detect(c, p, T, d_semi, d_semi_scale, k->w)) ||
+      (st = seq_words(c, p, T, d_desc, d_depth, k->w, &lm)))
+    return fail(st);
+  if ((st = mv_landmarks_speculate_impl(c, n_words, first_frame, n_warm, n_frames - 1, N, k->w.word, k->w.qc,
+                                        k->w.coords_in + 3 * (size_t)n_warm * N, &k->spec)))
+    return fail(st);
+  SeqScratch& b = k->b;
+  b = k->w;
+  b.idx += (size_t)n_warm * cells; b.prob += (size_t)n_warm * cells;
+  b.qp += (size_t)n_warm * N; b.qi += (size_t)n_warm * N; b.qpr += (size_t)n_warm * N;
+  b.qc += n_warm; b.ov += n_warm;
+  b.word += (size_t)n_warm * N; b.coords_in += 3 * (size_t)n_warm * N;
+  b.coords_out = mv_lm_spec_coords(k->spec);
+  if ((st = seq_match(c, p, n_frames, d_desc + (size_t)n_warm * cells * 256, b, nullptr))) return fail(st);
+  k->phase = 1;
+  *out = k;
+  return MV_OK;
+}
+
+static mv_status lm_block_check(mv_ctx* c, mv_lm_block* k, int phase, const char* fn) {
+  if (!k) { snprintf(c->err, sizeof(c->err), "bad argument: %s: NULL block", fn); return MV_ERR_BAD_ARG; }
+  if (k->ctx != c) { snprintf(c->err, sizeof(c->err), "bad argument: %s: block of another context", fn); return MV_ERR_BAD_ARG; }
+  if (k->phase != phase) {
+    snprintf(c->err, sizeof(c->err), "bad argument: %s: out of phase (prepare, step_table, solve, each once)", fn);
+    return MV_ERR_BAD_ARG;
+  }
+  return MV_OK;
+}
+
+extern "C" mv_status mv_track_landmarks_step_table(mv_ctx* c, mv_lm_block* k, mv_landmark* d_table,
+                                                   int32_t* d_n_rewalked) {
+  MV_ENTER(c);
+  mv_status st;
+  if ((st = lm_block_check(c, k, 1, "mv_track_landmarks_step_table"))) return st;
+  if (!d_table) MV_BAD_ARG(c, "mv_track_landmarks_step_table: NULL landmark table");
+  k->phase = 2;
+  return mv_landmarks_resolve_impl(c, k->spec, d_table, k->b.coords_out, d_n_rewalked);
+}
+
+extern "C" mv_status mv_track_landmarks_solve(mv_ctx* c, mv_lm_block* k, mv_pair_result* d_results,
+                                              int32_t* d_n_with_landmark) {
+  MV_ENTER(c);
+  mv_status st;
+  if ((st = lm_block_check(c, k, 2, "mv_track_landmarks_solve"))) return st;
+  if (!d_results) MV_BAD_ARG(c, "mv_track_landmarks_solve: NULL results");
+  k->phase = 3;
+  const SeqLandmarks lm = {0, k->n_words, nullptr, nullptr, d_n_with_landmark};
+  return seq_solve(c, &k->p, k->n_frames, nullptr, k->b, d_results, 0, &lm, nullptr);
+}
+
+extern "C" void mv_track_landmarks_release(mv_lm_block* k) {
+  if (k) lm_block_free(k);
 }
 
 // ---- selective staging of descriptors from pinned host memory ------------------------

@@ -337,22 +337,83 @@ __device__ __forceinline__ void landmark_age(mv_landmark& r, int first_frame, in
   }
 }
 
+// Speculation (mv_landmarks_speculate / mv_landmarks_resolve, DESIGN.md 4.6): what the speculative walk records of
+// one word, for the resolve step to turn the walk from the guessed entry record G into the walk from the true one.
+struct LmSpecWord {
+  mv_landmark guess;        // G: the record after the warm-up steps, the walk's entry record for the block
+  mv_landmark fin;          // the record after the block's last step
+  int32_t snap[8];          // frames[] at the first in-block delete or insert (the end of the block if none)
+  int32_t blk_beg;          // index in the word's sorted list of its first block occurrence
+  int32_t ins_idx;          // ... of its first in-block insert (the list's end if none)
+  uint32_t bits;            // slots written before the snapshot | after it << 8 | kSpecReset | kSpecInserted
+  int32_t pad;
+};
+constexpr uint32_t kSpecReset = 1u << 16, kSpecInserted = 1u << 17;
+enum { kWalkPlain = 0, kWalkSpec = 1, kWalkRewalk = 2 };
+
+// ring slots `n` consecutive from `s` (mod 8) as a bit mask
+__device__ __forceinline__ unsigned ring_slots(int s, int n) {
+  const unsigned m = n >= 8 ? 0xffu : (1u << n) - 1u;
+  return ((m << (s & 7)) | (m >> (8 - (s & 7)))) & 0xffu;
+}
+
+// the slots landmark_observe(f, w, frame, k, ...) writes, for a record of a valid shape (frame_ptr in [0, 8),
+// num_frames in [0, 8])
+__device__ __forceinline__ unsigned observe_slots(const mv_landmark& f, int k) {
+  int fp = f.frame_ptr, nf = f.num_frames;
+  unsigned m = 0;
+  if (f.word_id == -1) { m = 1u; fp = 0; nf = 1; k--; }
+  const int a = min(k, 8 - nf);
+  if (a > 0) { m |= ring_slots(fp + nf, a); k -= a; }
+  if (k > 0) m |= ring_slots(fp, k);
+  return m;
+}
+
 // One warp per word, every word (records age while unseen): its list in frame order, one observe per frame, the
 // ageing between its frames applied lazily; coords_out of each occurrence = the record's coordinates after that
 // frame's step (what mv_landmarks_lookup would return then).  Lists are very uneven (on the bench sequence one
 // word holds 95 k of 4.5 M occurrences), so the lanes read and write occurrences 32 at a time and only the
 // per-frame state machine is serial: every lane holds the same record and applies the same steps.
+// M = kWalkPlain is mv_landmarks_sequence's walk.  The speculation's two forms run over a list whose first n_warm
+// frames are warm-up: kWalkSpec starts from an empty record, takes the record at step n_warm as the guess and
+// records what LmSpecWord holds from there on (no coordinates exist for warm-up frames: their inserts take 0,0,0,
+// which only G and warm-up occurrences see); kWalkRewalk walks the block part of the list from `r`, the true entry
+// record, and writes coords_out at block-relative indices.
 constexpr int kWalkWarps = 4;
-__global__ void __launch_bounds__(32 * kWalkWarps)
-lmseq_walk_kernel(int n_words, mv_landmark* __restrict__ table, int first_frame, int n_steps, int top_n,
-                  const int32_t* __restrict__ start, const int32_t* __restrict__ sorted,
-                  const float* __restrict__ coords_in, float* __restrict__ coords_out) {
-  const int w = blockIdx.x * kWalkWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (w >= n_words) return;   // warp-uniform
-  mv_landmark r = table[w];
-  int aged = 0;     // steps before `aged` are applied, except the remove_old of the last observed frame
+template <int M>
+__device__ __forceinline__ void lmseq_walk(int w, int lane, mv_landmark& r, int first_frame, int n_steps, int top_n,
+                                           int beg, int end, int aged, const int32_t* __restrict__ sorted,
+                                           const float* __restrict__ coords_in, float* __restrict__ coords_out,
+                                           int n_warm, LmSpecWord* __restrict__ sw) {
   int cur_f = -1;   // frame of the last observed occurrence
-  const int beg = start[w], end = start[w + 1];
+  // kWalkSpec: the guess is taken, the slots written since then / the snapshot, reset / insert seen
+  bool crossed = M != kWalkSpec, reset = false, inserted = false;
+  unsigned wmask = 0, wbefore = 0;
+  int snap[8];
+  mv_landmark guess;
+  int blk_beg = end, ins_idx = end;
+  auto cross = [&](int at) {   // the record after step n_warm - 1 is G
+    landmark_age(r, first_frame, aged, n_warm);
+    aged = n_warm;
+    guess = r;
+    blk_beg = at;
+    crossed = true;
+  };
+  auto take_snapshot = [&]() {
+    for (int i = 0; i < 8; i++) snap[i] = r.frames[i];
+    wbefore = wmask;
+    wmask = 0;
+    reset = true;
+  };
+  auto age = [&](int to) {
+    if (M == kWalkSpec && crossed) {
+      const bool alive = r.word_id != -1;
+      landmark_age(r, first_frame, aged, to);
+      if (alive && r.word_id == -1 && !reset) take_snapshot();   // a delete: positions are absolute from here
+    } else {
+      landmark_age(r, first_frame, aged, to);
+    }
+  };
   for (int b = beg; b < end; b += 32) {
     const int i = b + lane;
     const bool in = i < end;
@@ -371,7 +432,8 @@ lmseq_walk_kernel(int n_words, mv_landmark* __restrict__ table, int first_frame,
       const unsigned mask = live & (e == 32 ? 0xffffffffu : (1u << e) - 1) & ~((1u << s) - 1);
       const int fs = __shfl_sync(0xffffffffu, f, s);
       if ((fresh >> s) & 1) {
-        landmark_age(r, first_frame, aged, fs);
+        if (M == kWalkSpec && !crossed && fs >= n_warm) cross(b + s);
+        age(fs);
         aged = cur_f = fs;   // this frame's remove_old comes with the next ageing: it never deletes a record just observed
       }
       const float* ins = nullptr;
@@ -385,7 +447,15 @@ lmseq_walk_kernel(int n_words, mv_landmark* __restrict__ table, int first_frame,
           if (__ballot_sync(0xffffffffu, !same)) break;   // frames are non-decreasing: the run ends here
         }
         for (int o = 16; o > 0; o >>= 1) gm = min(gm, __shfl_xor_sync(0xffffffffu, gm, o));
-        ins = coords_in + 3 * (size_t)gm;
+        if (M == kWalkPlain) ins = coords_in + 3 * (size_t)gm;
+        else if (fs >= n_warm) ins = coords_in + 3 * ((size_t)gm - (size_t)n_warm * top_n);
+      }
+      if (M == kWalkSpec && crossed) {
+        if (r.word_id == -1) {
+          if (!reset) take_snapshot();
+          if (!inserted) { inserted = true; ins_idx = b + s; }
+        }
+        wmask |= observe_slots(r, __popc(mask));
       }
       landmark_observe(r, w, first_frame + fs, __popc(mask), ins);
       if ((mask >> lane) & 1) {
@@ -393,9 +463,115 @@ lmseq_walk_kernel(int n_words, mv_landmark* __restrict__ table, int first_frame,
         X = ok ? r.coords[0] : 0.0f; Y = ok ? r.coords[1] : 0.0f; Z = ok ? r.coords[2] : 0.0f;
       }
     }
-    if (in) { coords_out[3 * (size_t)g] = X; coords_out[3 * (size_t)g + 1] = Y; coords_out[3 * (size_t)g + 2] = Z; }
+    if (in) {
+      const size_t o = M == kWalkRewalk ? (size_t)g - (size_t)n_warm * top_n : (size_t)g;
+      coords_out[3 * o] = X; coords_out[3 * o + 1] = Y; coords_out[3 * o + 2] = Z;
+    }
   }
-  landmark_age(r, first_frame, aged, n_steps);
+  if (M == kWalkSpec) {
+    if (!crossed) cross(end);
+    age(n_steps);
+    if (!reset) { for (int i = 0; i < 8; i++) snap[i] = r.frames[i]; wbefore = wmask; wmask = 0; }
+    if (lane == 0) {
+      LmSpecWord o;
+      o.guess = guess; o.fin = r;
+      for (int i = 0; i < 8; i++) o.snap[i] = snap[i];
+      o.blk_beg = blk_beg; o.ins_idx = ins_idx;
+      o.bits = wbefore | (wmask << 8) | (reset ? kSpecReset : 0u) | (inserted ? kSpecInserted : 0u);
+      o.pad = 0;
+      sw[w] = o;
+    }
+  } else {
+    landmark_age(r, first_frame, aged, n_steps);
+  }
+}
+
+__global__ void __launch_bounds__(32 * kWalkWarps)
+lmseq_walk_kernel(int n_words, mv_landmark* __restrict__ table, int first_frame, int n_steps, int top_n,
+                  const int32_t* __restrict__ start, const int32_t* __restrict__ sorted,
+                  const float* __restrict__ coords_in, float* __restrict__ coords_out) {
+  const int w = blockIdx.x * kWalkWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (w >= n_words) return;   // warp-uniform
+  mv_landmark r = table[w];
+  lmseq_walk<kWalkPlain>(w, lane, r, first_frame, n_steps, top_n, start[w], start[w + 1], 0, sorted, coords_in,
+                         coords_out, 0, nullptr);
+  if (lane == 0) table[w] = r;
+}
+
+// The speculative walk: warm-up and block of every word from an empty record, reading no table.  first_frame and
+// n_steps count from the first warm-up frame.
+__global__ void __launch_bounds__(32 * kWalkWarps)
+lmspec_walk_kernel(int n_words, int first_frame, int n_warm, int n_steps, int top_n, const int32_t* __restrict__ start,
+                   const int32_t* __restrict__ sorted, const float* __restrict__ coords_in,
+                   float* __restrict__ coords_out, LmSpecWord* __restrict__ sw) {
+  const int w = blockIdx.x * kWalkWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (w >= n_words) return;   // warp-uniform
+  mv_landmark r;
+  r.word_id = -1; r.frame_ptr = 0; r.num_frames = 0;
+  for (int i = 0; i < 8; i++) r.frames[i] = 0;
+  r.coords[0] = r.coords[1] = r.coords[2] = 0.0f;
+  lmseq_walk<kWalkSpec>(w, lane, r, first_frame, n_steps, top_n, start[w], start[w + 1], 0, sorted, coords_in,
+                        coords_out, n_warm, sw);
+}
+
+// Resolve, first half: one warp per word.  A word whose true entry record E has G's shape (word_id; if alive,
+// num_frames and the live frames in ring order) gets the speculative result corrected; any other word is queued
+// for the re-walk.  coords_out is block-relative.
+__global__ void __launch_bounds__(32 * kWalkWarps)
+lmspec_patch_kernel(int n_words, mv_landmark* __restrict__ table, int n_warm, int top_n,
+                    const int32_t* __restrict__ sorted, const LmSpecWord* __restrict__ sw,
+                    float* __restrict__ coords_out, int32_t* __restrict__ rewalk, int32_t* __restrict__ n_rewalk) {
+  const int w = blockIdx.x * kWalkWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (w >= n_words) return;   // warp-uniform
+  const mv_landmark E = table[w];
+  const LmSpecWord& s = sw[w];
+  const mv_landmark& G = s.guess;
+  bool same = E.word_id == G.word_id;
+  if (same && G.word_id != -1) {
+    same = E.num_frames == G.num_frames && E.frame_ptr >= 0 && E.frame_ptr < 8;
+    for (int i = 0; same && i < G.num_frames; i++)
+      same = E.frames[(E.frame_ptr + i) & 7] == G.frames[(G.frame_ptr + i) & 7];
+  }
+  if (!same) {
+    if (lane == 0) rewalk[atomicAdd(n_rewalk, 1)] = w;
+    return;
+  }
+  const bool reset = s.bits & kSpecReset, inserted = s.bits & kSpecInserted;
+  if (!reset && E.word_id == -1) return;   // no occurrence and nothing ages an empty record: E stays
+  if (lane == 0) {
+    const unsigned wb = s.bits & 0xffu, wa = (s.bits >> 8) & 0xffu;
+    const int d = E.word_id != -1 ? E.frame_ptr - G.frame_ptr : 0;   // G's slot q is E's slot q + d
+    mv_landmark R;
+    R.word_id = s.fin.word_id;
+    R.num_frames = s.fin.num_frames;
+    R.frame_ptr = reset ? s.fin.frame_ptr : (s.fin.frame_ptr + d) & 7;
+    for (int p = 0; p < 8; p++) {
+      const int q = (p - d) & 7;
+      R.frames[p] = (wa >> p) & 1 ? s.fin.frames[p] : (wb >> q) & 1 ? s.snap[q] : E.frames[p];
+    }
+    for (int c = 0; c < 3; c++) R.coords[c] = inserted ? s.fin.coords[c] : E.coords[c];
+    table[w] = R;
+  }
+  // before the first insert the record is E's, alive with word_id w: lookup gives E's coordinates
+  for (int i = s.blk_beg + lane; i < s.ins_idx; i += 32) {
+    const size_t o = (size_t)sorted[i] - (size_t)n_warm * top_n;
+    coords_out[3 * o] = E.coords[0]; coords_out[3 * o + 1] = E.coords[1]; coords_out[3 * o + 2] = E.coords[2];
+  }
+}
+
+// Resolve, second half: the queued words walked again over their block occurrences from the true entry record.
+__global__ void __launch_bounds__(32 * kWalkWarps)
+lmspec_rewalk_kernel(mv_landmark* __restrict__ table, int first_frame, int n_warm, int n_steps, int top_n,
+                     const int32_t* __restrict__ start, const int32_t* __restrict__ sorted,
+                     const float* __restrict__ coords_in, float* __restrict__ coords_out,
+                     const LmSpecWord* __restrict__ sw, const int32_t* __restrict__ rewalk,
+                     const int32_t* __restrict__ n_rewalk) {
+  const int k = blockIdx.x * kWalkWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (k >= *n_rewalk) return;   // warp-uniform
+  const int w = rewalk[k];
+  mv_landmark r = table[w];
+  lmseq_walk<kWalkRewalk>(w, lane, r, first_frame, n_steps, top_n, sw[w].blk_beg, start[w + 1], n_warm, sorted,
+                          coords_in, coords_out, n_warm, nullptr);
   if (lane == 0) table[w] = r;
 }
 
@@ -695,3 +871,124 @@ extern "C" mv_status mv_landmarks_sequence(mv_ctx* ctx, int n_words, mv_landmark
   return mv_landmarks_sequence_impl(ctx, n_words, d_table, first_frame, n_steps, top_n, d_word, d_q_count, d_coords_in,
                                     d_coords_out);
 }
+
+// ---------------------------------------------------------------- speculation: the table step split at the table
+struct mv_lm_spec {
+  mv_ctx* ctx;
+  int n_words, first_frame, n_warm, n_steps, top_n;   // first_frame: the block's; n_steps: the block's
+  void* mem;                                           // one allocation of the block pool, freed by mv_lm_spec_release
+  int32_t *start, *sorted, *rewalk, *n_rewalk;
+  float* coords;                                       // [n_warm + n_steps][top_n][3]: the walk's coords_out
+  LmSpecWord* sw;
+  const float* coords_in;                              // the caller's, block frames only: the re-walk reads it too
+  bool resolved;
+};
+
+float* mv_lm_spec_coords(mv_lm_spec* s) { return s->coords + 3 * (size_t)s->n_warm * s->top_n; }
+
+mv_status mv_landmarks_speculate_impl(mv_ctx* ctx, int n_words, int first_frame, int n_warm, int n_steps, int top_n,
+                                      const int32_t* d_word, const int32_t* d_q_count, const float* d_coords_in,
+                                      mv_lm_spec** out) {
+  const int T = n_warm + n_steps;   // steps of the sorted lists: warm-up, then block
+  int n_tiles, fb;
+  lmseq_tiles(n_words, T, &n_tiles, &fb);
+  const size_t occ = (size_t)T * top_n;
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t b_cnt = up(sizeof(int32_t) * (size_t)n_tiles * n_words), b_tot = up(sizeof(int32_t) * n_words),
+               b_start = up(sizeof(int32_t) * ((size_t)n_words + 1)), b_sorted = up(sizeof(int32_t) * occ),
+               b_coords = up(sizeof(float) * 3 * occ), b_sw = up(sizeof(LmSpecWord) * n_words),
+               b_list = up(sizeof(int32_t) * ((size_t)n_words + 1));
+  char* m = nullptr;
+  mv_status st;
+  if ((st = mv_block_alloc(ctx, b_cnt + b_tot + b_start + b_sorted + b_coords + b_sw + b_list, (void**)&m))) return st;
+  mv_lm_spec* s = new mv_lm_spec();
+  s->ctx = ctx; s->n_words = n_words; s->first_frame = first_frame; s->n_warm = n_warm; s->n_steps = n_steps;
+  s->top_n = top_n; s->mem = m; s->coords_in = d_coords_in; s->resolved = false;
+  int32_t* cnt = (int32_t*)m;
+  int32_t* tot = (int32_t*)(m + b_cnt);
+  s->start = (int32_t*)(m + b_cnt + b_tot);
+  s->sorted = (int32_t*)(m + b_cnt + b_tot + b_start);
+  s->coords = (float*)(m + b_cnt + b_tot + b_start + b_sorted);
+  s->sw = (LmSpecWord*)(m + b_cnt + b_tot + b_start + b_sorted + b_coords);
+  s->n_rewalk = (int32_t*)(m + b_cnt + b_tot + b_start + b_sorted + b_coords + b_sw);
+  s->rewalk = s->n_rewalk + 1;
+  *out = s;
+  {
+    mv_prof_scope ps(ctx, "spec_sort");
+    MV_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)n_tiles * n_words, ctx->stream));
+    const long long blocks = ((long long)occ + 255) / 256;
+    lmseq_count_kernel<<<(int)std::min<long long>(blocks, 8LL * ctx->sm_count), 256, 0, ctx->stream>>>(
+        T, top_n, n_words, fb, d_word, d_q_count, cnt, s->coords);
+    MV_CHECK_LAUNCH(ctx);
+    lmseq_colscan_kernel<<<(n_words + 127) / 128, 128, 0, ctx->stream>>>(n_words, n_tiles, cnt, tot);
+    MV_CHECK_LAUNCH(ctx);
+    lmseq_wordscan_kernel<<<1, 1024, 0, ctx->stream>>>(n_words, tot, s->start);
+    MV_CHECK_LAUNCH(ctx);
+    lmseq_scatter_kernel<<<n_tiles, 256, 0, ctx->stream>>>(T, top_n, n_words, fb, d_word, d_q_count, cnt, s->start,
+                                                          s->sorted);
+    MV_CHECK_LAUNCH(ctx);
+  }
+  mv_prof_scope ps(ctx, "spec_walk");
+  lmspec_walk_kernel<<<(n_words + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, ctx->stream>>>(
+      n_words, first_frame - n_warm, n_warm, T, top_n, s->start, s->sorted, d_coords_in, s->coords, s->sw);
+  MV_CHECK_LAUNCH(ctx);
+  return MV_OK;
+}
+
+mv_status mv_landmarks_resolve_impl(mv_ctx* ctx, mv_lm_spec* s, mv_landmark* d_table, float* d_coords_out,
+                                    int32_t* d_n_rewalked) {
+  const int n_words = s->n_words, top_n = s->top_n, n_warm = s->n_warm;
+  s->resolved = true;
+  mv_prof_scope ps(ctx, "resolve");
+  MV_CUDA(ctx, cudaMemsetAsync(s->n_rewalk, 0, sizeof(int32_t), ctx->stream));
+  if (d_coords_out != mv_lm_spec_coords(s))
+    MV_CUDA(ctx, cudaMemcpyAsync(d_coords_out, mv_lm_spec_coords(s), sizeof(float) * 3 * (size_t)s->n_steps * top_n,
+                                 cudaMemcpyDeviceToDevice, ctx->stream));
+  const int grid = (n_words + kWalkWarps - 1) / kWalkWarps;
+  lmspec_patch_kernel<<<grid, 32 * kWalkWarps, 0, ctx->stream>>>(n_words, d_table, n_warm, top_n, s->sorted, s->sw,
+                                                                 d_coords_out, s->rewalk, s->n_rewalk);
+  MV_CHECK_LAUNCH(ctx);
+  lmspec_rewalk_kernel<<<grid, 32 * kWalkWarps, 0, ctx->stream>>>(
+      d_table, s->first_frame - n_warm, n_warm, n_warm + s->n_steps, top_n, s->start, s->sorted, s->coords_in,
+      d_coords_out, s->sw, s->rewalk, s->n_rewalk);
+  MV_CHECK_LAUNCH(ctx);
+  if (d_n_rewalked)
+    MV_CUDA(ctx, cudaMemcpyAsync(d_n_rewalked, s->n_rewalk, sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+  return MV_OK;
+}
+
+void mv_lm_spec_free(mv_lm_spec* s) {
+  if (!s) return;
+  mv_device_guard guard(s->ctx->device);
+  cudaFreeAsync(s->mem, s->ctx->stream);
+  delete s;
+}
+
+extern "C" mv_status mv_landmarks_speculate(mv_ctx* ctx, int n_words, int first_frame, int n_warm, int n_steps,
+                                            int top_n, const int32_t* d_word, const int32_t* d_q_count,
+                                            const float* d_coords_in, mv_lm_spec** out) {
+  MV_ENTER(ctx);
+  if (!out) MV_BAD_ARG(ctx, "mv_landmarks_speculate: NULL out");
+  *out = nullptr;
+  if (n_words <= 0) MV_BAD_ARG(ctx, "mv_landmarks_speculate: n_words must be positive");
+  if (n_warm < 0 || n_steps < 1 || (long long)n_warm + n_steps > 65535 || top_n <= 0 ||
+      ((long long)n_warm + n_steps) * top_n > 0x7fffffffLL)
+    MV_BAD_ARG(ctx, "mv_landmarks_speculate: n_warm >= 0, n_steps >= 1, at most 65535 steps of top_n > 0 queries "
+                    "in all, fewer than 2^31 occurrences");
+  if (!d_word || !d_q_count || !d_coords_in) MV_BAD_ARG(ctx, "mv_landmarks_speculate");
+  return mv_landmarks_speculate_impl(ctx, n_words, first_frame, n_warm, n_steps, top_n, d_word, d_q_count,
+                                     d_coords_in, out);
+}
+
+extern "C" mv_status mv_landmarks_resolve(mv_ctx* ctx, mv_lm_spec* spec, mv_landmark* d_table, float* d_coords_out,
+                                          int32_t* d_n_rewalked) {
+  MV_ENTER(ctx);
+  if (!spec) MV_BAD_ARG(ctx, "mv_landmarks_resolve: NULL speculation");
+  if (spec->ctx != ctx) MV_BAD_ARG(ctx, "mv_landmarks_resolve: speculation of another context");
+  if (spec->resolved) MV_BAD_ARG(ctx, "mv_landmarks_resolve: speculation already resolved");
+  if (!d_table) MV_BAD_ARG(ctx, "mv_landmarks_resolve: NULL landmark table");
+  if (!d_coords_out) MV_BAD_ARG(ctx, "mv_landmarks_resolve: NULL coords_out");
+  return mv_landmarks_resolve_impl(ctx, spec, d_table, d_coords_out, d_n_rewalked);
+}
+
+extern "C" void mv_lm_spec_release(mv_lm_spec* spec) { mv_lm_spec_free(spec); }

@@ -44,6 +44,9 @@ struct mv_ctx {
 
   // scratch arena, grown on demand, never shrunk; owned by the context
   std::map<std::string, std::pair<void*, size_t>> scratch;
+  // stream-ordered memory of landmark speculations and blocks (mv_block_alloc): a pool of the context that keeps
+  // what they free, so a loop of prepare / release does not map and unmap device memory every time
+  cudaMemPool_t block_pool = nullptr;
   // Wait-site diagnostic of the mbarrier pipelines (tcgen05 matcher, TMA row gather): one int in mapped
   // pinned host memory, written by a kernel just before it traps on a barrier that never completed.  Host
   // memory survives the sticky error a trap leaves behind, so MV_CUDA can still name the wait site.
@@ -126,6 +129,8 @@ struct mv_device_guard {
 
 mv_status mv_scratch(mv_ctx* ctx, const char* name, size_t bytes, void** out);
 mv_status mv_pinned(mv_ctx* ctx, size_t bytes, void** out);
+// `bytes` of the context's block pool, ordered on its compute stream; freed with cudaFreeAsync
+mv_status mv_block_alloc(mv_ctx* ctx, size_t bytes, void** out);
 
 // Parameter rules of the batched calls, shared with the sequence calls (api.cu), which check them before they
 // enqueue anything.
@@ -155,6 +160,15 @@ mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_ta
 // allocates the scratch mv_landmarks_sequence_impl needs for n_steps steps (callers that must not grow scratch
 // while other streams run, i.e. the host-buffer pipeline, reserve it for their largest call up front)
 mv_status mv_landmarks_sequence_reserve(mv_ctx* ctx, int n_words, int n_steps, int top_n);
+// speculation of the table step (mv_landmarks_speculate / mv_landmarks_resolve without the argument checks); the
+// frame-level block (api.cu) resolves in place into mv_lm_spec_coords, the walk's block-relative coords_out
+mv_status mv_landmarks_speculate_impl(mv_ctx* ctx, int n_words, int first_frame, int n_warm, int n_steps, int top_n,
+                                      const int32_t* d_word, const int32_t* d_q_count, const float* d_coords_in,
+                                      mv_lm_spec** out);
+mv_status mv_landmarks_resolve_impl(mv_ctx* ctx, mv_lm_spec* s, mv_landmark* d_table, float* d_coords_out,
+                                    int32_t* d_n_rewalked);
+float* mv_lm_spec_coords(mv_lm_spec* s);
+void mv_lm_spec_free(mv_lm_spec* s);
 // mv_build_corr_landmarks_batch for pairs (p, p+1) with the 3-D side from mv_landmarks_sequence's coords_out
 mv_status mv_build_corr_landmarks_seq(mv_ctx* ctx, int n_pairs, int top_n, int stride, int n_words,
                                       const int32_t* d_q_patch, const int32_t* d_q_count, const int32_t* d_word,

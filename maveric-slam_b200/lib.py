@@ -28,7 +28,9 @@ NEW_SYMBOLS = [
     "mv_lba_solve_batch",
     "mv_bow_set_vocabulary", "mv_bow_assign_batch", "mv_landmarks_init", "mv_landmarks_observe",
     "mv_landmarks_remove_old", "mv_landmarks_lookup", "mv_build_corr_landmarks_batch", "mv_landmarks_sequence",
-    "mv_track_sequence_landmarks", "mv_track_sequence_landmarks_host",
+    "mv_track_sequence_landmarks", "mv_track_sequence_landmarks_host", "mv_landmarks_speculate",
+    "mv_landmarks_resolve", "mv_lm_spec_release", "mv_track_landmarks_prepare", "mv_track_landmarks_step_table",
+    "mv_track_landmarks_solve", "mv_track_landmarks_release",
 ]
 LEGACY_SYMBOLS = [
     "add_Vector2f", "add_Vector3f", "mult_Quaternionf", "create_Quaternionf", "Quaternionf_from_Vector3f",
@@ -142,6 +144,16 @@ def load() -> C.CDLL:
     L.mv_track_sequence_landmarks.argtypes = [vp, C.POINTER(TrackParams), i32, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     L.mv_track_sequence_landmarks_host.argtypes = [vp, C.POINTER(TrackParams), i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
                                                    vp, C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]
+    L.mv_landmarks_speculate.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, C.POINTER(vp)]
+    L.mv_landmarks_resolve.argtypes = [vp, vp, vp, vp, vp]
+    L.mv_lm_spec_release.argtypes = [vp]
+    L.mv_lm_spec_release.restype = None
+    L.mv_track_landmarks_prepare.argtypes = [vp, C.POINTER(TrackParams), i32, i32, i32, vp, vp, vp, vp, vp, i32,
+                                             C.POINTER(vp)]
+    L.mv_track_landmarks_step_table.argtypes = [vp, vp, vp, vp]
+    L.mv_track_landmarks_solve.argtypes = [vp, vp, vp, vp]
+    L.mv_track_landmarks_release.argtypes = [vp]
+    L.mv_track_landmarks_release.restype = None
     L.mv_synth_frames.argtypes = [vp, C.POINTER(SynthParams), i32, i32, vp, vp, vp, vp]
     L.mv_nms_batch.argtypes = [vp, i32, i32, i32, vp, vp]
     L.run_nms_ex.argtypes = [vp, i32, i32, vp, vp]

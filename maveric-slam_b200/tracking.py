@@ -497,6 +497,66 @@ class Tracker:
             _hp(depth), table.shape[0], self._d(table), _hp(out), _hp(n_with_landmark), C.byref(up), C.byref(down)))
         return out, n_with_landmark, up.value, down.value
 
+    def landmarks_speculate(self, n_words, first_frame, n_warm, word, q_count, coords_in):
+        """mv_landmarks_speculate: the table step of block frames first_frame .. from the table that the n_warm
+        frames before them give from an empty table.  word int32 [n_warm + n_steps, top_n], q_count int32
+        [n_warm + n_steps], coords_in float32 [n_steps, top_n, 3] (kept alive by the returned handle until release).
+        Returns a handle for :meth:`landmarks_resolve` / :meth:`landmarks_release`."""
+        n_total, top_n = word.shape
+        h = C.c_void_p()
+        self.ctx.check(self.lib.mv_landmarks_speculate(self.ctx.h, int(n_words), int(first_frame), int(n_warm),
+                                                       n_total - int(n_warm), top_n, self._d(word), self._d(q_count),
+                                                       self._d(coords_in), C.byref(h)))
+        return {"h": h, "n_steps": n_total - int(n_warm), "top_n": top_n, "keep": (word, q_count, coords_in)}
+
+    def landmarks_resolve(self, spec, table, coords_out=None, n_rewalked=None):
+        """mv_landmarks_resolve: steps `table` in place exactly as :meth:`landmarks_sequence` over the block would;
+        returns coords_out float32 [n_steps, top_n, 3]."""
+        if coords_out is None:
+            coords_out = self.torch.empty((spec["n_steps"], spec["top_n"], 3), dtype=self.torch.float32,
+                                          device=self.device)
+        self.ctx.check(self.lib.mv_landmarks_resolve(self.ctx.h, spec["h"], self._d(table), self._d(coords_out),
+                                                     self._d(n_rewalked)))
+        return coords_out
+
+    def landmarks_release(self, spec):
+        if spec["h"]:
+            self.lib.mv_lm_spec_release(spec["h"])
+            spec["h"] = C.c_void_p()
+
+    def track_landmarks_prepare(self, params: _lib.TrackParams, n_warm, first_frame, semi, semi_scale, desc,
+                                desc_scale, depth, n_words):
+        """mv_track_landmarks_prepare: everything of :meth:`track_sequence_landmarks` on a block that does not need
+        the table.  The inputs hold n_warm warm-up frames, then the block's frames (global numbers first_frame ..);
+        they must stay alive until :meth:`track_landmarks_solve`.  Returns a block handle."""
+        h = C.c_void_p()
+        n = semi.shape[0] - int(n_warm)
+        self.ctx.check(self.lib.mv_track_landmarks_prepare(
+            self.ctx.h, C.byref(params), int(n_warm), n, int(first_frame), self._d(semi), self._d(semi_scale),
+            self._d(desc), self._d(desc_scale), self._d(depth), int(n_words), C.byref(h)))
+        return {"h": h, "n_pairs": n - 1, "keep": (semi, semi_scale, desc, desc_scale, depth)}
+
+    def track_landmarks_step_table(self, block, table, n_rewalked=None):
+        """mv_track_landmarks_step_table: steps `table` in place over the block's frames."""
+        self.ctx.check(self.lib.mv_track_landmarks_step_table(self.ctx.h, block["h"], self._d(table),
+                                                              self._d(n_rewalked)))
+
+    def track_landmarks_solve(self, block, out=None, n_with_landmark=None):
+        """mv_track_landmarks_solve -> (uint8 [n_pairs, 64] results, int32 [n_pairs] matches with a landmark)."""
+        torch = self.torch
+        if out is None:
+            out = torch.empty((block["n_pairs"], 64), dtype=torch.uint8, device=self.device)
+        if n_with_landmark is None:
+            n_with_landmark = torch.empty((block["n_pairs"],), dtype=torch.int32, device=self.device)
+        self.ctx.check(self.lib.mv_track_landmarks_solve(self.ctx.h, block["h"], self._d(out),
+                                                         self._d(n_with_landmark)))
+        return out, n_with_landmark
+
+    def track_landmarks_release(self, block):
+        if block["h"]:
+            self.lib.mv_track_landmarks_release(block["h"])
+            block["h"] = C.c_void_p()
+
     def chain_transforms(self, transforms):
         """python/compute_trajectory.py:49-51,76-77 as a parallel scan: float64 [n, 3, 4] relative
         transforms -> float64 [n+1, 3, 4] frame poses, pose 0 the identity."""
@@ -654,6 +714,80 @@ class ResultGather:
             return self._recv[: self.n_pairs]
         torch.index_select(self._recv, 0, self._rows, out=self._out)   # unequal blocks: drop the padding rows
         return self._out
+
+
+def track_sequence_landmarks_sharded(tracker, params, frames, table, first_frame=0, n_warm=0, group=None,
+                                     timings=None):
+    """:meth:`Tracker.track_sequence_landmarks` over the whole sequence, its pairs sharded over the ranks of
+    `group` in the blocks of :func:`shard_pairs`, with the table relayed from rank to rank.
+
+    frames = (semi, semi_scale, desc, desc_scale, depth): the WHOLE sequence (n frames), on this rank's device;
+    each rank reads its block, its halo frame and up to n_warm frames before the block.  table: this rank's
+    landmark table, the entry table on rank 0 (it is read there only); on return every rank holds the final
+    table.  params.pnp.first_pair is the pair index of the sequence's first pair.  Each rank prepares its block
+    (reading no table), receives the table from rank r - 1, steps it, sends it to rank r + 1 and solves; the
+    records come back with one all_gather (:class:`ResultGather`), the landmark counts with another, the final
+    table with a broadcast from the last rank.  Every exchange is stream-ordered (NCCL on the current stream), so
+    nothing waits on the host.  Returns (uint8 [n - 1, 64] records, int32 [n - 1] counts, int32 re-walked words of
+    this rank's block).  `timings`: a list that receives this rank's CUDA events (prepare, table wait,
+    step_table, solve), for measurement."""
+    import copy
+    import torch
+    import torch.distributed as dist
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    semi, semi_scale, desc, desc_scale, depth = frames
+    n_pairs = semi.shape[0] - 1
+    gat = ResultGather(n_pairs, world, rank, tracker.device, group=group)
+    first, count = gat.first, gat.count
+    nl_send = torch.zeros((gat.per,), dtype=torch.int32, device=tracker.device)
+    rewalked = torch.zeros((1,), dtype=torch.int32, device=tracker.device)
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)] if timings is not None else None
+    if ev:
+        ev[0].record()
+    block = None
+    if count > 0:
+        w = min(int(n_warm), first)
+        lo, hi = first - w, first + count + 1
+        p = copy.copy(params)
+        p.pnp = copy.copy(params.pnp)
+        p.pnp.first_pair = params.pnp.first_pair + first
+        block = tracker.track_landmarks_prepare(p, w, first_frame + first, semi[lo:hi], semi_scale[lo:hi], desc[lo:hi],
+                                                desc_scale[lo:hi], depth[lo:hi], table.shape[0])
+    if ev:
+        ev[1].record()
+    src = _global_rank(group, rank - 1)
+    dst = _global_rank(group, rank + 1)
+    if rank > 0:
+        dist.recv(table, src=src, group=group)
+    if ev:
+        ev[2].record()
+    if block is not None:
+        tracker.track_landmarks_step_table(block, table, rewalked)
+    if ev:
+        ev[3].record()
+    if rank + 1 < world:
+        dist.send(table, dst=dst, group=group)
+    if block is not None:
+        tracker.track_landmarks_solve(block, out=gat.send, n_with_landmark=nl_send[:count])
+    if ev:
+        ev[4].record()
+        timings.extend(ev)
+    records = gat.gather()
+    if world > 1:
+        nl_all = torch.empty((world * gat.per,), dtype=torch.int32, device=tracker.device)
+        dist.all_gather_into_tensor(nl_all, nl_send, group=group)
+        dist.broadcast(table, src=_global_rank(group, world - 1), group=group)
+    else:
+        nl_all = nl_send
+    if block is not None:
+        tracker.track_landmarks_release(block)
+    return records, nl_all[:n_pairs], rewalked   # shard_pairs blocks start at rank * per: no padding between them
+
+
+def _global_rank(group, r):
+    import torch.distributed as dist
+    return r if group is None else dist.get_global_rank(group, r)
 
 
 # --------------------------------------------------------------------------------------
