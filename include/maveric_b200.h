@@ -405,8 +405,8 @@ mv_status mv_track_sequence_landmarks(mv_ctx* ctx, const mv_track_params* p, int
  *   - argument errors are MV_ERR_BAD_ARG before anything is enqueued (see above): the table is untouched.  After
  *     a CUDA error the streams are drained and the host buffers no longer read, but the table's state is
  *     unspecified.
- * Not sharded over GPUs: its pipeline steps the table chunk by chunk while it stages, so a rank could not run its
- * table-free half before the previous rank's table arrives.  The device call shards (below). */
+ * It steps the table chunk by chunk while it stages, so it runs on one GPU; over several, each rank stages its block
+ * with mv_track_landmarks_prepare_host (below) before the table arrives. */
 mv_status mv_track_sequence_landmarks_host(mv_ctx* ctx, const mv_track_params* p, int n_frames, int first_frame,
                                            const int8_t* h_semi, const float* h_semi_scale,
                                            const int8_t* h_desc, const float* h_desc_scale, const float* h_depth,
@@ -439,6 +439,28 @@ typedef struct mv_lm_block mv_lm_block;
 mv_status mv_track_landmarks_prepare(mv_ctx* ctx, const mv_track_params* p, int n_warm, int n_frames, int first_frame,
                                      const int8_t* d_semi, const float* d_semi_scale, const int8_t* d_desc,
                                      const float* d_desc_scale, const float* d_depth, int n_words, mv_lm_block** out);
+/* mv_track_landmarks_prepare from host (ideally pinned) buffers laid out the same way (n_warm warm-up frames, then
+ * the block's n_frames), over the staging pipeline of mv_track_sequence_landmarks_host
+ * (tracking.track_sequence_landmarks_host_sharded).  It returns the same kind of block: step_table, solve and
+ * release take it unchanged.
+ *   - equivalence: prepare_host, step_table, solve give records, counts and a final table byte for byte those of
+ *     mv_track_landmarks_prepare on the same frames (so of mv_track_sequence_landmarks and
+ *     mv_track_sequence_landmarks_host), for every n_warm, chunk size, pinned or pageable buffers and selective
+ *     staging on or off.  Blocks of either prepare chain with each other under the rule above;
+ *   - returns when the host buffers are no longer read (the staging streams are drained); the block's last device
+ *     work (the last chunk's matcher, the speculation) may still be queued on the context stream, ahead of anything
+ *     enqueued after it.  The block owns only what step_table and solve read: the detector planes stay in the
+ *     staging chunks;
+ *   - h2d_bytes (nullable, filled at return): for the block's frames exactly what mv_track_sequence_landmarks_host
+ *     moves for them; for each warm-up frame its logits, both scales and its query rows only (no depth: warm-up
+ *     words need no coordinates; no candidate rows: no matcher runs on them);
+ *   - errors: MV_ERR_BAD_ARG, before any allocation, enqueue or host read, for what mv_track_landmarks_prepare
+ *     refuses (more than 65535 frames in all included: the speculation's limit) and NULL host pointers.  After a CUDA
+ *     error the streams are drained, nothing is kept and *out is NULL. */
+mv_status mv_track_landmarks_prepare_host(mv_ctx* ctx, const mv_track_params* p, int n_warm, int n_frames,
+                                          int first_frame, const int8_t* h_semi, const float* h_semi_scale,
+                                          const int8_t* h_desc, const float* h_desc_scale, const float* h_depth,
+                                          int n_words, mv_lm_block** out, unsigned long long* h2d_bytes /* nullable */);
 mv_status mv_track_landmarks_step_table(mv_ctx* ctx, mv_lm_block* block, mv_landmark* d_table,
                                         int32_t* d_n_rewalked);
 mv_status mv_track_landmarks_solve(mv_ctx* ctx, mv_lm_block* block, mv_pair_result* d_results,

@@ -645,9 +645,11 @@ static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, 
   return MV_OK;
 }
 
-// own: allocate on the compute stream into this list instead of the context's arena (a block's scratch)
+// own: allocate on the compute stream into this list instead of the context's arena (a block's scratch).
+// planes = false leaves out the per-frame detector planes (idx, prob, qi, qpr, flags), which only the detector, the
+// row marking and the matcher read: a block prepared from host buffers keeps them in the staging chunks.
 static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, const char* ns, bool landmarks,
-                             SeqScratch* o, std::vector<void*>* own = nullptr) {
+                             SeqScratch* o, std::vector<void*>* own = nullptr, bool planes = true) {
   const int cells = p->match.rows * p->match.cols;
   const int n_pairs = n_frames - 1;
   const int N = p->top_n, M = p->match.max_matches;
@@ -662,14 +664,20 @@ static mv_status seq_scratch(mv_ctx* c, const mv_track_params* p, int n_frames, 
     return st;                                                               \
   }                                                                          \
   o->field = (type*)v
-  SCR(idx, int32_t, ".idx", sizeof(int32_t) * (size_t)n_frames * cells);
-  SCR(prob, float, ".prob", sizeof(float) * (size_t)n_frames * cells);
+  if (planes) {
+    SCR(idx, int32_t, ".idx", sizeof(int32_t) * (size_t)n_frames * cells);
+    SCR(prob, float, ".prob", sizeof(float) * (size_t)n_frames * cells);
+  }
   SCR(qp, int32_t, ".qp", sizeof(int32_t) * (size_t)n_frames * N);
-  SCR(qi, int32_t, ".qi", sizeof(int32_t) * (size_t)n_frames * N);
-  SCR(qpr, float, ".qpr", sizeof(float) * (size_t)n_frames * N);
+  if (planes) {
+    SCR(qi, int32_t, ".qi", sizeof(int32_t) * (size_t)n_frames * N);
+    SCR(qpr, float, ".qpr", sizeof(float) * (size_t)n_frames * N);
+  }
   SCR(qc, int32_t, ".qc", sizeof(int32_t) * (size_t)n_frames);
   SCR(ov, int32_t, ".ov", sizeof(int32_t) * (size_t)n_frames);
-  SCR(flags, uint8_t, ".flags", (size_t)n_frames * cells + 64);
+  if (planes) {
+    SCR(flags, uint8_t, ".flags", (size_t)n_frames * cells + 64);
+  }
   SCR(mp, float, ".mp", sizeof(float) * 4 * (size_t)n_pairs * M);
   SCR(mc, int32_t, ".mc", sizeof(int32_t) * (size_t)n_pairs);
   SCR(mcell, int32_t, ".mcell", sizeof(int32_t) * (size_t)n_pairs * M);
@@ -700,14 +708,15 @@ using SeqStageFn = std::function<mv_status(const char* stage)>;
 
 // The rest of a batch whose detector has run, in three parts that the landmark block calls apart (prepare: words,
 // speculation, matcher; step_table: the table; solve).  With `lm`, the word assignment of frames 0..n-2 with their
-// query keypoints back-projected in the same launch.
-static mv_status seq_words(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
+// query keypoints back-projected in the same launch (none where w.coords_in is NULL).  n_word_frames: the frames
+// that get words, 0 .. n_word_frames-1 (all but the last of a batch; every frame of a warm-up chunk).
+static mv_status seq_words(mv_ctx* c, const mv_track_params* p, int n_word_frames, const int8_t* d_desc,
                            const float* d_depth, const SeqScratch& w, const SeqLandmarks* lm) {
   MvBackProject bp;
   bp.q_idx = w.qi; bp.depth = d_depth; bp.rows = p->match.rows;
   bp.fx = p->pnp.fx; bp.fy = p->pnp.fy; bp.cx = p->pnp.cx; bp.cy = p->pnp.cy;
   bp.coords = w.coords_in;
-  return mv_bow_assign_impl(c, n_frames - 1, p->match.rows * p->match.cols, p->top_n, d_desc, lm->desc_scale, w.qp,
+  return mv_bow_assign_impl(c, n_word_frames, p->match.rows * p->match.cols, p->top_n, d_desc, lm->desc_scale, w.qp,
                             w.qc, w.word, nullptr, bp);
 }
 
@@ -760,7 +769,7 @@ static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, con
                           const SeqLandmarks* lm, const SeqStageFn& on_stage = nullptr) {
   mv_status st;
   if (lm) {
-    if ((st = seq_words(c, p, n_frames, d_desc, d_depth, w, lm))) return st;
+    if ((st = seq_words(c, p, n_frames - 1, d_desc, d_depth, w, lm))) return st;
     if ((st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_frames - 1, p->top_n, w.word,
                                          w.qc, w.coords_in, w.coords_out)))
       return st;
@@ -816,6 +825,19 @@ struct mv_lm_block {
   int phase = 0;   // 1 prepared, 2 table stepped, 3 solved
 };
 
+// k->b = the view of k->w at the block's first frame (coords_out aside: the speculation's)
+static void lm_block_view(mv_lm_block* k) {
+  const size_t W = k->n_warm, N = k->p.top_n, cells = (size_t)k->p.match.rows * k->p.match.cols;
+  SeqScratch& b = k->b;
+  b = k->w;
+  if (b.idx) {
+    b.idx += W * cells; b.prob += W * cells;
+    b.qi += W * N; b.qpr += W * N;
+  }
+  b.qp += W * N; b.qc += W; b.ov += W;
+  b.word += W * N; b.coords_in += 3 * W * N;
+}
+
 static void lm_block_free(mv_lm_block* k) {
   mv_device_guard guard(k->ctx->device);
   mv_lm_spec_free(k->spec);
@@ -844,19 +866,14 @@ extern "C" mv_status mv_track_landmarks_prepare(mv_ctx* c, const mv_track_params
   k->ctx = c; k->p = *p; k->n_warm = n_warm; k->n_frames = n_frames; k->n_words = n_words;
   auto fail = [&](mv_status e) { lm_block_free(k); return e; };
   if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem)) || (st = seq_detect(c, p, T, d_semi, d_semi_scale, k->w)) ||
-      (st = seq_words(c, p, T, d_desc, d_depth, k->w, &lm)))
+      (st = seq_words(c, p, T - 1, d_desc, d_depth, k->w, &lm)))
     return fail(st);
   if ((st = mv_landmarks_speculate_impl(c, n_words, first_frame, n_warm, n_frames - 1, N, k->w.word, k->w.qc,
                                         k->w.coords_in + 3 * (size_t)n_warm * N, &k->spec)))
     return fail(st);
-  SeqScratch& b = k->b;
-  b = k->w;
-  b.idx += (size_t)n_warm * cells; b.prob += (size_t)n_warm * cells;
-  b.qp += (size_t)n_warm * N; b.qi += (size_t)n_warm * N; b.qpr += (size_t)n_warm * N;
-  b.qc += n_warm; b.ov += n_warm;
-  b.word += (size_t)n_warm * N; b.coords_in += 3 * (size_t)n_warm * N;
-  b.coords_out = mv_lm_spec_coords(k->spec);
-  if ((st = seq_match(c, p, n_frames, d_desc + (size_t)n_warm * cells * 256, b, nullptr))) return fail(st);
+  lm_block_view(k);
+  k->b.coords_out = mv_lm_spec_coords(k->spec);
+  if ((st = seq_match(c, p, n_frames, d_desc + (size_t)n_warm * cells * 256, k->b, nullptr))) return fail(st);
   k->phase = 1;
   *out = k;
   return MV_OK;
@@ -1020,13 +1037,13 @@ struct PnpResidencyCap {  // cap the PnP kernel's CTAs per SM for a scope
 // meanwhile.  Consecutive chunks share one halo frame.  With `lm` (host desc_scale and
 // n_with_landmark) seq_step also steps the caller's landmark table over the chunk's frames but its
 // halo before matching; chunks run in order on that stream, so the table chains from chunk to chunk.
-static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames,
-                                          const int8_t* h_semi, const float* h_semi_scale, const int8_t* h_desc,
-                                          const float* h_depth, mv_pair_result* h_results,
-                                          unsigned long long* h2d_bytes, unsigned long long* d2h_bytes,
-                                          const SeqLandmarks* lm) {
-  const int cells = p->match.rows * p->match.cols;
-  const int n_pairs = n_frames - 1;
+// With `blk` (mv_track_landmarks_prepare_host; lm without a table) the host buffers start with blk->n_warm
+// warm-up frames, staged first in chunks of their own without a halo (logits and query rows; words only), and
+// each chunk of the block's n_frames runs the words and the matcher into the block's memory instead of seq_step;
+// the speculation follows the last chunk.  Returns once the host buffers are no longer read: that work may still
+// be queued on the compute stream.
+// Pairs per chunk of the host staging pipeline over n_pairs pairs.
+static int host_chunk_pairs(const mv_ctx* c, const mv_track_params* p, int n_pairs, bool landmarks) {
   // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see below); the
   // one-thread-per-hypothesis kernel covers 256 hypotheses per CTA, the multi-lane forms 16
   const int per_cta = p->pnp.lanes_per_hypothesis == 1 ? 256 : 16;
@@ -1041,14 +1058,26 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     if (v > 0) chunk_pairs = v;
   }
   if (chunk_pairs > n_pairs) chunk_pairs = n_pairs;
-  if (lm) {  // one table step per pair: mv_landmarks_sequence's limits on one call (top_n > 0 is checked below)
+  if (landmarks) {  // one table step per pair: mv_landmarks_sequence's limits on one call (top_n > 0 is checked)
     const int most = (int)std::min<long long>(65535, 0x7fffffffLL / std::max(p->top_n, 1));
     if (chunk_pairs > most) chunk_pairs = most;
   }
+  return chunk_pairs;
+}
+
+static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames,
+                                          const int8_t* h_semi, const float* h_semi_scale, const int8_t* h_desc,
+                                          const float* h_depth, mv_pair_result* h_results,
+                                          unsigned long long* h2d_bytes, unsigned long long* d2h_bytes,
+                                          const SeqLandmarks* lm, mv_lm_block* blk = nullptr) {
+  const int cells = p->match.rows * p->match.cols;
+  const int n_pairs = n_frames - 1;
+  const int n_warm = blk ? blk->n_warm : 0;
+  const int chunk_pairs = host_chunk_pairs(c, p, n_pairs, lm != nullptr);
   const int cf = chunk_pairs + 1;
   const int N = p->top_n;
   mv_status st;
-  if ((st = seq_check(c, fn, p, cf, nullptr, lm))) return st;
+  if ((st = seq_check(c, fn, p, cf, nullptr, lm, blk == nullptr))) return st;
 
   // zero-copy gather needs device-visible (pinned) descriptor and depth buffers
   bool gather = true;
@@ -1066,7 +1095,8 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   }
 
   // The PnP kernel (37 KB of shared memory per CTA) would otherwise fill an SM's shared memory with
-  // 6 CTAs and starve the one-warp row-gather kernel (17 KB) that must run beside it.
+  // 6 CTAs and starve the one-warp row-gather kernel (17 KB) that must run beside it.  The cap ends with this
+  // call: a block prepared here runs its PnP in mv_track_landmarks_solve, uncapped, after the staging.
   PnpResidencyCap residency(c, 5);
 
   constexpr int NB = 3;  // chunks in flight: staging DMA / row gather / compute
@@ -1083,7 +1113,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     if ((st = seq_scratch(c, p, cf, n.c_str(), lm != nullptr, &w[b]))) return st;
     if (lm && (st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
   }
-  if (lm) {
+  if (lm && !blk) {
     // the table update's shared sort scratch, for the full chunk and the last one: growing it between
     // enqueues would free memory (cudaFree) while the three streams run
     const int last_steps = n_pairs - (n_pairs - 1) / chunk_pairs * chunk_pairs;
@@ -1107,8 +1137,9 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   // pinned h_semi / h_desc / h_depth asynchronously.
   struct Drain {
     mv_ctx* c;
+    bool compute = true;   // cleared once a prepared block's work may stay queued (the host buffers are read by then)
     ~Drain() {
-      cudaStreamSynchronize(c->stream);
+      if (compute) cudaStreamSynchronize(c->stream);
       cudaStreamSynchronize(c->copy_stream);
       cudaStreamSynchronize(c->gather_stream);
     }
@@ -1152,15 +1183,38 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   mark("start", 0, c->stream);
 
   unsigned long long up = 0;
-  const int n_chunks = (n_pairs + chunk_pairs - 1) / chunk_pairs;
-  auto chunk_first = [&](int k) { return k * chunk_pairs; };
+  // chunks 0 .. n_warm_chunks-1: warm-up frames, chunk_pairs at most, no halo; then the pairs' chunks
+  const int n_warm_chunks = (n_warm + chunk_pairs - 1) / chunk_pairs;
+  const int n_chunks = n_warm_chunks + (n_pairs + chunk_pairs - 1) / chunk_pairs;
+  auto warm = [&](int k) { return k < n_warm_chunks; };
+  auto chunk_first = [&](int k) { return (k - n_warm_chunks) * chunk_pairs; };   // first pair of a pairs' chunk
+  auto chunk_frame0 = [&](int k) { return warm(k) ? k * chunk_pairs : n_warm + chunk_first(k); };  // in the buffers
   auto chunk_frames = [&](int k) {
-    const int p0 = k * chunk_pairs;
+    if (warm(k)) return std::min(chunk_pairs, n_warm - k * chunk_pairs);
+    const int p0 = chunk_first(k);
     return ((n_pairs - p0) < chunk_pairs ? (n_pairs - p0) : chunk_pairs) + 1;
+  };
+  // The scratch of chunk k: its buffer set, but a block being prepared keeps what step_table and solve read at the
+  // chunk's frames and pairs in its own memory.  The detector of chunk k+1 writes the halo frame's qp / qc / ov there
+  // again before the compute of chunk k reads them: the same bytes (the same frame, the same kernels), in the same
+  // stream order as the chunk-local copies of the host calls.
+  auto chunk_scratch = [&](int k) {
+    SeqScratch v = w[k % NB];
+    if (!blk) return v;
+    const size_t f0 = chunk_frame0(k), N = p->top_n, M = p->match.max_matches;
+    const SeqScratch& a = blk->w;
+    v.qp = a.qp + f0 * N; v.qc = a.qc + f0; v.ov = a.ov + f0;
+    v.word = a.word + f0 * N;
+    v.coords_in = warm(k) ? nullptr : a.coords_in + 3 * f0 * N;   // warm-up words need no coordinates
+    if (!warm(k)) {
+      const size_t p0 = chunk_first(k);
+      v.mp = a.mp + 4 * p0 * M; v.mc = a.mc + p0; v.mcell = a.mcell + p0 * M; v.rin = a.rin + p0;
+    }
+    return v;
   };
 
   auto stage_dma = [&](int k) -> mv_status {
-    const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
+    const int b = k % NB, p0 = chunk_frame0(k), nf = chunk_frames(k);
     cudaStream_t cs = c->copy_stream;
     // buffer set b may be refilled only after the compute that read it is done
     MV_CUDA(c, cudaStreamWaitEvent(cs, consumed[b], 0));
@@ -1168,9 +1222,12 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     MV_CUDA(c, cudaMemcpyAsync(bs[b], h_semi + (size_t)p0 * cells * 65, (size_t)nf * cells * 65,
                                cudaMemcpyHostToDevice, cs));
     MV_CUDA(c, cudaMemcpyAsync(bsc[b], h_semi_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice, cs));
-    MV_CUDA(c, cudaMemcpyAsync(bz[b], h_depth + (size_t)p0 * cells, sizeof(float) * (size_t)nf * cells,
-                               cudaMemcpyHostToDevice, cs));
-    up += (unsigned long long)nf * ((size_t)cells * (65 + 4) + 4);
+    up += (unsigned long long)nf * ((size_t)cells * 65 + 4);
+    if (!warm(k)) {
+      MV_CUDA(c, cudaMemcpyAsync(bz[b], h_depth + (size_t)p0 * cells, sizeof(float) * (size_t)nf * cells,
+                                 cudaMemcpyHostToDevice, cs));
+      up += (unsigned long long)nf * cells * 4;
+    }
     if (lm) {
       MV_CUDA(c, cudaMemcpyAsync(bdsc[b], lm->desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice,
                                  cs));
@@ -1193,7 +1250,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   cudaEvent_t matched;
   if ((st = new_event(&matched))) return st;
   auto launch_gather = [&](int k, cudaEvent_t after) -> mv_status {
-    const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
+    const int b = k % NB, p0 = chunk_frame0(k), nf = chunk_frames(k);
     cudaStream_t gs = c->gather_stream;
     MV_CUDA(c, cudaStreamWaitEvent(gs, detected[b], 0));
     if (after) MV_CUDA(c, cudaStreamWaitEvent(gs, after, 0));
@@ -1216,16 +1273,21 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     return MV_OK;
   };
   auto stage_detect = [&](int k) -> mv_status {
-    const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
+    const int b = k % NB, nf = chunk_frames(k);
+    const SeqScratch v = chunk_scratch(k);
     mv_status s2;
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, copied[b], 0));
-    if ((s2 = seq_detect(c, p, nf, (const int8_t*)bs[b], (const float*)bsc[b], w[b]))) return s2;
+    if ((s2 = seq_detect(c, p, nf, (const int8_t*)bs[b], (const float*)bsc[b], v))) return s2;
     if (gather) {
       dim3 g1((cells + 255) / 256, nf), g2((p->top_n + 255) / 256, nf);
-      mark_needed_rows_kernel<<<g1, 256, 0, c->stream>>>(nf, cells, p->top_n, mv_round_up(p->match.min_prob0),
-                                                         w[b].idx, w[b].prob, w[b].qp, w[b].qc, w[b].flags);
-      MV_CHECK_LAUNCH(c);
-      mark_query_rows_kernel<<<g2, 256, 0, c->stream>>>(cells, p->top_n, w[b].qp, w[b].qc, w[b].flags);
+      if (warm(k)) {   // no matcher runs on a warm-up frame: its query rows only
+        MV_CUDA(c, cudaMemsetAsync(v.flags, 0, (size_t)nf * cells, c->stream));
+      } else {
+        mark_needed_rows_kernel<<<g1, 256, 0, c->stream>>>(nf, cells, p->top_n, mv_round_up(p->match.min_prob0),
+                                                           v.idx, v.prob, v.qp, v.qc, v.flags);
+        MV_CHECK_LAUNCH(c);
+      }
+      mark_query_rows_kernel<<<g2, 256, 0, c->stream>>>(cells, p->top_n, v.qp, v.qc, v.flags);
       MV_CHECK_LAUNCH(c);
     }
     MV_CUDA(c, cudaEventRecord(detected[b], c->stream));
@@ -1241,24 +1303,39 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   };
   // In landmark mode seq_step runs the word assignment (a persistent CTA per SM with the vocabulary in shared
   // memory) after the chunk's `ready` and before its matcher, so it never runs beside a row gather.
+  // A block being prepared runs no K3: chunk k+1's gather is released after chunk k's whole compute (words,
+  // matcher, RANSAC-E) instead.  Released after the matcher it measured the same (profiles/r07).
+  auto release_gather = [&](int k) -> mv_status {
+    if (pending_gather != k + 1) return MV_OK;
+    pending_gather = -1;
+    MV_CUDA(c, cudaEventRecord(matched, c->stream));
+    return launch_gather(k + 1, matched);
+  };
   auto stage_compute = [&](int k) -> mv_status {
     const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, ready[b], 0));
     mark("cmp_beg", k, c->stream);
     const SeqStageFn on_stage = [&](const char* stage) -> mv_status {
       mark(stage, k, c->stream);
-      if (strcmp(stage, "match_end") || pending_gather != k + 1) return MV_OK;
-      pending_gather = -1;
-      MV_CUDA(c, cudaEventRecord(matched, c->stream));
-      return launch_gather(k + 1, matched);
+      if (strcmp(stage, "match_end") || blk) return MV_OK;
+      return release_gather(k);
     };
     SeqLandmarks chunk_lm{};
     if (lm)
       chunk_lm = {lm->first_frame + p0, lm->n_words, lm->table, (const float*)bdsc[b],
                   dnwl ? (int32_t*)dnwl + p0 : nullptr};
-    mv_status s2 = seq_step(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0,
-                            lm ? &chunk_lm : nullptr, on_stage);
-    if (s2) return s2;
+    mv_status s2;
+    if (!blk) {
+      s2 = seq_step(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0,
+                    lm ? &chunk_lm : nullptr, on_stage);
+    } else if (warm(k)) {
+      s2 = seq_words(c, p, nf, (const int8_t*)bd[b], nullptr, chunk_scratch(k), &chunk_lm);
+    } else {
+      const SeqScratch v = chunk_scratch(k);
+      if (!(s2 = seq_words(c, p, nf - 1, (const int8_t*)bd[b], (const float*)bz[b], v, &chunk_lm)))
+        s2 = seq_match(c, p, nf, (const int8_t*)bd[b], v, on_stage);
+    }
+    if (s2 || (blk && (s2 = release_gather(k)))) return s2;
     MV_CUDA(c, cudaEventRecord(consumed[b], c->stream));
     mark("cmp_end", k, c->stream);
     return MV_OK;
@@ -1273,19 +1350,30 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     if ((st = stage_compute(k))) return st;
   }
   unsigned long long moved = 0;
-  unsigned long long down = sizeof(mv_pair_result) * (unsigned long long)n_pairs;
-  MV_CUDA(c, cudaMemcpyAsync(h_results, dres, sizeof(mv_pair_result) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
-                             c->stream));
-  if (dnwl) {
-    MV_CUDA(c, cudaMemcpyAsync(lm->n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
+  unsigned long long down = 0;
+  if (blk) {
+    // one speculation over the warm-up and block words; the block's remaining work stays queued
+    if ((st = mv_landmarks_speculate_impl(c, lm->n_words, lm->first_frame, n_warm, n_pairs, p->top_n, blk->w.word,
+                                          blk->w.qc, blk->b.coords_in, &blk->spec)))
+      return st;
+    blk->b.coords_out = mv_lm_spec_coords(blk->spec);
+    drain.compute = false;
+  } else {
+    down = sizeof(mv_pair_result) * (unsigned long long)n_pairs;
+    MV_CUDA(c, cudaMemcpyAsync(h_results, dres, sizeof(mv_pair_result) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
                                c->stream));
-    down += sizeof(int32_t) * (unsigned long long)n_pairs;
+    if (dnwl) {
+      MV_CUDA(c, cudaMemcpyAsync(lm->n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs,
+                                 cudaMemcpyDeviceToHost, c->stream));
+      down += sizeof(int32_t) * (unsigned long long)n_pairs;
+    }
+    MV_CUDA(c, cudaStreamSynchronize(c->stream));
   }
-  MV_CUDA(c, cudaStreamSynchronize(c->stream));
   MV_CUDA(c, cudaStreamSynchronize(c->copy_stream));
   MV_CUDA(c, cudaMemcpyAsync(&moved, dmoved, 8, cudaMemcpyDeviceToHost, c->gather_stream));
   MV_CUDA(c, cudaStreamSynchronize(c->gather_stream));
   if (trace) {
+    if (blk) MV_CUDA(c, cudaStreamSynchronize(c->stream));
     for (auto& m : marks) {
       float ms = 0.f;
       cudaEventElapsedTime(&ms, marks[0].second, m.second);
@@ -1323,6 +1411,43 @@ extern "C" mv_status mv_track_sequence_landmarks_host(mv_ctx* c, const mv_track_
   const SeqLandmarks lm = {first_frame, n_words, d_table, h_desc_scale, h_n_with_landmark};
   return track_sequence_host_impl(c, "mv_track_sequence_landmarks_host", p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
                                   d2h_bytes, &lm);
+}
+
+extern "C" mv_status mv_track_landmarks_prepare_host(mv_ctx* c, const mv_track_params* p, int n_warm, int n_frames,
+                                                     int first_frame, const int8_t* h_semi, const float* h_semi_scale,
+                                                     const int8_t* h_desc, const float* h_desc_scale,
+                                                     const float* h_depth, int n_words, mv_lm_block** out,
+                                                     unsigned long long* h2d_bytes) {
+  MV_ENTER(c);
+  if (!out) MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: NULL out");
+  *out = nullptr;
+  if (!p || n_frames < 2 || n_warm < 0 || !h_semi || !h_semi_scale || !h_desc || !h_desc_scale || !h_depth)
+    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host");
+  if ((long long)n_warm + n_frames > 65535)
+    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: at most 65535 frames in all");
+  const int T = n_warm + n_frames;
+  const SeqLandmarks lm = {first_frame, n_words, nullptr, h_desc_scale, nullptr};
+  mv_status st;
+  // the whole block's limits, then those of the pipeline's chunks, before the block is allocated
+  if ((st = seq_check(c, "mv_track_landmarks_prepare_host", p, T, nullptr, &lm, false)) ||
+      (st = seq_check(c, "mv_track_landmarks_prepare_host", p, host_chunk_pairs(c, p, n_frames - 1, true) + 1, nullptr,
+                      &lm, false)))
+    return st;
+  if (p->match.use_tensor_cores == 1 && !mv_match_tc_feasible(&p->match, n_frames, n_frames - 1, p->top_n))
+    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: use_tensor_cores = 1 on a shape the tensor-core matcher does "
+                  "not take");
+  mv_lm_block* k = new mv_lm_block();
+  k->ctx = c; k->p = *p; k->n_warm = n_warm; k->n_frames = n_frames; k->n_words = n_words;
+  if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem, false))) { lm_block_free(k); return st; }
+  lm_block_view(k);
+  if ((st = track_sequence_host_impl(c, "mv_track_landmarks_prepare_host", p, n_frames, h_semi, h_semi_scale, h_desc,
+                                     h_depth, nullptr, h2d_bytes, nullptr, &lm, k))) {
+    lm_block_free(k);
+    return st;
+  }
+  k->phase = 1;
+  *out = k;
+  return MV_OK;
 }
 
 // ------------------------------------------------------------------------------------

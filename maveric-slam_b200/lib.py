@@ -30,7 +30,7 @@ NEW_SYMBOLS = [
     "mv_landmarks_remove_old", "mv_landmarks_lookup", "mv_build_corr_landmarks_batch", "mv_landmarks_sequence",
     "mv_track_sequence_landmarks", "mv_track_sequence_landmarks_host", "mv_landmarks_speculate",
     "mv_landmarks_resolve", "mv_lm_spec_release", "mv_track_landmarks_prepare", "mv_track_landmarks_step_table",
-    "mv_track_landmarks_solve", "mv_track_landmarks_release",
+    "mv_track_landmarks_solve", "mv_track_landmarks_release", "mv_track_landmarks_prepare_host",
 ]
 LEGACY_SYMBOLS = [
     "add_Vector2f", "add_Vector3f", "mult_Quaternionf", "create_Quaternionf", "Quaternionf_from_Vector3f",
@@ -150,6 +150,8 @@ def load() -> C.CDLL:
     L.mv_lm_spec_release.restype = None
     L.mv_track_landmarks_prepare.argtypes = [vp, C.POINTER(TrackParams), i32, i32, i32, vp, vp, vp, vp, vp, i32,
                                              C.POINTER(vp)]
+    L.mv_track_landmarks_prepare_host.argtypes = [vp, C.POINTER(TrackParams), i32, i32, i32, vp, vp, vp, vp, vp, i32,
+                                                  C.POINTER(vp), C.POINTER(C.c_ulonglong)]
     L.mv_track_landmarks_step_table.argtypes = [vp, vp, vp, vp]
     L.mv_track_landmarks_solve.argtypes = [vp, vp, vp, vp]
     L.mv_track_landmarks_release.argtypes = [vp]

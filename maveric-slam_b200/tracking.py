@@ -536,6 +536,20 @@ class Tracker:
             self._d(desc), self._d(desc_scale), self._d(depth), int(n_words), C.byref(h)))
         return {"h": h, "n_pairs": n - 1, "keep": (semi, semi_scale, desc, desc_scale, depth)}
 
+    def track_landmarks_prepare_host(self, params: _lib.TrackParams, n_warm, first_frame, semi, semi_scale, desc,
+                                     desc_scale, depth, n_words):
+        """mv_track_landmarks_prepare_host: :meth:`track_landmarks_prepare` from host tensors/arrays (pinned for
+        full copy bandwidth, as :meth:`track_sequence_landmarks_host`).  The host buffers are no longer read when it
+        returns.  Returns a block handle, as :meth:`track_landmarks_prepare`, whose "h2d_bytes" is the bytes
+        staged."""
+        h = C.c_void_p()
+        up = C.c_ulonglong(0)
+        n = semi.shape[0] - int(n_warm)
+        self.ctx.check(self.lib.mv_track_landmarks_prepare_host(
+            self.ctx.h, C.byref(params), int(n_warm), n, int(first_frame), _hp(semi), _hp(semi_scale), _hp(desc),
+            _hp(desc_scale), _hp(depth), int(n_words), C.byref(h), C.byref(up)))
+        return {"h": h, "n_pairs": n - 1, "h2d_bytes": up.value}
+
     def track_landmarks_step_table(self, block, table, n_rewalked=None):
         """mv_track_landmarks_step_table: steps `table` in place over the block's frames."""
         self.ctx.check(self.lib.mv_track_landmarks_step_table(self.ctx.h, block["h"], self._d(table),
@@ -731,14 +745,43 @@ def track_sequence_landmarks_sharded(tracker, params, frames, table, first_frame
     nothing waits on the host.  Returns (uint8 [n - 1, 64] records, int32 [n - 1] counts, int32 re-walked words of
     this rank's block).  `timings`: a list that receives this rank's CUDA events (prepare, table wait,
     step_table, solve), for measurement."""
+    semi, semi_scale, desc, desc_scale, depth = frames
+
+    def prepare(p, w, ff, lo, hi):
+        return tracker.track_landmarks_prepare(p, w, ff, semi[lo:hi], semi_scale[lo:hi], desc[lo:hi],
+                                               desc_scale[lo:hi], depth[lo:hi], table.shape[0])
+    return _relay_landmarks(tracker, params, semi.shape[0] - 1, table, first_frame, n_warm, group, None, timings,
+                            prepare)[:3]
+
+
+def track_sequence_landmarks_host_sharded(tracker, params, host_frames, table, first_frame=0, n_warm=0, group=None,
+                                          counts=None, timings=None):
+    """:func:`track_sequence_landmarks_sharded` from host buffers: each rank stages only its block, its halo frame
+    and up to n_warm warm-up frames through its own link (:meth:`Tracker.track_landmarks_prepare_host`), then the
+    table is relayed as there.
+
+    host_frames = (semi, semi_scale, desc, desc_scale, depth): the WHOLE sequence in host memory (pinned CPU
+    tensors or numpy arrays).  `counts`: pairs per rank of a weighted partition (:func:`shard_pairs_weighted`, for
+    ranks whose host links differ); default: the equal blocks of :func:`shard_pairs`.  Returns (uint8 [n - 1, 64]
+    records, int32 [n - 1] counts, int32 re-walked words of this rank's block, this rank's h2d bytes), the first
+    two on this rank's device.  `timings` as :func:`track_sequence_landmarks_sharded` (prepare is the device time
+    after the prepare call's start; the call itself returns once staging is done)."""
+    def prepare(p, w, ff, lo, hi):
+        return tracker.track_landmarks_prepare_host(p, w, ff, *[x[lo:hi] for x in host_frames], table.shape[0])
+    return _relay_landmarks(tracker, params, host_frames[0].shape[0] - 1, table, first_frame, n_warm, group, counts,
+                            timings, prepare)
+
+
+def _relay_landmarks(tracker, params, n_pairs, table, first_frame, n_warm, group, counts, timings, prepare):
+    """The relay of the sharded landmark calls.  prepare(params, n_warm, first_frame, lo, hi) prepares this rank's
+    block from frames [lo, hi) of the sequence (its warm-up frames, its pairs and its halo frame).  Returns
+    (records, counts, re-walked words, the block's "h2d_bytes" or 0)."""
     import copy
     import torch
     import torch.distributed as dist
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
-    semi, semi_scale, desc, desc_scale, depth = frames
-    n_pairs = semi.shape[0] - 1
-    gat = ResultGather(n_pairs, world, rank, tracker.device, group=group)
+    gat = ResultGather(n_pairs, world, rank, tracker.device, group=group, counts=counts)
     first, count = gat.first, gat.count
     nl_send = torch.zeros((gat.per,), dtype=torch.int32, device=tracker.device)
     rewalked = torch.zeros((1,), dtype=torch.int32, device=tracker.device)
@@ -748,12 +791,10 @@ def track_sequence_landmarks_sharded(tracker, params, frames, table, first_frame
     block = None
     if count > 0:
         w = min(int(n_warm), first)
-        lo, hi = first - w, first + count + 1
         p = copy.copy(params)
         p.pnp = copy.copy(params.pnp)
         p.pnp.first_pair = params.pnp.first_pair + first
-        block = tracker.track_landmarks_prepare(p, w, first_frame + first, semi[lo:hi], semi_scale[lo:hi], desc[lo:hi],
-                                                desc_scale[lo:hi], depth[lo:hi], table.shape[0])
+        block = prepare(p, w, first_frame + first, first - w, first + count + 1)
     if ev:
         ev[1].record()
     src = _global_rank(group, rank - 1)
@@ -780,9 +821,13 @@ def track_sequence_landmarks_sharded(tracker, params, frames, table, first_frame
         dist.broadcast(table, src=_global_rank(group, world - 1), group=group)
     else:
         nl_all = nl_send
+    h2d = 0
     if block is not None:
+        h2d = block.get("h2d_bytes", 0)
         tracker.track_landmarks_release(block)
-    return records, nl_all[:n_pairs], rewalked   # shard_pairs blocks start at rank * per: no padding between them
+    # equal blocks start at rank * per, so only the tail is padding; weighted ones drop it as the records do
+    nl = nl_all[:n_pairs] if gat._rows is None else nl_all.index_select(0, gat._rows)
+    return records, nl, rewalked, h2d
 
 
 def _global_rank(group, r):

@@ -13,7 +13,14 @@ cost at N = 1.
 For the landmark legs (W = warm-up frames per block: 0 is the plain relay, 8 / 16 / 32 speculate) each rank's
 median device times of prepare, the wait for the table, step_table and solve (CUDA events), and the words each rank
 walked again.  Checks, on every rank, that the gathered records, landmark counts and final table equal one
-mv_track_sequence_landmarks over the whole sequence on that rank's GPU."""
+mv_track_sequence_landmarks over the whole sequence on that rank's GPU.
+
+Host legs, from pinned host copies of the frames (each rank stages through its own link):
+    landmarks_host_one_call     mv_track_sequence_landmarks_host over the whole sequence, on each rank's GPU
+    landmarks_host_W<w>         tracking.track_sequence_landmarks_host_sharded (W = 0, 8, 32)
+    landmarks_upload_relay      the rank's frames uploaded whole (every descriptor), then the device relay (W = 0)
+with each rank's h2d bytes per step, the phase times and re-walked words of the sharded legs, and the same
+byte-equality check."""
 import json
 import os
 import subprocess
@@ -98,14 +105,56 @@ def one_call_step():   # the undivided call over the whole sequence, for the spl
     tr.track_sequence_landmarks(p, *frames, one_table, first_frame=0)
 
 
+# ---- host legs
+HOST_WARMS = (0, 8, 32)
+host = tuple(torch.empty(t.shape, dtype=t.dtype, pin_memory=True).copy_(t) for t in frames)
+torch.cuda.synchronize()
+h2d = {}
+host_last = {}
+
+
+def host_one_call_step():
+    tr.ctx.check(tr.lib.mv_landmarks_init(tr.ctx.h, tr.n_words, tr._d(one_table)))
+    _, _, up, _ = tr.track_sequence_landmarks_host(p, *host, one_table, first_frame=0)
+    h2d["landmarks_host_one_call"] = up
+
+
+def host_step(w, key):
+    tr.ctx.check(tr.lib.mv_landmarks_init(tr.ctx.h, tr.n_words, tr._d(table)))
+    ev = []
+    rec, nl, rw, up = tracking.track_sequence_landmarks_host_sharded(tr, p, host, table, first_frame=0, n_warm=w,
+                                                                     timings=ev)
+    host_last[key] = (rec, nl, rw, ev)
+    h2d[key] = up
+
+
+def upload_relay_step():
+    # what a user without prepare_host does: the rank's frames (block and halo) copied whole, then the device relay
+    if gat.count:
+        lo, hi = gat.first, gat.first + gat.count + 1
+        for d, hst in zip(frames, host):
+            d[lo:hi].copy_(hst[lo:hi], non_blocking=True)
+        h2d["landmarks_upload_relay"] = sum(x[lo:hi].numel() * x.element_size() for x in host)
+    landmark_step(0)
+    host_last["landmarks_upload_relay"] = last[0]
+
+
 legs = {"depth": depth_step, "landmarks_one_call": one_call_step}
 for w in WARMS:
     legs[f"landmarks_W{w}"] = (lambda w=w: landmark_step(w))
+legs["landmarks_host_one_call"] = host_one_call_step
+for w in HOST_WARMS:
+    legs[f"landmarks_host_W{w}"] = (lambda w=w: host_step(w, f"landmarks_host_W{w}"))
+legs["landmarks_upload_relay"] = upload_relay_step
+
+SHARDED = [k for k in legs if k.startswith("landmarks_host_W")] + ["landmarks_upload_relay"]
 for fn in legs.values():   # warm-up: modules, scratch, NCCL communicators
     fn()
 times = {k: [] for k in legs}
 phases = {w: [] for w in WARMS}
 rewalked = {w: [] for w in WARMS}
+host_phases = {k: [] for k in SHARDED}
+host_rewalked = {k: [] for k in SHARDED}
 for _ in range(STEPS):
     for k, fn in legs.items():
         times[k].append(timed(fn))
@@ -114,6 +163,10 @@ for _ in range(STEPS):
             ev = last[w][3]
             phases[w].append([ev[i].elapsed_time(ev[i + 1]) for i in range(4)])
             rewalked[w].append(int(last[w][2].item()))
+        if k in SHARDED:
+            ev = host_last[k][3]
+            host_phases[k].append([ev[i].elapsed_time(ev[i + 1]) for i in range(4)])
+            host_rewalked[k].append(int(host_last[k][2].item()))
 
 # byte-equality with one call over the whole sequence on this rank's GPU
 one = tr.landmarks_new(tr.n_words)
@@ -124,13 +177,28 @@ for w in WARMS:
     rec, nl, _, _ = last[w]
     equal[w] = bool(rec.cpu().numpy().tobytes() == res1.cpu().numpy().tobytes() and torch.equal(nl, nl1)
                     and torch.equal(table, one))
+host_equal = {}
+for k in SHARDED:
+    legs[k]()
+    rec, nl, _, _ = host_last[k]
+    host_equal[k] = bool(rec.cpu().numpy().tobytes() == res1.cpu().numpy().tobytes() and torch.equal(nl, nl1)
+                         and torch.equal(table, one))
+tr.ctx.check(tr.lib.mv_landmarks_init(tr.ctx.h, tr.n_words, tr._d(one_table)))
+h_res, h_nl, _, _ = tr.track_sequence_landmarks_host(p, *host, one_table, first_frame=0)
+host_equal["landmarks_host_one_call"] = bool(h_res.tobytes() == res1.cpu().numpy().tobytes()
+                                             and (h_nl == nl1.cpu().numpy()).all() and torch.equal(one_table, one))
 
 mine = {"rank": rank, "device": torch.cuda.get_device_name(local), "block": [gat.first, gat.count],
         "equal_to_one_gpu": {str(w): equal[w] for w in WARMS},
         "phase_ms_median": {str(w): dict(zip(("prepare", "table_wait", "step_table", "solve"),
                                              np.median(np.array(phases[w]), axis=0).round(4).tolist()))
                             for w in WARMS},
-        "rewalked_words": {str(w): rewalked[w][-1] for w in WARMS}}
+        "rewalked_words": {str(w): rewalked[w][-1] for w in WARMS},
+        "host_equal_to_one_gpu": host_equal, "h2d_bytes_per_step": h2d,
+        "host_phase_ms_median": {k: dict(zip(("prepare", "table_wait", "step_table", "solve"),
+                                             np.median(np.array(v), axis=0).round(4).tolist()))
+                                 for k, v in host_phases.items()},
+        "host_rewalked_words": {k: v[-1] for k, v in host_rewalked.items()}}
 ranks = [None] * world
 if world > 1:
     dist.all_gather_object(ranks, mine)
@@ -146,7 +214,8 @@ if rank == 0:
     out = {"gpus": world, "frames": NF, "pairs": n_pairs, "steps": STEPS, "gpu": power,
            "pairs_per_s": {k: n_pairs / m for k, m in med.items()}, "median_s": med,
            "all_s": times, "ranks": ranks,
-           "all_equal_to_one_gpu": all(all(r["equal_to_one_gpu"].values()) for r in ranks)}
+           "all_equal_to_one_gpu": all(all(r["equal_to_one_gpu"].values()) and all(r["host_equal_to_one_gpu"].values())
+                                       for r in ranks)}
     s = json.dumps(out, indent=1)
     print(s)
     if OUT:
