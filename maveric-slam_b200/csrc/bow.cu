@@ -708,7 +708,9 @@ static size_t bow_smem(int n_base, int wpb) {
   return sizeof(int32_t) * ((n_leaf + 3) & ~(size_t)3) + (size_t)n_base * 256 + sizeof(float) * 2 * n_base;
 }
 
-bool mv_bow_vocab_fits(const mv_ctx* ctx) { return bow_smem(ctx->bow_n_base, ctx->bow_wpb) <= 227 * 1024; }
+constexpr size_t kBowSmemMax = 227 * 1024;   // an SM's shared memory for one block (opt-in)
+
+bool mv_bow_vocab_fits(const mv_ctx* ctx) { return bow_smem(ctx->bow_n_base, ctx->bow_wpb) <= kBowSmemMax; }
 
 mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, const int8_t* d_desc,
                              const float* d_desc_scale, const int32_t* d_q_patch, const int32_t* d_q_count,
@@ -729,9 +731,12 @@ mv_status mv_bow_assign_impl(mv_ctx* ctx, int n_frames, int cells, int top_n, co
   v.leaves = (const int32_t*)dl; v.base_t = (const int8_t*)db;
   v.scale = (const float*)ds; v.bias = (const float*)ds + v.n_base;
   const size_t smem = bow_smem(v.n_base, v.wpb);
-  if (smem > ctx->bow_smem_attr) {   // a function attribute of the context's device: set once per size
-    MV_CUDA(ctx, cudaFuncSetAttribute(bow_assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ctx->bow_smem_attr = smem;
+  // The limit is an attribute of the kernel in the device's primary context, which every mv_ctx on that device
+  // shares: a context that set it to its own vocabulary's size would lower it under another context's larger
+  // one.  So every context sets the same bound, the largest any vocabulary that fits may need, and never less.
+  if (!ctx->bow_smem_attr_set) {
+    MV_CUDA(ctx, cudaFuncSetAttribute(bow_assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBowSmemMax));
+    ctx->bow_smem_attr_set = true;
   }
   const int per_cta = kBowThreads / kBowLanes;   // queries a CTA handles per trip
   const long long trips = ((long long)n_frames * top_n + per_cta - 1) / per_cta;

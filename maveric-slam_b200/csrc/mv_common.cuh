@@ -37,7 +37,7 @@ struct mv_ctx {
   bool pnp_work_live = false;           // profile mode: the PnP work counter holds launches not yet read
   int match_items = 0;                  // tiles of the last tensor-core matcher launch (mv_ctx_match_work)
   int bow_n_base = 0, bow_wpb = 0;      // vocabulary on the device (mv_bow_set_vocabulary)
-  size_t bow_smem_attr = 0;             // dynamic shared memory the word-assignment kernel is allowed so far
+  bool bow_smem_attr_set = false;       // the word-assignment kernel's shared-memory limit is set (bow.cu)
   int lm_words = 0;                     // size the landmark scratch was initialised for
   std::map<std::string, mv_prof_slot> prof;
   std::vector<mv_pending_event> pending;

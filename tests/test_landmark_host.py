@@ -4,7 +4,9 @@ mv_track_sequence_host with the landmark table carried from chunk to chunk on th
 The reference is the device-resident call mv_track_sequence_landmarks (itself checked against the composition of
 public calls and the oracle in tests/test_landmark_sequence.py): results, matches with a landmark and the final table
 must be byte-equal whatever the chunk size and staging mode.  The byte count is checked against what the staging
-needs, computed here from the public detector outputs."""
+needs, computed here from the public detector outputs.
+The device one-call is itself held to a CPU reference of the whole path, tests/landmark_reference.py
+(tests/test_landmark_reference.py)."""
 import ctypes as C
 import os
 

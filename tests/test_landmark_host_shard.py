@@ -4,7 +4,9 @@
 References: the device landmark path on the same 66-frame fixture (mv_track_sequence_landmarks, which
 tests/test_landmark_host.py equates with mv_track_sequence_landmarks_host) and the device-prepared block
 (tests/test_landmark_shard.py).  Staged bytes are checked against a formula computed from the public detector
-outputs, as tests/test_landmark_host.py does for the one host call."""
+outputs, as tests/test_landmark_host.py does for the one host call.
+The device one-call is itself held to a CPU reference of the whole path, tests/landmark_reference.py
+(tests/test_landmark_reference.py)."""
 import ctypes as C
 import os
 import sys

@@ -4,36 +4,19 @@
 References, all composed from pieces pinned elsewhere (tests/test_bow.py):
   * the per-frame loop of the existing kernels mv_landmarks_observe / mv_landmarks_remove_old, with
     mv_landmarks_lookup after each step -- the final table must be byte-equal, stale slots included;
-  * orc_landmarks_sequence below: the same loop on the oracle's table (orc_pool_observe / orc_pool_remove_old),
+  * orc_landmarks_sequence (tests/landmark_reference.py): the same loop on the oracle's table (orc_pool_observe / orc_pool_remove_old),
     itself checked against the contents of the host pool, which is pinned to the reference's header;
   * for the sequence path, the public calls softmax -> top_n -> bow_assign, the per-frame table loop,
     match -> ransac_identity, build_corr_landmarks per pair against its snapshot, pnp_gn; and the oracle's K3.
+The whole path against a CPU reference built from the oracle alone: tests/test_landmark_reference.py.
 """
 import numpy as np
 import pytest
 
+from landmark_reference import orc_landmarks_sequence
 from test_bow import drive_host_pool, table_contents
 
 CAM = (718.856, 718.856, 607.1928, 185.2157)
-
-
-def orc_landmarks_sequence(oracle, table, first_frame, word, q_count, coords, snapshots=None):
-    """The semantics of mv_landmarks_sequence on the oracle's table (updated in place): step f observes the first
-    q_count[f] words of frame first_frame + f, then removes old frames; returns each occurrence's lookup right after
-    its step (0 where the word has no record or q >= q_count)."""
-    n_steps, top_n = word.shape
-    out = np.zeros((n_steps, top_n, 3), np.float32)
-    for f in range(n_steps):
-        k = min(int(q_count[f]), top_n)
-        oracle.pool_observe(table, first_frame + f, word[f, :k], coords[f, :k])
-        oracle.pool_remove_old(table, first_frame + f)
-        for q in range(k):
-            w = int(word[f, q])
-            if 0 <= w < len(table) and table[w]["word_id"] == w:
-                out[f, q] = table[w]["coords"]
-        if snapshots is not None:
-            snapshots.append(table.copy())
-    return out
 
 
 # ------------------------------------------------------------------ CPU

@@ -4,6 +4,8 @@ frame-level block (mv_track_landmarks_prepare / step_table / solve) and the tabl
 
 References: mv_landmarks_sequence and mv_track_sequence_landmarks on the same inputs (themselves pinned to the
 per-frame kernels and the oracle in tests/test_landmark_sequence.py), and the oracle's table loop.
+The device one-call is itself held to a CPU reference of the whole path, tests/landmark_reference.py
+(tests/test_landmark_reference.py).
 """
 import os
 import socket
@@ -12,25 +14,11 @@ import sys
 import numpy as np
 import pytest
 
+from landmark_reference import orc_landmarks_sequence
 from test_bow import drive_host_pool
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 WARMS = (0, 1, 7, 8, 16, 64)
-
-
-def orc_landmarks_sequence(oracle, table, first_frame, word, q_count, coords):
-    """mv_landmarks_sequence on the oracle's table (updated in place) -> each occurrence's lookup after its step."""
-    n_steps, top_n = word.shape
-    out = np.zeros((n_steps, top_n, 3), np.float32)
-    for f in range(n_steps):
-        k = min(int(q_count[f]), top_n)
-        oracle.pool_observe(table, first_frame + f, word[f, :k], coords[f, :k])
-        oracle.pool_remove_old(table, first_frame + f)
-        for q in range(k):
-            w = int(word[f, q])
-            if 0 <= w < len(table) and table[w]["word_id"] == w:
-                out[f, q] = table[w]["coords"]
-    return out
 
 
 def _dev(tracker, a):
