@@ -239,27 +239,28 @@ def test_ransac_batch_device_pose(tracker, oracle, kat):
 
 def test_ransac_batch_inlier_cap(tracker, oracle):
     """pnp_solver.c:107,:146,:152: the inlier array holds 1000 entries.  Pairs of 1024 points with 0, 7,
-    999, 1000, 1001 and 1024 inliers: counts and the ordered inlier lists against T2 with cap = 1000
-    (T2 == T1 on these shapes: test_ransac_cap_and_empty_cases_vs_reference)."""
+    999, 1000, 1001 and 1024 inliers, and pairs of 16384 points (BASELINE configs[4]'s match cap) with 0, 1000,
+    1001, 9000 and 16384: counts and the ordered inlier lists against T2 with cap = 1000 (T2 == T1 on the
+    1024-point shapes: test_ransac_cap_and_empty_cases_vs_reference)."""
     import torch
     rng = np.random.default_rng(9)
-    wants = [0, 7, 999, 1000, 1001, 1024]
-    P, M = len(wants), 1024
-    pts = np.zeros((P, M, 4), np.float32)
-    for p, k in enumerate(wants):
-        a = (rng.random((M, 2)) * np.array([1241, 376])).astype(np.float32)
-        inl = np.zeros(M, bool)
-        inl[rng.permutation(M)[:k]] = True
-        off = np.where(inl[:, None], rng.random((M, 2)) * 1.2 - 0.6, 4.0 + rng.random((M, 2)))
-        pts[p, :, :2] = a
-        pts[p, :, 2:] = a + off.astype(np.float32)
-    cnt = np.full(P, M, np.int32)
-    ninl, inl, _ = tracker.ransac_identity(torch.from_numpy(pts).to(tracker.device),
-                                           torch.from_numpy(cnt).to(tracker.device))
-    for p, k in enumerate(wants):
-        E, ref_inl, n, _ = oracle.ransac_identity(pts[p, :, :2], pts[p, :, 2:], cap=1000)
-        assert n == min(k, 1000) == int(ninl[p])
-        assert (inl[p, :n].cpu().numpy() == ref_inl).all()
+    for M, wants in ((1024, [0, 7, 999, 1000, 1001, 1024]), (16384, [0, 1000, 1001, 9000, 16384])):
+        P = len(wants)
+        pts = np.zeros((P, M, 4), np.float32)
+        for p, k in enumerate(wants):
+            a = (rng.random((M, 2)) * np.array([1241, 376])).astype(np.float32)
+            inl = np.zeros(M, bool)
+            inl[rng.permutation(M)[:k]] = True
+            off = np.where(inl[:, None], rng.random((M, 2)) * 1.2 - 0.6, 4.0 + rng.random((M, 2)))
+            pts[p, :, :2] = a
+            pts[p, :, 2:] = a + off.astype(np.float32)
+        cnt = np.full(P, M, np.int32)
+        ninl, inl, _ = tracker.ransac_identity(torch.from_numpy(pts).to(tracker.device),
+                                               torch.from_numpy(cnt).to(tracker.device))
+        for p, k in enumerate(wants):
+            E, ref_inl, n, _ = oracle.ransac_identity(pts[p, :, :2], pts[p, :, 2:], cap=1000)
+            assert n == min(k, 1000) == int(ninl[p]), (M, k)
+            assert (inl[p, :n].cpu().numpy() == ref_inl).all(), (M, k)
 
 
 def test_matmul_shim(tk, kat):
@@ -293,11 +294,23 @@ def _pnp_lane_forms():
     return [(1, 8), (1, 7), (32, 8)]
 
 
+def _oracle_pnp(oracle, cfg, corr, n, want_hyp=True):
+    """oracle.pnp_gn of every pair of corr [P, 5, stride], the pairs on threads of their own (the oracle releases the
+    GIL) -> [(pose, stats, hypotheses)]."""
+    import os
+    from concurrent.futures import ThreadPoolExecutor
+    with ThreadPoolExecutor(min(len(corr), os.cpu_count() or 1)) as ex:
+        return list(ex.map(lambda p: oracle.pnp_gn(cfg, corr[p], n, pair_index=p, want_hyp=want_hyp), range(len(corr))))
+
+
+# H = 288 spans CTAs with a partial last one in both CTA sizes: 128 + 128 + 32 (MV_PNP_GPW=1) and 256 + 32 (=2).
+# n above 4096 walks the streaming kernel's staging chunks past 8 x 512; 16384 is BASELINE configs[4]'s match cap.
 @pytest.mark.parametrize("lanes,sample_size", _pnp_lane_forms())
-@pytest.mark.parametrize("n,stride", [(1000, 1024), (37, 64), (330, 1024), (480, 512), (1500, 1536), (2049, 2304), (8, 8)])
-def test_pnp_gn_vs_oracle(tracker, tk, oracle, synth, lanes, sample_size, n, stride):
+@pytest.mark.parametrize("n,stride", [(1000, 1024), (37, 64), (330, 1024), (480, 512), (1500, 1536), (2049, 2304), (8, 8),
+                                      (4100, 4608), (6900, 16384), (16384, 16384)])
+def test_pnp_gn_vs_oracle(tracker, tk, oracle, synth, monkeypatch, lanes, sample_size, n, stride):
     import torch
-    H, P = 96, 3
+    H, P = 288, 3
     corr = np.zeros((P, 5, stride), np.float32)
     truth = []
     for p in range(P):
@@ -306,36 +319,57 @@ def test_pnp_gn_vs_oracle(tracker, tk, oracle, synth, lanes, sample_size, n, str
         truth.append(pose)
     cnt = np.full(P, n, np.int32)
     prm = _pnp_params(tk, H, lanes, seed=4, sample_size=sample_size)
-    pose, stats, hyp = tracker.pnp_gn(prm, torch.from_numpy(corr).to(tracker.device),
-                                      torch.from_numpy(cnt).to(tracker.device), want_hyp=True)
-    pose, stats, hyp = pose.cpu().numpy(), stats.cpu().numpy(), hyp.cpu().numpy()
     cfg = orc.pnp_cfg(hypotheses=H, seed=4, lanes=lanes, sample_size=sample_size)
-    for p in range(P):
-        rp, rs, rh = oracle.pnp_gn(cfg, corr[p], n, pair_index=p, want_hyp=True)
-        # Every hypothesis, bit for bit: the kernel follows the oracle operation for operation (explicit RN
-        # ops, -fmad=false), so pose and inlier count of all H hypotheses are identical -- including the
-        # chaotic ones that never found a consensus.  A hypothesis that diverged to NaN is NaN in both
-        # (payload and sign of a NaN are not part of the contract).
-        g, r = hyp[p], rh
-        same = (g.view(np.int32) == r.view(np.int32)) | (np.isnan(g) & np.isnan(r))
-        bad = np.nonzero(~same.all(axis=1))[0]
-        assert bad.size == 0, (lanes, n, "hypotheses that differ:", bad[:8].tolist(),
-                               g[bad[:3]].tolist(), r[bad[:3]].tolist())
-        # the 1e-5 rad / 1e-5 relative tolerance of BASELINE.json is therefore met with zero error;
-        # kept as a statement of the contract on the hypotheses that found a consensus
-        good = rh[:, 7] >= 0.3 * n
-        assert good.sum() >= 1
-        ang = np.array([rot_angle(hyp[p, h, :4], rh[h, :4]) for h in np.nonzero(good)[0]])
-        dt = (np.linalg.norm(hyp[p, good, 4:7] - rh[good, 4:7], axis=1)
-              / np.maximum(1.0, np.linalg.norm(rh[good, 4:7], axis=1)))
-        assert (ang < 1e-5).all() and (dt < 1e-5).all()
-        # selected pose: tolerance stated in BASELINE.json north_star
-        assert stats[p, 0] == rs[0] and stats[p, 3] == rs[3]
+    want = _oracle_pnp(oracle, cfg, corr, n)
+    for gpw in ("1", "2"):
+        monkeypatch.setenv("MV_PNP_GPW", gpw)
+        pose, stats, hyp = tracker.pnp_gn(prm, torch.from_numpy(corr).to(tracker.device),
+                                          torch.from_numpy(cnt).to(tracker.device), want_hyp=True)
+        pose, stats, hyp = pose.cpu().numpy(), stats.cpu().numpy(), hyp.cpu().numpy()
+        for p in range(P):
+            rp, rs, rh = want[p]
+            # Every hypothesis, bit for bit: the kernel follows the oracle operation for operation (explicit RN
+            # ops, -fmad=false), so pose and inlier count of all H hypotheses are identical -- including the
+            # chaotic ones that never found a consensus.  A hypothesis that diverged to NaN is NaN in both
+            # (payload and sign of a NaN are not part of the contract).
+            g, r = hyp[p], rh
+            same = (g.view(np.int32) == r.view(np.int32)) | (np.isnan(g) & np.isnan(r))
+            bad = np.nonzero(~same.all(axis=1))[0]
+            assert bad.size == 0, (lanes, n, gpw, "hypotheses that differ:", bad[:8].tolist(),
+                                   g[bad[:3]].tolist(), r[bad[:3]].tolist())
+            # the 1e-5 rad / 1e-5 relative tolerance of BASELINE.json is therefore met with zero error;
+            # kept as a statement of the contract on the hypotheses that found a consensus
+            good = rh[:, 7] >= 0.3 * n
+            assert good.sum() >= 1
+            ang = np.array([rot_angle(hyp[p, h, :4], rh[h, :4]) for h in np.nonzero(good)[0]])
+            dt = (np.linalg.norm(hyp[p, good, 4:7] - rh[good, 4:7], axis=1)
+                  / np.maximum(1.0, np.linalg.norm(rh[good, 4:7], axis=1)))
+            assert (ang < 1e-5).all() and (dt < 1e-5).all()
+            # selected pose: tolerance stated in BASELINE.json north_star
+            assert stats[p, 0] == rs[0] and stats[p, 3] == rs[3]
+            assert rot_angle(pose[p, :4], rp[:4]) < 1e-5
+            assert np.linalg.norm(pose[p, 4:] - rp[4:]) <= 1e-5 * max(1.0, np.linalg.norm(rp[4:]))
+            if n >= 37:  # and it actually solves the problem
+                assert rot_angle(pose[p, :4], truth[p][:4]) < 2e-3
+                assert np.linalg.norm(pose[p, 4:] - truth[p][4:]) < 0.05
+
+
+def test_pnp_gn_4096_hypotheses_vs_oracle(tracker, tk, oracle, synth):
+    """BASELINE configs[4]'s K3 at its largest: 4096 hypotheses on 16384 correspondences, 32 CTAs of 128 or 16 of
+    256 per pair.  The selected pose and stats against the oracle."""
+    import torch
+    H, n, P = 4096, 16384, 2
+    corr = np.stack([synth.synth_pnp_problem(200 + p, n)[0] for p in range(P)])
+    pose, stats, _ = tracker.pnp_gn(_pnp_params(tk, H, 1, seed=4), torch.from_numpy(corr).to(tracker.device),
+                                    torch.full((P,), n, dtype=torch.int32, device=tracker.device))
+    pose, stats = pose.cpu().numpy(), stats.cpu().numpy()
+    for p, (rp, rs, _) in enumerate(_oracle_pnp(oracle, orc.pnp_cfg(hypotheses=H, seed=4, lanes=1), corr, n,
+                                               want_hyp=False)):
+        assert stats[p, 0] == rs[0] and stats[p, 2] == rs[2] and stats[p, 3] == rs[3], (p, stats[p], rs)
+        assert abs(stats[p, 1] - rs[1]) <= 1e-5 * abs(rs[1]), (p, stats[p], rs)
         assert rot_angle(pose[p, :4], rp[:4]) < 1e-5
         assert np.linalg.norm(pose[p, 4:] - rp[4:]) <= 1e-5 * max(1.0, np.linalg.norm(rp[4:]))
-        if n >= 37:  # and it actually solves the problem
-            assert rot_angle(pose[p, :4], truth[p][:4]) < 2e-3
-            assert np.linalg.norm(pose[p, 4:] - truth[p][4:]) < 0.05
+        assert rs[0] >= 0.5 * n
 
 
 def test_pnp_gn_empty_and_init(tracker, tk, oracle):

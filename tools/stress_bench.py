@@ -5,9 +5,10 @@ round 1 and the first half of round 2 ran --permille 550 = ~12.2k keypoints), 33
 under torchrun, sharded by contiguous pair blocks over N B200s with the one all_gather of 64-byte
 records (the same sharding as bench.py).  Device-resident frames, CUDA events, max over ranks, 2 warm-ups;
 prints one JSON line with the per-kernel breakdown of rank 0.  Also a scale check of the whole path: two
-runs must return identical bytes and both matchers must agree.
+runs must return identical bytes and both matchers must agree; and parity: rank 0's first 8 pairs against the CPU
+oracle (orc_bench_sequence on all host cores), compared as bench.py's cpu_baseline.parity (--no-parity skips it).
 
-    python tools/stress_bench.py [--frames F] [--steps K]
+    python tools/stress_bench.py [--frames F] [--steps K] [--no-parity]
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/stress_bench.py --frames 257
 """
 from __future__ import annotations
@@ -26,6 +27,7 @@ def main():
     ap.add_argument("--frames", type=int, default=33)
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--permille", type=int, default=850, help="keypoint density of the synthetic world")
+    ap.add_argument("--no-parity", action="store_true", help="skip the comparison with the CPU oracle")
     args = ap.parse_args()
     import torch
     import maveric_slam_b200  # noqa: F401
@@ -53,6 +55,7 @@ def main():
 
     out = tr.track_sequence(params(), semi, scale, desc, depth)
     ref = out.cpu().numpy().tobytes()
+    local = tracking.results_to_numpy(out)
     same = tr.track_sequence(params(), semi, scale, desc, depth).cpu().numpy().tobytes() == ref
     dp4a = tr.track_sequence(params(False), semi, scale, desc, depth).cpu().numpy().tobytes() == ref
     torch.cuda.synchronize()
@@ -82,6 +85,17 @@ def main():
     flags = torch.tensor([int(same), int(dp4a)], device=tr.device)
     if world > 1:
         dist.all_reduce(flags, op=dist.ReduceOp.MIN)
+    parity = None
+    if rank == 0 and not args.no_parity:
+        import numpy as np
+        from bench import parity_against_port
+        from oracle import orc
+        n_par = min(8, count)
+        cfg = orc.TrackCfg(orc.MatchCfg(rows, cols, 4, 4, 16, 16384, 0.9, 0.2),
+                           orc.pnp_cfg(hypotheses=4096, seed=0, lanes=1), 16000, 32768, 10, 1.1, float(synth.SEMI_SCALE))
+        _, cpu = orc.Oracle().bench_sequence(cfg, orc.SynthCfg(seed, rows, cols, args.permille, 6),
+                                             np.ascontiguousarray(off[:n_par + 1]), 0, n_par, os.cpu_count() or 1)
+        parity = parity_against_port(local, cpu, n_par)
     if rank == 0:
         print(json.dumps({
             "metric": "frame-pairs/sec (window match + PnP), BASELINE configs[4] stress shape, %d GPU(s)" % world,
@@ -91,7 +105,7 @@ def main():
                        "mean_matches_per_pair": float(res["num_matches"].mean()),
                        "mean_pnp_inliers": float(res["pnp_inliers"].mean())},
             "kernel_ms_rank0": prof, "deterministic": bool(flags[0].item()), "dp4a_matcher_same_bytes": bool(flags[1].item()),
-            "status_ok": bool((res["status"] == 0).all())}))
+            "status_ok": bool((res["status"] == 0).all()), "parity": parity}))
     if world > 1:
         dist.destroy_process_group()
 
