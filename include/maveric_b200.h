@@ -176,7 +176,9 @@ typedef struct {
   int   sample_iters;       /* GN iterations on the minimal sample */
   int   refine_iters;       /* GN iterations over all correspondences (gated) */
   float gate_sq;            /* squared-pixel inlier gate */
-  float min_depth;          /* cheirality guard on the camera-frame z */
+  float min_depth;          /* cheirality guard on the camera-frame z: a correspondence counts only
+                               where min_depth < z < 1e30.  At least FLT_MIN (a smaller value or
+                               NaN is MV_ERR_BAD_ARG): the GPU reciprocal flushes a subnormal z to 0 */
   float damping;            /* relative Levenberg damping added to diag(JtJ) */
   uint64_t seed;            /* counter-based sampling: splitmix64(seed, pair, h, i) */
   int   lanes_per_hypothesis; /* threads cooperating on one hypothesis: 1 (one thread each) or

@@ -630,7 +630,7 @@ static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, 
   if (m.radius < 0) return refuse("match.radius must be >= 0");
   if (!mv_pnp_params_ok(&p->pnp, m.max_matches))
     return refuse("max_matches <= 65535, pnp.hypotheses in [1,65536], pnp.sample_size in [1,255], "
-                  "pnp.lanes_per_hypothesis 1 or 32");
+                  "pnp.lanes_per_hypothesis 1 or 32, pnp.min_depth >= FLT_MIN");
   if (n_frames > 65535)
     return refuse("at most 65535 frames per call (grid y dimension); mv_track_sequence_host chunks longer sequences");
   if (m.use_tensor_cores != 0 && m.use_tensor_cores != 2 && !mv_match_tc_feasible(&m, n_frames, n_frames - 1, p->top_n))

@@ -941,7 +941,7 @@ void orc_pnp_gn(const orc_pnp_cfg* c, int pair_index, int n, int stride, const f
   int best_h = -1, best_cnt = -1;
   float best_cost = 0, best_pose[7];
   memcpy(best_pose, p0, sizeof(best_pose));
-  int sample[64];
+  int sample[255];   /* mv_pnp_params_ok (pnp_gn.cu) accepts sample_size up to 255 */
 
   for (int h = 0; h < c->hypotheses && n > 0; h++) {
     float q[4] = {p0[0], p0[1], p0[2], p0[3]}, t[3] = {p0[4], p0[5], p0[6]};

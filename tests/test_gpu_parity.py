@@ -305,9 +305,13 @@ def _oracle_pnp(oracle, cfg, corr, n, want_hyp=True):
 
 # H = 288 spans CTAs with a partial last one in both CTA sizes: 128 + 128 + 32 (MV_PNP_GPW=1) and 256 + 32 (=2).
 # n above 4096 walks the streaming kernel's staging chunks past 8 x 512; 16384 is BASELINE configs[4]'s match cap.
+# The lengths around 32 (a warp), 480 (the two-phase kernel's limit), 512 and 1024 (staging chunks) sit on either side
+# of a kernel boundary.
 @pytest.mark.parametrize("lanes,sample_size", _pnp_lane_forms())
 @pytest.mark.parametrize("n,stride", [(1000, 1024), (37, 64), (330, 1024), (480, 512), (1500, 1536), (2049, 2304), (8, 8),
-                                      (4100, 4608), (6900, 16384), (16384, 16384)])
+                                      (4100, 4608), (6900, 16384), (16384, 16384),
+                                      (1, 1), (31, 32), (32, 32), (33, 64), (479, 480), (481, 512), (511, 512),
+                                      (512, 512), (513, 1024), (1023, 1024), (1024, 1024), (1025, 1536)])
 def test_pnp_gn_vs_oracle(tracker, tk, oracle, synth, monkeypatch, lanes, sample_size, n, stride):
     import torch
     H, P = 288, 3
@@ -382,14 +386,26 @@ def test_pnp_gn_empty_and_init(tracker, tk, oracle):
 
 
 # ------------------------------------------------------------------ whole path
-@pytest.mark.parametrize("rows,cols,N,M,mv,H", [(24, 80, 100, 150, 1000, 64), (47, 155, 1000, 1024, 8192, 64)])
-def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, rows, cols, N, M, mv, H):
+# A camera with fx != fy and cx, cy off the KITTI values, with K3's gate, damping, iteration counts and sample size
+# away from their defaults: the back-projection (build_corr_kernel) and K3 both take the camera from the parameters.
+CAMERA_PNP = dict(fx=520.0, fy=910.0, cx=300.5, cy=260.25, gate_sq=16.0, damping=1e-3, sample_iters=3, refine_iters=6,
+                  sample_size=9)
+
+
+@pytest.mark.parametrize("rows,cols,N,M,mv,H,pnp", [
+    pytest.param(24, 80, 100, 150, 1000, 64, {}, id="24-80-100-150-1000-64"),
+    pytest.param(47, 155, 1000, 1024, 8192, 64, {}, id="47-155-1000-1024-8192-64"),
+    pytest.param(47, 155, 1000, 1024, 8192, 288, CAMERA_PNP, id="camera"),
+])
+def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, rows, cols, N, M, mv, H, pnp):
     import torch
     n_frames, seed = 4, 13
     off = synth.default_offsets(n_frames, seed)
     semi, desc, depth = tracker.synth_frames(seed, rows, cols, 0, off)
     scale = torch.full((n_frames,), float(synth.SEMI_SCALE), device=tracker.device)
     p = tk.track_params(rows, cols, top_n=N, max_valid=mv, max_matches=M, hypotheses=H)
+    for k, v in pnp.items():
+        setattr(p.pnp, k, v)
     res = tk.results_to_numpy(tracker.track_sequence(p, semi, scale, desc, depth))
     hs, hd, hz = semi.cpu().numpy(), desc.cpu().numpy(), depth.cpu().numpy()
     # same through host buffers (the e2e entry point)
@@ -402,16 +418,18 @@ def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, rows, cols, N, M, 
     finally:
         del os.environ["MV_HOST_CHUNK_PAIRS"]
     assert res_c.tobytes() == res.tobytes()
-    cfg = orc.TrackCfg(orc.MatchCfg(rows, cols, 4, 4, 4, M, 0.9, 0.2), orc.pnp_cfg(hypotheses=H, seed=0, lanes=1),
+    cfg = orc.TrackCfg(orc.MatchCfg(rows, cols, 4, 4, 4, M, 0.9, 0.2), orc.pnp_cfg(hypotheses=H, seed=0, lanes=1, **pnp),
                        N, mv, 10, 1.1, float(synth.SEMI_SCALE))
     for pi in range(n_frames - 1):
         ref = oracle.track_pair(cfg, pi, hs[pi], hd[pi], hz[pi], hs[pi + 1], hd[pi + 1])
         got = res[pi]
         assert got["status"] == 0 and got["num_matches"] == ref.num_matches > 0
         assert got["ransac_inliers"] == ref.ransac_inliers
-        assert got["pnp_inliers"] == ref.pnp_inliers
-        assert rot_angle(got["q"], np.array(list(ref.q))) < 1e-5
-        assert np.linalg.norm(got["t"] - np.array(list(ref.t))) <= 1e-5 * max(1.0, np.linalg.norm(list(ref.t)))
+        # every stage of the path is bit-exact, K3's pose and stats included
+        assert got["pnp_inliers"] == ref.pnp_inliers > 0 and got["best_hypothesis"] == ref.best_h
+        assert (bits(got["pnp_cost"]) == bits(np.float32(ref.pnp_cost))).all(), (pi, got["pnp_cost"], ref.pnp_cost)
+        assert (bits(got["q"]) == bits(np.array(list(ref.q), np.float32))).all(), (pi, got["q"], list(ref.q))
+        assert (bits(got["t"]) == bits(np.array(list(ref.t), np.float32))).all(), (pi, got["t"], list(ref.t))
 
 
 def test_gpu_pose_agrees_with_cv2_on_bench_pairs(tracker, tk, synth):

@@ -30,6 +30,9 @@ from landmark_reference import landmark_reference, track_cfg
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 f32 = np.float32
+# fx != fy, cx and cy off the KITTI values, K3's gate, damping, iteration counts and sample size off their defaults
+CAMERA_PNP = dict(fx=520.0, fy=910.0, cx=300.5, cy=260.25, gate_sq=16.0, damping=1e-3, sample_iters=3, refine_iters=6,
+                  sample_size=9)
 
 
 def _ref_vocab():
@@ -296,6 +299,21 @@ class _References:
                      rec=a["rec"][8:], nl=a["nl"][8:])
             assert np.unique(head[2]["word_id"]).size > 100
             return c
+        if name == "camera":   # case "scales" with another camera and K3 away from its defaults (only p.pnp changed)
+            a = self("scales")
+            c = dict(a)
+            c["p"] = copy.copy(a["p"])
+            c["p"].pnp = copy.copy(a["p"].pnp)
+            for k, v in CAMERA_PNP.items():
+                setattr(c["p"].pnp, k, v)
+            rec, nl, table = landmark_reference(o, o.bow_vocab(*c["vocab"]), c["p"], *c["frames"], table=c["entry"],
+                                                first_frame=c["first"], n_words=c["n_words"])
+            c.update(rec=rec, nl=nl, table=table)
+            _assert_case_reaches(name, c)
+            # the back-projected landmarks and the poses are the camera's own
+            assert table.tobytes() != a["table"].tobytes()
+            assert (rec["q"] != a["rec"]["q"]).any(axis=1).all()
+            return c
         c = _case_inputs(name, self.synth)
         rec, nl, table = landmark_reference(o, o.bow_vocab(*c["vocab"]), c["p"], *c["frames"], table=c["entry"],
                                             first_frame=c["first"], n_words=c["n_words"])
@@ -309,8 +327,10 @@ def _assert_case_reaches(name, c):
     rec, nl = c["rec"], c["nl"]
     nm = rec["num_matches"]
     assert (rec["pad"] == 0).all()
-    if name.startswith("scales"):
+    if name.startswith("scales") or name == "camera":
         assert (nm > 200).all() and (nl > 0).all()
+        if name == "camera":
+            assert (rec["pnp_inliers"] > 0).all()
     elif name == "degenerate":
         assert (rec["status"] == np.where(np.isin(np.arange(11), (5, 6)), 4, 0)).all()
         assert (nm[[1, 2, 3, 5, 8, 9]] == 0).all() and (nm[[0, 4, 6, 7, 10]] > 0).all()
@@ -442,7 +462,7 @@ ALL_ENTRIES = ("device", "host", "host:3", "host:pageable", "blocks:0", "blocks:
                "sharded", "host_sharded")
 SOME_ENTRIES = ("device", "host:3", "blocks:8")
 ENTRY_CASES = [(c, e) for c in ("scales", "scales_tc0", "degenerate") for e in ALL_ENTRIES] + \
-              [(c, e) for c in ("odd", "vocab60", "vocab200", "resume") for e in SOME_ENTRIES]
+              [(c, e) for c in ("odd", "vocab60", "vocab200", "resume", "camera") for e in SOME_ENTRIES]
 
 
 @pytest.mark.gpu
