@@ -1258,11 +1258,11 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     // An SM's L1/shared split is per-SM state: a kernel that asks for no shared memory
     // configures "all L1", and the PnP CTAs (5 x 37 KB shared) then cannot join that SM until
     // it drains.  Ask for the max-shared carveout so both kernels agree on the split.
-    static bool carveout_set = false;
-    if (!carveout_set) {
+    // The attribute belongs to the device: each context sets it on its own, so every GPU of the process gets it.
+    if (!c->gather_carveout_set) {
       cudaFuncSetAttribute(gather_rows_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                            cudaSharedmemCarveoutMaxShared);
-      carveout_set = true;
+      c->gather_carveout_set = true;
     }
     gather_rows_kernel<<<c->sm_count, 32, 0, gs>>>((long long)nf * cells, w[b].flags,
                                                    hd_desc + (size_t)p0 * cells * 256, (int8_t*)bd[b],

@@ -473,8 +473,12 @@ extern "C" mv_status mv_lba_schur_batch(mv_ctx* ctx, int n_windows, int n_ldmks,
   const int PD = 6 * n_poses, SH = PD + 1, LD = 3 * chunk, nf = chunk * n_poses;
   const size_t smem = sizeof(float) * ((size_t)SH * SH + (size_t)LD * LD + 2 * (size_t)SH * LD + (size_t)nf * 120);
   if (smem > 200 * 1024) MV_BAD_ARG(ctx, "mv_lba_schur_batch: window too large for shared memory");
-  if (smem > 48 * 1024)
-    MV_CUDA(ctx, cudaFuncSetAttribute(lba_schur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // The limit is shared by every mv_ctx on the device (see match_tc.cu): set once per context to the most this call
+  // admits, never to this call's own size.
+  if (smem > 48 * 1024 && !ctx->lba_schur_smem_attr_set) {
+    MV_CUDA(ctx, cudaFuncSetAttribute(lba_schur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    ctx->lba_schur_smem_attr_set = true;
+  }
   mv_prof_scope ps(ctx, "lba");
   const bool generic = getenv("MV_LBA_GENERIC") && atoi(getenv("MV_LBA_GENERIC"));   // A/B knob
   if (n_poses == kP8 && chunk == kC4 && !generic)
@@ -492,8 +496,12 @@ extern "C" mv_status mv_lba_solve_batch(mv_ctx* ctx, int n_windows, int n_poses,
   if (n_poses > 16) MV_BAD_ARG(ctx, "mv_lba_solve_batch: n_poses <= 16");
   const int n = 6 * n_poses;
   const size_t smem = sizeof(float) * (size_t)kSolveWarps * n * (n + 1);
-  if (smem > 48 * 1024)
-    MV_CUDA(ctx, cudaFuncSetAttribute(lba_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // as in mv_lba_schur_batch: the bound of n_poses = 16, once per context
+  if (smem > 48 * 1024 && !ctx->lba_solve_smem_attr_set) {
+    MV_CUDA(ctx, cudaFuncSetAttribute(lba_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)(sizeof(float) * kSolveWarps * 96 * 97)));
+    ctx->lba_solve_smem_attr_set = true;
+  }
   mv_prof_scope ps(ctx, "lba_solve");
   lba_solve_kernel<<<(n_windows + kSolveWarps - 1) / kSolveWarps, 32 * kSolveWarps, smem, ctx->stream>>>(
       n_windows, n_poses, damping, d_C, d_delta, d_ok);

@@ -667,10 +667,16 @@ static void tc_geom(const mv_match_params* p, int n_pairs, int top_n, TcGeom* g)
   g->prob_lt = mv_round_up(p->min_prob0);
 }
 
-static size_t tc_smem(const TcGeom& g) {
+static constexpr size_t tc_smem_of(int ystride) {
   return 1024 + (size_t)kBStages * kBStageBytes + (size_t)kAStages * (kAStageBytes + kRowBytes) +
-         (size_t)kBStages * 32u * g.ystride;
+         (size_t)kBStages * 32u * ystride;
 }
+static size_t tc_smem(const TcGeom& g) { return tc_smem_of(g.ystride); }
+// The most any launch needs, 198 400 B: mv_match_tc_feasible takes at most 256 rows, so ystride <= 260.  The
+// kernel's static shared memory (its mbarriers) counts against the same 227 KB a block may opt in to, so the
+// limit cannot be 227 KB itself.
+constexpr size_t kTcSmemMax = tc_smem_of((256 + 1 + 3) & ~3);
+static_assert(kTcSmemMax + 1024 <= 227 * 1024, "the largest matcher launch must fit beside the static shared memory");
 
 }  // namespace
 
@@ -755,7 +761,13 @@ mv_status mv_match_tc_launch(mv_ctx* ctx, const mv_match_params* p, int n_frames
   {
     mv_prof_scope p3(ctx, "match_gemm");
     const size_t smem = tc_smem(g);
-    MV_CUDA(ctx, cudaFuncSetAttribute(match_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // The limit is an attribute of the kernel in the device's primary context, which every mv_ctx on that device
+    // shares: set to this call's size, it could drop under the size another thread's context is about to launch
+    // with.  So every context sets the same bound, the most any launch needs, once.
+    if (!ctx->tc_smem_attr_set) {
+      MV_CUDA(ctx, cudaFuncSetAttribute(match_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemMax));
+      ctx->tc_smem_attr_set = true;
+    }
     const int grid = g.n_items < ctx->sm_count ? g.n_items : ctx->sm_count;
     match_tc_kernel<<<grid, kThreads, smem, ctx->stream>>>(tmap_a, tmap_b, g, d_f0, (const int4*)rinfo,
                                                           (const uint32_t*)cytab, (const int4*)spans, d_best_rank,

@@ -38,6 +38,10 @@ struct mv_ctx {
   int match_items = 0;                  // tiles of the last tensor-core matcher launch (mv_ctx_match_work)
   int bow_n_base = 0, bow_wpb = 0;      // vocabulary on the device (mv_bow_set_vocabulary)
   bool bow_smem_attr_set = false;       // the word-assignment kernel's shared-memory limit is set (bow.cu)
+  bool tc_smem_attr_set = false;        // the same for the tensor-core matcher (match_tc.cu)
+  bool lba_schur_smem_attr_set = false; // and for the generic Schur and the solve kernels (lba.cu)
+  bool lba_solve_smem_attr_set = false;
+  bool gather_carveout_set = false;     // the row gather's shared-memory carveout is set (api.cu)
   int lm_words = 0;                     // size the landmark scratch was initialised for
   std::map<std::string, mv_prof_slot> prof;
   std::vector<mv_pending_event> pending;

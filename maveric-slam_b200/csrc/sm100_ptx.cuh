@@ -213,14 +213,16 @@ typedef CUresult (*mv_tmap_encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint3
                                       const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
                                       CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
                                       CUtensorMapFloatOOBfill);
+// Looked up on first use.  The initialiser of a function-local static is thread-safe, so contexts used from
+// several threads at once may call this concurrently.
 static inline mv_tmap_encode_fn mv_get_tmap_encode() {
-  static mv_tmap_encode_fn fn = nullptr;
-  if (!fn) {
+  static const mv_tmap_encode_fn fn = []() -> mv_tmap_encode_fn {
     void* p = nullptr;
     cudaDriverEntryPointQueryResult q;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
         q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<mv_tmap_encode_fn>(p);
-  }
+      return reinterpret_cast<mv_tmap_encode_fn>(p);
+    return nullptr;
+  }();
   return fn;
 }

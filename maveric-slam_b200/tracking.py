@@ -51,6 +51,8 @@ _default_ctx: _lib.Context | None = None
 
 
 def default_context() -> _lib.Context:
+    """The context of the single-pair functions called without one.  It is one context for the whole process and
+    not safe to share across threads: a thread of its own passes a :class:`lib.Context` of its own as ``ctx``."""
     global _default_ctx
     if _default_ctx is None:
         _default_ctx = _lib.Context(0)
