@@ -13,7 +13,6 @@
 #include <stdlib.h>
 
 #include <algorithm>
-#include <functional>
 #include <mutex>
 
 #include "../../include/maveric_slam_compat.h"
@@ -593,12 +592,12 @@ __global__ void pack_results_kernel(int n_pairs, const float* __restrict__ pose,
   out[p] = r;
 }
 
-// Landmark mode of the sequence calls: the 3-D side of pair p's correspondences comes from the caller's table right
-// after step p instead of depth.  seq_step reads the descriptor of its batch, with device pointers; the host pipeline
-// keeps one for the whole call, with the caller's host desc_scale / n_with_landmark, and derives each chunk's.
+// Landmark mode of one batch of frames: the 3-D side of pair p's correspondences comes from the caller's table right
+// after step p instead of depth.  Device pointers of that batch only.
 struct SeqLandmarks {
-  int first_frame, n_words;
-  mv_landmark* table;
+  int first_frame;            // the table's frame number of the batch's frame 0
+  int n_words;
+  mv_landmark* table;         // NULL where the batch steps no table (a block's prepare and solve)
   const float* desc_scale;    // one per frame
   int32_t* n_with_landmark;   // one per pair, nullable
 };
@@ -613,16 +612,20 @@ struct SeqScratch {
   float *coords_in, *coords_out;   // landmark mode: [n_frames - 1][top_n][3]
 };
 
-// Every refusal seq_detect and seq_step could make from the arguments, so that a sequence call refuses before it
-// allocates or enqueues anything.  n_frames: the largest batch the call runs (the whole sequence for the
+// "bad argument: fn: why", or "bad argument: fn" without a reason
+static mv_status bad_arg(mv_ctx* c, const char* fn, const char* why) {
+  snprintf(c->err, sizeof(c->err), "bad argument: %s%s%s", fn, why ? ": " : "", why ? why : "");
+  return MV_ERR_BAD_ARG;
+}
+
+// Every refusal seq_detect and the parts of a batch could make from the arguments, so that a sequence call refuses
+// before it allocates or enqueues anything.  n_frames: the largest batch the call runs (the whole sequence for the
 // device-resident calls, the largest chunk for the host ones); d_desc: the caller's descriptors, or NULL when they
-// are staged into scratch.
+// are staged into scratch; landmarks: the batches assign words of an n_words vocabulary (the calls that step a table
+// refuse a NULL one themselves).
 static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                           const SeqLandmarks* lm, bool with_table = true) {
-  auto refuse = [&](const char* why) {
-    snprintf(c->err, sizeof(c->err), "bad argument: %s: %s", fn, why);
-    return MV_ERR_BAD_ARG;
-  };
+                           bool landmarks, int n_words = 0) {
+  auto refuse = [&](const char* why) { return bad_arg(c, fn, why); };
   const mv_match_params& m = p->match;
   if (m.rows <= 0 || m.cols <= 0 || p->top_n <= 0 || p->max_valid <= 0 || m.max_matches <= 0 ||
       (long long)m.rows * m.cols > 0x7fffffffLL)
@@ -636,11 +639,10 @@ static mv_status seq_check(mv_ctx* c, const char* fn, const mv_track_params* p, 
   if (m.use_tensor_cores != 0 && m.use_tensor_cores != 2 && !mv_match_tc_feasible(&m, n_frames, n_frames - 1, p->top_n))
     return refuse("use_tensor_cores = 1 on a shape the tensor-core matcher does not take (2 picks the matcher)");
   if (d_desc && (reinterpret_cast<uintptr_t>(d_desc) & 15)) return refuse("d_desc must be 16-byte aligned");
-  if (!lm) return MV_OK;
+  if (!landmarks) return MV_OK;
   if (c->bow_n_base <= 0) return refuse("no vocabulary (mv_bow_set_vocabulary first)");
   if (!mv_bow_vocab_fits(c)) return refuse("vocabulary larger than an SM's shared memory");
-  if (lm->n_words <= 0) return refuse("n_words must be positive");
-  if (with_table && !lm->table) return refuse("NULL landmark table");
+  if (n_words <= 0) return refuse("n_words must be positive");
   if ((long long)(n_frames - 1) * p->top_n > 0x7fffffffLL) return refuse("(n_frames - 1) * top_n must be below 2^31");
   return MV_OK;
 }
@@ -703,13 +705,10 @@ static mv_status seq_detect(mv_ctx* c, const mv_track_params* p, int n_frames, c
   return mv_top_n_batch(c, n_frames, cells, p->top_n, p->max_valid, w.idx, w.prob, w.qp, w.qi, w.qpr, w.qc, w.ov);
 }
 
-// Called by seq_step once the matcher ("match_end") and the correspondences ("corr_end") are enqueued.
-using SeqStageFn = std::function<mv_status(const char* stage)>;
-
-// The rest of a batch whose detector has run, in three parts that the landmark block calls apart (prepare: words,
-// speculation, matcher; step_table: the table; solve).  With `lm`, the word assignment of frames 0..n-2 with their
-// query keypoints back-projected in the same launch (none where w.coords_in is NULL).  n_word_frames: the frames
-// that get words, 0 .. n_word_frames-1 (all but the last of a batch; every frame of a warm-up chunk).
+// The rest of a batch whose detector has run, in the parts seq_step chains; the host pipeline and the landmark block
+// call them apart.  seq_words: the word assignment of frames 0..n_word_frames-1 (all but the last of a batch; every
+// frame of a warm-up chunk) with their query keypoints back-projected in the same launch (none where w.coords_in is
+// NULL).
 static mv_status seq_words(mv_ctx* c, const mv_track_params* p, int n_word_frames, const int8_t* d_desc,
                            const float* d_depth, const SeqScratch& w, const SeqLandmarks* lm) {
   MvBackProject bp;
@@ -720,41 +719,38 @@ static mv_status seq_words(mv_ctx* c, const mv_track_params* p, int n_word_frame
                             w.qc, w.word, nullptr, bp);
 }
 
-// Match and RANSAC-E.
 static mv_status seq_match(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                           const SeqScratch& w, const SeqStageFn& on_stage) {
-  const int n_pairs = n_frames - 1;
-  mv_status st;
-  if ((st = mv_match_batch(c, &p->match, n_frames, n_pairs, p->top_n, nullptr, nullptr, d_desc, w.idx, w.prob, w.qp,
-                           w.qi, w.qc, w.mp, w.mc, w.mcell, nullptr, nullptr)))
-    return st;
-  if (on_stage && (st = on_stage("match_end"))) return st;
-  if (p->ransac_iterations > 0)
-    return mv_ransac_identity_batch(c, n_pairs, p->match.max_matches, w.mp, w.mc, p->ransac_iterations,
-                                    p->ransac_threshold, w.rin, nullptr, nullptr);
-  return MV_OK;
+                           const SeqScratch& w) {
+  return mv_match_batch(c, &p->match, n_frames, n_frames - 1, p->top_n, nullptr, nullptr, d_desc, w.idx, w.prob, w.qp,
+                        w.qi, w.qc, w.mp, w.mc, w.mcell, nullptr, nullptr);
 }
 
-// Correspondences (with `lm`: from w.coords_out, each query's record right after its frame's step), K3, records.
-static mv_status seq_solve(mv_ctx* c, const mv_track_params* p, int n_frames, const float* d_depth,
-                           const SeqScratch& w, mv_pair_result* d_results, int first_pair, const SeqLandmarks* lm,
-                           const SeqStageFn& on_stage) {
-  const int cells = p->match.rows * p->match.cols;
+static mv_status seq_ransac(mv_ctx* c, const mv_track_params* p, int n_frames, const SeqScratch& w) {
+  if (p->ransac_iterations <= 0) return MV_OK;
+  return mv_ransac_identity_batch(c, n_frames - 1, p->match.max_matches, w.mp, w.mc, p->ransac_iterations,
+                                  p->ransac_threshold, w.rin, nullptr, nullptr);
+}
+
+// Correspondences: with `lm` from w.coords_out, each query's record right after its frame's step; else from depth.
+static mv_status seq_corr(mv_ctx* c, const mv_track_params* p, int n_frames, const float* d_depth,
+                          const SeqScratch& w, const SeqLandmarks* lm) {
+  const int n_pairs = n_frames - 1, M = p->match.max_matches;
+  if (lm)
+    return mv_build_corr_landmarks_seq(c, n_pairs, p->top_n, M, lm->n_words, w.qp, w.qc, w.word, w.coords_out, w.mp,
+                                       w.mc, w.mcell, w.corr, lm->n_with_landmark);
+  return mv_build_corr_batch(c, n_pairs, p->match.rows * p->match.cols, p->match.rows, M, nullptr, d_depth, p->pnp.fx,
+                             p->pnp.fy, p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr);
+}
+
+// K3 and the records; first_pair: the batch's first pair in the call (the PnP sampler is keyed on it).
+static mv_status seq_pose(mv_ctx* c, const mv_track_params* p, int n_frames, const SeqScratch& w,
+                          mv_pair_result* d_results, int first_pair) {
   const int n_pairs = n_frames - 1;
-  const int N = p->top_n, M = p->match.max_matches;
-  mv_status st;
-  if (lm) {
-    if ((st = mv_build_corr_landmarks_seq(c, n_pairs, N, M, lm->n_words, w.qp, w.qc, w.word, w.coords_out, w.mp,
-                                          w.mc, w.mcell, w.corr, lm->n_with_landmark)))
-      return st;
-  } else if ((st = mv_build_corr_batch(c, n_pairs, cells, p->match.rows, M, nullptr, d_depth, p->pnp.fx, p->pnp.fy,
-                                       p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr))) {
-    return st;
-  }
-  if (on_stage && (st = on_stage("corr_end"))) return st;
   mv_pnp_params pnp = p->pnp;
   pnp.first_pair += first_pair;
-  if ((st = mv_pnp_gn_batch(c, &pnp, n_pairs, M, w.corr, w.mc, nullptr, w.pose, w.stats, nullptr))) return st;
+  mv_status st;
+  if ((st = mv_pnp_gn_batch(c, &pnp, n_pairs, p->match.max_matches, w.corr, w.mc, nullptr, w.pose, w.stats, nullptr)))
+    return st;
   pack_results_kernel<<<(n_pairs + 127) / 128, 128, 0, c->stream>>>(
       n_pairs, w.pose, w.stats, w.mc, p->ransac_iterations > 0 ? w.rin : nullptr, w.ov, d_results);
   MV_CHECK_LAUNCH(c);
@@ -765,17 +761,17 @@ static mv_status seq_solve(mv_ctx* c, const mv_track_params* p, int n_frames, co
 // then match / RANSAC-E / correspondences / K3 / pack.  Only descriptor rows of candidate / query cells are read,
 // and depth only at matched frame-0 cells (or, with `lm`, at query cells).
 static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_desc,
-                          const float* d_depth, const SeqScratch& w, mv_pair_result* d_results, int first_pair,
-                          const SeqLandmarks* lm, const SeqStageFn& on_stage = nullptr) {
+                          const float* d_depth, const SeqScratch& w, mv_pair_result* d_results,
+                          const SeqLandmarks* lm) {
   mv_status st;
-  if (lm) {
-    if ((st = seq_words(c, p, n_frames - 1, d_desc, d_depth, w, lm))) return st;
-    if ((st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_frames - 1, p->top_n, w.word,
-                                         w.qc, w.coords_in, w.coords_out)))
-      return st;
-  }
-  if ((st = seq_match(c, p, n_frames, d_desc, w, on_stage))) return st;
-  return seq_solve(c, p, n_frames, d_depth, w, d_results, first_pair, lm, on_stage);
+  if (lm && ((st = seq_words(c, p, n_frames - 1, d_desc, d_depth, w, lm)) ||
+             (st = mv_landmarks_sequence_impl(c, lm->n_words, lm->table, lm->first_frame, n_frames - 1, p->top_n,
+                                              w.word, w.qc, w.coords_in, w.coords_out))))
+    return st;
+  if ((st = seq_match(c, p, n_frames, d_desc, w)) || (st = seq_ransac(c, p, n_frames, w)) ||
+      (st = seq_corr(c, p, n_frames, d_depth, w, lm)))
+    return st;
+  return seq_pose(c, p, n_frames, w, d_results, 0);
 }
 
 extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_semi,
@@ -786,10 +782,10 @@ extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int 
     MV_BAD_ARG(c, "mv_track_sequence");
   SeqScratch w;
   mv_status st;
-  if ((st = seq_check(c, "mv_track_sequence", p, n_frames, d_desc, nullptr)) ||
+  if ((st = seq_check(c, "mv_track_sequence", p, n_frames, d_desc, false)) ||
       (st = seq_scratch(c, p, n_frames, "seq", false, &w)) || (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
     return st;
-  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, 0, nullptr);
+  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, nullptr);
 }
 
 // Pair p = frames (p, p+1) with the 3-D side from the landmark table right after step p: detector, then seq_step in
@@ -805,11 +801,48 @@ extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_param
   const SeqLandmarks lm = {first_frame, n_words, d_table, d_desc_scale, d_n_with_landmark};
   SeqScratch w;
   mv_status st;
-  if ((st = seq_check(c, "mv_track_sequence_landmarks", p, n_frames, d_desc, &lm)) ||
-      (st = seq_scratch(c, p, n_frames, "lmseq", true, &w)) ||
-      (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
+  if ((st = seq_check(c, "mv_track_sequence_landmarks", p, n_frames, d_desc, true, n_words))) return st;
+  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks: NULL landmark table");
+  if ((st = seq_scratch(c, p, n_frames, "lmseq", true, &w)) || (st = seq_detect(c, p, n_frames, d_semi, d_semi_scale, w)))
     return st;
-  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, 0, &lm);
+  return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, &lm);
+}
+
+// ---- chunks of the host staging pipeline (track_sequence_host_impl below)
+// A call's host frames in chunks of `pairs` pairs: first the n_warm warm-up frames of a block being prepared, at most
+// `pairs` frames per chunk and no halo, then the n_pairs pairs, each chunk sharing its first frame with the last
+// frame of the chunk before.
+struct HostPlan {
+  int pairs, n_warm_chunks, n_chunks, n_warm, n_pairs;
+  bool warm(int k) const { return k < n_warm_chunks; }                                // words only, no matcher
+  int first_pair(int k) const { return (k - n_warm_chunks) * pairs; }                 // of a pairs' chunk
+  int frame0(int k) const { return warm(k) ? k * pairs : n_warm + first_pair(k); }   // in the host buffers
+  int frames(int k) const {
+    return warm(k) ? std::min(pairs, n_warm - k * pairs) : std::min(pairs, n_pairs - first_pair(k)) + 1;
+  }
+};
+
+static HostPlan host_plan(const mv_ctx* c, const mv_track_params* p, int n_warm, int n_pairs, bool landmarks) {
+  // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see PnpResidencyCap); the
+  // one-thread-per-hypothesis kernel covers 256 hypotheses per CTA, the multi-lane forms 16
+  const int per_cta = p->pnp.lanes_per_hypothesis == 1 ? 256 : 16;
+  const int pnp_ctas_per_pair = (p->pnp.hypotheses + per_cta - 1) / per_cta;
+  int chunk_pairs = 2 * (5 * c->sm_count) / (pnp_ctas_per_pair > 0 ? pnp_ctas_per_pair : 1);
+  if (chunk_pairs < 8) chunk_pairs = 8;
+  // short sequences (a rank's shard of a multi-GPU run): at least ~8 chunks, so that the staging
+  // pipeline has something to overlap with instead of one long fill and drain
+  if (chunk_pairs > (n_pairs + 7) / 8) chunk_pairs = (n_pairs + 7) / 8 > 32 ? (n_pairs + 7) / 8 : 32;
+  if (const char* e = getenv("MV_HOST_CHUNK_PAIRS")) {  // test hook: force small chunks
+    const int v = atoi(e);
+    if (v > 0) chunk_pairs = v;
+  }
+  if (chunk_pairs > n_pairs) chunk_pairs = n_pairs;
+  if (landmarks) {  // one table step per pair: mv_landmarks_sequence's limits on one call (top_n > 0 is checked)
+    const int most = (int)std::min<long long>(65535, 0x7fffffffLL / std::max(p->top_n, 1));
+    if (chunk_pairs > most) chunk_pairs = most;
+  }
+  const int n_warm_chunks = (n_warm + chunk_pairs - 1) / chunk_pairs;
+  return {chunk_pairs, n_warm_chunks, n_warm_chunks + (n_pairs + chunk_pairs - 1) / chunk_pairs, n_warm, n_pairs};
 }
 
 // ---- the landmark path split at the table (mv_track_landmarks_prepare / step_table / solve)
@@ -819,24 +852,12 @@ struct mv_lm_block {
   mv_ctx* ctx;
   mv_track_params p;
   int n_warm, n_frames, n_words;
+  int first_frame;   // the table's frame number of the block's first frame (after the warm-up)
   SeqScratch w, b;
   std::vector<void*> mem;
   mv_lm_spec* spec = nullptr;
   int phase = 0;   // 1 prepared, 2 table stepped, 3 solved
 };
-
-// k->b = the view of k->w at the block's first frame (coords_out aside: the speculation's)
-static void lm_block_view(mv_lm_block* k) {
-  const size_t W = k->n_warm, N = k->p.top_n, cells = (size_t)k->p.match.rows * k->p.match.cols;
-  SeqScratch& b = k->b;
-  b = k->w;
-  if (b.idx) {
-    b.idx += W * cells; b.prob += W * cells;
-    b.qi += W * N; b.qpr += W * N;
-  }
-  b.qp += W * N; b.qc += W; b.ov += W;
-  b.word += W * N; b.coords_in += 3 * W * N;
-}
 
 static void lm_block_free(mv_lm_block* k) {
   mv_device_guard guard(k->ctx->device);
@@ -845,47 +866,71 @@ static void lm_block_free(mv_lm_block* k) {
   delete k;
 }
 
+// Both prepare forms: checks the arguments (inputs: every input pointer is non-NULL), then allocates the block and
+// its scratch.  `plan`, the host form only: filled with the staging plan, whose chunks are checked too; that form
+// leaves the detector planes in the chunk buffers.  seq_check's tensor-core check over all n_warm + n_frames frames
+// also covers the matcher's n_frames: mv_match_tc_feasible only takes fewer shapes as the frames grow.
+static mv_status lm_block_new(mv_ctx* c, const char* fn, const mv_track_params* p, int n_warm, int n_frames,
+                              int first_frame, int n_words, bool inputs, const int8_t* d_desc, HostPlan* plan,
+                              mv_lm_block** out, mv_lm_block** block) {
+  if (!out) return bad_arg(c, fn, "NULL out");
+  *out = nullptr;
+  if (!p || n_frames < 2 || n_warm < 0 || !inputs) return bad_arg(c, fn, nullptr);
+  if ((long long)n_warm + n_frames > 65535) return bad_arg(c, fn, "at most 65535 frames in all");
+  const int T = n_warm + n_frames;
+  mv_status st;
+  if ((st = seq_check(c, fn, p, T, d_desc, true, n_words))) return st;
+  if (plan) {
+    *plan = host_plan(c, p, n_warm, n_frames - 1, true);
+    if ((st = seq_check(c, fn, p, plan->pairs + 1, nullptr, true, n_words))) return st;
+  }
+  mv_lm_block* k = new mv_lm_block{c, *p, n_warm, n_frames, n_words, first_frame};
+  if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem, !plan))) {
+    lm_block_free(k);
+    return st;
+  }
+  // k->b = the view of k->w at the block's first frame (coords_out aside: the speculation's)
+  const size_t W = n_warm, N = p->top_n, cells = (size_t)p->match.rows * p->match.cols;
+  SeqScratch& b = k->b = k->w;
+  if (b.idx) {
+    b.idx += W * cells; b.prob += W * cells;
+    b.qi += W * N; b.qpr += W * N;
+  }
+  b.qp += W * N; b.qc += W; b.ov += W;
+  b.word += W * N; b.coords_in += 3 * W * N;
+  *block = k;
+  return MV_OK;
+}
+
 extern "C" mv_status mv_track_landmarks_prepare(mv_ctx* c, const mv_track_params* p, int n_warm, int n_frames,
                                                 int first_frame, const int8_t* d_semi, const float* d_semi_scale,
                                                 const int8_t* d_desc, const float* d_desc_scale, const float* d_depth,
                                                 int n_words, mv_lm_block** out) {
   MV_ENTER(c);
-  if (!out) MV_BAD_ARG(c, "mv_track_landmarks_prepare: NULL out");
-  *out = nullptr;
-  if (!p || n_frames < 2 || n_warm < 0 || !d_semi || !d_semi_scale || !d_desc || !d_desc_scale || !d_depth)
-    MV_BAD_ARG(c, "mv_track_landmarks_prepare");
-  if ((long long)n_warm + n_frames > 65535) MV_BAD_ARG(c, "mv_track_landmarks_prepare: at most 65535 frames in all");
+  mv_lm_block* k;
+  mv_status st = lm_block_new(c, "mv_track_landmarks_prepare", p, n_warm, n_frames, first_frame, n_words,
+                              d_semi && d_semi_scale && d_desc && d_desc_scale && d_depth, d_desc, nullptr, out, &k);
+  if (st) return st;
   const int T = n_warm + n_frames;
   const SeqLandmarks lm = {first_frame - n_warm, n_words, nullptr, d_desc_scale, nullptr};
-  mv_status st;
-  if ((st = seq_check(c, "mv_track_landmarks_prepare", p, T, d_desc, &lm, false))) return st;
-  if (p->match.use_tensor_cores == 1 && !mv_match_tc_feasible(&p->match, n_frames, n_frames - 1, p->top_n))
-    MV_BAD_ARG(c, "mv_track_landmarks_prepare: use_tensor_cores = 1 on a shape the tensor-core matcher does not take");
-  const int cells = p->match.rows * p->match.cols, N = p->top_n;
-  mv_lm_block* k = new mv_lm_block();
-  k->ctx = c; k->p = *p; k->n_warm = n_warm; k->n_frames = n_frames; k->n_words = n_words;
-  auto fail = [&](mv_status e) { lm_block_free(k); return e; };
-  if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem)) || (st = seq_detect(c, p, T, d_semi, d_semi_scale, k->w)) ||
-      (st = seq_words(c, p, T - 1, d_desc, d_depth, k->w, &lm)))
-    return fail(st);
-  if ((st = mv_landmarks_speculate_impl(c, n_words, first_frame, n_warm, n_frames - 1, N, k->w.word, k->w.qc,
-                                        k->w.coords_in + 3 * (size_t)n_warm * N, &k->spec)))
-    return fail(st);
-  lm_block_view(k);
-  k->b.coords_out = mv_lm_spec_coords(k->spec);
-  if ((st = seq_match(c, p, n_frames, d_desc + (size_t)n_warm * cells * 256, k->b, nullptr))) return fail(st);
+  const int8_t* b_desc = d_desc + (size_t)n_warm * p->match.rows * p->match.cols * 256;
+  if ((st = seq_detect(c, p, T, d_semi, d_semi_scale, k->w)) || (st = seq_words(c, p, T - 1, d_desc, d_depth, k->w, &lm)) ||
+      (st = mv_landmarks_speculate_impl(c, n_words, first_frame, n_warm, n_frames - 1, p->top_n, k->w.word, k->w.qc,
+                                        k->b.coords_in, &k->spec)) ||
+      (st = seq_match(c, p, n_frames, b_desc, k->b)) || (st = seq_ransac(c, p, n_frames, k->b))) {
+    lm_block_free(k);
+    return st;
+  }
+  k->b.coords_out = mv_lm_spec_coords(k->spec);   // the matcher and RANSAC-E do not read it
   k->phase = 1;
   *out = k;
   return MV_OK;
 }
 
 static mv_status lm_block_check(mv_ctx* c, mv_lm_block* k, int phase, const char* fn) {
-  if (!k) { snprintf(c->err, sizeof(c->err), "bad argument: %s: NULL block", fn); return MV_ERR_BAD_ARG; }
-  if (k->ctx != c) { snprintf(c->err, sizeof(c->err), "bad argument: %s: block of another context", fn); return MV_ERR_BAD_ARG; }
-  if (k->phase != phase) {
-    snprintf(c->err, sizeof(c->err), "bad argument: %s: out of phase (prepare, step_table, solve, each once)", fn);
-    return MV_ERR_BAD_ARG;
-  }
+  if (!k) return bad_arg(c, fn, "NULL block");
+  if (k->ctx != c) return bad_arg(c, fn, "block of another context");
+  if (k->phase != phase) return bad_arg(c, fn, "out of phase (prepare, step_table, solve, each once)");
   return MV_OK;
 }
 
@@ -906,8 +951,9 @@ extern "C" mv_status mv_track_landmarks_solve(mv_ctx* c, mv_lm_block* k, mv_pair
   if ((st = lm_block_check(c, k, 2, "mv_track_landmarks_solve"))) return st;
   if (!d_results) MV_BAD_ARG(c, "mv_track_landmarks_solve: NULL results");
   k->phase = 3;
-  const SeqLandmarks lm = {0, k->n_words, nullptr, nullptr, d_n_with_landmark};
-  return seq_solve(c, &k->p, k->n_frames, nullptr, k->b, d_results, 0, &lm, nullptr);
+  const SeqLandmarks lm = {k->first_frame, k->n_words, nullptr, nullptr, d_n_with_landmark};
+  if ((st = seq_corr(c, &k->p, k->n_frames, nullptr, k->b, &lm))) return st;
+  return seq_pose(c, &k->p, k->n_frames, k->b, d_results, 0);
 }
 
 extern "C" void mv_track_landmarks_release(mv_lm_block* k) {
@@ -1031,53 +1077,30 @@ struct PnpResidencyCap {  // cap the PnP kernel's CTAs per SM for a scope
   ~PnpResidencyCap() { c->pnp_max_ctas_per_sm = saved; }
 };
 
-// Host inputs.  Chunks of frames are double-buffered: on the staging stream the logits are
-// copied and the detector runs, then descriptors arrive (selectively when the host buffers
-// are pinned, else as a plain copy); the compute stream runs seq_step on the previous chunk
-// meanwhile.  Consecutive chunks share one halo frame.  With `lm` (host desc_scale and
-// n_with_landmark) seq_step also steps the caller's landmark table over the chunk's frames but its
-// halo before matching; chunks run in order on that stream, so the table chains from chunk to chunk.
-// With `blk` (mv_track_landmarks_prepare_host; lm without a table) the host buffers start with blk->n_warm
-// warm-up frames, staged first in chunks of their own without a halo (logits and query rows; words only), and
-// each chunk of the block's n_frames runs the words and the matcher into the block's memory instead of seq_step;
-// the speculation follows the last chunk.  Returns once the host buffers are no longer read: that work may still
-// be queued on the compute stream.
-// Pairs per chunk of the host staging pipeline over n_pairs pairs.
-static int host_chunk_pairs(const mv_ctx* c, const mv_track_params* p, int n_pairs, bool landmarks) {
-  // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see below); the
-  // one-thread-per-hypothesis kernel covers 256 hypotheses per CTA, the multi-lane forms 16
-  const int per_cta = p->pnp.lanes_per_hypothesis == 1 ? 256 : 16;
-  const int pnp_ctas_per_pair = (p->pnp.hypotheses + per_cta - 1) / per_cta;
-  int chunk_pairs = 2 * (5 * c->sm_count) / (pnp_ctas_per_pair > 0 ? pnp_ctas_per_pair : 1);
-  if (chunk_pairs < 8) chunk_pairs = 8;
-  // short sequences (a rank's shard of a multi-GPU run): at least ~8 chunks, so that the staging
-  // pipeline has something to overlap with instead of one long fill and drain
-  if (chunk_pairs > (n_pairs + 7) / 8) chunk_pairs = (n_pairs + 7) / 8 > 32 ? (n_pairs + 7) / 8 : 32;
-  if (const char* e = getenv("MV_HOST_CHUNK_PAIRS")) {  // test hook: force small chunks
-    const int v = atoi(e);
-    if (v > 0) chunk_pairs = v;
-  }
-  if (chunk_pairs > n_pairs) chunk_pairs = n_pairs;
-  if (landmarks) {  // one table step per pair: mv_landmarks_sequence's limits on one call (top_n > 0 is checked)
-    const int most = (int)std::min<long long>(65535, 0x7fffffffLL / std::max(p->top_n, 1));
-    if (chunk_pairs > most) chunk_pairs = most;
-  }
-  return chunk_pairs;
-}
+// The call that stages host buffers through track_sequence_host_impl: mv_track_sequence_host,
+// mv_track_sequence_landmarks_host or mv_track_landmarks_prepare_host.
+enum class HostCall { depth, landmarks, prepare };
 
-static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_track_params* p, int n_frames,
+// Host inputs.  The chunks of `plan` are double-buffered: on the staging stream the logits are copied and the detector
+// runs, then descriptors arrive (selectively when the host buffers are pinned, else as a plain copy); the compute
+// stream runs the previous chunk's compute meanwhile.  Consecutive chunks share one halo frame.  HostCall::landmarks
+// also steps the caller's table over the chunk's frames but its halo before matching; chunks run in order on that
+// stream, so the table chains from chunk to chunk.  With HostCall::prepare the host buffers start with the block's
+// warm-up frames, staged first in chunks of their own without a halo (logits and query rows; words only), and each
+// chunk of the block's frames runs the words and the matcher into the block's memory; the speculation follows the
+// last chunk.  first_frame: the table's frame number of the first pair's frame.  Returns once the host buffers are no
+// longer read: a prepared block's work may still be queued on the compute stream.
+static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPlan& plan, const mv_track_params* p,
                                           const int8_t* h_semi, const float* h_semi_scale, const int8_t* h_desc,
-                                          const float* h_depth, mv_pair_result* h_results,
-                                          unsigned long long* h2d_bytes, unsigned long long* d2h_bytes,
-                                          const SeqLandmarks* lm, mv_lm_block* blk = nullptr) {
+                                          const float* h_desc_scale, const float* h_depth, int first_frame,
+                                          int n_words, mv_landmark* d_table, mv_pair_result* h_results,
+                                          int32_t* h_n_with_landmark, mv_lm_block* blk,
+                                          unsigned long long* h2d_bytes, unsigned long long* d2h_bytes) {
   const int cells = p->match.rows * p->match.cols;
-  const int n_pairs = n_frames - 1;
-  const int n_warm = blk ? blk->n_warm : 0;
-  const int chunk_pairs = host_chunk_pairs(c, p, n_pairs, lm != nullptr);
-  const int cf = chunk_pairs + 1;
+  const int n_pairs = plan.n_pairs, n_warm = plan.n_warm, cf = plan.pairs + 1;
   const int N = p->top_n;
+  const bool landmarks = call != HostCall::depth;
   mv_status st;
-  if ((st = seq_check(c, fn, p, cf, nullptr, lm, blk == nullptr))) return st;
 
   // zero-copy gather needs device-visible (pinned) descriptor and depth buffers
   bool gather = true;
@@ -1101,7 +1124,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
 
   constexpr int NB = 3;  // chunks in flight: staging DMA / row gather / compute
   void *bs[NB], *bd[NB], *bz[NB], *bsc[NB], *dres, *dmoved;
-  void *bdsc[NB], *dnwl = nullptr;   // landmark mode
+  void *bdsc[NB] = {}, *dnwl = nullptr;   // landmark mode
   SeqScratch w[NB];
   const size_t semi_pad = ((size_t)cf * cells * 65 + 255) & ~(size_t)255;
   for (int b = 0; b < NB; b++) {
@@ -1110,16 +1133,15 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     if ((st = mv_scratch(c, (n + ".desc").c_str(), (size_t)cf * cells * 256, &bd[b]))) return st;
     if ((st = mv_scratch(c, (n + ".depth").c_str(), sizeof(float) * (size_t)cf * cells, &bz[b]))) return st;
     if ((st = mv_scratch(c, (n + ".scale").c_str(), sizeof(float) * (size_t)cf, &bsc[b]))) return st;
-    if ((st = seq_scratch(c, p, cf, n.c_str(), lm != nullptr, &w[b]))) return st;
-    if (lm && (st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
+    if ((st = seq_scratch(c, p, cf, n.c_str(), landmarks, &w[b]))) return st;
+    if (landmarks && (st = mv_scratch(c, (n + ".dscale").c_str(), sizeof(float) * (size_t)cf, &bdsc[b]))) return st;
   }
-  if (lm && !blk) {
+  if (call == HostCall::landmarks) {
     // the table update's shared sort scratch, for the full chunk and the last one: growing it between
     // enqueues would free memory (cudaFree) while the three streams run
-    const int last_steps = n_pairs - (n_pairs - 1) / chunk_pairs * chunk_pairs;
-    if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, chunk_pairs, N))) return st;
-    if ((st = mv_landmarks_sequence_reserve(c, lm->n_words, last_steps, N))) return st;
-    if (lm->n_with_landmark &&
+    if ((st = mv_landmarks_sequence_reserve(c, n_words, plan.pairs, N))) return st;
+    if ((st = mv_landmarks_sequence_reserve(c, n_words, plan.frames(plan.n_chunks - 1) - 1, N))) return st;
+    if (h_n_with_landmark &&
         (st = mv_scratch(c, "host.n_with_landmark", sizeof(int32_t) * (size_t)n_pairs, &dnwl)))
       return st;
   }
@@ -1183,38 +1205,27 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   mark("start", 0, c->stream);
 
   unsigned long long up = 0;
-  // chunks 0 .. n_warm_chunks-1: warm-up frames, chunk_pairs at most, no halo; then the pairs' chunks
-  const int n_warm_chunks = (n_warm + chunk_pairs - 1) / chunk_pairs;
-  const int n_chunks = n_warm_chunks + (n_pairs + chunk_pairs - 1) / chunk_pairs;
-  auto warm = [&](int k) { return k < n_warm_chunks; };
-  auto chunk_first = [&](int k) { return (k - n_warm_chunks) * chunk_pairs; };   // first pair of a pairs' chunk
-  auto chunk_frame0 = [&](int k) { return warm(k) ? k * chunk_pairs : n_warm + chunk_first(k); };  // in the buffers
-  auto chunk_frames = [&](int k) {
-    if (warm(k)) return std::min(chunk_pairs, n_warm - k * chunk_pairs);
-    const int p0 = chunk_first(k);
-    return ((n_pairs - p0) < chunk_pairs ? (n_pairs - p0) : chunk_pairs) + 1;
-  };
   // The scratch of chunk k: its buffer set, but a block being prepared keeps what step_table and solve read at the
   // chunk's frames and pairs in its own memory.  The detector of chunk k+1 writes the halo frame's qp / qc / ov there
   // again before the compute of chunk k reads them: the same bytes (the same frame, the same kernels), in the same
   // stream order as the chunk-local copies of the host calls.
   auto chunk_scratch = [&](int k) {
     SeqScratch v = w[k % NB];
-    if (!blk) return v;
-    const size_t f0 = chunk_frame0(k), N = p->top_n, M = p->match.max_matches;
+    if (call != HostCall::prepare) return v;
+    const size_t f0 = plan.frame0(k), M = p->match.max_matches;
     const SeqScratch& a = blk->w;
     v.qp = a.qp + f0 * N; v.qc = a.qc + f0; v.ov = a.ov + f0;
     v.word = a.word + f0 * N;
-    v.coords_in = warm(k) ? nullptr : a.coords_in + 3 * f0 * N;   // warm-up words need no coordinates
-    if (!warm(k)) {
-      const size_t p0 = chunk_first(k);
+    v.coords_in = plan.warm(k) ? nullptr : a.coords_in + 3 * f0 * N;   // warm-up words need no coordinates
+    if (!plan.warm(k)) {
+      const size_t p0 = plan.first_pair(k);
       v.mp = a.mp + 4 * p0 * M; v.mc = a.mc + p0; v.mcell = a.mcell + p0 * M; v.rin = a.rin + p0;
     }
     return v;
   };
 
   auto stage_dma = [&](int k) -> mv_status {
-    const int b = k % NB, p0 = chunk_frame0(k), nf = chunk_frames(k);
+    const int b = k % NB, p0 = plan.frame0(k), nf = plan.frames(k);
     cudaStream_t cs = c->copy_stream;
     // buffer set b may be refilled only after the compute that read it is done
     MV_CUDA(c, cudaStreamWaitEvent(cs, consumed[b], 0));
@@ -1223,14 +1234,13 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
                                cudaMemcpyHostToDevice, cs));
     MV_CUDA(c, cudaMemcpyAsync(bsc[b], h_semi_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice, cs));
     up += (unsigned long long)nf * ((size_t)cells * 65 + 4);
-    if (!warm(k)) {
+    if (!plan.warm(k)) {
       MV_CUDA(c, cudaMemcpyAsync(bz[b], h_depth + (size_t)p0 * cells, sizeof(float) * (size_t)nf * cells,
                                  cudaMemcpyHostToDevice, cs));
       up += (unsigned long long)nf * cells * 4;
     }
-    if (lm) {
-      MV_CUDA(c, cudaMemcpyAsync(bdsc[b], lm->desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice,
-                                 cs));
+    if (landmarks) {
+      MV_CUDA(c, cudaMemcpyAsync(bdsc[b], h_desc_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice, cs));
       up += (unsigned long long)nf * 4;
     }
     if (!gather) {
@@ -1250,7 +1260,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   cudaEvent_t matched;
   if ((st = new_event(&matched))) return st;
   auto launch_gather = [&](int k, cudaEvent_t after) -> mv_status {
-    const int b = k % NB, p0 = chunk_frame0(k), nf = chunk_frames(k);
+    const int b = k % NB, p0 = plan.frame0(k), nf = plan.frames(k);
     cudaStream_t gs = c->gather_stream;
     MV_CUDA(c, cudaStreamWaitEvent(gs, detected[b], 0));
     if (after) MV_CUDA(c, cudaStreamWaitEvent(gs, after, 0));
@@ -1273,14 +1283,14 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     return MV_OK;
   };
   auto stage_detect = [&](int k) -> mv_status {
-    const int b = k % NB, nf = chunk_frames(k);
+    const int b = k % NB, nf = plan.frames(k);
     const SeqScratch v = chunk_scratch(k);
     mv_status s2;
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, copied[b], 0));
     if ((s2 = seq_detect(c, p, nf, (const int8_t*)bs[b], (const float*)bsc[b], v))) return s2;
     if (gather) {
       dim3 g1((cells + 255) / 256, nf), g2((p->top_n + 255) / 256, nf);
-      if (warm(k)) {   // no matcher runs on a warm-up frame: its query rows only
+      if (plan.warm(k)) {   // no matcher runs on a warm-up frame: its query rows only
         MV_CUDA(c, cudaMemsetAsync(v.flags, 0, (size_t)nf * cells, c->stream));
       } else {
         mark_needed_rows_kernel<<<g1, 256, 0, c->stream>>>(nf, cells, p->top_n, mv_round_up(p->match.min_prob0),
@@ -1297,64 +1307,67 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     } else if (k == 0) {
       return launch_gather(k, nullptr);
     } else {
-      pending_gather = k;   // released by chunk k-1's matcher, see stage_compute
+      pending_gather = k;   // released by chunk k-1's compute, see stage_compute
     }
     return MV_OK;
   };
-  // In landmark mode seq_step runs the word assignment (a persistent CTA per SM with the vocabulary in shared
-  // memory) after the chunk's `ready` and before its matcher, so it never runs beside a row gather.
-  // A block being prepared runs no K3: chunk k+1's gather is released after chunk k's whole compute (words,
-  // matcher, RANSAC-E) instead.  Released after the matcher it measured the same (profiles/r07).
   auto release_gather = [&](int k) -> mv_status {
     if (pending_gather != k + 1) return MV_OK;
     pending_gather = -1;
     MV_CUDA(c, cudaEventRecord(matched, c->stream));
     return launch_gather(k + 1, matched);
   };
+  // The word assignment (a persistent CTA per SM with the vocabulary in shared memory) runs after the chunk's `ready`
+  // and before its matcher, so it never runs beside a row gather.  Chunk k+1's gather is released once chunk k's
+  // matcher is enqueued, so that it runs beside K3.  A block being prepared runs no K3: there it is released after
+  // the chunk's whole compute (words, matcher, RANSAC-E; the words only for a warm-up chunk), which measured the
+  // same as after the matcher (profiles/r07).
   auto stage_compute = [&](int k) -> mv_status {
-    const int b = k % NB, p0 = chunk_first(k), nf = chunk_frames(k);
+    const int b = k % NB, nf = plan.frames(k), p0 = plan.first_pair(k);
+    const bool warm = plan.warm(k), prepare = call == HostCall::prepare;
+    const int8_t* desc = (const int8_t*)bd[b];
+    const float* depth = warm ? nullptr : (const float*)bz[b];
+    const SeqScratch v = chunk_scratch(k);
+    const SeqLandmarks lm = {first_frame - n_warm + plan.frame0(k), n_words, d_table, (const float*)bdsc[b],
+                             dnwl ? (int32_t*)dnwl + p0 : nullptr};
+    mv_status s2;
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, ready[b], 0));
     mark("cmp_beg", k, c->stream);
-    const SeqStageFn on_stage = [&](const char* stage) -> mv_status {
-      mark(stage, k, c->stream);
-      if (strcmp(stage, "match_end") || blk) return MV_OK;
-      return release_gather(k);
-    };
-    SeqLandmarks chunk_lm{};
-    if (lm)
-      chunk_lm = {lm->first_frame + p0, lm->n_words, lm->table, (const float*)bdsc[b],
-                  dnwl ? (int32_t*)dnwl + p0 : nullptr};
-    mv_status s2;
-    if (!blk) {
-      s2 = seq_step(c, p, nf, (const int8_t*)bd[b], (const float*)bz[b], w[b], (mv_pair_result*)dres + p0, p0,
-                    lm ? &chunk_lm : nullptr, on_stage);
-    } else if (warm(k)) {
-      s2 = seq_words(c, p, nf, (const int8_t*)bd[b], nullptr, chunk_scratch(k), &chunk_lm);
-    } else {
-      const SeqScratch v = chunk_scratch(k);
-      if (!(s2 = seq_words(c, p, nf - 1, (const int8_t*)bd[b], (const float*)bz[b], v, &chunk_lm)))
-        s2 = seq_match(c, p, nf, (const int8_t*)bd[b], v, on_stage);
+    if (landmarks && (s2 = seq_words(c, p, warm ? nf : nf - 1, desc, depth, v, &lm))) return s2;
+    if (call == HostCall::landmarks &&
+        (s2 = mv_landmarks_sequence_impl(c, n_words, d_table, lm.first_frame, nf - 1, N, v.word, v.qc, v.coords_in,
+                                         v.coords_out)))
+      return s2;
+    if (!warm) {
+      if ((s2 = seq_match(c, p, nf, desc, v))) return s2;
+      mark("match_end", k, c->stream);
+      if ((!prepare && (s2 = release_gather(k))) || (s2 = seq_ransac(c, p, nf, v))) return s2;
     }
-    if (s2 || (blk && (s2 = release_gather(k)))) return s2;
+    if (prepare && (s2 = release_gather(k))) return s2;
+    if (!prepare) {
+      if ((s2 = seq_corr(c, p, nf, depth, v, landmarks ? &lm : nullptr))) return s2;
+      mark("corr_end", k, c->stream);
+      if ((s2 = seq_pose(c, p, nf, v, (mv_pair_result*)dres + p0, p0))) return s2;
+    }
     MV_CUDA(c, cudaEventRecord(consumed[b], c->stream));
     mark("cmp_end", k, c->stream);
     return MV_OK;
   };
 
   if ((st = stage_dma(0))) return st;
-  if (n_chunks > 1 && (st = stage_dma(1))) return st;
+  if (plan.n_chunks > 1 && (st = stage_dma(1))) return st;
   if ((st = stage_detect(0))) return st;
-  for (int k = 0; k < n_chunks; k++) {
-    if (k + 2 < n_chunks && (st = stage_dma(k + 2))) return st;
-    if (k + 1 < n_chunks && (st = stage_detect(k + 1))) return st;
+  for (int k = 0; k < plan.n_chunks; k++) {
+    if (k + 2 < plan.n_chunks && (st = stage_dma(k + 2))) return st;
+    if (k + 1 < plan.n_chunks && (st = stage_detect(k + 1))) return st;
     if ((st = stage_compute(k))) return st;
   }
   unsigned long long moved = 0;
   unsigned long long down = 0;
-  if (blk) {
+  if (call == HostCall::prepare) {
     // one speculation over the warm-up and block words; the block's remaining work stays queued
-    if ((st = mv_landmarks_speculate_impl(c, lm->n_words, lm->first_frame, n_warm, n_pairs, p->top_n, blk->w.word,
-                                          blk->w.qc, blk->b.coords_in, &blk->spec)))
+    if ((st = mv_landmarks_speculate_impl(c, n_words, first_frame, n_warm, n_pairs, p->top_n, blk->w.word, blk->w.qc,
+                                          blk->b.coords_in, &blk->spec)))
       return st;
     blk->b.coords_out = mv_lm_spec_coords(blk->spec);
     drain.compute = false;
@@ -1363,8 +1376,8 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
     MV_CUDA(c, cudaMemcpyAsync(h_results, dres, sizeof(mv_pair_result) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
                                c->stream));
     if (dnwl) {
-      MV_CUDA(c, cudaMemcpyAsync(lm->n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs,
-                                 cudaMemcpyDeviceToHost, c->stream));
+      MV_CUDA(c, cudaMemcpyAsync(h_n_with_landmark, dnwl, sizeof(int32_t) * (size_t)n_pairs, cudaMemcpyDeviceToHost,
+                                 c->stream));
       down += sizeof(int32_t) * (unsigned long long)n_pairs;
     }
     MV_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -1373,7 +1386,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, const char* fn, const mv_tr
   MV_CUDA(c, cudaMemcpyAsync(&moved, dmoved, 8, cudaMemcpyDeviceToHost, c->gather_stream));
   MV_CUDA(c, cudaStreamSynchronize(c->gather_stream));
   if (trace) {
-    if (blk) MV_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (call == HostCall::prepare) MV_CUDA(c, cudaStreamSynchronize(c->stream));
     for (auto& m : marks) {
       float ms = 0.f;
       cudaEventElapsedTime(&ms, marks[0].second, m.second);
@@ -1395,8 +1408,10 @@ extern "C" mv_status mv_track_sequence_host(mv_ctx* c, const mv_track_params* p,
   MV_ENTER(c);
   if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_depth || !h_results)
     MV_BAD_ARG(c, "mv_track_sequence_host");
-  return track_sequence_host_impl(c, "mv_track_sequence_host", p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
-                                  d2h_bytes, nullptr);
+  const HostPlan plan = host_plan(c, p, 0, n_frames - 1, false);
+  if (mv_status st = seq_check(c, "mv_track_sequence_host", p, plan.pairs + 1, nullptr, false)) return st;
+  return track_sequence_host_impl(c, HostCall::depth, plan, p, h_semi, h_semi_scale, h_desc, nullptr, h_depth, 0, 0,
+                                  nullptr, h_results, nullptr, nullptr, h2d_bytes, d2h_bytes);
 }
 
 extern "C" mv_status mv_track_sequence_landmarks_host(mv_ctx* c, const mv_track_params* p, int n_frames,
@@ -1408,9 +1423,13 @@ extern "C" mv_status mv_track_sequence_landmarks_host(mv_ctx* c, const mv_track_
   MV_ENTER(c);
   if (!p || n_frames < 2 || !h_semi || !h_semi_scale || !h_desc || !h_desc_scale || !h_depth || !h_results)
     MV_BAD_ARG(c, "mv_track_sequence_landmarks_host");
-  const SeqLandmarks lm = {first_frame, n_words, d_table, h_desc_scale, h_n_with_landmark};
-  return track_sequence_host_impl(c, "mv_track_sequence_landmarks_host", p, n_frames, h_semi, h_semi_scale, h_desc, h_depth, h_results, h2d_bytes,
-                                  d2h_bytes, &lm);
+  const HostPlan plan = host_plan(c, p, 0, n_frames - 1, true);
+  if (mv_status st = seq_check(c, "mv_track_sequence_landmarks_host", p, plan.pairs + 1, nullptr, true, n_words))
+    return st;
+  if (!d_table) MV_BAD_ARG(c, "mv_track_sequence_landmarks_host: NULL landmark table");
+  return track_sequence_host_impl(c, HostCall::landmarks, plan, p, h_semi, h_semi_scale, h_desc, h_desc_scale, h_depth,
+                                  first_frame, n_words, d_table, h_results, h_n_with_landmark, nullptr, h2d_bytes,
+                                  d2h_bytes);
 }
 
 extern "C" mv_status mv_track_landmarks_prepare_host(mv_ctx* c, const mv_track_params* p, int n_warm, int n_frames,
@@ -1419,29 +1438,13 @@ extern "C" mv_status mv_track_landmarks_prepare_host(mv_ctx* c, const mv_track_p
                                                      const float* h_depth, int n_words, mv_lm_block** out,
                                                      unsigned long long* h2d_bytes) {
   MV_ENTER(c);
-  if (!out) MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: NULL out");
-  *out = nullptr;
-  if (!p || n_frames < 2 || n_warm < 0 || !h_semi || !h_semi_scale || !h_desc || !h_desc_scale || !h_depth)
-    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host");
-  if ((long long)n_warm + n_frames > 65535)
-    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: at most 65535 frames in all");
-  const int T = n_warm + n_frames;
-  const SeqLandmarks lm = {first_frame, n_words, nullptr, h_desc_scale, nullptr};
-  mv_status st;
-  // the whole block's limits, then those of the pipeline's chunks, before the block is allocated
-  if ((st = seq_check(c, "mv_track_landmarks_prepare_host", p, T, nullptr, &lm, false)) ||
-      (st = seq_check(c, "mv_track_landmarks_prepare_host", p, host_chunk_pairs(c, p, n_frames - 1, true) + 1, nullptr,
-                      &lm, false)))
-    return st;
-  if (p->match.use_tensor_cores == 1 && !mv_match_tc_feasible(&p->match, n_frames, n_frames - 1, p->top_n))
-    MV_BAD_ARG(c, "mv_track_landmarks_prepare_host: use_tensor_cores = 1 on a shape the tensor-core matcher does "
-                  "not take");
-  mv_lm_block* k = new mv_lm_block();
-  k->ctx = c; k->p = *p; k->n_warm = n_warm; k->n_frames = n_frames; k->n_words = n_words;
-  if ((st = seq_scratch(c, p, T, "", true, &k->w, &k->mem, false))) { lm_block_free(k); return st; }
-  lm_block_view(k);
-  if ((st = track_sequence_host_impl(c, "mv_track_landmarks_prepare_host", p, n_frames, h_semi, h_semi_scale, h_desc,
-                                     h_depth, nullptr, h2d_bytes, nullptr, &lm, k))) {
+  HostPlan plan;
+  mv_lm_block* k;
+  mv_status st = lm_block_new(c, "mv_track_landmarks_prepare_host", p, n_warm, n_frames, first_frame, n_words,
+                              h_semi && h_semi_scale && h_desc && h_desc_scale && h_depth, nullptr, &plan, out, &k);
+  if (st) return st;
+  if ((st = track_sequence_host_impl(c, HostCall::prepare, plan, p, h_semi, h_semi_scale, h_desc, h_desc_scale, h_depth,
+                                     first_frame, n_words, nullptr, nullptr, nullptr, k, h2d_bytes, nullptr))) {
     lm_block_free(k);
     return st;
   }

@@ -831,6 +831,29 @@ mv_status mv_landmarks_sequence_reserve(mv_ctx* ctx, int n_words, int n_steps, i
   return lmseq_scratch(ctx, n_words, n_steps, top_n, &cnt, &tot, &start, &sorted);
 }
 
+// Enqueues the counting sort of n_steps steps' occurrences by word into start / sorted, with cnt / tot as its
+// scratch (sized as lmseq_scratch's), timed under `tag`; the occurrences without a word get zero coords_out.
+static mv_status lmseq_sort(mv_ctx* ctx, const char* tag, int n_words, int n_steps, int top_n, const int32_t* d_word,
+                            const int32_t* d_q_count, int32_t* cnt, int32_t* tot, int32_t* start, int32_t* sorted,
+                            float* d_coords_out) {
+  int n_tiles, fb;
+  lmseq_tiles(n_words, n_steps, &n_tiles, &fb);
+  mv_prof_scope ps(ctx, tag);
+  MV_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)n_tiles * n_words, ctx->stream));
+  const long long blocks = ((long long)n_steps * top_n + 255) / 256;
+  lmseq_count_kernel<<<(int)std::min<long long>(blocks, 8LL * ctx->sm_count), 256, 0, ctx->stream>>>(
+      n_steps, top_n, n_words, fb, d_word, d_q_count, cnt, d_coords_out);
+  MV_CHECK_LAUNCH(ctx);
+  lmseq_colscan_kernel<<<(n_words + 127) / 128, 128, 0, ctx->stream>>>(n_words, n_tiles, cnt, tot);
+  MV_CHECK_LAUNCH(ctx);
+  lmseq_wordscan_kernel<<<1, 1024, 0, ctx->stream>>>(n_words, tot, start);
+  MV_CHECK_LAUNCH(ctx);
+  lmseq_scatter_kernel<<<n_tiles, 256, 0, ctx->stream>>>(n_steps, top_n, n_words, fb, d_word, d_q_count, cnt, start,
+                                                        sorted);
+  MV_CHECK_LAUNCH(ctx);
+  return MV_OK;
+}
+
 mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_table, int first_frame, int n_steps,
                                      int top_n, const int32_t* d_word, const int32_t* d_q_count,
                                      const float* d_coords_in, float* d_coords_out) {
@@ -840,27 +863,12 @@ mv_status mv_landmarks_sequence_impl(mv_ctx* ctx, int n_words, mv_landmark* d_ta
     MV_BAD_ARG(ctx, "mv_landmarks_sequence: 0..65535 steps of top_n > 0 queries, fewer than 2^31 in all");
   if (n_steps == 0) return MV_OK;
   if (!d_word || !d_q_count || !d_coords_in || !d_coords_out) MV_BAD_ARG(ctx, "mv_landmarks_sequence");
-  int n_tiles, fb;
-  lmseq_tiles(n_words, n_steps, &n_tiles, &fb);
-  const long long total = (long long)n_steps * top_n;
   void *cnt, *tot, *start, *sorted;
   mv_status st;
-  if ((st = lmseq_scratch(ctx, n_words, n_steps, top_n, &cnt, &tot, &start, &sorted))) return st;
-  {
-    mv_prof_scope ps(ctx, "sort");
-    MV_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)n_tiles * n_words, ctx->stream));
-    const long long blocks = (total + 255) / 256;
-    lmseq_count_kernel<<<(int)std::min<long long>(blocks, 8LL * ctx->sm_count), 256, 0, ctx->stream>>>(
-        n_steps, top_n, n_words, fb, d_word, d_q_count, (int32_t*)cnt, d_coords_out);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_colscan_kernel<<<(n_words + 127) / 128, 128, 0, ctx->stream>>>(n_words, n_tiles, (int32_t*)cnt, (int32_t*)tot);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_wordscan_kernel<<<1, 1024, 0, ctx->stream>>>(n_words, (const int32_t*)tot, (int32_t*)start);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_scatter_kernel<<<n_tiles, 256, 0, ctx->stream>>>(n_steps, top_n, n_words, fb, d_word, d_q_count, (int32_t*)cnt,
-                                                          (const int32_t*)start, (int32_t*)sorted);
-    MV_CHECK_LAUNCH(ctx);
-  }
+  if ((st = lmseq_scratch(ctx, n_words, n_steps, top_n, &cnt, &tot, &start, &sorted)) ||
+      (st = lmseq_sort(ctx, "sort", n_words, n_steps, top_n, d_word, d_q_count, (int32_t*)cnt, (int32_t*)tot,
+                       (int32_t*)start, (int32_t*)sorted, d_coords_out)))
+    return st;
   mv_prof_scope ps(ctx, "walk");
   lmseq_walk_kernel<<<(n_words + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, ctx->stream>>>(
       n_words, d_table, first_frame, n_steps, top_n, (const int32_t*)start, (const int32_t*)sorted, d_coords_in,
@@ -918,21 +926,9 @@ mv_status mv_landmarks_speculate_impl(mv_ctx* ctx, int n_words, int first_frame,
   s->n_rewalk = (int32_t*)(m + b_cnt + b_tot + b_start + b_sorted + b_coords + b_sw);
   s->rewalk = s->n_rewalk + 1;
   *out = s;
-  {
-    mv_prof_scope ps(ctx, "spec_sort");
-    MV_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (size_t)n_tiles * n_words, ctx->stream));
-    const long long blocks = ((long long)occ + 255) / 256;
-    lmseq_count_kernel<<<(int)std::min<long long>(blocks, 8LL * ctx->sm_count), 256, 0, ctx->stream>>>(
-        T, top_n, n_words, fb, d_word, d_q_count, cnt, s->coords);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_colscan_kernel<<<(n_words + 127) / 128, 128, 0, ctx->stream>>>(n_words, n_tiles, cnt, tot);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_wordscan_kernel<<<1, 1024, 0, ctx->stream>>>(n_words, tot, s->start);
-    MV_CHECK_LAUNCH(ctx);
-    lmseq_scatter_kernel<<<n_tiles, 256, 0, ctx->stream>>>(T, top_n, n_words, fb, d_word, d_q_count, cnt, s->start,
-                                                          s->sorted);
-    MV_CHECK_LAUNCH(ctx);
-  }
+  if ((st = lmseq_sort(ctx, "spec_sort", n_words, T, top_n, d_word, d_q_count, cnt, tot, s->start, s->sorted,
+                       s->coords)))
+    return st;
   mv_prof_scope ps(ctx, "spec_walk");
   lmspec_walk_kernel<<<(n_words + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, ctx->stream>>>(
       n_words, first_frame - n_warm, n_warm, T, top_n, s->start, s->sorted, d_coords_in, s->coords, s->sw);
