@@ -12,9 +12,13 @@ It follows the semantics list of DESIGN §4.6 ("Words", "Inserted coordinates", 
     after step p (the matched frame-0 cell's query, its word in [0, n_words) with a live record; NaN otherwise, and
     only the former counted in n_with_landmark), orc_pnp_gn keyed on pnp.first_pair + p;
   * status 4 (MV_ERR_TOO_MANY_VALID) where either frame of the pair overflowed max_valid.
+
+Below the reference: the inputs of the cases the modules hold to it, the word-assignment checks beyond the reference
+vocabulary, and run_entry, which runs one of the library's landmark-path entry points on a case.
 """
 import numpy as np
 
+from helpers import blocks_then_rest, dev, pinned, ref_vocab, upload_table, with_first_pair
 from oracle import orc
 
 STATUS_TOO_MANY_VALID = 4
@@ -24,17 +28,19 @@ f32 = np.float32
 def orc_landmarks_sequence(oracle, table, first_frame, word, q_count, coords, snapshots=None):
     """The semantics of mv_landmarks_sequence on the oracle's table (updated in place): step f observes the first
     q_count[f] words of frame first_frame + f, then removes old frames; returns each occurrence's lookup right after
-    its step (0 where the word has no record or q >= q_count)."""
+    its step (0 where the word has no record or q >= q_count).  snapshots: a list that receives a copy of the table
+    after every step."""
     n_steps, top_n = word.shape
     out = np.zeros((n_steps, top_n, 3), np.float32)
     for f in range(n_steps):
         k = min(int(q_count[f]), top_n)
-        oracle.pool_observe(table, first_frame + f, word[f, :k], coords[f, :k])
+        w = word[f, :k]
+        oracle.pool_observe(table, first_frame + f, w, coords[f, :k])
         oracle.pool_remove_old(table, first_frame + f)
-        for q in range(k):
-            w = int(word[f, q])
-            if 0 <= w < len(table) and table[w]["word_id"] == w:
-                out[f, q] = table[w]["coords"]
+        ok = (w >= 0) & (w < len(table))
+        wc = np.where(ok, w, 0)
+        ok &= table["word_id"][wc] == wc
+        out[f, :k][ok] = table["coords"][wc[ok]]
         if snapshots is not None:
             snapshots.append(table.copy())
     return out
@@ -174,3 +180,203 @@ def landmark_reference(oracle, vocab, params, semi, semi_scale, desc, desc_scale
     if depth_mode:
         return rec, None, None
     return rec, np.array([k for _, k in out], np.int32).reshape(n - 1), table
+
+
+# ------------------------------------------------------------------ the reference's cases and the calls held to it
+def random_vocab(rng, n_base, wpb):
+    base = rng.integers(-128, 128, (256, n_base)).astype(np.int8)
+    scale = rng.uniform(0.5, 2.0, n_base).astype(f32)
+    bias = rng.uniform(-0.3, 0.3, n_base).astype(f32)
+    leaves = rng.integers(-2 ** 31, 2 ** 31, (n_base, wpb, 4)).astype(np.int32)
+    return base, scale, bias, leaves
+
+
+# one frame per (descriptor kind, desc_scale): random, zero, all -128, all 127, one row repeated
+BOW_SCALES = (4.3353, -1.5, 0.0, 1e-30, 1e30, np.inf, -np.inf, np.nan)
+BOW_KINDS = ("random", "zero", "min", "max", "repeated")
+
+
+def bow_vocab(name):
+    """(n_base, wpb) shapes with random contents, the reference vocabulary, and vocabularies built to tie."""
+    rng = np.random.default_rng(sum(map(ord, name)))
+    if name == "10x1000":
+        return ref_vocab()
+    if "x" in name:
+        nb, wpb = (int(x) for x in name.split("x"))
+        return random_vocab(rng, nb, wpb)
+    if name == "repeated_leaves":      # leaf w = L[w % 5]: every 8-word window occurs at 4 leaves of different lanes
+        base, scale, bias, _ = random_vocab(rng, 3, 20)
+        L = rng.integers(-2 ** 31, 2 ** 31, (5, 4)).astype(np.int32)
+        return base, scale, bias, np.ascontiguousarray(np.broadcast_to(L[np.arange(20) % 5], (3, 20, 4)))
+    if name == "zero_leaves":          # every window ties
+        base, scale, bias, leaves = random_vocab(rng, 2, 16)
+        return base, scale, bias, np.zeros_like(leaves)
+    if name == "nonpositive_scores":   # no score exceeds 0: base 0
+        base, scale, bias, leaves = random_vocab(rng, 4, 11)
+        scale[:2], bias[:2], bias[2:] = 0.0, 0.0, -1.2
+        return base, scale, bias, leaves
+    if name == "equal_bases":          # bases 2..4 identical and the only ones that can win: base 2
+        base, scale, bias, leaves = random_vocab(rng, 5, 12)
+        base[:, 3] = base[:, 4] = base[:, 2]
+        scale[3:] = scale[2]
+        bias[3:] = bias[2] = 0.25
+        bias[:2] = -1.0
+        return base, scale, bias, leaves
+    raise KeyError(name)
+
+
+def bow_inputs(seed, top_n, cells=48, reps=1):
+    """Descriptors of len(BOW_KINDS) x len(BOW_SCALES) x reps frames, their scales, query cells (duplicates
+    included) and counts (0 and top_n among them)."""
+    rng = np.random.default_rng(seed)
+    n = len(BOW_KINDS) * len(BOW_SCALES) * reps
+    desc = rng.integers(-128, 128, (n, cells, 256)).astype(np.int8)
+    dscale = np.zeros(n, f32)
+    for f in range(n):
+        kind = BOW_KINDS[(f // len(BOW_SCALES)) % len(BOW_KINDS)]
+        dscale[f] = BOW_SCALES[f % len(BOW_SCALES)]
+        if kind == "zero":
+            desc[f] = 0
+        elif kind == "min":
+            desc[f] = -128
+        elif kind == "max":
+            desc[f] = 127
+        elif kind == "repeated":
+            desc[f] = desc[f, 0]
+    qp = rng.integers(0, cells, (n, top_n)).astype(np.int32)
+    qp[:, 1::3] = qp[:, 0::3][:, :qp[:, 1::3].shape[1]]       # the same cell queried twice
+    qc = rng.integers(1, top_n + 1, n).astype(np.int32)
+    qc[::7] = top_n
+    qc[3::11] = 0
+    for f in range(n):
+        qp[f, qc[f]:] = 0
+    return desc, dscale, qp, qc
+
+
+def bow_check(tr, oracle, vocab, desc, dscale, qp, qc):
+    """mv_bow_assign_batch on tr against oracle.bow_assign, frame by frame -> the device's words."""
+    v = oracle.bow_vocab(*vocab)
+    wpb = vocab[3].shape[1]
+    word, base = tr.bow_assign(dev(tr, desc), dev(tr, dscale), dev(tr, qp), dev(tr, qc))
+    word, base = word.cpu().numpy(), base.cpu().numpy()
+    for f in range(desc.shape[0]):
+        k = int(qc[f])
+        assert (word[f, k:] == -1).all() and (base[f, k:] == -1).all(), f
+        rb, rw = oracle.bow_assign(v, dscale[f], desc[f][qp[f, :k]])
+        assert (base[f, :k] == rb).all(), (f, dscale[f])
+        assert (word[f, :k] == rb * wpb + rw).all(), (f, dscale[f])
+    return word
+
+
+def case_inputs(name, synth):
+    """Host inputs and parameters of one case -> dict(p, frames (semi, semi_scale, desc, desc_scale, depth), first,
+    n_words, vocab, entry table or None)."""
+    import maveric_slam_b200  # noqa: F401
+    from maveric_slam_b200 import tracking
+    rng = np.random.default_rng(sum(map(ord, name)))
+    vocab = ref_vocab()
+    n_words, first, entry = 10000, 0, None
+    if name == "scales":
+        rows, cols, n = 47, 155, 20
+        semi, desc, depth, _ = synth.synth_sequence(31, rows, cols, n)
+        rng = np.random.default_rng(8)
+        sscale = (synth.SEMI_SCALE * rng.uniform(0.9, 1.1, n)).astype(f32)
+        dscale = (synth.DESC_SCALE * rng.uniform(0.5, 2.0, n)).astype(f32)
+        dscale[4], dscale[11] = -dscale[4], 0.0
+        p = tracking.kitti_track_params(hypotheses=256)
+        first = 500
+    elif name == "degenerate":
+        rows, cols, n = 24, 80, 12
+        semi, desc, depth, off = synth.synth_sequence(5, rows, cols, n)
+        semi[2:4, :, :64], semi[2:4, :, 64] = -128, 127                    # no keypoints
+        semi[6] = synth.synth_frame(5, rows, cols, 6, int(off[6, 0]), int(off[6, 1]), keypoint_permille=1000)[0]
+        desc[8], desc[9] = -128, 0
+        sscale = np.full(n, synth.SEMI_SCALE, f32)
+        dscale = np.full(n, synth.DESC_SCALE, f32)
+        p = tracking.track_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=64)
+    elif name == "odd":
+        rows, cols, n = 13, 37, 14
+        semi, desc, depth, _ = synth.synth_sequence(9, rows, cols, n, offsets=synth.default_offsets(n, 9, step=0),
+                                                    keypoint_permille=300, noise_amp=2)
+        sscale = np.full(n, synth.SEMI_SCALE, f32)
+        dscale = (synth.DESC_SCALE * rng.uniform(0.5, 2.0, n)).astype(f32)
+        # a query has at most one match, so the cap binds only below top_n
+        p = tracking.track_params(rows, cols, top_n=37, max_valid=482, max_matches=16, hypotheses=32, radius=6,
+                                  shift=(-2, 1), lanes=32)
+        first = -20
+    elif name in ("vocab60", "vocab200"):
+        rows, cols, n = 24, 80, 16
+        semi, desc, depth, _ = synth.synth_sequence(13, rows, cols, n)
+        sscale = np.full(n, synth.SEMI_SCALE, f32)
+        dscale = np.full(n, synth.DESC_SCALE, f32)
+        vocab = random_vocab(np.random.default_rng(77), 7, 13)
+        vocab[3][:, 6:9] = vocab[3][:, 2:5]                                  # repeated leaves
+        p = tracking.track_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=64)
+        n_words, first = int(name[5:]), 40
+    else:
+        raise KeyError(name)
+    return dict(p=p, frames=[semi, sscale, desc, dscale, depth], first=first, n_words=n_words, vocab=vocab,
+                entry=entry)
+
+
+def run_entry(tr, c, entry, monkeypatch):
+    """Runs one entry point on the case -> (records bytes, n_with_landmark int32, final table bytes)."""
+    import torch
+    from maveric_slam_b200 import tracking
+    p, first, n_words = c["p"], c["first"], c["n_words"]
+    host = c["frames"]
+    dframes = [dev(tr, x) for x in host]
+    n_pairs = host[0].shape[0] - 1
+    table = tr.landmarks_new(n_words) if c["entry"] is None else upload_table(tr, c["entry"])
+    kind, _, opt = entry.partition(":")
+    if kind == "device":
+        res, nl = tr.track_sequence_landmarks(p, *dframes, table, first_frame=first)
+        res, nl = res.cpu().numpy(), nl.cpu().numpy()
+    elif kind == "host":
+        if opt == "pageable":
+            bufs = [np.ascontiguousarray(x) for x in host]
+        else:
+            bufs = [pinned(x) for x in host]
+            if opt:
+                monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", opt)
+        res, nl, _, _ = tr.track_sequence_landmarks_host(p, *bufs, table, first_frame=first)
+    elif kind in ("blocks", "blocks_host"):
+        n_warm = int(opt)
+        bufs = dframes if kind == "blocks" else [pinned(x) for x in host]
+        prep = tr.track_landmarks_prepare if kind == "blocks" else tr.track_landmarks_prepare_host
+        blocks = blocks_then_rest(n_pairs, (1, 5))
+        prepared = {}
+        for i, (lo, cnt) in reversed(list(enumerate(blocks))):
+            w = min(n_warm, lo)
+            prepared[i] = prep(with_first_pair(p, p.pnp.first_pair + lo), w, first + lo,
+                               *[x[lo - w:lo + cnt + 1] for x in bufs], n_words)
+        res, nl = [], []
+        for i in range(len(blocks)):
+            tr.track_landmarks_step_table(prepared[i], table)
+            r, n = tr.track_landmarks_solve(prepared[i])
+            res.append(r.cpu().numpy()); nl.append(n.cpu().numpy())
+            tr.track_landmarks_release(prepared[i])
+        res, nl = np.concatenate(res), np.concatenate(nl)
+    elif kind == "sharded":
+        res, nl, _ = tracking.track_sequence_landmarks_sharded(tr, p, dframes, table, first_frame=first, n_warm=8)
+        res, nl = res.cpu().numpy(), nl.cpu().numpy()
+    elif kind == "host_sharded":
+        bufs = [pinned(x) for x in host]
+        res, nl, _, _ = tracking.track_sequence_landmarks_host_sharded(tr, p, bufs, table, first_frame=first, n_warm=8)
+        res, nl = res.cpu().numpy(), nl.cpu().numpy()
+    else:
+        raise KeyError(entry)
+    torch.cuda.synchronize()
+    return np.ascontiguousarray(res).view(np.uint8).reshape(-1).tobytes(), np.asarray(nl, np.int32), \
+        table.cpu().numpy().tobytes()
+
+
+def first_difference(want, got):
+    """Pair and field of the first differing byte of two record arrays."""
+    from maveric_slam_b200 import tracking
+    g = np.frombuffer(got, tracking.PAIR_RESULT_DTYPE)
+    for q in range(len(want)):
+        for f in tracking.PAIR_RESULT_DTYPE.names:
+            if want[q][f].tobytes() != g[q][f].tobytes():
+                return "pair %d %s: reference %r, got %r" % (q, f, want[q][f], g[q][f])
+    return "lengths %d, %d" % (len(want), len(g))

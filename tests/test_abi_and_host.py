@@ -9,6 +9,8 @@ import subprocess
 import numpy as np
 import pytest
 
+from helpers import InsertResult, LocalFeature, Pool
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -91,23 +93,6 @@ def test_numpy_generator_equals_c_generator(oracle, synth):
 
 
 # ---------------------------------------------------------------- local feature pool (host side)
-class LocalFeature(C.Structure):
-    _fields_ = [("word_id", C.c_int), ("frame_ptr", C.c_int), ("num_frames", C.c_int), ("frames", C.c_int * 8),
-                ("coords_3D", C.c_float * 3)]
-
-
-class HashEntry(C.Structure):
-    _fields_ = [("key", C.c_int), ("value", LocalFeature), ("is_occupied", C.c_bool)]
-
-
-class Pool(C.Structure):
-    _fields_ = [("entries", HashEntry * 3000), ("size", C.c_int), ("capacity", C.c_int)]
-
-
-class InsertResult(C.Structure):
-    _fields_ = [("feature", C.POINTER(LocalFeature)), ("inserted", C.c_bool)]
-
-
 def _drive_pool(L, frames=60, per_frame=200, seed=0):
     """The churn of src/local_feature_matching.c:129-170: per frame insert-or-update ids, age out,
     check the invariant.  Returns a trace of (size, occupied slots)."""

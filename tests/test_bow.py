@@ -13,22 +13,17 @@ What is pinned and what is not:
     sequence of src/local_feature_matching.c:153-163.
 GPU tests: the CUDA kernels against the oracle, through the C ABI.
 """
-import ctypes as C
-import os
-
 import numpy as np
 import pytest
 
 from conftest import RECORD_T1, T1Calls
+from helpers import drive_host_pool, ref_vocab, table_contents
 from oracle import orc
-
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
 def vocab_np():
-    v = np.load(os.path.join(GOLDEN, "ref_vocab.npz"))
-    return v["base_desc"], v["scale"], v["bias"], v["leaves"]
+    return ref_vocab()
 
 
 @pytest.fixture(scope="module")
@@ -103,72 +98,6 @@ def test_oracle_word_assignment_follows_its_definition(oracle, vocab_np, image0)
 
 
 # ------------------------------------------------------------------ CPU: landmark table == contents of the pool
-class LocalFeature(C.Structure):
-    _fields_ = [("word_id", C.c_int), ("frame_ptr", C.c_int), ("num_frames", C.c_int), ("frames", C.c_int * 8),
-                ("coords_3D", C.c_float * 3)]
-
-
-class HashEntry(C.Structure):
-    _fields_ = [("key", C.c_int), ("value", LocalFeature), ("is_occupied", C.c_bool)]
-
-
-class Pool(C.Structure):
-    _fields_ = [("entries", HashEntry * 3000), ("size", C.c_int), ("capacity", C.c_int)]
-
-
-class InsertResult(C.Structure):
-    _fields_ = [("feature", C.POINTER(LocalFeature)), ("inserted", C.c_bool)]
-
-
-def frame_ids(rng, prev, per_frame=200, n_words=10000):
-    keep = rng.choice(prev, 75, replace=False)
-    fresh = rng.choice(np.setdiff1d(np.arange(n_words), keep), per_frame - 75, replace=False)
-    return np.concatenate([keep, fresh]).astype(np.int32)
-
-
-def pool_contents(pool):
-    out = {}
-    for e in pool.entries:
-        if e.is_occupied:
-            f = e.value
-            out[e.key] = (tuple(f.frames[(f.frame_ptr + k) % 8] for k in range(f.num_frames)), tuple(f.coords_3D))
-    return out
-
-
-def table_contents(table):
-    out = {}
-    for r in table[table["word_id"] >= 0]:
-        assert r["word_id"] >= 0
-        out[int(r["word_id"])] = (tuple(int(r["frames"][(r["frame_ptr"] + k) % 8]) for k in range(r["num_frames"])),
-                                  tuple(float(c) for c in r["coords"]))
-    return out
-
-
-def drive_host_pool(L, frames=60, seed=0):
-    """src/local_feature_matching.c:153-163 on the product's host pool (pinned to the reference's header)."""
-    L.local_feature_pool_insert.restype = InsertResult
-    L.local_feature_pool_insert.argtypes = [C.POINTER(Pool), C.c_int, LocalFeature]
-    pool = Pool()
-    L.init_local_feature_pool(C.byref(pool))
-    rng = np.random.default_rng(seed)
-    prev = rng.choice(10000, 200, replace=False)
-    snaps = []
-    for f in range(frames):
-        ids = frame_ids(rng, prev)
-        coords = rng.normal(size=(len(ids), 3)).astype(np.float32)
-        for wid, c in zip(ids, coords):
-            feat = LocalFeature()
-            L.init_local_feature_with_id(C.byref(feat), int(wid), f)
-            feat.coords_3D = (C.c_float * 3)(*c)
-            res = L.local_feature_pool_insert(C.byref(pool), int(wid), feat)
-            if not res.inserted:
-                L.update_local_feature(res.feature, f)
-        L.local_feature_pool_remove_old(C.byref(pool), f)
-        snaps.append((ids, coords, pool_contents(pool)))
-        prev = ids
-    return snaps
-
-
 def test_oracle_landmark_table_equals_pool_contents(oracle):
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import lib

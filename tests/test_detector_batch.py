@@ -21,7 +21,7 @@ import numpy as np
 import pytest
 
 from adversarial import adversarial_logits
-from test_lba import same_bits
+from helpers import dev, same_bits
 
 F32 = np.float32
 FLT_MAX = F32(np.finfo(np.float32).max)
@@ -344,11 +344,6 @@ def test_builders_reach_their_cases(oracle, synth):
 
 
 # ------------------------------------------------------------------ GPU
-def _dev(tracker, a):
-    import torch
-    return torch.from_numpy(np.ascontiguousarray(a)).to(tracker.device)
-
-
 def _check_top_n(got, want_per_frame):
     qp, qi, qpr, qc, ov = (t.cpu().numpy() for t in got)
     for f, (pa, ix, pp, n, o) in enumerate(want_per_frame):
@@ -362,12 +357,12 @@ def test_softmax_batch_across_frame_boundaries(tracker, oracle, synth, cells, al
     import torch
     semi, scale, ref = softmax_batch(oracle, synth, cells)
     if aligned:
-        dsemi = _dev(tracker, semi)
+        dsemi = dev(tracker, semi)
     else:                                                   # not 16-byte aligned: the byte-wise staging path
         buf = torch.zeros(semi.size + 64, dtype=torch.int8, device=tracker.device)
         dsemi = buf[5:5 + semi.size].view(semi.shape)
         dsemi.copy_(torch.from_numpy(semi))
-    idx, prob, nv = (t.cpu().numpy() for t in tracker.softmax(dsemi, _dev(tracker, scale)))
+    idx, prob, nv = (t.cpu().numpy() for t in tracker.softmax(dsemi, dev(tracker, scale)))
     for f, (i2, p2, n2) in enumerate(ref):
         assert (idx[f] == i2).all() and same_bits(prob[f], p2) and nv[f] == n2, (cells, f, float(scale[f]))
 
@@ -377,7 +372,7 @@ def test_softmax_batch_across_frame_boundaries(tracker, oracle, synth, cells, al
 @pytest.mark.parametrize("K", TOP_N_KS)
 def test_top_n_batch_at_count_limits(tracker, oracle, synth, K):
     semi, scale, max_valids = top_n_batch(oracle, synth, K)
-    idx, prob, _ = tracker.softmax(_dev(tracker, semi), _dev(tracker, scale))
+    idx, prob, _ = tracker.softmax(dev(tracker, semi), dev(tracker, scale))
     for mv in max_valids:
         want = []
         for f in range(len(semi)):
@@ -397,7 +392,7 @@ def test_nms_on_built_frames(tracker, oracle, rows, cols):
     N = max(1, cells // 10)
     for B in (1, 4, 5, 7):
         sel = [(B + j) % n for j in range(B)]
-        di, dp = _dev(tracker, mi[sel]), _dev(tracker, pr[sel])
+        di, dp = dev(tracker, mi[sel]), dev(tracker, pr[sel])
         tracker.nms(rows, cols, di, dp)
         gi, gp = di.cpu().numpy(), dp.cpu().numpy()
         once = [oracle.nms(rows, cols, mi[f], pr[f]) for f in sel]
@@ -456,7 +451,7 @@ def test_softmax_nms_top_n_on_the_device(tracker, oracle, synth, rows, cols, N):
     semi = np.stack(frames)
     scale = np.array([SEMI_SCALE, 3.0, 1.0, SEMI_SCALE, 0.01, 1e10, SEMI_SCALE, SEMI_SCALE, 0.5], np.float32)
     mv = cells + 1
-    di, dp, _ = tracker.softmax(_dev(tracker, semi), _dev(tracker, scale))
+    di, dp, _ = tracker.softmax(dev(tracker, semi), dev(tracker, scale))
     tracker.nms(rows, cols, di, dp)
     got = tracker.top_n(di, dp, N, mv)
     gi, gp = di.cpu().numpy(), dp.cpu().numpy()

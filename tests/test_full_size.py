@@ -8,24 +8,19 @@ modules stop at KITTI-sized or smaller ones.
     n_words, n_steps) tiles of fb = ceil(n_steps / t) frames): mv_landmarks_sequence at fb = 9, 2, 8 and 20, the
     speculation over 8 blocks of the bench sequence, and the whole landmark path on the 4 541-frame bench sequence.
 """
-import copy
 import os
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pytest
 
-from landmark_reference import back_project, detect, landmark_reference, pair_record, table_xyz, track_cfg
+from helpers import dev, pinned, ref_vocab, upload_table, with_first_pair
+from landmark_reference import (back_project, detect, landmark_reference, orc_landmarks_sequence, pair_record, table_xyz,
+                                track_cfg)
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 THREADS = os.cpu_count() or 1
 ROWS, COLS, PERMILLE, SEED = 94, 310, 850, 0     # tools/stress_bench.py
 f32 = np.float32
-
-
-def _ref_vocab():
-    v = np.load(os.path.join(GOLDEN, "ref_vocab.npz"))
-    return v["base_desc"], v["scale"], v["bias"], v["leaves"]
 
 
 def _stress_params(first_pair=0, tc=True, lanes=1):
@@ -48,23 +43,6 @@ def _tiles(n_words, n_steps):
     t = max(1, min(512, (1 << 24) // n_words, n_steps))
     fb = -(-n_steps // t)
     return -(-n_steps // fb), fb
-
-
-def _params(p, first_pair):
-    q = copy.copy(p)
-    q.pnp = copy.copy(p.pnp)
-    q.pnp.first_pair = first_pair
-    return q
-
-
-def _dev(tr, a):
-    import torch
-    return torch.from_numpy(np.ascontiguousarray(a)).to(tr.device)
-
-
-def _pinned(t):
-    import torch
-    return torch.empty(t.shape, dtype=t.dtype, pin_memory=True).copy_(t)
 
 
 # ------------------------------------------------------------------ CPU: the oracle of the stress legs
@@ -131,7 +109,7 @@ def test_stress_depth_path_vs_oracle(tracker, oracle, synth, stress_refs, monkey
     _check_parity(want, ref, "tcgen05")
     assert run(tc=False).tobytes() == want.tobytes(), "dp4a"
     _check_parity(run(lanes=32), stress_refs[(first, 32)], "lanes 32")
-    host = [_pinned(t) for t in (semi, scale, desc, depth)]
+    host = [pinned(t) for t in (semi, scale, desc, depth)]
     for chunk in (None, "3"):
         if chunk:
             monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", chunk)
@@ -149,7 +127,7 @@ def lm_tracker():
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import tracking
     tr = tracking.Tracker(0)
-    tr.bow_set_vocabulary(*_ref_vocab())
+    tr.bow_set_vocabulary(*ref_vocab())
     return tr
 
 
@@ -164,7 +142,7 @@ def test_stress_landmark_path_vs_reference(lm_tracker, oracle, synth):
     dscale = torch.full((n,), float(synth.DESC_SCALE), device=tr.device)
     frames = (semi, sscale, desc, dscale, depth)
     p = _stress_params()
-    rec, nl, table = landmark_reference(oracle, oracle.bow_vocab(*_ref_vocab()), p,
+    rec, nl, table = landmark_reference(oracle, oracle.bow_vocab(*ref_vocab()), p,
                                         *[t.cpu().numpy() for t in frames], n_words=10000, threads=THREADS)
     assert (rec["num_matches"] > 5000).all() and (nl > 0).all()
     t_dev = tr.landmarks_new(10000)
@@ -172,32 +150,12 @@ def test_stress_landmark_path_vs_reference(lm_tracker, oracle, synth):
     assert res.cpu().numpy().tobytes() == rec.tobytes()
     assert (got_nl.cpu().numpy() == nl).all() and t_dev.cpu().numpy().tobytes() == table.tobytes()
     t_host = tr.landmarks_new(10000)
-    res, got_nl, _, _ = tr.track_sequence_landmarks_host(p, *[_pinned(t) for t in frames], t_host)
+    res, got_nl, _, _ = tr.track_sequence_landmarks_host(p, *[pinned(t) for t in frames], t_host)
     assert res.tobytes() == rec.tobytes()
     assert (got_nl == nl).all() and t_host.cpu().numpy().tobytes() == table.tobytes()
 
 
 # ------------------------------------------------------------------ E: sequence sorts whose tiles span several frames
-def orc_sequence(oracle, table, first_frame, word, q_count, coords, snapshot_at=()):
-    """landmark_reference.orc_landmarks_sequence with its lookup vectorised; table updated in place.  Also returns
-    copies of the table right after the steps in snapshot_at."""
-    n_steps, top_n = word.shape
-    out = np.zeros((n_steps, top_n, 3), np.float32)
-    snaps = {}
-    for f in range(n_steps):
-        k = min(int(q_count[f]), top_n)
-        w = word[f, :k]
-        oracle.pool_observe(table, first_frame + f, w, coords[f, :k])
-        oracle.pool_remove_old(table, first_frame + f)
-        ok = (w >= 0) & (w < len(table))
-        wc = np.where(ok, w, 0)
-        ok &= table["word_id"][wc] == wc
-        out[f, :k][ok] = table["coords"][wc[ok]]
-        if f in snapshot_at:
-            snaps[f] = table.copy()
-    return out, snaps
-
-
 def _stream(oracle, name):
     """Words, counts and coordinates of one table sequence, its entry table (None: empty) and tiling."""
     n, top_n, n_words, first, seed = {"bench": (4541, 1000, 10000, 7000, 41), "fb2": (513, 300, 10000, 0, 42),
@@ -221,8 +179,8 @@ def _stream(oracle, name):
     entry = None
     if name == "bench":                  # a live entry table: 30 frames before the sequence
         entry = oracle.pool_new(n_words)
-        orc_sequence(oracle, entry, first - 30, rng.integers(0, n_words, (30, top_n)).astype(np.int32),
-                     np.full(30, top_n, np.int32), rng.standard_normal((30, top_n, 3), dtype=np.float32))
+        orc_landmarks_sequence(oracle, entry, first - 30, rng.integers(0, n_words, (30, top_n)).astype(np.int32),
+                               np.full(30, top_n, np.int32), rng.standard_normal((30, top_n, 3), dtype=np.float32))
     return dict(n_words=n_words, first=first, word=word, qc=qc, coords=coords, entry=entry,
                 tiles=_tiles(n_words, n))
 
@@ -237,7 +195,7 @@ class _Streams:
         if name not in self.done:
             c = _stream(self.oracle, name)
             table = self.oracle.pool_new(c["n_words"]) if c["entry"] is None else c["entry"].copy()
-            c["out"], _ = orc_sequence(self.oracle, table, c["first"], c["word"], c["qc"], c["coords"])
+            c["out"] = orc_landmarks_sequence(self.oracle, table, c["first"], c["word"], c["qc"], c["coords"])
             c["table"] = table
             self.done[name] = c
         return self.done[name]
@@ -251,7 +209,7 @@ def streams(oracle):
 def _entry_table(tr, c):
     if c["entry"] is None:
         return tr.landmarks_new(c["n_words"])
-    return _dev(tr, c["entry"].view(np.uint8).reshape(-1, 56))
+    return upload_table(tr, c["entry"])
 
 
 def _same_table(t_dev, table):
@@ -271,8 +229,8 @@ def test_landmarks_sequence_tiles_of_several_frames(tracker, streams, case, tili
     c = streams(case)
     assert c["tiles"] == tiling
     table = _entry_table(tracker, c)
-    out = tracker.landmarks_sequence(table, c["first"], _dev(tracker, c["word"]), _dev(tracker, c["qc"]),
-                                     _dev(tracker, c["coords"]))
+    out = tracker.landmarks_sequence(table, c["first"], dev(tracker, c["word"]), dev(tracker, c["qc"]),
+                                     dev(tracker, c["coords"]))
     assert np.array_equal(out.cpu().numpy().view(np.int32), c["out"].view(np.int32))
     assert _same_table(table, c["table"])
     if case == "bench":
@@ -291,7 +249,7 @@ def test_speculate_resolve_blocks_of_the_bench_stream(tracker, streams, n_warm):
     n = c["word"].shape[0]
     blocks = [tracking.shard_pairs(n - 1, 8, r)[:2] for r in range(8)]
     blocks[-1] = (blocks[-1][0], n - blocks[-1][0])
-    word, qc, coords = (_dev(tracker, c[k]) for k in ("word", "qc", "coords"))
+    word, qc, coords = (dev(tracker, c[k]) for k in ("word", "qc", "coords"))
     specs = {}
     for r in reversed(range(8)):
         lo, cnt = blocks[r]
@@ -348,7 +306,7 @@ def test_landmark_path_bench_sequence(lm_tracker, oracle, synth):
     res, nl, final = res.cpu().numpy(), nl.cpu().numpy(), table.cpu().numpy()
 
     blocks = [tracking.shard_pairs(NF - 1, 8, r)[:2] for r in range(8)]
-    prepared = [tr.track_landmarks_prepare(_params(p, lo), 0, lo, *[x[lo:lo + cnt + 1] for x in frames], n_words)
+    prepared = [tr.track_landmarks_prepare(with_first_pair(p, lo), 0, lo, *[x[lo:lo + cnt + 1] for x in frames], n_words)
                 for lo, cnt in blocks]
     t_blk = tr.landmarks_new(n_words)
     got, got_nl = [], []
@@ -366,7 +324,7 @@ def test_landmark_path_bench_sequence(lm_tracker, oracle, synth):
     word, _ = tr.bow_assign(desc[:NF - 1], dscale[:NF - 1], qp[:NF - 1], qc[:NF - 1])
     qp, qi, qc, word, hdepth = (t.cpu().numpy() for t in (qp, qi, qc, word, depth))
     del semi, desc, frames
-    vocab = oracle.bow_vocab(*_ref_vocab())
+    vocab = oracle.bow_vocab(*ref_vocab())
 
     def oracle_frame(f):
         return oracle.synth_frame(SEED, rows, cols, f, int(off[f, 0]), int(off[f, 1]))

@@ -4,12 +4,11 @@ test_oracle_vs_ref.py) and against the golden vectors produced by the reference 
 Bit-exact for integers, indices, candidate/match lists (incl. tie order) and the fp32 of
 the detector / RANSAC / SVD; the Gauss-Newton PnP is held to 1e-5 rad / 1e-5 relative
 against its (reference-unpinned) oracle."""
-import ctypes as C
-
 import numpy as np
 import pytest
 
 from conftest import bits
+from helpers import pnp_params
 from oracle import orc
 
 pytestmark = pytest.mark.gpu
@@ -279,15 +278,6 @@ def test_matmul_shim(tk, kat):
 
 
 # ------------------------------------------------------------------ Gauss-Newton PnP
-def _pnp_params(tk, H, lanes, seed=0, refine=10, sample_size=8):
-    from maveric_slam_b200 import lib
-    p = lib.PnpParams()
-    lib.load().mv_pnp_params_default(C.byref(p))
-    p.hypotheses, p.lanes_per_hypothesis, p.seed, p.refine_iters = H, lanes, seed, refine
-    p.sample_size = sample_size
-    return p
-
-
 # lanes = 1: one thread per hypothesis (two-phase kernel for n <= 480, streaming kernel above); lanes = 32: one warp
 # per hypothesis.
 def _pnp_lane_forms():
@@ -322,7 +312,7 @@ def test_pnp_gn_vs_oracle(tracker, tk, oracle, synth, monkeypatch, lanes, sample
         corr[p] = c
         truth.append(pose)
     cnt = np.full(P, n, np.int32)
-    prm = _pnp_params(tk, H, lanes, seed=4, sample_size=sample_size)
+    prm = pnp_params(H, lanes, seed=4, sample_size=sample_size)
     cfg = orc.pnp_cfg(hypotheses=H, seed=4, lanes=lanes, sample_size=sample_size)
     want = _oracle_pnp(oracle, cfg, corr, n)
     for gpw in ("1", "2"):
@@ -364,7 +354,7 @@ def test_pnp_gn_4096_hypotheses_vs_oracle(tracker, tk, oracle, synth):
     import torch
     H, n, P = 4096, 16384, 2
     corr = np.stack([synth.synth_pnp_problem(200 + p, n)[0] for p in range(P)])
-    pose, stats, _ = tracker.pnp_gn(_pnp_params(tk, H, 1, seed=4), torch.from_numpy(corr).to(tracker.device),
+    pose, stats, _ = tracker.pnp_gn(pnp_params(H, 1, seed=4), torch.from_numpy(corr).to(tracker.device),
                                     torch.full((P,), n, dtype=torch.int32, device=tracker.device))
     pose, stats = pose.cpu().numpy(), stats.cpu().numpy()
     for p, (rp, rs, _) in enumerate(_oracle_pnp(oracle, orc.pnp_cfg(hypotheses=H, seed=4, lanes=1), corr, n,
@@ -381,7 +371,7 @@ def test_pnp_gn_empty_and_init(tracker, tk, oracle):
     corr = torch.zeros((2, 5, 16), device=tracker.device)
     cnt = torch.zeros((2,), dtype=torch.int32, device=tracker.device)
     init = torch.tensor([[1, 0, 0, 0, 0.1, 0.2, 0.3], [1, 0, 0, 0, 0, 0, 0]], dtype=torch.float32, device=tracker.device)
-    pose, stats, _ = tracker.pnp_gn(_pnp_params(tk, 32, 1), corr, cnt, init_pose=init)
+    pose, stats, _ = tracker.pnp_gn(pnp_params(32, 1), corr, cnt, init_pose=init)
     assert (pose.cpu().numpy() == init.cpu().numpy()).all() and (stats.cpu().numpy()[:, 3] == 0).all()
 
 
@@ -397,7 +387,7 @@ CAMERA_PNP = dict(fx=520.0, fy=910.0, cx=300.5, cy=260.25, gate_sq=16.0, damping
     pytest.param(47, 155, 1000, 1024, 8192, 64, {}, id="47-155-1000-1024-8192-64"),
     pytest.param(47, 155, 1000, 1024, 8192, 288, CAMERA_PNP, id="camera"),
 ])
-def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, rows, cols, N, M, mv, H, pnp):
+def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, monkeypatch, rows, cols, N, M, mv, H, pnp):
     import torch
     n_frames, seed = 4, 13
     off = synth.default_offsets(n_frames, seed)
@@ -411,12 +401,8 @@ def test_track_sequence_vs_oracle(tracker, tk, oracle, synth, rows, cols, N, M, 
     # same through host buffers (the e2e entry point)
     res_h, up, down = tracker.track_sequence_host(p, hs, np.full(n_frames, synth.SEMI_SCALE, np.float32), hd, hz)
     assert res_h.tobytes() == res.tobytes() and down == 64 * (n_frames - 1)
-    import os
-    os.environ["MV_HOST_CHUNK_PAIRS"] = "2"     # chunked staging must not change any result
-    try:
-        res_c, _, _ = tracker.track_sequence_host(p, hs, np.full(n_frames, synth.SEMI_SCALE, np.float32), hd, hz)
-    finally:
-        del os.environ["MV_HOST_CHUNK_PAIRS"]
+    monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", "2")     # chunked staging must not change any result
+    res_c, _, _ = tracker.track_sequence_host(p, hs, np.full(n_frames, synth.SEMI_SCALE, np.float32), hd, hz)
     assert res_c.tobytes() == res.tobytes()
     cfg = orc.TrackCfg(orc.MatchCfg(rows, cols, 4, 4, 4, M, 0.9, 0.2), orc.pnp_cfg(hypotheses=H, seed=0, lanes=1, **pnp),
                        N, mv, 10, 1.1, float(synth.SEMI_SCALE))

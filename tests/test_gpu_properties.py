@@ -8,10 +8,11 @@ result from the entry point (device-resident vs host buffers).  Everything goes 
   configs[4]  4096 hypotheses (the 16k-keypoint matcher shape is in test_gpu_parity.py)
 """
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
+
+from helpers import pinned, pnp_params, pnp_problems
 
 pytestmark = pytest.mark.gpu
 
@@ -24,62 +25,31 @@ def tk(tracker):
     return tracking
 
 
-def _pnp_params(H, lanes=1, seed=0):
-    from maveric_slam_b200 import lib
-    p = lib.PnpParams()
-    lib.load().mv_pnp_params_default(C.byref(p))
-    p.hypotheses, p.lanes_per_hypothesis, p.seed = H, lanes, seed
-    return p
-
-
-def _problems(synth, P, n, stride):
-    corr = np.zeros((P, 5, stride), np.float32)
-    for p in range(P):
-        corr[p], _, _ = synth.synth_pnp_problem(500 + p, n, stride=stride)
-    return corr
-
-
-class _Env:
-    """An environment variable for the duration of a block (the library reads its knobs per call)."""
-
-    def __init__(self, name, value):
-        self.name, self.value = name, value
-
-    def __enter__(self):
-        self.old = os.environ.get(self.name)
-        os.environ[self.name] = self.value
-
-    def __exit__(self, *a):
-        if self.old is None:
-            del os.environ[self.name]
-        else:
-            os.environ[self.name] = self.old
-
-
 @pytest.mark.parametrize("n,stride", [(1000, 1024), (330, 1024), (480, 480), (481, 512), (513, 640), (31, 32), (3, 1024)])
-def test_pnp_forms_return_identical_bytes(tracker, synth, n, stride):
+def test_pnp_forms_return_identical_bytes(tracker, synth, monkeypatch, n, stride):
     """configs[2]: the product's two one-thread-per-hypothesis kernels -- the two-phase kernel (gate every
     slot, re-deal by exact count, packed-FFMA2 walk; pairs of up to 480 correspondences) and the streaming
     kernel (larger pairs; MV_PNP_STREAM=1 forces it for every pair) -- with 128 or 256 hypotheses per CTA:
     same bytes for every one of 1024 hypotheses and for the selected pose."""
     import torch
     P, H = 3, 1024
-    corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
+    corr = torch.from_numpy(pnp_problems(synth, P, n, stride)).to(tracker.device)
     cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
 
     def run():
-        pose, stats, hyp = tracker.pnp_gn(_pnp_params(H), corr, cnt, want_hyp=True)
+        pose, stats, hyp = tracker.pnp_gn(pnp_params(H), corr, cnt, want_hyp=True)
         return (pose.cpu().numpy().tobytes(), stats.cpu().numpy().tobytes(), hyp.cpu().numpy().tobytes())
 
     want = run()
     for gpw in ("1", "2"):
-        with _Env("MV_PNP_GPW", gpw):
+        with monkeypatch.context() as m:
+            m.setenv("MV_PNP_GPW", gpw)
             assert run() == want, ("two-phase", gpw)
-            with _Env("MV_PNP_STREAM", "1"):
-                assert run() == want, ("streaming", gpw)
+            m.setenv("MV_PNP_STREAM", "1")
+            assert run() == want, ("streaming", gpw)
 
 
-def test_pnp_split_launch_returns_identical_bytes(tracker, synth):
+def test_pnp_split_launch_returns_identical_bytes(tracker, synth, monkeypatch):
     """How K3 cuts a batch into CTAs does not change a byte: 128-hypothesis CTAs for every pair (short
     launches), 256-hypothesis CTAs for every pair, or the split launch (the shortest pairs of the
     longest-first order as 128-hypothesis CTAs in a programmatic dependent launch) -- on a batch whose pairs differ in
@@ -87,21 +57,22 @@ def test_pnp_split_launch_returns_identical_bytes(tracker, synth):
     import torch
     P, stride, H = 11, 1024, 1024
     counts = [330, 5, 0, 480, 600, 17, 330, 1000, 128, 3, 250]
-    corr = torch.from_numpy(_problems(synth, P, 1000, stride)).to(tracker.device)
+    corr = torch.from_numpy(pnp_problems(synth, P, 1000, stride)).to(tracker.device)
     cnt = torch.tensor(counts, dtype=torch.int32, device=tracker.device)
 
     def run():
-        pose, stats, hyp = tracker.pnp_gn(_pnp_params(H), corr, cnt, want_hyp=True)
+        pose, stats, hyp = tracker.pnp_gn(pnp_params(H), corr, cnt, want_hyp=True)
         return (pose.cpu().numpy().tobytes(), stats.cpu().numpy().tobytes(), hyp.cpu().numpy().tobytes())
 
     want = run()                                   # 11 pairs: every pair as 128-hypothesis CTAs
-    with _Env("MV_PNP_K3_SMALL_BELOW", "0"):       # never the short-launch form
-        assert run() == want, "split launch, 5 tail pairs"
-        for tail in ("0", "1", "3"):
-            with _Env("MV_PNP_TAIL_PAIRS", tail):
-                assert run() == want, ("tail pairs", tail)
-        with _Env("MV_PNP_ORDER", "0"):            # index order: no split
-            assert run() == want, "index order"
+    monkeypatch.setenv("MV_PNP_K3_SMALL_BELOW", "0")   # never the short-launch form
+    assert run() == want, "split launch, 5 tail pairs"
+    for tail in ("0", "1", "3"):
+        with monkeypatch.context() as m:
+            m.setenv("MV_PNP_TAIL_PAIRS", tail)
+            assert run() == want, ("tail pairs", tail)
+    monkeypatch.setenv("MV_PNP_ORDER", "0")            # index order: no split
+    assert run() == want, "index order"
 
 
 @pytest.mark.parametrize("lanes", [0, 2, 3, 4, 8, 16, 64])
@@ -111,12 +82,12 @@ def test_pnp_refuses_lanes_without_a_kernel(tracker, synth, lanes):
     import torch
     from maveric_slam_b200 import lib
     P, n, stride = 2, 100, 128
-    corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
+    corr = torch.from_numpy(pnp_problems(synth, P, n, stride)).to(tracker.device)
     cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
     pose = torch.zeros((P, 7), dtype=torch.float32, device=tracker.device)
     stats = torch.zeros((P, 4), dtype=torch.float32, device=tracker.device)
     launches = tracker.ctx.launches
-    st = tracker.lib.mv_pnp_gn_batch(tracker.ctx.h, C.byref(_pnp_params(64, lanes=lanes)), P, stride,
+    st = tracker.lib.mv_pnp_gn_batch(tracker.ctx.h, C.byref(pnp_params(64, lanes=lanes)), P, stride,
                                      tracker._d(corr), tracker._d(cnt), None, tracker._d(pose), tracker._d(stats),
                                      None)
     assert st == lib.MV_ERR_BAD_ARG, (lanes, st)
@@ -129,10 +100,10 @@ def test_pnp_hypothesis_does_not_depend_on_hypothesis_count(tracker, synth):
     the best key (inliers, then cost, then index) over the per-hypothesis records."""
     import torch
     P, n, stride = 2, 1000, 1024
-    corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
+    corr = torch.from_numpy(pnp_problems(synth, P, n, stride)).to(tracker.device)
     cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
-    pose4, stats4, hyp4 = tracker.pnp_gn(_pnp_params(4096), corr, cnt, want_hyp=True)
-    pose1, stats1, hyp1 = tracker.pnp_gn(_pnp_params(1024), corr, cnt, want_hyp=True)
+    pose4, stats4, hyp4 = tracker.pnp_gn(pnp_params(4096), corr, cnt, want_hyp=True)
+    pose1, stats1, hyp1 = tracker.pnp_gn(pnp_params(1024), corr, cnt, want_hyp=True)
     hyp4, hyp1 = hyp4.cpu().numpy(), hyp1.cpu().numpy()
     assert hyp4[:, :1024].tobytes() == hyp1.tobytes()
     stats4, pose4 = stats4.cpu().numpy(), pose4.cpu().numpy()
@@ -151,12 +122,12 @@ def test_pnp_pair_does_not_depend_on_batch(tracker, synth):
     with first_pair = 0 and 3 (what sharding across GPUs and chunked staging rely on)."""
     import torch
     P, n, stride, H = 6, 700, 1024, 512
-    corr = torch.from_numpy(_problems(synth, P, n, stride)).to(tracker.device)
+    corr = torch.from_numpy(pnp_problems(synth, P, n, stride)).to(tracker.device)
     cnt = torch.full((P,), n, dtype=torch.int32, device=tracker.device)
-    pose, stats, _ = tracker.pnp_gn(_pnp_params(H), corr, cnt)
+    pose, stats, _ = tracker.pnp_gn(pnp_params(H), corr, cnt)
     parts = []
     for first in (0, 3):
-        prm = _pnp_params(H)
+        prm = pnp_params(H)
         prm.first_pair = first
         pp, ss, _ = tracker.pnp_gn(prm, corr[first:first + 3].contiguous(), cnt[first:first + 3].contiguous())
         parts.append((pp.cpu().numpy(), ss.cpu().numpy()))
@@ -179,21 +150,21 @@ def test_pnp_ragged_counts_and_work_counter(tracker, synth):
     dcnt = torch.tensor(counts, dtype=torch.int32, device=tracker.device)
     tracker.ctx.profile(True)
     tracker.ctx.pnp_work()
-    pose, stats, hyp = tracker.pnp_gn(_pnp_params(H), dcorr, dcnt, want_hyp=True)
+    pose, stats, hyp = tracker.pnp_gn(pnp_params(H), dcorr, dcnt, want_hyp=True)
     work = tracker.ctx.pnp_work()
     tracker.ctx.profile(False)
     assert 0 < work <= H * sum(counts) * 10
     pose, stats = pose.cpu().numpy(), stats.cpu().numpy()
     assert stats[0, 3] == 0 and (pose[0] == np.array([1, 0, 0, 0, 0, 0, 0], np.float32)).all()
     for p, n in enumerate(counts):
-        prm = _pnp_params(H)
+        prm = pnp_params(H)
         prm.first_pair = p
         p1, s1, _ = tracker.pnp_gn(prm, dcorr[p:p + 1].contiguous(), dcnt[p:p + 1].contiguous())
         assert p1.cpu().numpy().tobytes() == pose[p:p + 1].tobytes(), n
         assert s1.cpu().numpy().tobytes() == stats[p:p + 1].tobytes(), n
 
 
-def test_sequence_full_config_properties(tracker, tk, synth):
+def test_sequence_full_config_properties(tracker, tk, synth, monkeypatch):
     """configs[3] at its real parameters (47x155 cells, top-1000 queries, 1024 matches, 1024
     hypotheses), 97 frames: two runs are identical (determinism); two shards with one halo frame
     and first_pair = 0 / 48 reproduce the unsharded records (multi-GPU sharding); the host-buffer
@@ -222,10 +193,7 @@ def test_sequence_full_config_properties(tracker, tk, synth):
     dp4a = tracker.track_sequence(params(tc=False), semi, scale, desc, depth).cpu().numpy()
     assert dp4a.tobytes() == full.tobytes()
 
-    hs = torch.empty(semi.shape, dtype=torch.int8, pin_memory=True).copy_(semi)
-    hd = torch.empty(desc.shape, dtype=torch.int8, pin_memory=True).copy_(desc)
-    hz = torch.empty(depth.shape, dtype=torch.float32, pin_memory=True).copy_(depth)
-    hsc = torch.empty(scale.shape, dtype=torch.float32, pin_memory=True).copy_(scale)
+    hs, hsc, hd, hz = (pinned(t) for t in (semi, scale, desc, depth))
     torch.cuda.synchronize()
     host, up, down = tracker.track_sequence_host(params(), hs, hsc, hd, hz)
     assert host.tobytes() == full.tobytes() and down == 64 * (n_frames - 1)
@@ -233,11 +201,8 @@ def test_sequence_full_config_properties(tracker, tk, synth):
     assert up < semi.numel() + 4 * depth.numel() + desc.numel() // 2
     # the chunk size of the staging pipeline must not change a byte (7: a last chunk of 5 pairs; 40: 40 + 40 + 16)
     for chunk_pairs in ("7", "40"):
-        os.environ["MV_HOST_CHUNK_PAIRS"] = chunk_pairs
-        try:
-            chunked, _, _ = tracker.track_sequence_host(params(), hs, hsc, hd, hz)
-        finally:
-            del os.environ["MV_HOST_CHUNK_PAIRS"]
+        monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", chunk_pairs)
+        chunked, _, _ = tracker.track_sequence_host(params(), hs, hsc, hd, hz)
         assert chunked.tobytes() == full.tobytes(), chunk_pairs
 
 
@@ -376,7 +341,7 @@ def test_contexts_of_two_gpus_from_one_thread(synth):
     thread's current device left on GPU 0 throughout, return the bytes a single-GPU run returns."""
     import torch
     if not torch.cuda.is_available() or torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     from maveric_slam_b200 import tracking
     rows, cols, n_frames = 24, 80, 5
     off = synth.default_offsets(n_frames, 3)

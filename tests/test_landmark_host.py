@@ -8,65 +8,31 @@ needs, computed here from the public detector outputs.
 The device one-call is itself held to a CPU reference of the whole path, tests/landmark_reference.py
 (tests/test_landmark_reference.py)."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
 
-from test_landmark_sequence import N_FRAMES, _table_bytes
+from helpers import FIRST, N_FRAMES, landmark_sequence, landmarks_host, table_bytes
 
 pytestmark = pytest.mark.gpu
-
-ROWS, COLS, FIRST = 47, 155, 500
-
-
-def _pinned(torch, t):
-    h = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
-    h.copy_(t)
-    return h
 
 
 @pytest.fixture(scope="module")
 def lmseq(tracker, synth):
     """A 66-frame KITTI-shaped sequence, its pinned host copies, and the device landmark path's answer from an
     empty table at frame 500."""
-    import torch
-    from maveric_slam_b200 import tracking
-    v = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_vocab.npz"))
-    tracker.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    n = N_FRAMES
-    p = tracking.kitti_track_params(hypotheses=256)
-    semi, desc, depth = tracker.synth_frames(21, ROWS, COLS, 0, synth.default_offsets(n, 21))
-    sscale = torch.full((n,), float(synth.SEMI_SCALE), device=tracker.device)
-    dscale = torch.full((n,), 4.3353, device=tracker.device)
-    table = tracker.landmarks_new(tracker.n_words)
-    res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=FIRST)
-    h = dict(semi=_pinned(torch, semi), sscale=_pinned(torch, sscale), desc=_pinned(torch, desc),
-             dscale=_pinned(torch, dscale), depth=_pinned(torch, depth))
-    torch.cuda.synchronize()
-    return dict(p=p, d=dict(semi=semi, sscale=sscale, desc=desc, dscale=dscale, depth=depth), h=h,
-                n_words=tracker.n_words, res=res.cpu().numpy().tobytes(), nl=nl.cpu().numpy(), table=_table_bytes(table))
-
-
-def _host(tracker, s, h=None, first=FIRST, lo=0, hi=N_FRAMES, table=None, p=None):
-    from maveric_slam_b200 import tracking
-    h = h or s["h"]
-    table = tracker.landmarks_new(s["n_words"]) if table is None else table
-    p = p or (s["p"] if lo == 0 else tracking.kitti_track_params(hypotheses=256, first_pair=lo))
-    res, nl, up, down = tracker.track_sequence_landmarks_host(
-        p, h["semi"][lo:hi], h["sscale"][lo:hi], h["desc"][lo:hi], h["dscale"][lo:hi], h["depth"][lo:hi], table,
-        first_frame=first)
-    return res, nl, table, up, down
+    s = landmark_sequence(tracker, synth, host=True)
+    return dict(s, res=s["res"].tobytes())
 
 
 def _assert_equal_device(s, res, nl, table, what=""):
     assert res.tobytes() == s["res"], what
     assert nl.tobytes() == s["nl"].tobytes(), what
-    assert _table_bytes(table) == s["table"], what
+    assert table_bytes(table) == s["table"], what
 
 
 def test_host_equals_device(tracker, lmseq):
-    res, nl, table, _, down = _host(tracker, lmseq)
+    res, nl, table, _, down = landmarks_host(tracker, lmseq)
     _assert_equal_device(lmseq, res, nl, table)
     assert down == 68 * (N_FRAMES - 1)
     assert (nl > 0).all()
@@ -76,7 +42,7 @@ def test_host_equals_device(tracker, lmseq):
 def test_chunk_size_changes_nothing(tracker, lmseq, monkeypatch, chunk):
     # 1: one-pair chunks (every chunk a single table step); 7: a short last chunk of 2; 40: 40 + 25
     monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", chunk)
-    res, nl, table, _, _ = _host(tracker, lmseq)
+    res, nl, table, _, _ = landmarks_host(tracker, lmseq)
     _assert_equal_device(lmseq, res, nl, table, chunk)
 
 
@@ -84,13 +50,13 @@ def test_staging_mode_changes_nothing(tracker, lmseq, monkeypatch):
     import torch
     h = lmseq["h"]
     monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", "9")
-    _, _, _, up_gather, _ = _host(tracker, lmseq)
+    _, _, _, up_gather, _ = landmarks_host(tracker, lmseq)
     pageable = {k: v.numpy().copy() for k, v in h.items()}
-    res, nl, table, up_pageable, _ = _host(tracker, lmseq, h=pageable)
+    res, nl, table, up_pageable, _ = landmarks_host(tracker, lmseq, h=pageable)
     _assert_equal_device(lmseq, res, nl, table, "pageable")
     with monkeypatch.context() as m:
         m.setenv("MV_HOST_GATHER", "0")
-        res, nl, table, up_copy, _ = _host(tracker, lmseq)
+        res, nl, table, up_copy, _ = landmarks_host(tracker, lmseq)
         _assert_equal_device(lmseq, res, nl, table, "MV_HOST_GATHER=0")
     assert up_copy == up_pageable
     # a depth buffer 4 bytes off a 16-byte boundary
@@ -99,7 +65,7 @@ def test_staging_mode_changes_nothing(tracker, lmseq, monkeypatch):
     odd = buf[1:1 + n * cells].view(n, cells)
     odd.copy_(h["depth"])
     assert odd.data_ptr() % 16 == 4
-    res, nl, table, up_odd, _ = _host(tracker, lmseq, h=dict(h, depth=odd))
+    res, nl, table, up_odd, _ = landmarks_host(tracker, lmseq, h=dict(h, depth=odd))
     _assert_equal_device(lmseq, res, nl, table, "unaligned depth")
     assert up_odd == up_gather < up_copy
 
@@ -111,13 +77,13 @@ def test_resume_and_halo(tracker, lmseq):
     table = tracker.landmarks_new(s["n_words"])
     res_a, nl_a = tracker.track_sequence_landmarks(s["p"], d["semi"][:k + 1], d["sscale"][:k + 1], d["desc"][:k + 1],
                                                    d["dscale"][:k + 1], d["depth"][:k + 1], table, first_frame=FIRST)
-    res_b, nl_b, table, _, _ = _host(tracker, s, first=FIRST + k, lo=k, table=table)
+    res_b, nl_b, table, _, _ = landmarks_host(tracker, s, first=FIRST + k, lo=k, table=table)
     res = np.concatenate([res_a.cpu().numpy().reshape(-1), res_b.view(np.uint8).reshape(-1)])
     _assert_equal_device(s, res, np.concatenate([nl_a.cpu().numpy(), nl_b]), table, "device then host")
     # two host calls sharing a halo frame
     table = tracker.landmarks_new(s["n_words"])
-    res_a, nl_a, table, _, _ = _host(tracker, s, hi=k + 1, table=table)
-    res_b, nl_b, table, _, _ = _host(tracker, s, first=FIRST + k, lo=k, table=table,
+    res_a, nl_a, table, _, _ = landmarks_host(tracker, s, hi=k + 1, table=table)
+    res_b, nl_b, table, _, _ = landmarks_host(tracker, s, first=FIRST + k, lo=k, table=table,
                                      p=tracking.kitti_track_params(hypotheses=256, first_pair=k))
     _assert_equal_device(s, np.concatenate([res_a, res_b]), np.concatenate([nl_a, nl_b]), table, "host then host")
 
@@ -127,7 +93,7 @@ def test_byte_accounting(tracker, lmseq, monkeypatch):
     candidate-or-query cell (the word assignment reads query rows only)."""
     s, p, chunk = lmseq, lmseq["p"], 9
     monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", str(chunk))
-    res, nl, _, up, down = _host(tracker, s)
+    res, nl, _, up, down = landmarks_host(tracker, s)
     assert res.tobytes() == s["res"]
     idx, prob, _ = tracker.softmax(s["d"]["semi"], s["d"]["sscale"])
     qp, _, _, qc, _ = tracker.top_n(idx, prob, p.top_n, p.max_valid)
@@ -153,34 +119,28 @@ def test_byte_accounting(tracker, lmseq, monkeypatch):
         tracker.ctx.h, C.byref(p), n, FIRST, *inputs, s["n_words"], tracker._d(table), out.ctypes.data_as(C.c_void_p),
         None, C.byref(u), C.byref(dn)))
     assert out.tobytes() == s["res"] and u.value == up and dn.value == 64 * n_pairs
-    assert _table_bytes(table) == s["table"]
+    assert table_bytes(table) == s["table"]
 
 
 def test_degenerate_frames(tracker, synth):
     """Frames without keypoints (2, 3), with saturated (5) and zero (7) descriptors, at a 24x80 grid: the host path
     equals the device landmark path, from pinned and from pageable buffers."""
-    import torch
     from maveric_slam_b200 import tracking
-    v = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_vocab.npz"))
-    tracker.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    rows, cols, n, seed = 24, 80, 9, 2
-    semi, desc, depth = tracker.synth_frames(seed, rows, cols, 0, synth.default_offsets(n, seed))
-    semi[2:4] = -5
-    desc[5] = -128
-    desc[7] = 0
-    sscale = torch.full((n,), float(synth.SEMI_SCALE), device=tracker.device)
-    dscale = torch.full((n,), 4.3353, device=tracker.device)
-    p = tracking.track_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=64)
-    table = tracker.landmarks_new(tracker.n_words)
-    res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=7)
-    want = (res.cpu().numpy().tobytes(), nl.cpu().numpy().tobytes(), _table_bytes(table))
-    assert tracking.results_to_numpy(res)[1:4]["num_matches"].tolist() == [0, 0, 0]
-    pinned = [_pinned(torch, t) for t in (semi, sscale, desc, dscale, depth)]
-    torch.cuda.synchronize()
-    for bufs in (pinned, [t.cpu().numpy() for t in (semi, sscale, desc, dscale, depth)]):
+
+    def degenerate(semi, desc, depth):
+        semi[2:4] = -5
+        desc[5] = -128
+        desc[7] = 0
+
+    p = tracking.track_params(24, 80, top_n=100, max_valid=1000, max_matches=150, hypotheses=64)
+    s = landmark_sequence(tracker, synth, n_frames=9, rows=24, cols=80, seed=2, params=p, first_frame=7,
+                          edit=degenerate, host=True)
+    want = (s["res"].tobytes(), s["nl"].tobytes(), s["table"])
+    assert s["res"][1:4]["num_matches"].tolist() == [0, 0, 0]
+    for bufs in (s["h"].values(), [t.cpu().numpy() for t in s["d"].values()]):
         t2 = tracker.landmarks_new(tracker.n_words)
         r2, nl2, _, _ = tracker.track_sequence_landmarks_host(p, *bufs, t2, first_frame=7)
-        assert (r2.tobytes(), nl2.tobytes(), _table_bytes(t2)) == want
+        assert (r2.tobytes(), nl2.tobytes(), table_bytes(t2)) == want
 
 
 def test_depth_path_untouched(tracker, lmseq):
@@ -188,7 +148,7 @@ def test_depth_path_untouched(tracker, lmseq):
     h = lmseq["h"]
     p = tracking.kitti_track_params(hypotheses=256)
     before = tracker.track_sequence_host(p, h["semi"], h["sscale"], h["desc"], h["depth"])
-    _host(tracker, lmseq)
+    landmarks_host(tracker, lmseq)
     after = tracker.track_sequence_host(p, h["semi"], h["sscale"], h["desc"], h["depth"])
     assert before[0].tobytes() == after[0].tobytes() and before[1:] == after[1:]
 
@@ -197,8 +157,8 @@ def test_argument_errors(tracker, lmseq):
     from maveric_slam_b200 import lib, tracking
     s, h = lmseq, lmseq["h"]
     table = tracker.landmarks_new(s["n_words"])
-    _host(tracker, s, hi=4, table=table)          # a non-empty table that must survive every refused call
-    before = _table_bytes(table)
+    landmarks_host(tracker, s, hi=4, table=table)          # a non-empty table that must survive every refused call
+    before = table_bytes(table)
 
     def call(tr=tracker, p=None, n=4, n_words=None, tab=table, **over):
         hb = dict(h, **over)
@@ -238,13 +198,13 @@ def test_argument_errors(tracker, lmseq):
         with pytest.raises(lib.MvError, match="bad argument"):
             call(p=p)
         assert tracker.ctx.launches == launches, field
-        assert _table_bytes(table) == before, field
-    assert _table_bytes(table) == before
+        assert table_bytes(table) == before, field
+    assert table_bytes(table) == before
     # the context still works and continues the same table
-    res, nl, table, _, _ = _host(tracker, s, first=FIRST + 3, lo=3, table=table,
+    res, nl, table, _, _ = landmarks_host(tracker, s, first=FIRST + 3, lo=3, table=table,
                                  p=tracking.kitti_track_params(hypotheses=256, first_pair=3))
     assert res.tobytes() == s["res"][3 * 64:] and nl.tobytes() == s["nl"][3:].tobytes()
-    assert _table_bytes(table) == s["table"]
+    assert table_bytes(table) == s["table"]
 
 
 def test_oversize_vocabulary_refused_up_front(tracker, lmseq):
@@ -258,13 +218,13 @@ def test_oversize_vocabulary_refused_up_front(tracker, lmseq):
     fresh.bow_set_vocabulary(np.zeros((256, 64), np.int8), np.ones(64, np.float32), np.zeros(64, np.float32),
                              np.zeros((64, 211, 4), np.int32))
     table = fresh.landmarks_new(fresh.n_words)
-    before, launches = _table_bytes(table), fresh.ctx.launches
+    before, launches = table_bytes(table), fresh.ctx.launches
     with pytest.raises(lib.MvError, match="shared memory"):
         fresh.track_sequence_landmarks(s["p"], d["semi"], d["sscale"], d["desc"], d["dscale"], d["depth"], table)
     with pytest.raises(lib.MvError, match="shared memory"):
         fresh.track_sequence_landmarks_host(s["p"], h["semi"], h["sscale"], h["desc"], h["dscale"], h["depth"], table)
     assert fresh.ctx.launches == launches
-    assert _table_bytes(table) == before
+    assert table_bytes(table) == before
     assert fresh.track_sequence(s["p"], d["semi"], d["sscale"], d["desc"], d["depth"]).cpu().numpy().tobytes() == want
     res, _, _ = fresh.track_sequence_host(s["p"], h["semi"], h["sscale"], h["desc"], h["depth"])
     assert res.tobytes() == want

@@ -14,12 +14,17 @@ import sys
 import numpy as np
 import pytest
 
-from test_landmark_host import FIRST, _host, _pinned, lmseq  # noqa: F401  (lmseq: the module's fixture)
-from test_landmark_sequence import N_FRAMES, _table_bytes
-from test_landmark_shard import WARMS, _blocks, _free_port, _StandIn
+from helpers import (FIRST, KEYS, N_FRAMES, WARMS, HostStandIn, StandIn, cycled_blocks, free_port, landmark_sequence,
+                     landmarks_host, pinned, ref_vocab, table_bytes)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-KEYS = ("semi", "sscale", "desc", "dscale", "depth")
+
+
+@pytest.fixture(scope="module")
+def lmseq(tracker, synth):
+    """The 66-frame sequence of tests/test_landmark_host.py, its pinned host copies and the device path's answer."""
+    s = landmark_sequence(tracker, synth, host=True)
+    return dict(s, res=s["res"].tobytes())
 
 
 def _params(lo):
@@ -49,7 +54,7 @@ def _chain(s, prepared, trs):
         r, nl = tr.track_landmarks_solve(b)
         res.append(r.cpu().numpy()); nls.append(nl.cpu().numpy())
         tr.track_landmarks_release(b)
-    return np.concatenate(res).tobytes(), np.concatenate(nls), _table_bytes(table)
+    return np.concatenate(res).tobytes(), np.concatenate(nls), table_bytes(table)
 
 
 def _assert_one_call(s, got, what=""):
@@ -62,25 +67,24 @@ def _assert_one_call(s, got, what=""):
 def _second(tracker, s):
     from maveric_slam_b200 import tracking
     other = tracking.Tracker(0)
-    v = np.load(os.path.join(ROOT, "tests", "golden", "ref_vocab.npz"))
-    other.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
+    other.bow_set_vocabulary(*ref_vocab())
     return other
 
 
 @pytest.mark.gpu
-def test_whole_sequence(tracker, lmseq):  # noqa: F811
+def test_whole_sequence(tracker, lmseq):
     b = _prep_host(tracker, lmseq, 0, N_FRAMES - 1, 0)
     _assert_one_call(lmseq, _chain(lmseq, [b], [tracker]))
-    res, nl, table, _, _ = _host(tracker, lmseq)
-    assert (res.tobytes(), nl.tobytes(), _table_bytes(table)) == (lmseq["res"], lmseq["nl"].tobytes(), lmseq["table"])
+    res, nl, table, _, _ = landmarks_host(tracker, lmseq)
+    assert (res.tobytes(), nl.tobytes(), table_bytes(table)) == (lmseq["res"], lmseq["nl"].tobytes(), lmseq["table"])
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("two_contexts", [False, True])
-def test_blocks_in_reverse_with_a_device_block(tracker, lmseq, two_contexts):  # noqa: F811
+def test_blocks_in_reverse_with_a_device_block(tracker, lmseq, two_contexts):
     s = lmseq
     other = _second(tracker, s) if two_contexts else tracker
-    blocks = _blocks([1, 2, 3, 7, 40], N_FRAMES - 1)
+    blocks = cycled_blocks([1, 2, 3, 7, 40], N_FRAMES - 1)
     for n_warm in WARMS:
         trs = [(tracker, other)[i % 2] for i in range(len(blocks))]
         prepared = {}
@@ -93,7 +97,7 @@ def test_blocks_in_reverse_with_a_device_block(tracker, lmseq, two_contexts):  #
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("mode", ["chunk1", "chunk7", "chunk40", "pageable", "no_gather"])
-def test_chunking_and_staging_change_nothing(tracker, lmseq, monkeypatch, mode):  # noqa: F811
+def test_chunking_and_staging_change_nothing(tracker, lmseq, monkeypatch, mode):
     s = lmseq
     h = s["h"]
     if mode.startswith("chunk"):
@@ -121,7 +125,7 @@ def _rows_per_frame(tracker, s):
 
 
 @pytest.mark.gpu
-def test_byte_accounting(tracker, lmseq, monkeypatch):  # noqa: F811
+def test_byte_accounting(tracker, lmseq, monkeypatch):
     """Block frames: per chunk of pairs (one halo frame), the logits, depth, both scales and 256 B per candidate-or-query
     row, as the one host call; warm-up frames, in chunks without a halo: logits, both scales and query rows only."""
     s, chunk = lmseq, 9
@@ -141,18 +145,18 @@ def test_byte_accounting(tracker, lmseq, monkeypatch):  # noqa: F811
         assert b["h2d_bytes"] < whole
         tracker.track_landmarks_release(b)
         if n_warm == 0:   # the same frames through the one host call move the same bytes
-            _, _, _, up, _ = _host(tracker, s, first=FIRST + lo, lo=lo, hi=lo + count + 1, p=_params(lo))
+            _, _, _, up, _ = landmarks_host(tracker, s, first=FIRST + lo, lo=lo, hi=lo + count + 1, p=_params(lo))
             assert up == want
 
 
 @pytest.mark.gpu
-def test_host_buffers_free_at_return(tracker, lmseq):  # noqa: F811
+def test_host_buffers_free_at_return(tracker, lmseq):
     import torch
     s = lmseq
     prepared = []
     for lo, c in ((0, 30), (30, 35)):
         w = min(8, lo)
-        h = {k: _pinned(torch, s["h"][k][lo - w:lo + c + 1]) for k in KEYS}
+        h = {k: pinned(s["h"][k][lo - w:lo + c + 1]) for k in KEYS}
         prepared.append(tracker.track_landmarks_prepare_host(_params(lo), w, FIRST + lo, *[h[k] for k in KEYS],
                                                              s["n_words"]))
         for k in KEYS:   # overwritten as soon as the call returns, before any later stream work
@@ -161,7 +165,7 @@ def test_host_buffers_free_at_return(tracker, lmseq):  # noqa: F811
 
 
 @pytest.mark.gpu
-def test_refusals(tracker, lmseq):  # noqa: F811
+def test_refusals(tracker, lmseq):
     from maveric_slam_b200 import lib, tracking
     s, h = lmseq, lmseq["h"]
 
@@ -207,12 +211,12 @@ def test_refusals(tracker, lmseq):  # noqa: F811
         if steps:
             tracker.track_landmarks_step_table(b, tracker.landmarks_new(s["n_words"]))
         tracker.track_landmarks_release(b)
-    res, nl, table, _, _ = _host(tracker, s)
-    assert (res.tobytes(), nl.tobytes(), _table_bytes(table)) == (s["res"], s["nl"].tobytes(), s["table"])
+    res, nl, table, _, _ = landmarks_host(tracker, s)
+    assert (res.tobytes(), nl.tobytes(), table_bytes(table)) == (s["res"], s["nl"].tobytes(), s["table"])
 
 
 @pytest.mark.gpu
-def test_existing_host_calls_unchanged(tracker, lmseq):  # noqa: F811
+def test_existing_host_calls_unchanged(tracker, lmseq):
     """The depth and landmark host calls on a fresh context: results, byte counts and launches per call are the same
     before and after a prepare_host on that context."""
     s, h = lmseq, lmseq["h"]
@@ -224,8 +228,8 @@ def test_existing_host_calls_unchanged(tracker, lmseq):  # noqa: F811
         r = tr.track_sequence_host(s["p"], h["semi"], h["sscale"], h["desc"], h["depth"])
         out.append((r[0].tobytes(), r[1], r[2], tr.ctx.launches - n0))
         n0 = tr.ctx.launches
-        res, nl, table, up, down = _host(tr, s)
-        out.append((res.tobytes(), nl.tobytes(), _table_bytes(table), up, down, tr.ctx.launches - n0))
+        res, nl, table, up, down = landmarks_host(tr, s)
+        out.append((res.tobytes(), nl.tobytes(), table_bytes(table), up, down, tr.ctx.launches - n0))
         return out
 
     both()   # first calls on the context: modules, scratch
@@ -248,24 +252,16 @@ def _gpu_worker(rank, world, port, out_dir, n_warm, weighted):
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import synth, tracking
     tr = tracking.Tracker(rank)
-    v = np.load(os.path.join(ROOT, "tests", "golden", "ref_vocab.npz"))
-    tr.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    p = tracking.kitti_track_params(hypotheses=256)
-    semi, desc, depth = tr.synth_frames(21, 47, 155, 0, synth.default_offsets(N_FRAMES, 21))
-    sscale = torch.full((N_FRAMES,), float(synth.SEMI_SCALE), device=tr.device)
-    dscale = torch.full((N_FRAMES,), 4.3353, device=tr.device)
-    host = tuple(_pinned(torch, t) for t in (semi, sscale, desc, dscale, depth))
-    torch.cuda.synchronize()
+    s = landmark_sequence(tr, synth, host=True)
     counts = None
     if weighted:
         counts = [c for _, c in tracking.shard_pairs_weighted(N_FRAMES - 1, [1.0 + 2.0 * r for r in range(world)])]
-    table = tr.landmarks_new(tr.n_words)
-    rec, nl, _, up = tracking.track_sequence_landmarks_host_sharded(tr, p, host, table, first_frame=500,
-                                                                    n_warm=n_warm, counts=counts)
-    one = tr.landmarks_new(tr.n_words)
-    res1, nl1 = tr.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, one, first_frame=500)
-    ok = (rec.cpu().numpy().tobytes() == res1.cpu().numpy().tobytes() and bool((nl == nl1).all().item())
-          and _table_bytes(table) == _table_bytes(one) and up > 0)
+    table = tr.landmarks_new(s["n_words"])
+    rec, nl, _, up = tracking.track_sequence_landmarks_host_sharded(tr, s["p"], tuple(s["h"].values()), table,
+                                                                    first_frame=s["first"], n_warm=n_warm,
+                                                                    counts=counts)
+    ok = (rec.cpu().numpy().tobytes() == s["res"].tobytes() and bool((nl.cpu().numpy() == s["nl"]).all())
+          and table_bytes(table) == s["table"] and up > 0)
     open(os.path.join(out_dir, f"rank{rank}_{n_warm}_{weighted}.txt"), "w").write("ok" if ok else "differs")
     dist.destroy_process_group()
 
@@ -279,16 +275,9 @@ def test_host_sharded_equals_one_gpu(tmp_path, world):
         pytest.skip(f"needs {world} GPUs")
     for weighted in (False, True):
         for n_warm in (0, 16):
-            mp.spawn(_gpu_worker, args=(world, _free_port(), str(tmp_path), n_warm, weighted), nprocs=world, join=True)
+            mp.spawn(_gpu_worker, args=(world, free_port(), str(tmp_path), n_warm, weighted), nprocs=world, join=True)
             for r in range(world):
                 assert open(tmp_path / f"rank{r}_{n_warm}_{weighted}.txt").read() == "ok", (r, n_warm, weighted)
-
-
-class _HostStandIn(_StandIn):
-    def track_landmarks_prepare_host(self, p, n_warm, first_frame, semi, *rest):
-        b = self.track_landmarks_prepare(p, n_warm, first_frame, semi, *rest)
-        b["h2d_bytes"] = 1000 * semi.shape[0]
-        return b
 
 
 COUNTS = {1: [11], 3: [2, 6, 3], 4: [5, 0, 4, 2]}
@@ -307,7 +296,7 @@ def _relay_worker(rank, world, port, n_pairs, out_dir):
     frames = tuple(torch.zeros((n_pairs + 1, 1)) for _ in range(5))
     table = torch.arange(128, dtype=torch.uint8).reshape(2, 64).clone() if rank == 0 else \
         torch.full((2, 64), 99, dtype=torch.uint8)
-    rec, nl, rw, up = tracking.track_sequence_landmarks_host_sharded(_HostStandIn(), p, frames, table, first_frame=10,
+    rec, nl, rw, up = tracking.track_sequence_landmarks_host_sharded(HostStandIn(), p, frames, table, first_frame=10,
                                                                      n_warm=4, counts=COUNTS[world])
     np.savez(os.path.join(out_dir, f"rank{rank}.npz"), rec=rec.numpy(), nl=nl.numpy(), table=table.numpy(),
              rw=rw.numpy(), up=np.array(up))
@@ -321,8 +310,8 @@ def test_host_relay_order_uneven_cpu(tmp_path):
     import torch.multiprocessing as mp
     n_pairs = 11
     for world, counts in COUNTS.items():
-        mp.spawn(_relay_worker, args=(world, _free_port(), n_pairs, str(tmp_path)), nprocs=world, join=True)
-        st = _StandIn()
+        mp.spawn(_relay_worker, args=(world, free_port(), n_pairs, str(tmp_path)), nprocs=world, join=True)
+        st = StandIn()
         chain = torch.arange(128, dtype=torch.uint8).reshape(2, 64).clone()
         want_rec = np.zeros((n_pairs, 64), np.uint8)
         first = 0

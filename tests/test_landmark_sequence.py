@@ -13,8 +13,8 @@ The whole path against a CPU reference built from the oracle alone: tests/test_l
 import numpy as np
 import pytest
 
+from helpers import N_FRAMES, dev, drive_host_pool, landmark_sequence, table_bytes, table_contents, upload_table
 from landmark_reference import orc_landmarks_sequence
-from test_bow import drive_host_pool, table_contents
 
 CAM = (718.856, 718.856, 607.1928, 185.2157)
 
@@ -37,19 +37,6 @@ def test_oracle_sequence_equals_pool_contents(oracle):
 
 
 # ------------------------------------------------------------------ GPU: mv_landmarks_sequence
-def _dev(tracker, a):
-    import torch
-    return torch.from_numpy(np.ascontiguousarray(a)).to(tracker.device)
-
-
-def _table_bytes(t):
-    return t.cpu().numpy().tobytes()
-
-
-def _upload_table(tracker, host_table):
-    return _dev(tracker, host_table.view(np.uint8).reshape(-1, 56))
-
-
 def _per_frame_loop(tracker, table, first_frame, word, q_count, coords):
     """The existing kernels, one frame at a time; lookups after each step."""
     n_steps, top_n = word.shape
@@ -57,10 +44,10 @@ def _per_frame_loop(tracker, table, first_frame, word, q_count, coords):
     for f in range(n_steps):
         k = min(int(q_count[f]), top_n)
         if k:
-            tracker.landmarks_observe(table, first_frame + f, _dev(tracker, word[f, :k]), _dev(tracker, coords[f, :k]))
+            tracker.landmarks_observe(table, first_frame + f, dev(tracker, word[f, :k]), dev(tracker, coords[f, :k]))
         tracker.landmarks_remove_old(table, first_frame + f)
         if k:
-            c, _ = tracker.landmarks_lookup(table, _dev(tracker, word[f, :k]))
+            c, _ = tracker.landmarks_lookup(table, dev(tracker, word[f, :k]))
             out[f, :k] = c.cpu().numpy()
     return out
 
@@ -68,7 +55,7 @@ def _per_frame_loop(tracker, table, first_frame, word, q_count, coords):
 def _cases():
     rng = np.random.default_rng(11)
     cases = {}
-    # the 60-frame churn of the reference driver (tests/test_bow.py)
+    # the 60-frame churn of the reference driver (helpers.drive_host_pool, pinned in tests/test_bow.py)
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import lib
     snaps = drive_host_pool(lib.load())
@@ -109,16 +96,16 @@ def test_landmarks_sequence_equals_per_frame_loop_and_oracle(tracker, oracle, ca
     c = _cases()[case]
     word, qc, coords, n_words, first = c["word"], c["qc"], c["coords"], c["n_words"], c["first"]
     init = c["init"] if c["init"] is not None else oracle.pool_new(n_words)
-    t_loop = _upload_table(tracker, init)
+    t_loop = upload_table(tracker, init)
     want = _per_frame_loop(tracker, t_loop, first, word, qc, coords)
-    t_seq = _upload_table(tracker, init)
-    got = tracker.landmarks_sequence(t_seq, first, _dev(tracker, word), _dev(tracker, qc), _dev(tracker, coords))
+    t_seq = upload_table(tracker, init)
+    got = tracker.landmarks_sequence(t_seq, first, dev(tracker, word), dev(tracker, qc), dev(tracker, coords))
     got = got.cpu().numpy()
-    assert _table_bytes(t_seq) == _table_bytes(t_loop)
+    assert table_bytes(t_seq) == table_bytes(t_loop)
     assert got.view(np.int32).tobytes() == want.view(np.int32).tobytes()
     o_table = init.copy()
     o_out = orc_landmarks_sequence(oracle, o_table, first, word, qc, coords)
-    assert _table_bytes(t_seq) == o_table.tobytes()
+    assert table_bytes(t_seq) == o_table.tobytes()
     assert got.tobytes() == o_out.tobytes()
     if case == "churn_dups":   # word 42 really was deleted and re-inserted with the coordinates of its new frame
         rec = t_seq.cpu().numpy().view(oracle.pool_new(1).dtype).reshape(-1)[42]
@@ -130,37 +117,24 @@ def test_landmarks_sequence_equals_per_frame_loop_and_oracle(tracker, oracle, ca
 def test_landmarks_sequence_split_equals_one_call(tracker, oracle):
     c = _cases()["churn_dups"]
     word, qc, coords = c["word"], c["qc"], c["coords"]
-    one = _upload_table(tracker, oracle.pool_new(500))
-    out1 = tracker.landmarks_sequence(one, 0, _dev(tracker, word), _dev(tracker, qc), _dev(tracker, coords)).cpu().numpy()
+    one = upload_table(tracker, oracle.pool_new(500))
+    out1 = tracker.landmarks_sequence(one, 0, dev(tracker, word), dev(tracker, qc), dev(tracker, coords)).cpu().numpy()
     for k in (1, 17, 39):
-        two = _upload_table(tracker, oracle.pool_new(500))
-        a = tracker.landmarks_sequence(two, 0, _dev(tracker, word[:k]), _dev(tracker, qc[:k]), _dev(tracker, coords[:k]))
-        b = tracker.landmarks_sequence(two, k, _dev(tracker, word[k:]), _dev(tracker, qc[k:]), _dev(tracker, coords[k:]))
-        assert _table_bytes(two) == _table_bytes(one), k
+        two = upload_table(tracker, oracle.pool_new(500))
+        a = tracker.landmarks_sequence(two, 0, dev(tracker, word[:k]), dev(tracker, qc[:k]), dev(tracker, coords[:k]))
+        b = tracker.landmarks_sequence(two, k, dev(tracker, word[k:]), dev(tracker, qc[k:]), dev(tracker, coords[k:]))
+        assert table_bytes(two) == table_bytes(one), k
         assert np.concatenate([a.cpu().numpy(), b.cpu().numpy()]).tobytes() == out1.tobytes(), k
 
 
 # ------------------------------------------------------------------ GPU: mv_track_sequence_landmarks
-N_FRAMES = 66
-
-
 @pytest.fixture(scope="module")
 def seq(tracker, synth):
     """A KITTI-shaped synthetic sequence, the path's results, and the composition of public calls."""
-    import os
     import torch
-    from maveric_slam_b200 import tracking
-    v = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_vocab.npz"))
-    tracker.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    n_words = tracker.n_words
-    rows, cols, n = 47, 155, N_FRAMES
-    p = tracking.kitti_track_params(hypotheses=256)
-    semi, desc, depth = tracker.synth_frames(21, rows, cols, 0, synth.default_offsets(n, 21))
-    sscale = torch.full((n,), float(synth.SEMI_SCALE), device=tracker.device)
-    dscale = torch.full((n,), 4.3353, device=tracker.device)
-    first = 500
-    table = tracker.landmarks_new(n_words)
-    res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=first)
+    s = landmark_sequence(tracker, synth)
+    semi, sscale, desc, dscale, depth = s["d"].values()
+    p, first, n_words, rows, n = s["p"], s["first"], s["n_words"], 47, N_FRAMES
     # the composition
     idx, prob, _ = tracker.softmax(semi, sscale)
     qp, qi, _, qc, ov = tracker.top_n(idx, prob, p.top_n, p.max_valid)
@@ -176,7 +150,7 @@ def seq(tracker, synth):
     snaps = []
     for f in range(n - 1):
         k = min(int(hc[f]), p.top_n)
-        tracker.landmarks_observe(ref_table, first + f, _dev(tracker, hw[f, :k]), _dev(tracker, coords[f, :k]))
+        tracker.landmarks_observe(ref_table, first + f, dev(tracker, hw[f, :k]), dev(tracker, coords[f, :k]))
         tracker.landmarks_remove_old(ref_table, first + f)
         snaps.append(ref_table.clone())
     pts, cnt, cell0, _, _ = tracker.match(p.match, desc, idx, prob, qp, qi, qc)
@@ -188,9 +162,7 @@ def seq(tracker, synth):
         corr.append(c); nls.append(l)
     corr = torch.cat(corr)
     pose, stats, _ = tracker.pnp_gn(p.pnp, corr, cnt)
-    return dict(p=p, semi=semi, sscale=sscale, desc=desc, dscale=dscale, depth=depth, first=first, n_words=n_words,
-                res=tracking.results_to_numpy(res), nl=nl.cpu().numpy(), table=_table_bytes(table),
-                ref_table=_table_bytes(ref_table), pose=pose.cpu().numpy(), stats=stats.cpu().numpy(),
+    return dict(s, **s["d"], ref_table=table_bytes(ref_table), pose=pose.cpu().numpy(), stats=stats.cpu().numpy(),
                 cnt=cnt.cpu().numpy(), rin=rin.cpu().numpy(), ov=ov.cpu().numpy(), nls=torch.cat(nls).cpu().numpy(),
                 corr=corr.cpu().numpy())
 
@@ -239,7 +211,7 @@ def test_track_sequence_landmarks_halo_split_equals_one_call(tracker, seq):
         parts.append(tracking.results_to_numpy(res)); nls.append(nl.cpu().numpy())
     assert np.concatenate(parts).tobytes() == seq["res"].tobytes()
     assert (np.concatenate(nls) == seq["nl"]).all()
-    assert _table_bytes(table) == seq["table"]
+    assert table_bytes(table) == seq["table"]
 
 
 @pytest.mark.gpu
@@ -278,7 +250,7 @@ def test_track_sequence_landmarks_argument_errors(tracker, seq):
         tracker.ctx.check(tracker.lib.mv_landmarks_sequence(tracker.ctx.h, 0, tracker._d(table), 0, 1, 1, None, None,
                                                             None, None))
     # refusals of the PnP and the matcher: checked before the table is stepped, nothing launched
-    before = _table_bytes(table)
+    before = table_bytes(table)
     for part, field, val in (("pnp", "lanes_per_hypothesis", 4), ("pnp", "hypotheses", 0), ("pnp", "sample_size", 0),
                              ("match", "radius", -1)):
         bad = tracking.kitti_track_params(hypotheses=256)
@@ -287,8 +259,8 @@ def test_track_sequence_landmarks_argument_errors(tracker, seq):
         with pytest.raises(lib.MvError, match="bad argument"):
             tracker.track_sequence_landmarks(bad, semi, sscale, desc, dscale, depth, table, first_frame=seq["first"])
         assert tracker.ctx.launches == launches, field
-        assert _table_bytes(table) == before, field
+        assert table_bytes(table) == before, field
     # the context still works and the table gives the stored answer
     res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=seq["first"])
     assert tracking.results_to_numpy(res).tobytes() == seq["res"].tobytes() and (nl.cpu().numpy() == seq["nl"]).all()
-    assert _table_bytes(table) == seq["table"]
+    assert table_bytes(table) == seq["table"]

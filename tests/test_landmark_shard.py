@@ -8,30 +8,16 @@ The device one-call is itself held to a CPU reference of the whole path, tests/l
 (tests/test_landmark_reference.py).
 """
 import os
-import socket
 import sys
 
 import numpy as np
 import pytest
 
+from helpers import (N_FRAMES, WARMS, StandIn, cycled_blocks, dev, drive_host_pool, free_port, landmark_sequence,
+                     ref_vocab, table_bytes, upload_table)
 from landmark_reference import orc_landmarks_sequence
-from test_bow import drive_host_pool
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-WARMS = (0, 1, 7, 8, 16, 64)
-
-
-def _dev(tracker, a):
-    import torch
-    return torch.from_numpy(np.ascontiguousarray(a)).to(tracker.device)
-
-
-def _table_bytes(t):
-    return t.cpu().numpy().tobytes()
-
-
-def _upload_table(tracker, host_table):
-    return _dev(tracker, host_table.view(np.uint8).reshape(-1, 56))
 
 
 def _cases():
@@ -104,9 +90,9 @@ def _split(tracker, oracle, c, k, n_warm, rng):
     """-> (entry table on the device, warm-up + block words / counts, block coordinates)."""
     word, qc, coords, n_words, first = c["word"], c["qc"], c["coords"], c["n_words"], c["first"]
     init = c["init"] if c["init"] is not None else oracle.pool_new(n_words)
-    entry = _upload_table(tracker, init)
+    entry = upload_table(tracker, init)
     if k > 0:
-        tracker.landmarks_sequence(entry, first, _dev(tracker, word[:k]), _dev(tracker, qc[:k]), _dev(tracker, coords[:k]))
+        tracker.landmarks_sequence(entry, first, dev(tracker, word[:k]), dev(tracker, qc[:k]), dev(tracker, coords[:k]))
     # warm-up frames: the stream's, and where it has too few, made-up frames (a guess that is simply wrong)
     pad = max(0, n_warm - k)
     ww = np.concatenate([rng.integers(-1, n_words, (pad, word.shape[1])).astype(np.int32), word[k - n_warm + pad:k]])
@@ -126,21 +112,21 @@ def test_speculate_resolve_equals_sequence(tracker, oracle, cases, case):
             entry, word, qc, coords = _split(tracker, oracle, c, k, n_warm, rng)
             first = c["first"] + k
             want_t = entry.clone()
-            want = tracker.landmarks_sequence(want_t, first, _dev(tracker, word[n_warm:]), _dev(tracker, qc[n_warm:]),
-                                              _dev(tracker, coords)).cpu().numpy()
-            spec = tracker.landmarks_speculate(c["n_words"], first, n_warm, _dev(tracker, word), _dev(tracker, qc),
-                                               _dev(tracker, coords))
+            want = tracker.landmarks_sequence(want_t, first, dev(tracker, word[n_warm:]), dev(tracker, qc[n_warm:]),
+                                              dev(tracker, coords)).cpu().numpy()
+            spec = tracker.landmarks_speculate(c["n_words"], first, n_warm, dev(tracker, word), dev(tracker, qc),
+                                               dev(tracker, coords))
             got_t = entry.clone()
             n_rw = torch.full((1,), -1, dtype=torch.int32, device=tracker.device)
             got = tracker.landmarks_resolve(spec, got_t, n_rewalked=n_rw).cpu().numpy()
             tracker.landmarks_release(spec)
-            assert _table_bytes(got_t) == _table_bytes(want_t), (k, n_warm)
+            assert table_bytes(got_t) == table_bytes(want_t), (k, n_warm)
             assert got.tobytes() == want.tobytes(), (k, n_warm)
             rewalked.append(int(n_rw.item()))
             if case != "random_table" and n_warm in (0, 16):
                 o_table = entry.cpu().numpy().view(oracle.pool_new(1).dtype).reshape(-1).copy()
                 o_out = orc_landmarks_sequence(oracle, o_table, first, word[n_warm:], qc[n_warm:], coords)
-                assert _table_bytes(got_t) == o_table.tobytes() and got.tobytes() == o_out.tobytes(), (k, n_warm)
+                assert table_bytes(got_t) == o_table.tobytes() and got.tobytes() == o_out.tobytes(), (k, n_warm)
     assert min(rewalked) >= 0
     if case in ("branches", "churn"):   # both paths of the resolve step run
         assert min(rewalked) == 0 and max(rewalked) > 0, rewalked
@@ -151,7 +137,7 @@ def test_speculate_resolve_refusals(tracker, cases):
     import torch
     from maveric_slam_b200 import lib
     c = cases["churn_dups"]
-    word, qc, coords = (_dev(tracker, c[x]) for x in ("word", "qc", "coords"))
+    word, qc, coords = (dev(tracker, c[x]) for x in ("word", "qc", "coords"))
     with pytest.raises(lib.MvError, match="bad argument"):
         tracker.landmarks_speculate(c["n_words"], 0, 40, word, qc, coords)   # no block step left
     from maveric_slam_b200 import tracking
@@ -170,34 +156,10 @@ def test_speculate_resolve_refusals(tracker, cases):
 
 
 # ------------------------------------------------------------------ frame level
-N_FRAMES = 66
-
-
 @pytest.fixture(scope="module")
 def seq(tracker, synth):
-    import torch
-    from maveric_slam_b200 import tracking
-    v = np.load(os.path.join(ROOT, "tests", "golden", "ref_vocab.npz"))
-    tracker.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    rows, cols, n = 47, 155, N_FRAMES
-    p = tracking.kitti_track_params(hypotheses=256)
-    semi, desc, depth = tracker.synth_frames(21, rows, cols, 0, synth.default_offsets(n, 21))
-    sscale = torch.full((n,), float(synth.SEMI_SCALE), device=tracker.device)
-    dscale = torch.full((n,), 4.3353, device=tracker.device)
-    first = 500
-    table = tracker.landmarks_new(tracker.n_words)
-    res, nl = tracker.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, table, first_frame=first)
-    return dict(p=p, frames=(semi, sscale, desc, dscale, depth), first=first, n_words=tracker.n_words, vocab=v,
-                res=tracking.results_to_numpy(res), nl=nl.cpu().numpy(), table=_table_bytes(table))
-
-
-def _blocks(sizes, n_pairs):
-    out, lo, i = [], 0, 0
-    while lo < n_pairs:
-        c = min(sizes[i % len(sizes)], n_pairs - lo)
-        out.append((lo, c))
-        lo, i = lo + c, i + 1
-    return out
+    s = landmark_sequence(tracker, synth)
+    return dict(s, frames=tuple(s["d"].values()))
 
 
 def _prepare(tr, seq, lo, count, n_warm):
@@ -217,7 +179,7 @@ def test_prepare_step_solve_whole_sequence(tracker, seq):
     res, nl = tracker.track_landmarks_solve(block)
     tracker.track_landmarks_release(block)
     assert tracking.results_to_numpy(res).tobytes() == seq["res"].tobytes()
-    assert (nl.cpu().numpy() == seq["nl"]).all() and _table_bytes(table) == seq["table"]
+    assert (nl.cpu().numpy() == seq["nl"]).all() and table_bytes(table) == seq["table"]
 
 
 @pytest.mark.gpu
@@ -228,10 +190,9 @@ def test_blocks_prepared_first_then_stepped_in_order(tracker, seq, two_contexts)
     other = tracker
     if two_contexts:
         other = tracking.Tracker(0)
-        v = seq["vocab"]
-        other.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
+        other.bow_set_vocabulary(*ref_vocab())
     for n_warm in WARMS:
-        blocks = _blocks([1, 2, 3, 7], N_FRAMES - 1)
+        blocks = cycled_blocks([1, 2, 3, 7], N_FRAMES - 1)
         trs = [(tracker, other)[i % 2] for i in range(len(blocks))]
         # prepared in reverse order, all before the first table step
         prepared = {i: _prepare(trs[i], seq, lo, c, n_warm) for i, (lo, c) in reversed(list(enumerate(blocks)))}
@@ -248,7 +209,7 @@ def test_blocks_prepared_first_then_stepped_in_order(tracker, seq, two_contexts)
             trs[i].track_landmarks_release(prepared[i])
         assert np.concatenate(res).tobytes() == seq["res"].tobytes(), n_warm
         assert (np.concatenate(nls) == seq["nl"]).all(), n_warm
-        assert _table_bytes(table) == seq["table"], n_warm
+        assert table_bytes(table) == seq["table"], n_warm
 
 
 @pytest.mark.gpu
@@ -257,7 +218,7 @@ def test_block_refusals(tracker, seq):
     from maveric_slam_b200 import lib, tracking
     semi, sscale, desc, dscale, depth = seq["frames"]
     table = tracker.landmarks_new(seq["n_words"])
-    before = _table_bytes(table)
+    before = table_bytes(table)
     for part, field, val in (("pnp", "lanes_per_hypothesis", 4), ("pnp", "hypotheses", 0), ("pnp", "sample_size", 0),
                              ("match", "radius", -1)):
         bad = tracking.kitti_track_params(hypotheses=256)
@@ -275,7 +236,7 @@ def test_block_refusals(tracker, seq):
     with pytest.raises(lib.MvError, match="n_words must be positive"):
         tracker.track_landmarks_prepare(seq["p"], 0, 0, semi[:4], sscale[:4], desc[:4], dscale[:4], depth[:4], 0)
     assert tracker.ctx.launches == launches
-    assert _table_bytes(table) == before
+    assert table_bytes(table) == before
     # phases
     block = _prepare(tracker, seq, 0, 5, 0)
     launches = tracker.ctx.launches
@@ -286,7 +247,7 @@ def test_block_refusals(tracker, seq):
     other = tracking.Tracker(0)
     with pytest.raises(lib.MvError, match="another context"):
         other.track_landmarks_step_table(block, table)
-    assert tracker.ctx.launches == launches and _table_bytes(table) == before
+    assert tracker.ctx.launches == launches and table_bytes(table) == before
     tracker.track_landmarks_step_table(block, table)
     with pytest.raises(lib.MvError, match="out of phase"):
         tracker.track_landmarks_step_table(block, table)
@@ -303,19 +264,11 @@ def test_block_refusals(tracker, seq):
     table = tracker.landmarks_new(seq["n_words"])
     res, nl = tracker.track_sequence_landmarks(seq["p"], *seq["frames"], table, first_frame=seq["first"])
     assert tracking.results_to_numpy(res).tobytes() == seq["res"].tobytes() and (nl.cpu().numpy() == seq["nl"]).all()
-    assert _table_bytes(table) == seq["table"]
+    assert table_bytes(table) == seq["table"]
     torch.cuda.synchronize()
 
 
 # ------------------------------------------------------------------ ranks
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    p = s.getsockname()[1]
-    s.close()
-    return p
-
-
 def _gpu_worker(rank, world, port, out_dir, n_warm):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -328,19 +281,12 @@ def _gpu_worker(rank, world, port, out_dir, n_warm):
     import maveric_slam_b200  # noqa: F401
     from maveric_slam_b200 import synth, tracking
     tr = tracking.Tracker(rank)
-    v = np.load(os.path.join(ROOT, "tests", "golden", "ref_vocab.npz"))
-    tr.bow_set_vocabulary(v["base_desc"], v["scale"], v["bias"], v["leaves"])
-    p = tracking.kitti_track_params(hypotheses=256)
-    semi, desc, depth = tr.synth_frames(21, 47, 155, 0, synth.default_offsets(N_FRAMES, 21))
-    sscale = torch.full((N_FRAMES,), float(synth.SEMI_SCALE), device=tr.device)
-    dscale = torch.full((N_FRAMES,), 4.3353, device=tr.device)
-    table = tr.landmarks_new(tr.n_words)
-    rec, nl, _ = tracking.track_sequence_landmarks_sharded(tr, p, (semi, sscale, desc, dscale, depth), table,
-                                                           first_frame=500, n_warm=n_warm)
-    one = tr.landmarks_new(tr.n_words)
-    res1, nl1 = tr.track_sequence_landmarks(p, semi, sscale, desc, dscale, depth, one, first_frame=500)
-    ok = (rec.cpu().numpy().tobytes() == res1.cpu().numpy().tobytes() and bool((nl == nl1).all().item())
-          and _table_bytes(table) == _table_bytes(one))
+    s = landmark_sequence(tr, synth)
+    table = tr.landmarks_new(s["n_words"])
+    rec, nl, _ = tracking.track_sequence_landmarks_sharded(tr, s["p"], tuple(s["d"].values()), table,
+                                                           first_frame=s["first"], n_warm=n_warm)
+    ok = (rec.cpu().numpy().tobytes() == s["res"].tobytes() and bool((nl.cpu().numpy() == s["nl"]).all())
+          and table_bytes(table) == s["table"])
     open(os.path.join(out_dir, f"rank{rank}_{n_warm}.txt"), "w").write("ok" if ok else "differs")
     dist.destroy_process_group()
 
@@ -353,38 +299,9 @@ def test_sharded_equals_one_gpu(tmp_path, world):
     if torch.cuda.device_count() < world:
         pytest.skip(f"needs {world} GPUs")
     for n_warm in (0, 16):
-        mp.spawn(_gpu_worker, args=(world, _free_port(), str(tmp_path), n_warm), nprocs=world, join=True)
+        mp.spawn(_gpu_worker, args=(world, free_port(), str(tmp_path), n_warm), nprocs=world, join=True)
         for r in range(world):
             assert open(tmp_path / f"rank{r}_{n_warm}.txt").read() == "ok", (r, n_warm)
-
-
-class _StandIn:
-    """The block calls of a Tracker on the CPU, with a table step that is not associative: any other order of the
-    relay than rank order, or a table read before it arrives, changes the final table and the records."""
-
-    def __init__(self):
-        import torch
-        self.torch = torch
-        self.device = torch.device("cpu")
-
-    def track_landmarks_prepare(self, p, n_warm, first_frame, semi, *rest):
-        return {"first": p.pnp.first_pair, "n_pairs": semi.shape[0] - n_warm - 1, "n_warm": n_warm,
-                "frame": first_frame}
-
-    def track_landmarks_step_table(self, block, table, n_rewalked=None):
-        for i in range(block["n_pairs"]):
-            table.copy_(((table.to(self.torch.int64) * 7 + block["first"] + i + 3) % 251).to(self.torch.uint8))
-        block["state"] = table.clone()
-        if n_rewalked is not None:
-            n_rewalked.fill_(block["n_warm"])
-
-    def track_landmarks_solve(self, block, out, n_with_landmark):
-        for i in range(block["n_pairs"]):
-            out[i] = block["state"].reshape(-1)[:64] + i
-            n_with_landmark[i] = block["frame"] + i
-
-    def track_landmarks_release(self, block):
-        block.clear()
 
 
 def _relay_worker(rank, world, port, n_pairs, out_dir):
@@ -400,7 +317,7 @@ def _relay_worker(rank, world, port, n_pairs, out_dir):
     frames = tuple(torch.zeros((n_pairs + 1, 1)) for _ in range(5))
     table = torch.arange(128, dtype=torch.uint8).reshape(2, 64).clone() if rank == 0 else \
         torch.full((2, 64), 99, dtype=torch.uint8)
-    rec, nl, rw = tracking.track_sequence_landmarks_sharded(_StandIn(), p, frames, table, first_frame=10, n_warm=4)
+    rec, nl, rw = tracking.track_sequence_landmarks_sharded(StandIn(), p, frames, table, first_frame=10, n_warm=4)
     np.savez(os.path.join(out_dir, f"rank{rank}.npz"), rec=rec.numpy(), nl=nl.numpy(), table=table.numpy(),
              rw=rw.numpy())
     dist.destroy_process_group()
@@ -416,8 +333,8 @@ def test_relay_order_cpu(tmp_path):
     from maveric_slam_b200 import tracking
     n_pairs = 11
     for world in (1, 3):
-        mp.spawn(_relay_worker, args=(world, _free_port(), n_pairs, str(tmp_path)), nprocs=world, join=True)
-        st = _StandIn()
+        mp.spawn(_relay_worker, args=(world, free_port(), n_pairs, str(tmp_path)), nprocs=world, join=True)
+        st = StandIn()
         table = torch.arange(128, dtype=torch.uint8).reshape(2, 64).clone()
         block = {"first": 0, "n_pairs": n_pairs, "n_warm": 0, "frame": 10}
         st.track_landmarks_step_table(block, table)

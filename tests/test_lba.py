@@ -17,14 +17,8 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from helpers import same_bits, spd_system
 from oracle import orc
-
-
-def same_bits(a, b):
-    a = np.ascontiguousarray(a, np.float32)
-    b = np.ascontiguousarray(b, np.float32)
-    na, nb = np.isnan(a), np.isnan(b)
-    return a.shape == b.shape and (na == nb).all() and (a[~na].view(np.int32) == b[~nb].view(np.int32)).all()
 
 
 @pytest.fixture(scope="module")
@@ -85,24 +79,10 @@ def test_oracle_solves_a_real_window(oracle):
     assert np.abs(got[6 * P, :6 * P] - want[6 * P, :6 * P]).max() < 1e-4 * scale   # gradient row: no Schur term
 
 
-def _spd_system(rng, P, cond=1.0):
-    """(C as lba_schur lays it out, S, g) for a random SPD pose block."""
-    n = 6 * P
-    A = rng.normal(size=(n + 24, n)) * np.logspace(0, np.log10(cond), n)
-    S = (A.T @ A).astype(np.float32)
-    S = np.tril(S) + np.tril(S, -1).T
-    g = rng.normal(size=n).astype(np.float32)
-    C = np.zeros((n + 1, n + 1), np.float32)
-    C[:n, :n] = S.T                     # [column, row]
-    C[:n, n] = g                        # last row
-    C[n, n] = 3.0
-    return C, S, g
-
-
 def test_oracle_solve_against_float64(oracle):
     rng = np.random.default_rng(5)
     for P in (1, 2, 5, 8, 11, 16):
-        C, S, g = _spd_system(rng, P)
+        C, S, g = spd_system(rng, P)
         ok, d = oracle.lba_solve(C, 0.0)
         want = np.linalg.solve(S.astype(np.float64), -g.astype(np.float64))
         assert ok == 1 and np.abs(d - want).max() < 1e-4 * np.abs(want).max(), P
@@ -120,7 +100,7 @@ def test_oracle_solve_against_float64(oracle):
 
 def test_oracle_solve_rejects_what_is_not_positive_definite(oracle, golden):
     rng = np.random.default_rng(6)
-    C, S, g = _spd_system(rng, 3)
+    C, S, g = spd_system(rng, 3)
     C[4, 4] = -1.0
     ok, d = oracle.lba_solve(C, 0.0)
     assert ok == 0 and not d.any()
@@ -128,7 +108,7 @@ def test_oracle_solve_rejects_what_is_not_positive_definite(oracle, golden):
     ok, d = oracle.lba_solve(golden["C"][0], 0.0)
     assert ok == 0 and not d.any()
     # one pose, 6 x 6: the PnP solve's definition (ascending back substitution differs in order only)
-    C, S, g = _spd_system(rng, 1)
+    C, S, g = spd_system(rng, 1)
     ok, d = oracle.lba_solve(C, 1e-3)
     want = np.linalg.solve(S.astype(np.float64) * (np.eye(6) * 1e-3 + 1), -g.astype(np.float64))
     assert ok == 1 and np.abs(d - want).max() < 1e-5 * np.abs(want).max()
@@ -197,7 +177,7 @@ def test_gpu_solve_equals_oracle(tracker, oracle, golden):
     for P in (1, 2, 3, 5, 6, 8, 11, 16):
         Cs = []
         for w in range(9):
-            C, _, _ = _spd_system(rng, P, cond=(1.0, 30.0, 1000.0)[w % 3])
+            C, _, _ = spd_system(rng, P, cond=(1.0, 30.0, 1000.0)[w % 3])
             if w == 4:
                 C[2 * P, 2 * P] = -abs(C[2 * P, 2 * P])          # a negative pivot in the middle
             if w == 7:
@@ -228,7 +208,7 @@ def test_gpu_solve_full_batch_and_residual(tracker):
     system (float64 residual)."""
     import torch
     rng = np.random.default_rng(22)
-    base = np.stack([_spd_system(rng, 8)[0] for _ in range(37)])
+    base = np.stack([spd_system(rng, 8)[0] for _ in range(37)])
     Cs = torch.from_numpy(np.tile(base, (64, 1, 1))).to(tracker.device)
     d, ok = tracker.lba_solve(Cs, 0.0)
     assert int(ok.sum()) == Cs.shape[0]

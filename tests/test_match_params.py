@@ -30,7 +30,8 @@ import numpy as np
 import pytest
 
 from conftest import bits
-from landmark_reference import detect, landmark_reference, match_cfg
+from helpers import pinned, ref_vocab
+from landmark_reference import detect, first_difference, landmark_reference, match_cfg, run_entry
 from oracle import orc
 
 f32 = np.float32
@@ -622,12 +623,6 @@ def test_sequence_case_reaches(seq_refs, name):
     _assert_seq_reaches(name, seq_refs)
 
 
-def _pinned(torch, a):
-    h = torch.empty(a.shape, dtype=torch.from_numpy(a[:0]).dtype, pin_memory=True)
-    h.copy_(torch.from_numpy(np.ascontiguousarray(a)))
-    return h
-
-
 def _run_sequence(tracker, p, frames, entry, monkeypatch):
     import torch
     from maveric_slam_b200 import tracking
@@ -648,10 +643,10 @@ def _run_sequence(tracker, p, frames, entry, monkeypatch):
         q.match = copy.copy(p.match)
         q.match.min_prob0 = -INF
         reversed_desc = np.ascontiguousarray(desc[::-1])
-        tracker.track_sequence_host(q, *[_pinned(torch, x) for x in (semi, sscale, reversed_desc, depth)])
+        tracker.track_sequence_host(q, *[pinned(x) for x in (semi, sscale, reversed_desc, depth)])
         if entry == "host_no_gather":
             m.setenv("MV_HOST_GATHER", "0")
-        return tracker.track_sequence_host(p, *[_pinned(torch, x) for x in frames])[0]
+        return tracker.track_sequence_host(p, *[pinned(x) for x in frames])[0]
 
 
 @pytest.mark.gpu
@@ -660,13 +655,12 @@ def test_sequence_vs_oracle(tracker, seq_refs, monkeypatch, name):
     """Whole records of every pair, byte for byte, through the device call and the host call from pinned buffers
     (row gather, chunks of 2 pairs: the three staging buffer sets are reused, so a row the gather skipped holds an
     earlier frame's descriptor), pageable buffers and pinned buffers without the gather."""
-    from test_landmark_reference import _first_difference
     want = seq_refs.records(name)
     frames = seq_refs.inputs(SEQ_CASES[name]["shape"])
     p = seq_refs.params(name)
     for entry in SEQ_ENTRIES:
         got = np.ascontiguousarray(_run_sequence(tracker, p, frames, entry, monkeypatch)).tobytes()
-        assert got == want.tobytes(), (entry, _first_difference(want, got))
+        assert got == want.tobytes(), (entry, first_difference(want, got))
 
 
 # ------------------------------------------------------------------ landmark path
@@ -678,7 +672,6 @@ class _LmRef:
     6 .. 9), RANSAC-E at 1 iteration and 1e30 (every match an inlier)."""
 
     def __init__(self, oracle, synth):
-        from test_landmark_reference import _ref_vocab
         self.oracle = oracle
         rows, cols, n = 24, 80, 12
         semi, desc, depth, _ = synth.synth_sequence(41, rows, cols, n)
@@ -687,7 +680,7 @@ class _LmRef:
         p = _seq_params(24, thr=0.7, ransac=(1, 1e30))
         self.gate = _gate_cell(oracle, p, semi, sscale, desc, range(6, 10))
         p.match.min_prob0 = self.gate[2]
-        self.vocab = _ref_vocab()
+        self.vocab = ref_vocab()
         self.c = dict(p=p, frames=[semi, sscale, desc, dscale, depth], first=0, n_words=10000, vocab=self.vocab,
                       entry=None)
         self.c["rec"], self.c["nl"], self.c["table"] = self.reference(p)
@@ -723,22 +716,20 @@ def lm_tracker():
     import torch
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
-    from test_landmark_reference import _ref_vocab
     from maveric_slam_b200 import tracking
     tr = tracking.Tracker(0)
-    tr.bow_set_vocabulary(*_ref_vocab())
+    tr.bow_set_vocabulary(*ref_vocab())
     return tr
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("entry", LM_ENTRIES)
 def test_landmark_path_vs_reference(lm_tracker, lm_ref, monkeypatch, entry):
-    from test_landmark_reference import _first_difference, _run
     c = lm_ref.c
     monkeypatch.delenv("MV_HOST_CHUNK_PAIRS", raising=False)
     monkeypatch.delenv("MV_HOST_GATHER", raising=False)
-    res, nl, table = _run(lm_tracker, c, entry, monkeypatch)
-    assert res == c["rec"].tobytes(), _first_difference(c["rec"], res)
+    res, nl, table = run_entry(lm_tracker, c, entry, monkeypatch)
+    assert res == c["rec"].tobytes(), first_difference(c["rec"], res)
     assert (nl == c["nl"]).all(), (nl, c["nl"])
     assert table == c["table"].tobytes()
 
@@ -750,14 +741,13 @@ def test_nan_threshold_with_forced_tensor_cores_is_refused(tracker, lm_tracker, 
     it with MV_ERR_BAD_ARG before anything is enqueued, and the context then still gives the oracle's answers."""
     import torch
     from maveric_slam_b200 import lib
-    from test_landmark_reference import _first_difference, _run
     I = refs.inputs["syn24"]
     dev = [torch.from_numpy(np.ascontiguousarray(a)).to(tracker.device) for a in _frames(I)]
     frames = seq_refs.inputs(24)
     dframes = [torch.from_numpy(np.ascontiguousarray(x)).to(tracker.device) for x in frames]
     lm = lm_ref.c["frames"]
     lm_dev = [torch.from_numpy(np.ascontiguousarray(x)).to(lm_tracker.device) for x in lm]
-    lm_pin = [_pinned(torch, x) for x in lm]
+    lm_pin = [pinned(x) for x in lm]
     mp = _mparams(I, NAN, DEFAULT_GATE, 1)
     tp = seq_refs.params("low")
     tp.match.match_threshold, tp.match.use_tensor_cores = NAN, 1
@@ -769,7 +759,7 @@ def test_nan_threshold_with_forced_tensor_cores_is_refused(tracker, lm_tracker, 
         ("mv_match_batch", tracker, lambda: tracker.match(mp, *dev)),
         ("mv_track_sequence", tracker, lambda: tracker.track_sequence(tp, *dframes)),
         ("mv_track_sequence_host", tracker,
-         lambda: tracker.track_sequence_host(tp, *[_pinned(torch, x) for x in frames])),
+         lambda: tracker.track_sequence_host(tp, *[pinned(x) for x in frames])),
         ("mv_track_landmarks_prepare", lm_tracker,
          lambda: lm_tracker.track_landmarks_prepare(lp, 0, 0, *lm_dev, 10000)),
         ("mv_track_landmarks_prepare_host", lm_tracker,
@@ -785,6 +775,6 @@ def test_nan_threshold_with_forced_tensor_cores_is_refused(tracker, lm_tracker, 
         _assert_same(g, refs.answer("thr_0.9", "syn24")[i], ("after refusal", i))
     want = seq_refs.records("low")
     got = np.ascontiguousarray(_run_sequence(tracker, seq_refs.params("low"), frames, "host_pinned", monkeypatch))
-    assert got.tobytes() == want.tobytes(), _first_difference(want, got.tobytes())
-    res, nl, table = _run(lm_tracker, lm_ref.c, "blocks_host:8", monkeypatch)
+    assert got.tobytes() == want.tobytes(), first_difference(want, got.tobytes())
+    res, nl, table = run_entry(lm_tracker, lm_ref.c, "blocks_host:8", monkeypatch)
     assert res == lm_ref.c["rec"].tobytes() and table == lm_ref.c["table"].tobytes()

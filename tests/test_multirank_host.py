@@ -2,7 +2,6 @@
 blocks, each rank computes its own block (here with the CPU oracle standing in for the GPU),
 and one all_gather of 64-byte records reproduces the single-rank result on every rank."""
 import os
-import socket
 import sys
 
 import numpy as np
@@ -10,15 +9,9 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
+from helpers import free_port
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    p = s.getsockname()[1]
-    s.close()
-    return p
 
 
 def _records(first, count):
@@ -105,7 +98,7 @@ def test_weighted_blocks_and_balancing():
 
 def test_two_rank_gather_equals_single_rank(tmp_path):
     n_pairs, world = 37, 2
-    port = _free_port()
+    port = free_port()
     mp.spawn(_worker, args=(world, port, n_pairs, str(tmp_path)), nprocs=world, join=True)
     want = _records(0, n_pairs).view(np.uint8).reshape(-1, 64)
     for r in range(world):

@@ -26,9 +26,8 @@ import numpy as np
 import pytest
 
 from conftest import bits
-from landmark_reference import landmark_reference, orc_landmarks_sequence
-from test_landmark_reference import _bow_check, _bow_inputs, _bow_vocab, _case_inputs, _params, _pinned, _ref_vocab
-from test_lba import same_bits
+from helpers import dev, pinned, pnp_params, pnp_problems, ref_vocab, same_bits, spd_system, with_first_pair
+from landmark_reference import bow_check, bow_inputs, bow_vocab, case_inputs, landmark_reference, orc_landmarks_sequence
 
 pytestmark = pytest.mark.gpu
 
@@ -78,11 +77,6 @@ def _both(side, plain, work, *args):
     return got
 
 
-def _up(tr, a):
-    import torch
-    return torch.from_numpy(np.ascontiguousarray(a)).to(tr.device)
-
-
 def _b(t):
     return t.cpu().numpy().tobytes()
 
@@ -119,7 +113,7 @@ def test_track_sequence_on_callers_stream(side, plain, depth_case, monkeypatch, 
     monkeypatch.setenv("MV_PNP_K3_SMALL_BELOW", "0")      # the split launch at 7 pairs
 
     def work(tr):
-        d = [_up(tr, x) for x in (semi, sscale, desc, depth)]
+        d = [dev(tr, x) for x in (semi, sscale, desc, depth)]
         return {"records": _b(tr.track_sequence(_depth_params(tc), *d))}
     got = _both(side, plain, work)
     assert got["records"] == want
@@ -128,7 +122,6 @@ def test_track_sequence_on_callers_stream(side, plain, depth_case, monkeypatch, 
 @pytest.mark.parametrize("mode", ["pinned", "pageable", "chunks_of_3"])
 def test_track_sequence_host_on_callers_stream(side, plain, depth_case, monkeypatch, mode):
     """mv_track_sequence_host: pinned buffers (the row gather), pageable ones, and staging chunks of 3 pairs."""
-    import torch
     (semi, sscale, desc, depth), want = depth_case
     monkeypatch.setenv("MV_PNP_K3_SMALL_BELOW", "0")
     monkeypatch.delenv("MV_HOST_CHUNK_PAIRS", raising=False)
@@ -138,7 +131,7 @@ def test_track_sequence_host_on_callers_stream(side, plain, depth_case, monkeypa
 
     def work(tr):
         bufs = [np.ascontiguousarray(x) for x in (semi, sscale, desc, depth)] if mode == "pageable" else \
-            [_pinned(torch, x) for x in (semi, sscale, desc, depth)]
+            [pinned(x) for x in (semi, sscale, desc, depth)]
         res, _, down = tr.track_sequence_host(_depth_params(1), *bufs)
         assert down == 64 * (semi.shape[0] - 1)
         return {"records": res.tobytes()}
@@ -151,7 +144,7 @@ def test_track_sequence_host_on_callers_stream(side, plain, depth_case, monkeypa
 def lm_case(oracle, synth):
     """tests/test_landmark_reference.py's "degenerate" case (frames without keypoints, an overflowing frame,
     saturated and zero descriptors) and its reference."""
-    c = _case_inputs("degenerate", synth)
+    c = case_inputs("degenerate", synth)
     rec, nl, table = landmark_reference(oracle, oracle.bow_vocab(*c["vocab"]), c["p"], *c["frames"],
                                         first_frame=c["first"], n_words=c["n_words"])
     return c, rec.tobytes(), nl.tobytes(), table.tobytes()
@@ -159,28 +152,27 @@ def lm_case(oracle, synth):
 
 def _landmark_entry(tr, c, entry):
     """One landmark-path entry point on the case, from an empty table -> dict of bytes."""
-    import torch
     p, first, n_words, host = c["p"], c["first"], c["n_words"], c["frames"]
     tr.bow_set_vocabulary(*c["vocab"])
     table = tr.landmarks_new(n_words)
     n_pairs = host[0].shape[0] - 1
     if entry == "device":
-        res, nl = tr.track_sequence_landmarks(p, *[_up(tr, x) for x in host], table, first_frame=first)
+        res, nl = tr.track_sequence_landmarks(p, *[dev(tr, x) for x in host], table, first_frame=first)
         res, nl = _b(res), _b(nl)
     elif entry == "host":
-        res, nl, _, _ = tr.track_sequence_landmarks_host(p, *[_pinned(torch, x) for x in host], table, first_frame=first)
+        res, nl, _, _ = tr.track_sequence_landmarks_host(p, *[pinned(x) for x in host], table, first_frame=first)
         res, nl = res.tobytes(), nl.tobytes()
     else:   # two blocks, 8 warm-up frames, prepared in reverse order
         n_warm = 8
-        bufs = [_up(tr, x) for x in host] if entry == "blocks" else [_pinned(torch, x) for x in host]
+        bufs = [dev(tr, x) for x in host] if entry == "blocks" else [pinned(x) for x in host]
         prep = tr.track_landmarks_prepare if entry == "blocks" else tr.track_landmarks_prepare_host
         half = n_pairs // 2
         blocks = [(0, half), (half, n_pairs - half)]
         prepared = {}
         for i, (lo, cnt) in reversed(list(enumerate(blocks))):
             w = min(n_warm, lo)
-            prepared[i] = prep(_params(p, p.pnp.first_pair + lo), w, first + lo, *[x[lo - w:lo + cnt + 1] for x in bufs],
-                               n_words)
+            prepared[i] = prep(with_first_pair(p, p.pnp.first_pair + lo), w, first + lo,
+                               *[x[lo - w:lo + cnt + 1] for x in bufs], n_words)
         rs, ns = [], []
         for i in range(len(blocks)):
             tr.track_landmarks_step_table(prepared[i], table)
@@ -203,11 +195,11 @@ def _table_walk(tr, oracle, n_words, first, k, n_warm, word, qc, coords):
     """mv_landmarks_sequence over frames 0 .. k-1, then the block k .. by mv_landmarks_sequence and by
     speculate / resolve from the same entry table -> dict of bytes."""
     entry = tr.landmarks_new(n_words)
-    head = tr.landmarks_sequence(entry, first, _up(tr, word[:k]), _up(tr, qc[:k]), _up(tr, coords[:k]))
+    head = tr.landmarks_sequence(entry, first, dev(tr, word[:k]), dev(tr, qc[:k]), dev(tr, coords[:k]))
     seq_t = entry.clone()
-    seq = tr.landmarks_sequence(seq_t, first + k, _up(tr, word[k:]), _up(tr, qc[k:]), _up(tr, coords[k:]))
-    spec = tr.landmarks_speculate(n_words, first + k, n_warm, _up(tr, word[k - n_warm:]), _up(tr, qc[k - n_warm:]),
-                                  _up(tr, coords[k:]))
+    seq = tr.landmarks_sequence(seq_t, first + k, dev(tr, word[k:]), dev(tr, qc[k:]), dev(tr, coords[k:]))
+    spec = tr.landmarks_speculate(n_words, first + k, n_warm, dev(tr, word[k - n_warm:]), dev(tr, qc[k - n_warm:]),
+                                  dev(tr, coords[k:]))
     spec_t = entry.clone()
     res = tr.landmarks_resolve(spec, spec_t)
     out = {"head": _b(head), "entry": _b(entry), "seq": _b(seq), "seq_table": _b(seq_t), "resolve": _b(res),
@@ -247,12 +239,12 @@ def test_detector_and_matchers_on_callers_stream(side, plain, oracle, synth):
     def work(tr):
         from maveric_slam_b200 import tracking
         out = {}
-        idx, prob, nv = tr.softmax(_up(tr, semi), _up(tr, sscale))
+        idx, prob, nv = tr.softmax(dev(tr, semi), dev(tr, sscale))
         out.update(idx=_b(idx), prob=_b(prob), nv=_b(nv))
         qp, qi, qpr, qc, ov = tr.top_n(idx, prob, N, mv)
         out.update(qp=_b(qp), qi=_b(qi), qpr=_b(qpr), qc=_b(qc), ov=_b(ov))
         for tc in (0, 1):
-            m = tr.match(tracking.match_params(rows, cols, use_tensor_cores=tc), _up(tr, desc), idx, prob, qp, qi, qc)
+            m = tr.match(tracking.match_params(rows, cols, use_tensor_cores=tc), dev(tr, desc), idx, prob, qp, qi, qc)
             cnt = m[1].cpu().numpy()
             out["count%d" % tc] = cnt.tobytes()
             for name, t in zip(("pts", "cell0", "query", "score"), (m[0], m[2], m[3], m[4])):
@@ -298,9 +290,6 @@ def test_ransac_and_pnp_on_callers_stream(side, plain, oracle, synth, monkeypatc
     """RANSAC-E of a batch, and mv_pnp_gn_batch on test_pnp_split_launch_returns_identical_bytes's batch (pairs of 0 to
     1000 correspondences, the split launch forced): every hypothesis bit for bit against the oracle."""
     from oracle import orc
-    from test_gpu_parity import _pnp_params
-    from test_gpu_properties import _problems
-    from maveric_slam_b200 import tracking
     monkeypatch.setenv("MV_PNP_K3_SMALL_BELOW", "0")
     rng = np.random.default_rng(5)
     P, M = 5, 300
@@ -311,13 +300,13 @@ def test_ransac_and_pnp_on_callers_stream(side, plain, oracle, synth, monkeypatc
         pts[p, :, :2] = a
         pts[p, :, 2:] = a + rng.integers(-1, 2, size=(M, 2))
     counts = np.array([330, 5, 0, 480, 600, 17, 330, 1000, 128, 3, 250], np.int32)
-    corr = _problems(synth, len(counts), 1000, 1024)
+    corr = pnp_problems(synth, len(counts), 1000, 1024)
     H = 1024
-    prm = _pnp_params(tracking, H, 1)
+    prm = pnp_params(H, 1)
 
     def work(tr):
-        ninl, inl, pose = tr.ransac_identity(_up(tr, pts), _up(tr, cnt))
-        kp, ks, kh = tr.pnp_gn(prm, _up(tr, corr), _up(tr, counts), want_hyp=True)
+        ninl, inl, pose = tr.ransac_identity(dev(tr, pts), dev(tr, cnt))
+        kp, ks, kh = tr.pnp_gn(prm, dev(tr, corr), dev(tr, counts), want_hyp=True)
         return {"ninl": _b(ninl), "inl": _b(inl), "pose": _b(pose), "k3_pose": _b(kp), "k3_stats": _b(ks),
                 "k3_hyp": _b(kh)}
     got = _both(side, plain, work)
@@ -353,11 +342,10 @@ def test_bow_lba_and_trajectory_on_callers_stream(side, plain, oracle):
     from oracle import traj_oracle
     from maveric_slam_b200 import tracking
     rng = np.random.default_rng(29)
-    vocab = _ref_vocab()
-    bow_in = _bow_inputs(7, 37)
+    vocab = ref_vocab()
+    bow_in = bow_inputs(7, 37)
     J = {(P, ch): rng.normal(size=(2, 8 * ch, P, 20)).astype(f32) for P, ch in ((8, 4), (16, 8), (5, 2))}
-    from test_lba import _spd_system
-    Cs = {P: np.stack([_spd_system(rng, P)[0] for _ in range(3)]) for P in (16, 12, 3)}
+    Cs = {P: np.stack([spd_system(rng, P)[0] for _ in range(3)]) for P in (16, 12, 3)}
     T = np.zeros((40, 3, 4))
     for k in range(40):
         q = rng.normal(size=4) * [1, 0.01, 0.02, 0.01] + [1, 0, 0, 0]
@@ -369,14 +357,14 @@ def test_bow_lba_and_trajectory_on_callers_stream(side, plain, oracle):
 
     def work(tr):
         tr.bow_set_vocabulary(*vocab)
-        out = {"words": _bow_check(tr, oracle, vocab, *bow_in).tobytes()}
+        out = {"words": bow_check(tr, oracle, vocab, *bow_in).tobytes()}
         for key, j in J.items():
-            out["schur%s" % (key,)] = _b(tr.lba_schur(_up(tr, j), key[1]))
+            out["schur%s" % (key,)] = _b(tr.lba_schur(dev(tr, j), key[1]))
         for P, c in Cs.items():
-            d, ok = tr.lba_solve(_up(tr, c), 1e-3)
+            d, ok = tr.lba_solve(dev(tr, c), 1e-3)
             out["solve%d" % P] = _b(d) + _b(ok)
-        out["chain"] = _b(tr.chain_transforms(_up(tr, T)))
-        out["transforms"] = _b(tr.results_to_transforms(_up(tr, rec.view(np.uint8).reshape(20, 64))))
+        out["chain"] = _b(tr.chain_transforms(dev(tr, T)))
+        out["transforms"] = _b(tr.results_to_transforms(dev(tr, rec.view(np.uint8).reshape(20, 64))))
         return out
     got = _both(side, plain, work)
     for (P, ch), j in J.items():
@@ -444,7 +432,7 @@ def _path_job(torch, oracle, synth, rows, cols, seed):
     s = torch.cuda.Stream(0)
     with torch.cuda.stream(s):
         tr = tracking.Tracker(0)
-        d = [_up(tr, x) for x in (semi, sscale, desc, depth)]
+        d = [dev(tr, x) for x in (semi, sscale, desc, depth)]
         s.synchronize()
     return s, lambda: _b(tr.track_sequence(p, *d)), rec.tobytes()
 
@@ -467,8 +455,7 @@ def test_contexts_on_several_threads_at_once(torch_cuda, oracle, synth, lm_case)
     for name, shapes, solves in (("lba_large", ((16, 8),), (16,)), ("lba_small", ((8, 8), (8, 4)), (12, 10))):
         s = torch.cuda.Stream(0)
         J = [(ch, rng.normal(size=(2, 2 * 8, P, 20)).astype(f32)) for P, ch in shapes]
-        from test_lba import _spd_system
-        Cs = [np.stack([_spd_system(rng, P)[0] for _ in range(4)]) for P in solves]
+        Cs = [np.stack([spd_system(rng, P)[0] for _ in range(4)]) for P in solves]
         expect = b"".join(oracle.lba_schur(j[w], ch).tobytes() for ch, j in J for w in range(2))
         for c in Cs:
             sol = [oracle.lba_solve(c[w], 0.0) for w in range(4)]
@@ -476,8 +463,8 @@ def test_contexts_on_several_threads_at_once(torch_cuda, oracle, synth, lm_case)
             expect += np.stack([d for _, d in sol]).astype(f32).tobytes() + np.ones(4, np.int32).tobytes()
         with torch.cuda.stream(s):
             tr = tracking.Tracker(0)
-            dj = [(ch, _up(tr, j)) for ch, j in J]
-            dc = [_up(tr, c) for c in Cs]
+            dj = [(ch, dev(tr, j)) for ch, j in J]
+            dc = [dev(tr, c) for c in Cs]
             s.synchronize()
 
         def lba(tr=tr, dj=dj, dc=dc):
@@ -489,14 +476,14 @@ def test_contexts_on_several_threads_at_once(torch_cuda, oracle, synth, lm_case)
         jobs.append((name, s, lba))
         want[name] = expect
 
-    bow_in = _bow_inputs(7, 37)
-    for name, vocab in (("bow_ref", _ref_vocab()), ("bow_64x210", _bow_vocab("64x210"))):
+    bow_in = bow_inputs(7, 37)
+    for name, vocab in (("bow_ref", ref_vocab()), ("bow_64x210", bow_vocab("64x210"))):
         s = torch.cuda.Stream(0)
         with torch.cuda.stream(s):
             tr = tracking.Tracker(0)
             tr.bow_set_vocabulary(*vocab)
-            words = _bow_check(tr, oracle, vocab, *bow_in)     # the serial run, held to the oracle
-            d = [_up(tr, x) for x in bow_in]
+            words = bow_check(tr, oracle, vocab, *bow_in)     # the serial run, held to the oracle
+            d = [dev(tr, x) for x in bow_in]
             s.synchronize()
         jobs.append((name, s, lambda tr=tr, d=d: _b(tr.bow_assign(*d)[0])))
         want[name] = words.tobytes()
@@ -506,7 +493,7 @@ def test_contexts_on_several_threads_at_once(torch_cuda, oracle, synth, lm_case)
     with torch.cuda.stream(s):
         tr = tracking.Tracker(0)
         tr.bow_set_vocabulary(*c["vocab"])
-        bufs = [_pinned(torch, x) for x in c["frames"]]
+        bufs = [pinned(x) for x in c["frames"]]
 
     def landmarks(tr=tr, bufs=bufs):
         t = tr.landmarks_new(c["n_words"])
@@ -547,9 +534,9 @@ def test_contexts_of_two_gpus_from_two_threads(torch_cuda, synth):
     p = _depth_params(None, hypotheses=64, rows=rows, cols=cols, top_n=100, max_matches=150, thr=0.9)
     ctxs = {}
     for t in (0, 1):
-        for dev in (0, 1):
-            tr = tracking.Tracker(dev)
-            ctxs[t, dev] = (tr, [_up(tr, x) for x in (semi, sscale, desc, depth)])
+        for gpu in (0, 1):
+            tr = tracking.Tracker(gpu)
+            ctxs[t, gpu] = (tr, [dev(tr, x) for x in (semi, sscale, desc, depth)])
     torch.cuda.set_device(0)
     want = _b(ctxs[0, 0][0].track_sequence(p, *ctxs[0, 0][1]))
     got, errors = {}, []
@@ -559,12 +546,12 @@ def test_contexts_of_two_gpus_from_two_threads(torch_cuda, synth):
             torch.cuda.set_device(t)
             outs = []
             for _ in range(3):
-                for dev in (0, 1):
-                    tr, d = ctxs[t, dev]
+                for gpu in (0, 1):
+                    tr, d = ctxs[t, gpu]
                     res = tr.track_sequence(p, *d)
-                    assert torch.cuda.current_device() == t, (t, dev)
+                    assert torch.cuda.current_device() == t, (t, gpu)
                     tr.ctx.sync()
-                    assert torch.cuda.current_device() == t, (t, dev)
+                    assert torch.cuda.current_device() == t, (t, gpu)
                     outs.append(_b(res))
             got[t] = outs
         except BaseException as e:
