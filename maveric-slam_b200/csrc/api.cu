@@ -1104,17 +1104,14 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
 
   // zero-copy gather needs device-visible (pinned) descriptor and depth buffers
   bool gather = true;
-  if (const char* e = getenv("MV_HOST_GATHER")) gather = atoi(e) != 0;
   const int8_t* hd_desc = nullptr;
-  if (gather) {
-    cudaPointerAttributes a1;
-    if (cudaPointerGetAttributes(&a1, h_desc) == cudaSuccess && a1.type == cudaMemoryTypeHost && a1.devicePointer &&
-        (reinterpret_cast<uintptr_t>(a1.devicePointer) & 15) == 0) {
-      hd_desc = (const int8_t*)a1.devicePointer;
-    } else {
-      cudaGetLastError();
-      gather = false;  // pageable memory: plain staged copies
-    }
+  cudaPointerAttributes a1;
+  if (cudaPointerGetAttributes(&a1, h_desc) == cudaSuccess && a1.type == cudaMemoryTypeHost && a1.devicePointer &&
+      (reinterpret_cast<uintptr_t>(a1.devicePointer) & 15) == 0) {
+    hd_desc = (const int8_t*)a1.devicePointer;
+  } else {
+    cudaGetLastError();
+    gather = false;  // pageable memory: plain staged copies
   }
 
   // The PnP kernel (37 KB of shared memory per CTA) would otherwise fill an SM's shared memory with
@@ -1192,18 +1189,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
   MV_CUDA(c, cudaStreamWaitEvent(c->gather_stream, start, 0));
   MV_CUDA(c, cudaMemsetAsync(dmoved, 0, 8, c->gather_stream));
 
-  // MV_HOST_TRACE=1: timestamp every stage of every chunk (debug aid, prints to stderr)
-  const bool trace = getenv("MV_HOST_TRACE") != nullptr;
-  std::vector<std::pair<std::string, cudaEvent_t>> marks;
-  auto mark = [&](const char* what, int chunk, cudaStream_t s) {
-    if (!trace) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, s);
-    marks.push_back({std::string(what) + "#" + std::to_string(chunk), e});
-  };
-  mark("start", 0, c->stream);
-
   unsigned long long up = 0;
   // The scratch of chunk k: its buffer set, but a block being prepared keeps what step_table and solve read at the
   // chunk's frames and pairs in its own memory.  The detector of chunk k+1 writes the halo frame's qp / qc / ov there
@@ -1229,7 +1214,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
     cudaStream_t cs = c->copy_stream;
     // buffer set b may be refilled only after the compute that read it is done
     MV_CUDA(c, cudaStreamWaitEvent(cs, consumed[b], 0));
-    mark("dma_beg", k, cs);
     MV_CUDA(c, cudaMemcpyAsync(bs[b], h_semi + (size_t)p0 * cells * 65, (size_t)nf * cells * 65,
                                cudaMemcpyHostToDevice, cs));
     MV_CUDA(c, cudaMemcpyAsync(bsc[b], h_semi_scale + p0, sizeof(float) * (size_t)nf, cudaMemcpyHostToDevice, cs));
@@ -1249,7 +1233,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
       up += (unsigned long long)nf * (size_t)cells * 256;
     }
     MV_CUDA(c, cudaEventRecord(copied[b], cs));
-    mark("dma_end", k, cs);
     return MV_OK;
   };
   // The row gather of chunk k+1 runs beside the pose kernels of chunk k, not beside its matcher:
@@ -1264,7 +1247,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
     cudaStream_t gs = c->gather_stream;
     MV_CUDA(c, cudaStreamWaitEvent(gs, detected[b], 0));
     if (after) MV_CUDA(c, cudaStreamWaitEvent(gs, after, 0));
-    mark("gat_beg", k, gs);
     // An SM's L1/shared split is per-SM state: a kernel that asks for no shared memory
     // configures "all L1", and the PnP CTAs (5 x 37 KB shared) then cannot join that SM until
     // it drains.  Ask for the max-shared carveout so both kernels agree on the split.
@@ -1279,7 +1261,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
                                                    (unsigned long long*)dmoved, abort_flag);
     MV_CHECK_LAUNCH(c);
     MV_CUDA(c, cudaEventRecord(ready[b], gs));
-    mark("gat_end", k, gs);
     return MV_OK;
   };
   auto stage_detect = [&](int k) -> mv_status {
@@ -1301,7 +1282,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
       MV_CHECK_LAUNCH(c);
     }
     MV_CUDA(c, cudaEventRecord(detected[b], c->stream));
-    mark("det_end", k, c->stream);
     if (!gather) {
       MV_CUDA(c, cudaEventRecord(ready[b], c->stream));
     } else if (k == 0) {
@@ -1332,7 +1312,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
                              dnwl ? (int32_t*)dnwl + p0 : nullptr};
     mv_status s2;
     MV_CUDA(c, cudaStreamWaitEvent(c->stream, ready[b], 0));
-    mark("cmp_beg", k, c->stream);
     if (landmarks && (s2 = seq_words(c, p, warm ? nf : nf - 1, desc, depth, v, &lm))) return s2;
     if (call == HostCall::landmarks &&
         (s2 = mv_landmarks_sequence_impl(c, n_words, d_table, lm.first_frame, nf - 1, N, v.word, v.qc, v.coords_in,
@@ -1340,17 +1319,14 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
       return s2;
     if (!warm) {
       if ((s2 = seq_match(c, p, nf, desc, v))) return s2;
-      mark("match_end", k, c->stream);
       if ((!prepare && (s2 = release_gather(k))) || (s2 = seq_ransac(c, p, nf, v))) return s2;
     }
     if (prepare && (s2 = release_gather(k))) return s2;
     if (!prepare) {
       if ((s2 = seq_corr(c, p, nf, depth, v, landmarks ? &lm : nullptr))) return s2;
-      mark("corr_end", k, c->stream);
       if ((s2 = seq_pose(c, p, nf, v, (mv_pair_result*)dres + p0, p0))) return s2;
     }
     MV_CUDA(c, cudaEventRecord(consumed[b], c->stream));
-    mark("cmp_end", k, c->stream);
     return MV_OK;
   };
 
@@ -1385,15 +1361,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
   MV_CUDA(c, cudaStreamSynchronize(c->copy_stream));
   MV_CUDA(c, cudaMemcpyAsync(&moved, dmoved, 8, cudaMemcpyDeviceToHost, c->gather_stream));
   MV_CUDA(c, cudaStreamSynchronize(c->gather_stream));
-  if (trace) {
-    if (call == HostCall::prepare) MV_CUDA(c, cudaStreamSynchronize(c->stream));
-    for (auto& m : marks) {
-      float ms = 0.f;
-      cudaEventElapsedTime(&ms, marks[0].second, m.second);
-      fprintf(stderr, "[mv trace] %-12s %9.3f ms\n", m.first.c_str(), ms);
-    }
-    for (auto& m : marks) cudaEventDestroy(m.second);
-  }
   if (gather) up += moved * 256ull;  // one 256 B descriptor row per staged cell
   if (h2d_bytes) *h2d_bytes = up;
   if (d2h_bytes) *d2h_bytes = down;

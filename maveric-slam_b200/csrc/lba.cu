@@ -480,8 +480,7 @@ extern "C" mv_status mv_lba_schur_batch(mv_ctx* ctx, int n_windows, int n_ldmks,
     ctx->lba_schur_smem_attr_set = true;
   }
   mv_prof_scope ps(ctx, "lba");
-  const bool generic = getenv("MV_LBA_GENERIC") && atoi(getenv("MV_LBA_GENERIC"));   // A/B knob
-  if (n_poses == kP8 && chunk == kC4 && !generic)
+  if (n_poses == kP8 && chunk == kC4)
     lba_schur_p8c4_kernel<<<n_windows, 256, 0, ctx->stream>>>(n_ldmks, d_J, d_C);
   else
     lba_schur_kernel<<<n_windows, kLbaThreads, smem, ctx->stream>>>(n_ldmks, n_poses, chunk, d_J, d_C);

@@ -71,8 +71,6 @@ def test_pnp_split_launch_returns_identical_bytes(tracker, synth, monkeypatch):
         with monkeypatch.context() as m:
             m.setenv("MV_PNP_TAIL_PAIRS", tail)
             assert run() == want, ("tail pairs", tail)
-    monkeypatch.setenv("MV_PNP_ORDER", "0")            # index order: no split
-    assert run() == want, "index order"
 
 
 @pytest.mark.parametrize("lanes", [0, 2, 3, 4, 8, 16, 64])

@@ -46,28 +46,28 @@ def test_chunk_size_changes_nothing(tracker, lmseq, monkeypatch, chunk):
     _assert_equal_device(lmseq, res, nl, table, chunk)
 
 
-def test_staging_mode_changes_nothing(tracker, lmseq, monkeypatch):
+def test_pageable_and_unaligned_staging_change_nothing(tracker, lmseq, monkeypatch):
+    """Pageable buffers (plain staged copies) and a pinned depth buffer off a 16-byte boundary give the pinned
+    path's answer; pageable staging moves whole descriptor planes, the row gather fewer bytes."""
     import torch
-    h = lmseq["h"]
-    monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", "9")
+    h, chunk = lmseq["h"], 9
+    monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", str(chunk))
     _, _, _, up_gather, _ = landmarks_host(tracker, lmseq)
     pageable = {k: v.numpy().copy() for k, v in h.items()}
     res, nl, table, up_pageable, _ = landmarks_host(tracker, lmseq, h=pageable)
     _assert_equal_device(lmseq, res, nl, table, "pageable")
-    with monkeypatch.context() as m:
-        m.setenv("MV_HOST_GATHER", "0")
-        res, nl, table, up_copy, _ = landmarks_host(tracker, lmseq)
-        _assert_equal_device(lmseq, res, nl, table, "MV_HOST_GATHER=0")
-    assert up_copy == up_pageable
+    # pageable staging moves whole descriptor planes: every byte of a chunk's frames, the halo frame included
+    n, cells = h["depth"].shape
+    frame = cells * (65 + 4 + 256) + 4 + 4
+    assert up_pageable == sum((min(chunk, n - 1 - p0) + 1) * frame for p0 in range(0, n - 1, chunk))
     # a depth buffer 4 bytes off a 16-byte boundary
-    n, cells = lmseq["h"]["depth"].shape
     buf = torch.empty(n * cells + 4, dtype=torch.float32, pin_memory=True)
     odd = buf[1:1 + n * cells].view(n, cells)
     odd.copy_(h["depth"])
     assert odd.data_ptr() % 16 == 4
     res, nl, table, up_odd, _ = landmarks_host(tracker, lmseq, h=dict(h, depth=odd))
     _assert_equal_device(lmseq, res, nl, table, "unaligned depth")
-    assert up_odd == up_gather < up_copy
+    assert up_odd == up_gather < up_pageable
 
 
 def test_resume_and_halo(tracker, lmseq):

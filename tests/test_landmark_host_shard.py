@@ -96,16 +96,14 @@ def test_blocks_in_reverse_with_a_device_block(tracker, lmseq, two_contexts):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("mode", ["chunk1", "chunk7", "chunk40", "pageable", "no_gather"])
+@pytest.mark.parametrize("mode", ["chunk1", "chunk7", "chunk40", "pageable"])
 def test_chunking_and_staging_change_nothing(tracker, lmseq, monkeypatch, mode):
     s = lmseq
     h = s["h"]
     if mode.startswith("chunk"):
         monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", mode[5:])
-    elif mode == "pageable":
-        h = {k: v.numpy().copy() for k, v in h.items()}
     else:
-        monkeypatch.setenv("MV_HOST_GATHER", "0")
+        h = {k: v.numpy().copy() for k, v in h.items()}
     blocks = [(0, 10), (10, 40), (50, 15)]
     prepared = [_prep_host(tracker, s, lo, c, 8, h=h) for lo, c in blocks]
     _assert_one_call(s, _chain(s, prepared, [tracker] * 3), mode)

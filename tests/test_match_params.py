@@ -498,7 +498,7 @@ SEQ_CASES = {
     "ransac_0": dict(shape=47, ransac=(0, 1.1)),
     **{"ransac_1_%r" % t: dict(shape=47, ransac=(1, t)) for t in (0.0, 0.25, 1e30)},
 }
-SEQ_ENTRIES = ("device", "host_pinned", "host_pageable", "host_no_gather")
+SEQ_ENTRIES = ("device", "host_pinned", "host_pageable", "host_pageable_chunk2")
 
 
 def _seq_params(shape, thr=DEFAULT_THR, gate=DEFAULT_GATE, ransac=(10, 1.1)):
@@ -627,7 +627,6 @@ def _run_sequence(tracker, p, frames, entry, monkeypatch):
     import torch
     from maveric_slam_b200 import tracking
     monkeypatch.delenv("MV_HOST_CHUNK_PAIRS", raising=False)
-    monkeypatch.delenv("MV_HOST_GATHER", raising=False)
     if entry == "device":
         dev = [torch.from_numpy(np.ascontiguousarray(x)).to(tracker.device) for x in frames]
         return tracking.results_to_numpy(tracker.track_sequence(p, *dev))
@@ -644,9 +643,8 @@ def _run_sequence(tracker, p, frames, entry, monkeypatch):
         q.match.min_prob0 = -INF
         reversed_desc = np.ascontiguousarray(desc[::-1])
         tracker.track_sequence_host(q, *[pinned(x) for x in (semi, sscale, reversed_desc, depth)])
-        if entry == "host_no_gather":
-            m.setenv("MV_HOST_GATHER", "0")
-        return tracker.track_sequence_host(p, *[pinned(x) for x in frames])[0]
+        stage = np.ascontiguousarray if entry == "host_pageable_chunk2" else pinned
+        return tracker.track_sequence_host(p, *[stage(x) for x in frames])[0]
 
 
 @pytest.mark.gpu
@@ -654,7 +652,7 @@ def _run_sequence(tracker, p, frames, entry, monkeypatch):
 def test_sequence_vs_oracle(tracker, seq_refs, monkeypatch, name):
     """Whole records of every pair, byte for byte, through the device call and the host call from pinned buffers
     (row gather, chunks of 2 pairs: the three staging buffer sets are reused, so a row the gather skipped holds an
-    earlier frame's descriptor), pageable buffers and pinned buffers without the gather."""
+    earlier frame's descriptor), and pageable buffers, in the default chunks and in chunks of 2 pairs."""
     want = seq_refs.records(name)
     frames = seq_refs.inputs(SEQ_CASES[name]["shape"])
     p = seq_refs.params(name)
@@ -727,7 +725,6 @@ def lm_tracker():
 def test_landmark_path_vs_reference(lm_tracker, lm_ref, monkeypatch, entry):
     c = lm_ref.c
     monkeypatch.delenv("MV_HOST_CHUNK_PAIRS", raising=False)
-    monkeypatch.delenv("MV_HOST_GATHER", raising=False)
     res, nl, table = run_entry(lm_tracker, c, entry, monkeypatch)
     assert res == c["rec"].tobytes(), first_difference(c["rec"], res)
     assert (nl == c["nl"]).all(), (nl, c["nl"])

@@ -325,7 +325,7 @@ def test_pnp_params_vs_oracle(tracker, refs, monkeypatch, name):
     import torch
     c = refs.case(name)
     dev = lambda a: None if a is None else torch.from_numpy(np.ascontiguousarray(a)).to(tracker.device)  # noqa: E731
-    for var in ("MV_PNP_STREAM", "MV_PNP_GPW", "MV_PNP_K3_SMALL_BELOW", "MV_PNP_TAIL_PAIRS", "MV_PNP_ORDER"):
+    for var in ("MV_PNP_STREAM", "MV_PNP_GPW", "MV_PNP_K3_SMALL_BELOW", "MV_PNP_TAIL_PAIRS"):
         monkeypatch.delenv(var, raising=False)
     for label, lanes, env in _forms(c):
         want = refs.answer(name, lanes)

@@ -125,7 +125,6 @@ def test_track_sequence_host_on_callers_stream(side, plain, depth_case, monkeypa
     (semi, sscale, desc, depth), want = depth_case
     monkeypatch.setenv("MV_PNP_K3_SMALL_BELOW", "0")
     monkeypatch.delenv("MV_HOST_CHUNK_PAIRS", raising=False)
-    monkeypatch.delenv("MV_HOST_GATHER", raising=False)
     if mode == "chunks_of_3":
         monkeypatch.setenv("MV_HOST_CHUNK_PAIRS", "3")
 

@@ -4,7 +4,7 @@ hypotheses): one process, the knob read per call, CUDA-event kernel times from t
 profile mode (K3_AB_TAG: pnp by default, or match, detect, ...), results compared byte for byte
 with the default's.
 
-    python tools/k3_ab.py [ENV=VALUE[,ENV=VALUE] ...]     e.g.  MV_PNP_STREAM=1 MV_PNP_GPW=1 MV_PNP_ORDER=0
+    python tools/k3_ab.py [ENV=VALUE[,ENV=VALUE] ...]     e.g.  MV_PNP_STREAM=1 MV_PNP_GPW=1 MV_PNP_TAIL_PAIRS=0
     K3_AB_TAG=match python tools/k3_ab.py                 (another kernel's time; K3_AB_FRAMES=569 a shorter sequence)
     MV_LIB_PATH=/path/variant.so python tools/k3_ab.py    (an A/B build of the library: build.py MV_EXTRA_NVCC / MV_OUT)
 """
