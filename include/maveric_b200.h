@@ -470,6 +470,94 @@ mv_status mv_track_landmarks_solve(mv_ctx* ctx, mv_lm_block* block, mv_pair_resu
 void mv_track_landmarks_release(mv_lm_block* block);
 
 /* ------------------------------------------------------------------------- */
+/* Loop closure: BoW candidates (src/lcd_main.c), verified by match + PnP      */
+/* ------------------------------------------------------------------------- */
+
+/* The reference's lcd_main.c intersects the sorted BoW id lists of two frames.  The score below is this library's
+ * definition (PARITY UNPINNED: the reference program cannot be run here); with unit weights it is the number of
+ * distinct shared words, which is what a sorted-list intersection counts on duplicate-free lists.  All integer,
+ * so exact:
+ *   P[f][w]       1 where word w in [0, n_words) occurs among frame f's first min(q_count[f], top_n) words
+ *                 (duplicates count once; ids outside the range, -1 included, are skipped), else 0
+ *   score(i, j)   sum_w weight[w] * P[i][w] * P[j][w], int32; weights in [0, 127] (d_weight NULL: all 1)
+ *   candidates    of frame i: the frames j <= i - min_gap of the same call (indices within the call) with
+ *                 score >= min_score, the best k by score, descending, the smaller j first on equal scores;
+ *                 reported as global frame numbers first_frame + j
+ * Each call stands alone: a frame is scored against the earlier frames of its own call only.
+ *   d_word int32 [n_frames][top_n], d_q_count int32 [n_frames]   as mv_bow_assign_batch writes them
+ *   d_weight int8 [n_words] (nullable)
+ *   d_cand int32 [n_frames][k]    candidate frames, -1 in unused slots
+ *   d_score int32 [n_frames][k]   their scores, 0 in unused slots
+ * With first_frame < 0 a candidate's global number can itself be -1 (j = -1 - first_frame), which reads like an
+ * unused slot; a caller with negative frame numbers that must tell them apart passes first_frame 0 and adds its
+ * offset to the non-negative entries (mv_detect_loops does so).
+ * The similarity is an int8 GEMM on the tensor cores over the lower triangle of 128 x 128 frame tiles; the score
+ * matrix is never stored.  Context scratch: the presence matrix, n_frames (rounded up to 128) x n_words (rounded up
+ * to 64) bytes, twice with weights, and the per-tile lists, 8 * k bytes per frame and 128-frame column tile
+ * (n_frames^2 * k / 16 bytes: 5 MB at 4 541 frames and k = 4, 2.1 GB at 65 535 frames and k = 8).  MV_ERR_BAD_ARG, with no kernel launched: n_frames outside [1, 65535], top_n <= 0, n_words
+ * outside [1, 2^24], k outside [1, 8], min_gap < 0, first_frame + n_frames - 1 beyond int32, a NULL buffer, and a
+ * negative weight (d_weight is copied to the host to check it, so a call with weights synchronises the context's
+ * stream). */
+mv_status mv_loop_candidates(mv_ctx* ctx, int n_frames, int first_frame, int top_n, int n_words,
+                             const int32_t* d_word, const int32_t* d_q_count, const int8_t* d_weight,
+                             int min_gap, int k, int min_score, int32_t* d_cand, int32_t* d_score);
+
+/* idf weights for mv_loop_candidates from the frames given:
+ *   weight[w] = df ? rint(127 * ln(n_frames / df) / ln(n_frames)) : 0,   computed in double,
+ * df = the number of the n_frames frames whose first min(q_count, top_n) words hold w.  A word in every frame weighs
+ * 0, a word in one frame 127.  n_frames in [2, 65535]; d_weight int8 [n_words] (device). */
+mv_status mv_lcd_word_weights(mv_ctx* ctx, int n_frames, int top_n, int n_words, const int32_t* d_word,
+                              const int32_t* d_q_count, int8_t* d_weight);
+
+typedef struct {
+  mv_match_params match;   /* default: shift 0 and a radius that covers the grid (a revisit's offset is unknown) */
+  mv_pnp_params   pnp;     /* the sampler of candidate r of frame i is keyed on pnp.first_pair + i * k + r */
+  int top_n;               /* queries per frame (words per frame) */
+  int max_valid;           /* MAX_VALID_FEATURES analogue */
+  int min_gap;             /* candidates of frame i are frames j <= i - min_gap (default 30) */
+  int k;                   /* candidates verified per frame, 1..8 (default 4) */
+  int min_score;           /* least BoW score of a candidate (default 1) */
+  int min_inliers;         /* least PnP inliers of an accepted loop (default 30) */
+} mv_loop_params;
+
+void mv_loop_params_default(mv_loop_params* p, int rows, int cols);
+
+/* One record per frame (64 bytes). */
+typedef struct {
+  int32_t frame;           /* the accepted earlier frame j (global number: first_frame + its index in the call), -1
+                            * if none; with first_frame < 0 an accepted frame can be -1 too: test bow_rank */
+  int32_t bow_score;       /* its score and its rank (0 = best) in the frame's candidate list; 0 / -1 if none, */
+  int32_t bow_rank;        /* so bow_rank >= 0 exactly where a loop was accepted */
+  int32_t num_matches;     /* matches of pair (f0 = j, f1 = i) */
+  float pnp_inliers;       /* Gauss-Newton PnP inliers and cost of that pair */
+  float pnp_cost;
+  float q[4];              /* the pose that takes frame j's camera points into frame i's (w,x,y,z), the */
+  float t[3];              /* convention of mv_pair_result with f0 = j and f1 = i; zero if none */
+  int32_t status;          /* 0 ok; MV_ERR_TOO_MANY_VALID if frame i, or the accepted j, overflowed max_valid */
+  int32_t pad[2];
+} mv_loop_result;
+
+/* Loop closures of n_frames device-resident frames (inputs as mv_track_sequence, plus mv_bow_assign_batch's desc
+ * scales), in context scratch:
+ *   1. the detector and top-N of every frame;  2. their words (the context's vocabulary, n_words of it);
+ *   3. mv_loop_candidates(p->min_gap, p->k, p->min_score, d_weight) with first_frame 0, so that a slot's -1 is
+ *      unambiguous (first_frame is added to the accepted frame's index in the record);
+ *   4. ONE mv_match_batch launch over the pairs (f0 = j, f1 = i) of every candidate slot;
+ *   5. mv_build_corr_batch from frame j's depth;  6. ONE mv_pnp_gn_batch launch, slot r of frame i being pair
+ *      i * k + r (so the sampler key is pnp.first_pair + i * k + r whatever the candidates are);
+ *   7. per frame the candidate with the most PnP inliers, the better BoW rank on equal inliers, accepted where it
+ *      has at least min_inliers.
+ * Slots without a candidate run as pairs (i, i) and their matches are discarded before step 5.  Each record equals
+ * what those calls give when made one by one.  d_results mv_loop_result [n_frames].
+ * MV_ERR_BAD_ARG with no kernel launched: what mv_track_sequence refuses (bar n_frames >= 2: one frame is
+ * allowed), what mv_loop_candidates refuses, no vocabulary, n_frames * k > 65535 (one batched matcher / PnP call),
+ * and a NULL d_desc_scale or d_results. */
+mv_status mv_detect_loops(mv_ctx* ctx, const mv_loop_params* p, int n_frames, int first_frame,
+                          const int8_t* d_semi, const float* d_semi_scale,
+                          const int8_t* d_desc, const float* d_desc_scale, const float* d_depth,
+                          const int8_t* d_weight, mv_loop_result* d_results);
+
+/* ------------------------------------------------------------------------- */
 /* NMS between the detector and the matcher (src/run_nms.c)                     */
 /* ------------------------------------------------------------------------- */
 

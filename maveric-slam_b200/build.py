@@ -27,7 +27,7 @@ if os.environ.get("MV_EXTRA_NVCC"):
 if os.environ.get("MV_OUT"):
     OUT = os.path.abspath(os.environ["MV_OUT"])
     OBJ = OUT + ".obj"
-SOURCES = ["api.cu", "detector.cu", "match.cu", "match_tc.cu", "ransac.cu", "pnp_gn.cu", "traj.cu", "nms.cu", "lba.cu", "bow.cu", "synth.cu", "pool.cpp"]
+SOURCES = ["api.cu", "detector.cu", "match.cu", "match_tc.cu", "ransac.cu", "pnp_gn.cu", "traj.cu", "nms.cu", "lba.cu", "bow.cu", "lcd.cu", "synth.cu", "pool.cpp"]
 
 
 def _newer(src_list, target):

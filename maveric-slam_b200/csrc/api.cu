@@ -808,6 +808,155 @@ extern "C" mv_status mv_track_sequence_landmarks(mv_ctx* c, const mv_track_param
   return seq_step(c, p, n_frames, d_desc, d_depth, w, d_results, &lm);
 }
 
+// ------------------------------------------------------------------------------------
+// loop closure: BoW candidates (lcd.cu), then one matcher launch, depth correspondences and one K3 launch over
+// every candidate slot
+// ------------------------------------------------------------------------------------
+extern "C" void mv_loop_params_default(mv_loop_params* p, int rows, int cols) {
+  memset(p, 0, sizeof(*p));
+  mv_match_params_default(&p->match, rows, cols);
+  p->match.shift_x = p->match.shift_y = 0;   // a revisit's offset is unknown: search the whole grid
+  p->match.radius = std::max(rows, cols);
+  mv_pnp_params_default(&p->pnp);
+  p->top_n = 100;
+  p->max_valid = 1000;
+  p->min_gap = 30;
+  p->k = 4;
+  p->min_score = 1;
+  p->min_inliers = 30;
+}
+
+// The candidate stage of mv_detect_loops runs with first_frame 0: cand holds indices within the call, so -1 marks an
+// empty slot whatever the caller's first_frame (a global frame number may itself be -1).
+// slot s = i * k + r: pair (f0 = j, f1 = i) of candidate r of frame i, or (i, i) where the slot has no candidate
+__global__ void loop_pairs_kernel(int n_slots, int k, const int32_t* __restrict__ cand, int32_t* __restrict__ f0,
+                                  int32_t* __restrict__ f1) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_slots) return;
+  const int i = s / k, c = cand[s];
+  f0[s] = c >= 0 ? c : i;
+  f1[s] = i;
+}
+
+// the matches of slots without a candidate are dropped before the correspondences
+__global__ void loop_drop_empty_kernel(int n_slots, const int32_t* __restrict__ cand, int32_t* __restrict__ match_count) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s < n_slots && cand[s] < 0) match_count[s] = 0;
+}
+
+// per frame: the candidate with the most PnP inliers (the earlier slot, i.e. the better BoW rank, on equal inliers),
+// accepted where it has at least min_inliers
+__global__ void loop_select_kernel(int n_frames, int k, int first_frame, int min_inliers, const int32_t* __restrict__ cand,
+                                   const int32_t* __restrict__ score, const int32_t* __restrict__ match_count,
+                                   const float* __restrict__ pose, const float* __restrict__ stats,
+                                   const int32_t* __restrict__ overflow, mv_loop_result* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_frames) return;
+  int best = -1;
+  float best_inl = 0.0f;
+  for (int r = 0; r < k; r++) {
+    const size_t s = (size_t)i * k + r;
+    if (cand[s] < 0) continue;
+    const float inl = stats[s * 4];
+    if (best < 0 || inl > best_inl) { best = r; best_inl = inl; }
+  }
+  mv_loop_result res;
+  memset(&res, 0, sizeof(res));
+  res.frame = -1;
+  res.bow_rank = -1;
+  if (best >= 0 && best_inl >= (float)min_inliers) {
+    const size_t s = (size_t)i * k + best;
+    res.frame = first_frame + cand[s];
+    res.bow_score = score[s];
+    res.bow_rank = best;
+    res.num_matches = match_count[s];
+    res.pnp_inliers = stats[s * 4];
+    res.pnp_cost = stats[s * 4 + 1];
+    for (int c = 0; c < 4; c++) res.q[c] = pose[s * 7 + c];
+    for (int c = 0; c < 3; c++) res.t[c] = pose[s * 7 + 4 + c];
+  }
+  res.status = (overflow[i] || (res.bow_rank >= 0 && overflow[res.frame - first_frame])) ? (int)MV_ERR_TOO_MANY_VALID : 0;
+  out[i] = res;
+}
+
+extern "C" mv_status mv_detect_loops(mv_ctx* c, const mv_loop_params* p, int n_frames, int first_frame,
+                                     const int8_t* d_semi, const float* d_semi_scale, const int8_t* d_desc,
+                                     const float* d_desc_scale, const float* d_depth, const int8_t* d_weight,
+                                     mv_loop_result* d_results) {
+  MV_ENTER(c);
+  const char* fn = "mv_detect_loops";
+  if (!p || n_frames < 1 || !d_semi || !d_semi_scale || !d_desc || !d_desc_scale || !d_depth || !d_results)
+    MV_BAD_ARG(c, "mv_detect_loops");
+  // the detector, matcher and K3 refusals of the sequence calls; the matcher's tensor-core shape is checked below
+  // for the call's real pair count
+  mv_track_params tp;
+  memset(&tp, 0, sizeof(tp));
+  tp.match = p->match;
+  tp.match.use_tensor_cores = 2;
+  tp.pnp = p->pnp;
+  tp.top_n = p->top_n;
+  tp.max_valid = p->max_valid;
+  const int n_words = c->bow_n_base * c->bow_wpb;
+  mv_status st;
+  if ((st = seq_check(c, fn, &tp, n_frames, d_desc, true, n_words))) return st;
+  if (p->k < 1 || p->k > 8 || (long long)n_frames * p->k > 65535)
+    return bad_arg(c, fn, "k in [1, 8] and n_frames * k <= 65535 (one batched matcher and PnP call)");
+  const int n = n_frames, K = p->k, n_slots = n * K, N = p->top_n, M = p->match.max_matches;
+  if (p->match.use_tensor_cores != 0 && p->match.use_tensor_cores != 2 && !mv_match_tc_feasible(&p->match, n, n_slots, N))
+    return bad_arg(c, fn, "use_tensor_cores = 1 on a shape the tensor-core matcher does not take (2 picks the matcher)");
+  if ((st = mv_loop_candidates_check(c, fn, n, first_frame, N, n_words, d_weight, p->min_gap, K))) return st;
+
+  const int cells = p->match.rows * p->match.cols;
+  SeqScratch w;
+  memset(&w, 0, sizeof(w));
+  int32_t *word, *cand, *score, *f0, *f1;
+  void* v;
+#define SCR(ptr, type, name, bytes)                                   \
+  if ((st = mv_scratch(c, "loop." name, (bytes), &v))) return st;     \
+  ptr = (type*)v
+  SCR(w.idx, int32_t, "idx", sizeof(int32_t) * (size_t)n * cells);
+  SCR(w.prob, float, "prob", sizeof(float) * (size_t)n * cells);
+  SCR(w.qp, int32_t, "qp", sizeof(int32_t) * (size_t)n * N);
+  SCR(w.qi, int32_t, "qi", sizeof(int32_t) * (size_t)n * N);
+  SCR(w.qpr, float, "qpr", sizeof(float) * (size_t)n * N);
+  SCR(w.qc, int32_t, "qc", sizeof(int32_t) * (size_t)n);
+  SCR(w.ov, int32_t, "ov", sizeof(int32_t) * (size_t)n);
+  SCR(word, int32_t, "word", sizeof(int32_t) * (size_t)n * N);
+  SCR(cand, int32_t, "cand", sizeof(int32_t) * (size_t)n_slots);
+  SCR(score, int32_t, "score", sizeof(int32_t) * (size_t)n_slots);
+  SCR(f0, int32_t, "f0", sizeof(int32_t) * (size_t)n_slots);
+  SCR(f1, int32_t, "f1", sizeof(int32_t) * (size_t)n_slots);
+  SCR(w.mp, float, "mp", sizeof(float) * 4 * (size_t)n_slots * M);
+  SCR(w.mc, int32_t, "mc", sizeof(int32_t) * (size_t)n_slots);
+  SCR(w.mcell, int32_t, "mcell", sizeof(int32_t) * (size_t)n_slots * M);
+  SCR(w.corr, float, "corr", sizeof(float) * 5 * (size_t)n_slots * M);
+  SCR(w.pose, float, "pose", sizeof(float) * 7 * (size_t)n_slots);
+  SCR(w.stats, float, "stats", sizeof(float) * 4 * (size_t)n_slots);
+#undef SCR
+
+  if ((st = seq_detect(c, &tp, n, d_semi, d_semi_scale, w)) ||
+      (st = mv_bow_assign_impl(c, n, cells, N, d_desc, d_desc_scale, w.qp, w.qc, word, nullptr, MvBackProject())) ||
+      (st = mv_loop_candidates_impl(c, n, 0, N, n_words, word, w.qc, d_weight, p->min_gap, K, p->min_score,
+                                    cand, score)))
+    return st;
+  const unsigned slot_blocks = (unsigned)((n_slots + 255) / 256);
+  loop_pairs_kernel<<<slot_blocks, 256, 0, c->stream>>>(n_slots, K, cand, f0, f1);
+  MV_CHECK_LAUNCH(c);
+  if ((st = mv_match_batch(c, &p->match, n, n_slots, N, f0, f1, d_desc, w.idx, w.prob, w.qp, w.qi, w.qc, w.mp, w.mc,
+                           w.mcell, nullptr, nullptr)))
+    return st;
+  loop_drop_empty_kernel<<<slot_blocks, 256, 0, c->stream>>>(n_slots, cand, w.mc);
+  MV_CHECK_LAUNCH(c);
+  if ((st = mv_build_corr_batch(c, n_slots, cells, p->match.rows, M, f0, d_depth, p->pnp.fx, p->pnp.fy, p->pnp.cx,
+                                p->pnp.cy, w.mp, w.mc, w.mcell, w.corr)) ||
+      (st = mv_pnp_gn_batch(c, &p->pnp, n_slots, M, w.corr, w.mc, nullptr, w.pose, w.stats, nullptr)))
+    return st;
+  loop_select_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, K, first_frame, p->min_inliers, cand, score, w.mc,
+                                                             w.pose, w.stats, w.ov, d_results);
+  MV_CHECK_LAUNCH(c);
+  return MV_OK;
+}
+
 // ---- chunks of the host staging pipeline (track_sequence_host_impl below)
 // A call's host frames in chunks of `pairs` pairs: first the n_warm warm-up frames of a block being prepared, at most
 // `pairs` frames per chunk and no halo, then the n_pairs pairs, each chunk sharing its first frame with the last

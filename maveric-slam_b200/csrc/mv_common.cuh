@@ -42,6 +42,7 @@ struct mv_ctx {
   bool lba_schur_smem_attr_set = false; // and for the generic Schur and the solve kernels (lba.cu)
   bool lba_solve_smem_attr_set = false;
   bool gather_carveout_set = false;     // the row gather's shared-memory carveout is set (api.cu)
+  bool lcd_smem_attr_set = false;       // the loop-candidate tile kernel's shared-memory limit is set (lcd.cu)
   int lm_words = 0;                     // size the landmark scratch was initialised for
   std::map<std::string, mv_prof_slot> prof;
   std::vector<mv_pending_event> pending;
@@ -178,6 +179,15 @@ mv_status mv_build_corr_landmarks_seq(mv_ctx* ctx, int n_pairs, int top_n, int s
                                       const int32_t* d_q_patch, const int32_t* d_q_count, const int32_t* d_word,
                                       const float* d_coords_out, const float* d_match_pts, const int32_t* d_match_count,
                                       const int32_t* d_match_cell0, float* d_corr, int32_t* d_n_with_landmark);
+
+// ---- loop closure (lcd.cu), called by mv_detect_loops (api.cu)
+// the refusals of mv_loop_candidates (reads d_weight back to check its sign), before anything is enqueued
+mv_status mv_loop_candidates_check(mv_ctx* ctx, const char* fn, int n_frames, int first_frame, int top_n, int n_words,
+                                   const int8_t* d_weight, int min_gap, int k);
+// mv_loop_candidates after its checks
+mv_status mv_loop_candidates_impl(mv_ctx* ctx, int n_frames, int first_frame, int top_n, int n_words,
+                                  const int32_t* d_word, const int32_t* d_q_count, const int8_t* d_weight, int min_gap,
+                                  int k, int min_score, int32_t* d_cand, int32_t* d_score);
 
 // float bounds that make a float-vs-double comparison exact in fp32:
 //   (double)s >  T  <=>  s >  mv_round_down(T)

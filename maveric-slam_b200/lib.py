@@ -31,6 +31,7 @@ NEW_SYMBOLS = [
     "mv_track_sequence_landmarks", "mv_track_sequence_landmarks_host", "mv_landmarks_speculate",
     "mv_landmarks_resolve", "mv_lm_spec_release", "mv_track_landmarks_prepare", "mv_track_landmarks_step_table",
     "mv_track_landmarks_solve", "mv_track_landmarks_release", "mv_track_landmarks_prepare_host",
+    "mv_loop_candidates", "mv_lcd_word_weights", "mv_loop_params_default", "mv_detect_loops",
 ]
 LEGACY_SYMBOLS = [
     "add_Vector2f", "add_Vector3f", "mult_Quaternionf", "create_Quaternionf", "Quaternionf_from_Vector3f",
@@ -70,12 +71,24 @@ class PairResult(C.Structure):
                 ("status", C.c_int32), ("pad", C.c_int32 * 3)]
 
 
+class LoopParams(C.Structure):
+    _fields_ = [("match", MatchParams), ("pnp", PnpParams), ("top_n", C.c_int), ("max_valid", C.c_int),
+                ("min_gap", C.c_int), ("k", C.c_int), ("min_score", C.c_int), ("min_inliers", C.c_int)]
+
+
+class LoopResult(C.Structure):
+    _fields_ = [("frame", C.c_int32), ("bow_score", C.c_int32), ("bow_rank", C.c_int32), ("num_matches", C.c_int32),
+                ("pnp_inliers", C.c_float), ("pnp_cost", C.c_float), ("q", C.c_float * 4), ("t", C.c_float * 3),
+                ("status", C.c_int32), ("pad", C.c_int32 * 2)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("rows", C.c_int), ("cols", C.c_int), ("keypoint_permille", C.c_int),
                 ("noise_amp", C.c_int)]
 
 
 assert C.sizeof(PairResult) == 64
+assert C.sizeof(LoopResult) == 64
 
 _lib = None
 
@@ -156,6 +169,11 @@ def load() -> C.CDLL:
     L.mv_track_landmarks_solve.argtypes = [vp, vp, vp, vp]
     L.mv_track_landmarks_release.argtypes = [vp]
     L.mv_track_landmarks_release.restype = None
+    L.mv_loop_candidates.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, vp, vp]
+    L.mv_lcd_word_weights.argtypes = [vp, i32, i32, i32, vp, vp, vp]
+    L.mv_loop_params_default.argtypes = [C.POINTER(LoopParams), i32, i32]
+    L.mv_loop_params_default.restype = None
+    L.mv_detect_loops.argtypes = [vp, C.POINTER(LoopParams), i32, i32, vp, vp, vp, vp, vp, vp, vp]
     L.mv_synth_frames.argtypes = [vp, C.POINTER(SynthParams), i32, i32, vp, vp, vp, vp]
     L.mv_nms_batch.argtypes = [vp, i32, i32, i32, vp, vp]
     L.run_nms_ex.argtypes = [vp, i32, i32, vp, vp]

@@ -22,6 +22,11 @@ PAIR_RESULT_DTYPE = np.dtype([
     ("num_matches", np.int32), ("ransac_inliers", np.int32), ("best_hypothesis", np.int32),
     ("status", np.int32), ("pad", np.int32, 3)])
 assert PAIR_RESULT_DTYPE.itemsize == 64
+LOOP_RESULT_DTYPE = np.dtype([
+    ("frame", np.int32), ("bow_score", np.int32), ("bow_rank", np.int32), ("num_matches", np.int32),
+    ("pnp_inliers", np.float32), ("pnp_cost", np.float32), ("q", np.float32, 4), ("t", np.float32, 3),
+    ("status", np.int32), ("pad", np.int32, 2)])
+assert LOOP_RESULT_DTYPE.itemsize == 64
 
 
 @dataclass
@@ -232,6 +237,30 @@ def kitti_track_params(**kw) -> _lib.TrackParams:
     return track_params(**d)
 
 
+def loop_params(rows, cols, top_n=100, max_valid=1000, max_matches=150, hypotheses=1024, min_gap=30, k=4,
+                min_score=1, min_inliers=30, radius=None, shift=(0, 0), refine_iters=10, sample_iters=4, lanes=1, seed=0,
+                use_tensor_cores=None, first_pair=0) -> _lib.LoopParams:
+    """mv_loop_params_default with these fields set; radius None keeps the default, which covers the grid."""
+    p = _lib.LoopParams()
+    _lib.load().mv_loop_params_default(C.byref(p), rows, cols)
+    p.top_n, p.max_valid = top_n, max_valid
+    p.min_gap, p.k, p.min_score, p.min_inliers = min_gap, k, min_score, min_inliers
+    p.match.max_matches = max_matches
+    if radius is not None:
+        p.match.radius = radius
+    p.match.shift_x, p.match.shift_y = shift
+    if use_tensor_cores is not None:
+        p.match.use_tensor_cores = 1 if use_tensor_cores else 0
+    p.pnp.hypotheses, p.pnp.refine_iters, p.pnp.sample_iters = hypotheses, refine_iters, sample_iters
+    p.pnp.lanes_per_hypothesis, p.pnp.seed, p.pnp.first_pair = lanes, seed, first_pair
+    return p
+
+
+def loop_results_to_numpy(t) -> np.ndarray:
+    """uint8 [n, 64] loop records (device or host tensor) -> structured array of LOOP_RESULT_DTYPE."""
+    return np.ascontiguousarray(t.cpu().numpy()).view(LOOP_RESULT_DTYPE).reshape(-1)
+
+
 class Tracker:
     """Batched hot path on one GPU.  Tensors are torch CUDA tensors; calls are asynchronous
     on torch's current stream (bound at construction)."""
@@ -418,6 +447,43 @@ class Tracker:
         self.ctx.check(self.lib.mv_bow_assign_batch(self.ctx.h, n, cells, top_n, self._d(desc), self._d(desc_scale),
                                                     self._d(q_patch), self._d(q_count), self._d(word), self._d(base)))
         return word, base
+
+    # -- loop closure: BoW candidates on the tensor cores, verified by the matcher and the Gauss-Newton PnP
+    def lcd_word_weights(self, word, q_count, n_words=None):
+        """idf weights int8 [n_words] of the given frames' words (mv_lcd_word_weights):
+        rint(127 ln(n / df) / ln(n)), 0 for a word no frame holds."""
+        n, top_n = word.shape
+        n_words = self.n_words if n_words is None else n_words
+        weight = self.torch.empty((n_words,), dtype=self.torch.int8, device=self.device)
+        self.ctx.check(self.lib.mv_lcd_word_weights(self.ctx.h, n, top_n, n_words, self._d(word), self._d(q_count),
+                                                    self._d(weight)))
+        return weight
+
+    def loop_candidates(self, word, q_count, weight=None, min_gap=30, k=4, min_score=1, first_frame=0, n_words=None):
+        """The best k earlier frames of every frame by BoW score (mv_loop_candidates): word int32 [n, top_n] and
+        q_count int32 [n] as :meth:`bow_assign` / :meth:`top_n` return them, weight int8 [n_words] or None (all 1).
+        Returns (cand int32 [n, k] global frame numbers or -1, score int32 [n, k])."""
+        torch = self.torch
+        n, top_n = word.shape
+        n_words = self.n_words if n_words is None else n_words
+        cand = torch.empty((n, k), dtype=torch.int32, device=self.device)
+        score = torch.empty((n, k), dtype=torch.int32, device=self.device)
+        self.ctx.check(self.lib.mv_loop_candidates(self.ctx.h, n, int(first_frame), top_n, n_words, self._d(word),
+                                                   self._d(q_count), self._d(weight), int(min_gap), int(k),
+                                                   int(min_score), self._d(cand), self._d(score)))
+        return cand, score
+
+    def detect_loops(self, params: _lib.LoopParams, semi, semi_scale, desc, desc_scale, depth, weight=None,
+                     first_frame=0, out=None):
+        """Loop closures of device-resident frames in one call (mv_detect_loops; vocabulary set first with
+        :meth:`bow_set_vocabulary`) -> uint8 [n_frames, 64] records (view with :func:`loop_results_to_numpy`)."""
+        n = semi.shape[0]
+        if out is None:
+            out = self.torch.empty((n, 64), dtype=self.torch.uint8, device=self.device)
+        self.ctx.check(self.lib.mv_detect_loops(self.ctx.h, C.byref(params), n, int(first_frame), self._d(semi),
+                                                self._d(semi_scale), self._d(desc), self._d(desc_scale),
+                                                self._d(depth), self._d(weight), self._d(out)))
+        return out
 
     def landmarks_new(self, n_words):
         """Empty device landmark table: uint8 [n_words, 56] (view with LANDMARK_DTYPE after .cpu().numpy())."""
