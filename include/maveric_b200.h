@@ -504,7 +504,8 @@ mv_status mv_loop_candidates(mv_ctx* ctx, int n_frames, int first_frame, int top
 
 /* idf weights for mv_loop_candidates from the frames given:
  *   weight[w] = df ? rint(127 * ln(n_frames / df) / ln(n_frames)) : 0,   computed in double,
- * df = the number of the n_frames frames whose first min(q_count, top_n) words hold w.  A word in every frame weighs
+ * df = the number of the n_frames frames whose first min(q_count, top_n) words hold w.  The one exact tie,
+ * df * df == n_frames (63.5), is decided in integers and weighs 64.  A word in every frame weighs
  * 0, a word in one frame 127.  n_frames in [2, 65535]; d_weight int8 [n_words] (device). */
 mv_status mv_lcd_word_weights(mv_ctx* ctx, int n_frames, int top_n, int n_words, const int32_t* d_word,
                               const int32_t* d_q_count, int8_t* d_weight);

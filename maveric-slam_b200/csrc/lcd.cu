@@ -80,14 +80,23 @@ __global__ void presence_kernel(int n, int top_n, int n_words, int kpad, const i
   }
 }
 
-// weight[w] = df ? rint(127 ln(n / df) / ln(n)) : 0 in double, df = frames whose presence row holds w
+// weight[w] = df ? rint(127 ln(n / df) / ln(n)) : 0, df = frames whose presence row holds w.
+// The value is a half-integer exactly when df * df == n, and then it is 63.5, which rint takes to 64.  Proof: for
+// 1 <= df < n, x = ln(n / df) / ln(n) is rational only when n / df and n are powers of one integer base, so x = q / p
+// with p <= 16 (n < 2^16); 127 q / p = (2a + 1) / 2 forces p = 2 (127 is prime and p <= 16), so x = 1/2 and
+// df^2 = n.  In double the tie can land an ulp either side of 63.5 (with the host C library's log it does at 82 of
+// the 254 squares up to 65 025, and rint then gives 63 at 44), so it is decided in integers.  Everywhere else the
+// value is at least 2.1e-10 from a half-integer for n <= 65 535 (tools/idf_tie_scan.c), 15 000 ulp of 64: far beyond
+// the few ulp of error of a double evaluation whose log is within an ulp or two.
 __global__ void word_weights_kernel(int n, int n_words, int kpad, const int8_t* __restrict__ P,
                                     int8_t* __restrict__ weight) {
   const int w = blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= n_words) return;
   int df = 0;
   for (int f = 0; f < n; f++) df += P[(size_t)f * kpad + w];
-  weight[w] = df ? (int8_t)rint(127.0 * log((double)n / (double)df) / log((double)n)) : (int8_t)0;
+  if (!df) weight[w] = 0;
+  else if ((long long)df * df == n) weight[w] = 64;
+  else weight[w] = (int8_t)rint(127.0 * log((double)n / (double)df) / log((double)n));
 }
 
 __global__ void __launch_bounds__(kThreads)

@@ -90,7 +90,10 @@ void orc_lcd_word_weights(int n, int top_n, int n_words, const int32_t* word, co
   distinct_words(n, top_n, n_words, word, q_count, &ids, &off);
   int* df = (int*)calloc((size_t)n_words, sizeof(int));
   for (long long e = 0; e < off[n]; e++) df[ids[e]]++;
+  /* df^2 = n is the one exact half (63.5 -> 64), decided in integers: in double it lands an ulp either side */
   for (int w = 0; w < n_words; w++)
-    weight[w] = df[w] ? (int8_t)rint(127.0 * log((double)n / (double)df[w]) / log((double)n)) : (int8_t)0;
+    weight[w] = !df[w] ? (int8_t)0
+              : (long long)df[w] * df[w] == n ? (int8_t)64
+              : (int8_t)rint(127.0 * log((double)n / (double)df[w]) / log((double)n));
   free(df); free(ids); free(off);
 }

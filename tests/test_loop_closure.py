@@ -8,9 +8,7 @@ oracle without a GPU.  Verification is the composition of calls that are each he
 (matcher, depth correspondences, K3), and is checked here both against those calls made one by one on the GPU and
 against the CPU oracle chain.
 """
-import copy
 import ctypes as C
-import math
 
 import numpy as np
 import pytest
@@ -18,72 +16,8 @@ import pytest
 import lcd_oracle
 from helpers import dev, ref_vocab
 from landmark_reference import depth_xyz, detect, match_cfg, pnp_cfg
-
-STATUS_TOO_MANY_VALID = 4
-
-
-# ------------------------------------------------------------------ the definition, restated in numpy
-def presence(word, q_count, n_words):
-    n, top_n = word.shape
-    P = np.zeros((n, n_words), np.float32)
-    for f in range(n):
-        w = word[f, :min(max(int(q_count[f]), 0), top_n)]
-        P[f, w[(w >= 0) & (w < n_words)]] = 1
-    return P
-
-
-def ref_candidates(word, q_count, n_words, weight, min_gap, k, min_score, first_frame):
-    """-> (cand int32 [n, k], score int32 [n, k]).  Scores in float32 are exact: every partial sum is an integer
-    below 127 * top_n < 2^24."""
-    assert 127 * word.shape[1] < 2 ** 24
-    P = presence(word, q_count, n_words)
-    W = P if weight is None else P * weight.astype(np.float32)
-    S = (W @ P.T).astype(np.int64)
-    n = len(P)
-    cand = np.full((n, k), -1, np.int32)
-    score = np.zeros((n, k), np.int32)
-    for i in range(n):
-        hi = i - min_gap + 1
-        if hi <= 0:
-            continue
-        s = S[i, :hi]
-        j = np.nonzero(s >= min_score)[0]
-        order = j[np.lexsort((j, -s[j]))][:k]
-        cand[i, :len(order)] = first_frame + order
-        score[i, :len(order)] = s[order]
-    return cand, score
-
-
-def ref_word_weights(word, q_count, n_words):
-    P = presence(word, q_count, n_words)
-    n = len(P)
-    df = P.sum(0).astype(np.int64)
-    return np.array([round(127.0 * math.log(n / d) / math.log(n)) if d else 0 for d in df], np.int8)
-
-
-def random_words(rng, n, top_n, n_words, bad=True):
-    """Word lists with duplicates, ids -1 and >= n_words, and query counts 0 and above top_n."""
-    word = rng.integers(0, n_words, size=(n, top_n)).astype(np.int32)
-    if bad:
-        word[rng.random((n, top_n)) < 0.05] = -1
-        word[rng.random((n, top_n)) < 0.05] = n_words + 3
-    q_count = rng.integers(0, top_n + 4, size=n).astype(np.int32)
-    q_count[::7] = 0
-    q_count[1::5] = top_n + 9
-    return word, q_count
-
-
-def random_weights(rng, n_words):
-    w = rng.integers(0, 128, size=n_words).astype(np.int8)
-    w[rng.random(n_words) < 0.1] = 0
-    return w
-
-
-def run_candidates(tracker, word, q_count, n_words, weight, min_gap, k, min_score, first_frame):
-    cand, score = tracker.loop_candidates(dev(tracker, word), dev(tracker, q_count),
-                                          None if weight is None else dev(tracker, weight), min_gap=min_gap, k=k,
-                                          min_score=min_score, first_frame=first_frame, n_words=n_words)
-    return cand.cpu().numpy(), score.cpu().numpy()
+from loop_reference import (COLS, ROWS, frames, loop_offsets, random_weights, random_words, ref_candidates,
+                            ref_word_weights, run_candidates, select, small_params, verify_by_parts)
 
 
 # ------------------------------------------------------------------ 1. candidates
@@ -185,95 +119,10 @@ def test_word_weights_equal_reference(tracker, n, top_n, n_words):
 
 
 # ------------------------------------------------------------------ 3. the whole call equals its parts
-ROWS, COLS = 47, 155
-
-
 @pytest.fixture(scope="module")
 def vocab_tracker(tracker):
     tracker.bow_set_vocabulary(*ref_vocab())
     return tracker
-
-
-def loop_offsets(n, returns):
-    """A (4, 4) cells/frame drift; with `returns`, the last frame comes back next to frame 2's offset (one cell
-    off): the planted revisit of DESIGN §4.7's probe."""
-    off = np.array([(4 * f, 4 * f) for f in range(n)], np.int32)
-    if returns:
-        off[-1] = (9, 8)
-    return off
-
-
-def frames(tracker, synth, off, seed=0):
-    semi, desc, depth = tracker.synth_frames(seed, ROWS, COLS, 0, off)
-    n = off.shape[0]
-    sscale = dev(tracker, np.full(n, synth.SEMI_SCALE, np.float32))
-    dscale = dev(tracker, np.full(n, synth.DESC_SCALE, np.float32))
-    return semi, sscale, desc, dscale, depth
-
-
-def select(params, first_frame, cand, score, cnt, pose, stats, ov):
-    """The selection rule of mv_detect_loops, restated, from candidates as indices within the call (-1: empty slot)
-    -> LOOP_RESULT_DTYPE [n]."""
-    from maveric_slam_b200 import tracking
-    n, k = cand.shape
-    out = np.zeros(n, tracking.LOOP_RESULT_DTYPE)
-    for i in range(n):
-        best = -1
-        for r in range(k):
-            if cand[i, r] >= 0 and (best < 0 or stats[i, r, 0] > stats[i, best, 0]):
-                best = r
-        rec = out[i]
-        rec["frame"], rec["bow_rank"] = -1, -1
-        accepted = best >= 0 and stats[i, best, 0] >= np.float32(params.min_inliers)
-        if accepted:
-            rec["frame"], rec["bow_score"], rec["bow_rank"] = first_frame + cand[i, best], score[i, best], best
-            rec["num_matches"] = cnt[i, best]
-            rec["pnp_inliers"], rec["pnp_cost"] = stats[i, best, 0], stats[i, best, 1]
-            rec["q"], rec["t"] = pose[i, best, :4], pose[i, best, 4:]
-        rec["status"] = STATUS_TOO_MANY_VALID if (ov[i] or (accepted and ov[cand[i, best]])) else 0
-    return out
-
-
-def small_params(**kw):
-    from maveric_slam_b200 import tracking
-    d = dict(top_n=300, max_valid=8192, max_matches=150, hypotheses=64, min_gap=3, k=2, min_score=1, min_inliers=20)
-    d.update(kw)
-    return tracking.loop_params(ROWS, COLS, **d)
-
-
-def verify_by_parts(tr, p, n, args, weight):
-    """Every candidate of every frame through the separate GPU calls: detector, words, mv_loop_candidates (first frame
-    0: indices within the call), mv_match_batch over the explicit list of real candidate pairs only,
-    mv_build_corr_batch and one mv_pnp_gn_batch per pair keyed on pnp.first_pair + i * k + r.
-    -> dict of cand, score [n, k] and per slot cnt [n, k], pose [n, k, 7], stats [n, k, 4], and ov [n]."""
-    semi, sscale, desc, dscale, depth = args
-    idx, prob, _ = tr.softmax(semi, sscale)
-    qp, qi, _, qc, ov = tr.top_n(idx, prob, p.top_n, p.max_valid)
-    word, _ = tr.bow_assign(desc, dscale, qp, qc)
-    if weight == "idf":
-        weight = tr.lcd_word_weights(word, qc)
-    cand, score = tr.loop_candidates(word, qc, weight, p.min_gap, p.k, p.min_score, 0)
-    cand, score = cand.cpu().numpy(), score.cpu().numpy()
-    K = p.k
-    out = dict(cand=cand, score=score, ov=ov.cpu().numpy(), weight=weight, word=word, qc=qc,
-               cnt=np.zeros((n, K), np.int32), pose=np.zeros((n, K, 7), np.float32),
-               stats=np.zeros((n, K, 4), np.float32))
-    slots = [(i, r) for i in range(n) for r in range(K) if cand[i, r] >= 0]
-    out["slots"] = slots
-    if not slots:
-        return out
-    f0 = dev(tr, np.array([cand[i, r] for i, r in slots], np.int32))
-    f1 = dev(tr, np.array([i for i, r in slots], np.int32))
-    pts, cnt, cell0, _, _ = tr.match(p.match, desc, idx, prob, qp, qi, qc, f0=f0, f1=f1)
-    corr = tr.build_corr(pts, cnt, cell0, depth, (p.pnp.fx, p.pnp.fy, p.pnp.cx, p.pnp.cy), ROWS, f0=f0)
-    cnt_h = cnt.cpu().numpy()
-    for m, (i, r) in enumerate(slots):
-        pnp = copy.copy(p.pnp)
-        pnp.first_pair = p.pnp.first_pair + i * K + r
-        pose, stats, _ = tr.pnp_gn(pnp, corr[m:m + 1].contiguous(), cnt[m:m + 1])
-        out["cnt"][i, r], out["pose"][i, r] = cnt_h[m], pose.cpu().numpy()[0]
-        out["stats"][i, r] = stats.cpu().numpy()[0]
-    return out
 
 
 @pytest.mark.gpu
