@@ -742,14 +742,16 @@ static mv_status seq_corr(mv_ctx* c, const mv_track_params* p, int n_frames, con
                              p->pnp.fy, p->pnp.cx, p->pnp.cy, w.mp, w.mc, w.mcell, w.corr);
 }
 
-// K3 and the records; first_pair: the batch's first pair in the call (the PnP sampler is keyed on it).
+// K3 and the records; first_pair: the batch's first pair in the call (the PnP sampler is keyed on it);
+// max_ctas_per_sm: K3's residency cap (0: none).
 static mv_status seq_pose(mv_ctx* c, const mv_track_params* p, int n_frames, const SeqScratch& w,
-                          mv_pair_result* d_results, int first_pair) {
+                          mv_pair_result* d_results, int first_pair, int max_ctas_per_sm) {
   const int n_pairs = n_frames - 1;
   mv_pnp_params pnp = p->pnp;
   pnp.first_pair += first_pair;
   mv_status st;
-  if ((st = mv_pnp_gn_batch(c, &pnp, n_pairs, p->match.max_matches, w.corr, w.mc, nullptr, w.pose, w.stats, nullptr)))
+  if ((st = mv_pnp_gn_batch_impl(c, &pnp, n_pairs, p->match.max_matches, w.corr, w.mc, nullptr, w.pose, w.stats,
+                                 nullptr, max_ctas_per_sm)))
     return st;
   pack_results_kernel<<<(n_pairs + 127) / 128, 128, 0, c->stream>>>(
       n_pairs, w.pose, w.stats, w.mc, p->ransac_iterations > 0 ? w.rin : nullptr, w.ov, d_results);
@@ -771,7 +773,7 @@ static mv_status seq_step(mv_ctx* c, const mv_track_params* p, int n_frames, con
   if ((st = seq_match(c, p, n_frames, d_desc, w)) || (st = seq_ransac(c, p, n_frames, w)) ||
       (st = seq_corr(c, p, n_frames, d_depth, w, lm)))
     return st;
-  return seq_pose(c, p, n_frames, w, d_results, 0);
+  return seq_pose(c, p, n_frames, w, d_results, 0, 0);
 }
 
 extern "C" mv_status mv_track_sequence(mv_ctx* c, const mv_track_params* p, int n_frames, const int8_t* d_semi,
@@ -971,12 +973,14 @@ struct HostPlan {
   }
 };
 
+// K3's CTAs per SM while the pipeline stages: the PnP kernel (37 KB of shared memory per CTA) would otherwise fill an
+// SM's shared memory with 6 CTAs and starve the one-warp row-gather kernel (17 KB) that must run beside it.
+constexpr int kStagingPnpCtasPerSm = 5;
+
 static HostPlan host_plan(const mv_ctx* c, const mv_track_params* p, int n_warm, int n_pairs, bool landmarks) {
-  // chunk = two full waves of the PnP kernel at its capped residency (5 CTAs/SM, see PnpResidencyCap); the
-  // one-thread-per-hypothesis kernel covers 256 hypotheses per CTA, the multi-lane forms 16
-  const int per_cta = p->pnp.lanes_per_hypothesis == 1 ? 256 : 16;
-  const int pnp_ctas_per_pair = (p->pnp.hypotheses + per_cta - 1) / per_cta;
-  int chunk_pairs = 2 * (5 * c->sm_count) / (pnp_ctas_per_pair > 0 ? pnp_ctas_per_pair : 1);
+  // chunk = two full waves of the PnP kernel at its staging residency
+  const int pnp_ctas_per_pair = mv_pnp_ctas_per_pair(&p->pnp);
+  int chunk_pairs = 2 * (kStagingPnpCtasPerSm * c->sm_count) / (pnp_ctas_per_pair > 0 ? pnp_ctas_per_pair : 1);
   if (chunk_pairs < 8) chunk_pairs = 8;
   // short sequences (a rank's shard of a multi-GPU run): at least ~8 chunks, so that the staging
   // pipeline has something to overlap with instead of one long fill and drain
@@ -1102,7 +1106,7 @@ extern "C" mv_status mv_track_landmarks_solve(mv_ctx* c, mv_lm_block* k, mv_pair
   k->phase = 3;
   const SeqLandmarks lm = {k->first_frame, k->n_words, nullptr, nullptr, d_n_with_landmark};
   if ((st = seq_corr(c, &k->p, k->n_frames, nullptr, k->b, &lm))) return st;
-  return seq_pose(c, &k->p, k->n_frames, k->b, d_results, 0);
+  return seq_pose(c, &k->p, k->n_frames, k->b, d_results, 0, 0);
 }
 
 extern "C" void mv_track_landmarks_release(mv_lm_block* k) {
@@ -1219,13 +1223,6 @@ gather_rows_kernel(long long total_cells, const uint8_t* __restrict__ flags, con
   if (lane == 0 && moved) atomicAdd(rows_moved, moved);
 }
 
-struct PnpResidencyCap {  // cap the PnP kernel's CTAs per SM for a scope
-  mv_ctx* c;
-  int saved;
-  PnpResidencyCap(mv_ctx* ctx, int cap) : c(ctx), saved(ctx->pnp_max_ctas_per_sm) { ctx->pnp_max_ctas_per_sm = cap; }
-  ~PnpResidencyCap() { c->pnp_max_ctas_per_sm = saved; }
-};
-
 // The call that stages host buffers through track_sequence_host_impl: mv_track_sequence_host,
 // mv_track_sequence_landmarks_host or mv_track_landmarks_prepare_host.
 enum class HostCall { depth, landmarks, prepare };
@@ -1262,11 +1259,6 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
     cudaGetLastError();
     gather = false;  // pageable memory: plain staged copies
   }
-
-  // The PnP kernel (37 KB of shared memory per CTA) would otherwise fill an SM's shared memory with
-  // 6 CTAs and starve the one-warp row-gather kernel (17 KB) that must run beside it.  The cap ends with this
-  // call: a block prepared here runs its PnP in mv_track_landmarks_solve, uncapped, after the staging.
-  PnpResidencyCap residency(c, 5);
 
   constexpr int NB = 3;  // chunks in flight: staging DMA / row gather / compute
   void *bs[NB], *bd[NB], *bz[NB], *bsc[NB], *dres, *dmoved;
@@ -1327,7 +1319,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
   //   copy_stream    DMA of a chunk's logits (and descriptors/depth when not gathering)
   //   stream         in order: detector + row marking of chunk k+1, then match + pose of chunk k
   //   gather_stream  zero-copy pull of chunk k+1's marked descriptor rows, concurrent with the
-  //                  PnP launch of chunk k.  That launch is capped at 5 CTAs per SM (above), which
+  //                  PnP launch of chunk k.  That launch is capped at kStagingPnpCtasPerSm, which
   //                  leaves registers and 38 KB of shared memory free; the gather kernel is a
   //                  one-warp CTA that fits in them, so it is resident alongside.
   // whatever the caller queued on the compute stream must be ordered before the staging
@@ -1473,7 +1465,7 @@ static mv_status track_sequence_host_impl(mv_ctx* c, HostCall call, const HostPl
     if (prepare && (s2 = release_gather(k))) return s2;
     if (!prepare) {
       if ((s2 = seq_corr(c, p, nf, depth, v, landmarks ? &lm : nullptr))) return s2;
-      if ((s2 = seq_pose(c, p, nf, v, (mv_pair_result*)dres + p0, p0))) return s2;
+      if ((s2 = seq_pose(c, p, nf, v, (mv_pair_result*)dres + p0, p0, kStagingPnpCtasPerSm))) return s2;
     }
     MV_CUDA(c, cudaEventRecord(consumed[b], c->stream));
     return MV_OK;

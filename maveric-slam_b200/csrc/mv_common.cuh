@@ -30,7 +30,6 @@ struct mv_ctx {
   bool own_stream = true;
   cudaStream_t copy_stream = nullptr; // host-buffer sequence call: logits DMA + detector (high priority)
   cudaStream_t gather_stream = nullptr; // host-buffer sequence call: selective descriptor staging
-  int pnp_max_ctas_per_sm = 0;        // >0: cap K3 residency so staging kernels can co-reside
   char err[512] = {0};
   unsigned long long launches = 0;
   bool profile = false;
@@ -145,6 +144,15 @@ bool mv_pnp_params_ok(const mv_pnp_params* p, int stride);
 bool mv_match_tc_feasible(const mv_match_params* p, int n_frames, int n_pairs, int top_n);
 // the context's vocabulary fits the word-assignment kernel's shared memory (bow.cu)
 bool mv_bow_vocab_fits(const mv_ctx* ctx);
+
+// ---- K3 (pnp_gn.cu), called by the sequence calls (api.cu)
+// mv_pnp_gn_batch with at most max_ctas_per_sm CTAs of its slot kernels per SM (0: no cap), so that the host staging
+// pipeline's row gather fits beside them
+mv_status mv_pnp_gn_batch_impl(mv_ctx* ctx, const mv_pnp_params* p, int n_pairs, int stride, const float* d_corr,
+                               const int32_t* d_count, const float* d_init_pose, float* d_pose, float* d_stats,
+                               float* d_hyp_pose, int max_ctas_per_sm);
+// K3's CTAs per pair that the host staging pipeline sizes its chunks by
+int mv_pnp_ctas_per_pair(const mv_pnp_params* p);
 
 // ---- landmark sequence path (bow.cu), called by mv_track_sequence_landmarks (api.cu)
 // Back-projection of every query keypoint with its frame's depth, fused into the word assignment launch:
